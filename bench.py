@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- body2hand frames/sec on B200 (contract: see the task statement / DESIGN.md §Measurement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Headline workload (N GPUs): BASELINE.json config 3/4 -- the training step (forward + mask_output +
 maskedPoseL1 + backward + Adam) on batch 256 x 64 frames per GPU, C=30, synthetic How2Sign-shaped
@@ -26,7 +26,6 @@ FWD_FLOP_PER_WINDOW = 2 * (5 * T - 6) * S_MAC                # 2 373 840 at T=64
 TRAIN_FLOP_PER_WINDOW = 2 * (5 * T - 6) * (3 * S_MAC - 24 * C)   # 6 669 360
 PRE_BYTES_PER_FRAME = 804 + 648                              # K0 figure of record (SURVEY.md §8d)
 N_SLOTS = 40                                                 # resident batches rotated so the working set > L2
-MIN_TIMED_STEPS = 20000                                      # the timed region lasts >= ~0.5 s whatever --steps is
 
 
 def dp_parity_check(b2h, synthetic, DataParallelTrainer, TrainStepRunner, dev, rank, world, prec, exchange, multicast):
@@ -112,10 +111,11 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
-def cpu_reference_arm(steps, warmup, budget_s=25.0):
+def cpu_reference_arm(steps, warmup, budget_s=None):
     """The reference's CPU path for the headline config: its ConvModel + mask_output + maskedPoseL1 + Adam
     (restated in oracle/b2h_oracle.py from traintest.py:87-123; the reference is pure Python/PyTorch, nothing
-    to compile -> kind 'port'), all host threads, same seeded batch."""
+    to compile -> kind 'port'), all host threads, same seeded batch.  With `budget_s`, stops early once the
+    timed steps have taken that long."""
     import torch
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import b2h_oracle as oracle
@@ -131,7 +131,7 @@ def cpu_reference_arm(steps, warmup, budget_s=25.0):
     for _ in range(steps):
         oracle.train_step(st, batch["input_kp"], batch["target_kp"], batch["n_frames"])
         done += 1
-        if time.perf_counter() - t0 > budget_s:
+        if budget_s is not None and time.perf_counter() - t0 > budget_s:
             break
     dt = time.perf_counter() - t0
     # SURVEY 8d: also the "loops vectorised" variant (closed-form masked L1, one multiply for mask_output), so the
@@ -166,10 +166,21 @@ def cpu_reference_arm(steps, warmup, budget_s=25.0):
             "value_loops_vectorised": (B_TRAIN * T / (vec_ms * 1e-3)) if vec_ms else None}, done, dt
 
 
+def dump_outputs(out_dir, loss, model):
+    """What the last timed train step hands its caller, as float32 .npy files: the step's loss (`loss.npy`) and the
+    updated parameters (`<state-dict key>.npy`).  The inputs are seeded, so two builds run with the same arguments can
+    be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.reshape(1), **model.state_dict()}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_reference(args, rank):
     if rank != 0:
         return
-    base, done, dt = cpu_reference_arm(args.steps, args.warmup, budget_s=150.0)
+    base, done, dt = cpu_reference_arm(args.steps, args.warmup)
     line = {"impl": "reference", "metric": "body2hand_train_frames_per_sec", "value": base["value"], "unit": "frames/s",
             "n_gpus": args.gpus, "steps": done, "warmup": args.warmup, "ms_per_step": dt / done * 1e3,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -194,7 +205,11 @@ def main():
     ap.add_argument("--strong", action="store_true", help="strong scaling (SURVEY 8d config 4): the GLOBAL batch stays 256 windows, "
                                                          "each of the N ranks trains 256/N; the default (and the driver's contract) is weak")
     ap.add_argument("--no-numa-bind", action="store_true", help="leave the rank's threads / pinned buffers where the OS puts them")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's loss and the updated "
+                                                          "parameters to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 train step (--impl b200)")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -259,9 +274,6 @@ def main():
         staged.append(runner.host_stage(b))                   # ONE pinned buffer per batch (x | target | lengths)
         runner.load_staged(staged[-1], slot=s, non_blocking=False)
     chunk = min(N_SLOTS, args.steps)
-    # The driver's --steps can be as small as 20 (0.6 ms of GPU time): the timed region repeats the K-step unit R times
-    # so that it lasts >= ~0.5 s at any K (clock samples under load, no start-up skew); ms_per_step = region / (K * R).
-    repeats = max(1, -(-MIN_TIMED_STEPS // args.steps))
     graphed = True
     try:
         runner.capture(chunk)
@@ -289,10 +301,11 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     run_steps(args.steps)                                     # untimed, not synchronised: the ranks meet inside these steps
     ev0.record()                                              # ... so every rank's clock starts in lock-step with its peers
-    for _ in range(repeats):
-        run_steps(args.steps)
+    run_steps(args.steps)
     ev1.record()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:                       # before the steps below move the weights on
+        dump_outputs(args.dump_outputs, runner.loss[(args.steps - 1) % N_SLOTS], model)
     if world > 1:
         dist.barrier()
     ms = ev0.elapsed_time(ev1)
@@ -301,7 +314,7 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     clocks = sampler.stop() if rank == 0 else None
-    timed_steps = args.steps * repeats
+    timed_steps = args.steps
     torch.cuda.synchronize()
     c0 = _lib.launch_count()
     runner.step(0)                                            # count the kernels of ONE step (outside the timed region)
@@ -382,12 +395,12 @@ def main():
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms / timed_steps, "higher_is_better": True,
             "scaling": "strong" if args.strong else "weak", "vs_baseline": None,
             "dtype": "f32" if train_prec.startswith("fp32") else "bf16", "data": "synthetic",
-            "repeats": repeats, "timed_steps": timed_steps, "timed_region_ms": ms,
+            "timed_steps": timed_steps, "timed_region_ms": ms,
             "config": {"workload": f"train step (fwd+mask+L1+bwd+Adam), batch {B_TRAIN}x{T} frames per GPU, C={C} (BASELINE config 3/4)",
                        "global_batch": B_TRAIN * world, "frames_per_window": T, "conv_channels": C,
                        "parallelism": f"dp{world}", "cuda_graph": graphed, "host_numa": host_numa,
                        "grad_exchange": (getattr(runner, "exchange", None) if world > 1 else None),
-                       "timing": f"{repeats} x {args.steps} steps timed back to back after {max(args.warmup, chunk)} warm-up steps "
+                       "timing": f"{args.steps} steps timed back to back after {max(args.warmup, chunk)} warm-up steps "
                                  f"of the same CUDA graph and one untimed {args.steps}-step pass that aligns the ranks",
                        "l2": f"{N_SLOTS} resident batches rotated ({N_SLOTS * (h2d) / 1e6:.0f} MB inputs + "
                              f"{_lib.workspace_bytes(B_TRAIN, T, 24, C, 0, _lib.PRECISIONS[train_prec]) / 1e6:.0f} MB gradient partials) > 126 MB L2"},

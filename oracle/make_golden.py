@@ -1,6 +1,6 @@
 """Generates tests/golden/*.npz by EXECUTING THE UNMODIFIED REFERENCE (oracle/ref_loader.py) on seeded
-synthetic inputs.  Run in the build container only:  python oracle/make_golden.py
-The fixtures travel to the GPU box; /root/reference does not.  TEST INFRASTRUCTURE ONLY."""
+synthetic inputs:  B2H_REFERENCE_ROOT=<checkout of the original project> python oracle/make_golden.py
+tests/test_oracle_golden.py reads only the fixtures, so it runs without the reference.  TEST INFRASTRUCTURE ONLY."""
 import os
 import random
 import sys

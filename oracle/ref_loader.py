@@ -1,10 +1,11 @@
-"""TEST INFRASTRUCTURE ONLY -- loads the *unmodified* reference classes from /root/reference.
+"""TEST INFRASTRUCTURE ONLY -- loads the *unmodified* reference classes from a checkout of the original
+project (benoriol/hand_pose_sl) named by the environment variable B2H_REFERENCE_ROOT.
 
-This file is used in the build container (where /root/reference is mounted) to
- (a) validate the restatement in oracle/b2h_oracle.py and
+With that checkout available it is used to
+ (a) validate the restatement in oracle/b2h_oracle.py (tests/test_oracle_vs_reference.py) and
  (b) generate the golden vectors committed under tests/golden/ (oracle/make_golden.py).
-It never runs on the GPU box (no /root/reference there) and nothing in the product
-package imports it.
+Without it the live comparisons skip; tests/test_oracle_golden.py checks the oracle against the stored
+vectors.  Nothing in the product package imports this file.
 
 Recipe (SURVEY.md §8c): the reference's package __init__ files import fairseq / h5py and two
 classes that do not exist, so the three hot-path source files are loaded *by file path* with
@@ -16,12 +17,12 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("B2H_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("B2H_REFERENCE_ROOT", "")
 _SRC = os.path.join(REF_ROOT, "body2hand", "src")
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(_SRC, "models", "HandPoseModels.py"))
+    return bool(REF_ROOT) and os.path.isfile(os.path.join(_SRC, "models", "HandPoseModels.py"))
 
 
 def _stub(name, **attrs):
@@ -74,7 +75,7 @@ def load():
     """Returns (models_mod, utils_mod, dataset_mod) = the reference's HandPoseModels.py,
     steps/utils.py and dataloaders/text_pose_dataset.py executed unmodified."""
     if not available():
-        raise FileNotFoundError(f"reference not mounted at {REF_ROOT}")
+        raise FileNotFoundError(f"no reference checkout: set B2H_REFERENCE_ROOT (now {REF_ROOT!r})")
     if not _cache:
         _install_stubs()
         _cache["models"] = _load("b2h_ref_HandPoseModels", "models/HandPoseModels.py")
@@ -91,7 +92,7 @@ def load_function(rel_path, name):
     import numpy as np
     import torch
     if not available():
-        raise FileNotFoundError(f"reference not mounted at {REF_ROOT}")
+        raise FileNotFoundError(f"no reference checkout: set B2H_REFERENCE_ROOT (now {REF_ROOT!r})")
     path = os.path.join(REF_ROOT, "body2hand", "src", rel_path)
     src = open(path).read()
     for node in ast.parse(src).body:

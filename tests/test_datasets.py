@@ -76,7 +76,7 @@ def test_gpu_dataset_matches_reference_items(selection):
     assert b["n_frames"].device.type == "cpu" and b["n_frames"].dtype == torch.int64      # traintest.py:91
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not mounted")
+@pytest.mark.skipif(not ref_loader.available(), reason="needs B2H_REFERENCE_ROOT: a checkout of the original project")
 def test_pack_metadata_feeds_reference_identically():
     """The packed arrays hold exactly the numbers the reference's load_keypoints reads from the same metadata."""
     _, _, D = ref_loader.load()

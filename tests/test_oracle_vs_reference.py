@@ -1,5 +1,5 @@
-"""CPU tier, build container only: the oracle against the live, unmodified reference classes
-(skipped on the GPU box where /root/reference does not exist)."""
+"""CPU tier: the oracle against the live, unmodified reference classes (skipped unless B2H_REFERENCE_ROOT names a
+checkout of the original project; tests/test_oracle_golden.py checks the oracle against its stored outputs)."""
 import numpy as np
 import pytest
 import torch
@@ -8,7 +8,7 @@ import b2h_oracle as oracle
 import ref_loader
 from hand_pose_sl_b200 import synthetic
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not mounted")
+pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="needs B2H_REFERENCE_ROOT: a checkout of the original project")
 
 
 @pytest.mark.parametrize("C,B,T,pe", [(30, 3, 64, False), (30, 2, 100, True), (48, 2, 37, False)])
