@@ -59,11 +59,6 @@ _SIGNATURES = {
     "b2h_train_step": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_double, c_double, c_double,
                                c_double, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
-    "b2h_train_forward_backward_dp": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                                              c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
-                                              c_void_p, c_int64, c_void_p]),
-    "b2h_adam_step_dp": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int64, c_double, c_double, c_double,
-                                 c_double, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_int, c_int, c_int, c_void_p]),
     "b2h_train_step_dp": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_double, c_double, c_double,
                                   c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_float,

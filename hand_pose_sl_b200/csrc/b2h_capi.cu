@@ -110,7 +110,8 @@ extern "C" int64_t b2h_param_offset(int n_in, int C, int pos_emb, int layer, int
   return is_bias ? g.b_off[layer - 1] : g.w_off[layer - 1];
 }
 /* Host-side self-check of the gradient-partial slot layout (no GPU): every flat parameter index maps to a distinct
- * slot and back, every other slot decodes as padding.  Returns the number of violations (0 = consistent). */
+ * slot and back, every other slot decodes as padding.  gp_index_of_flat goes through gp_slot_of_flat, the decode the
+ * packed-weight scatter uses.  Returns the number of violations (0 = consistent). */
 extern "C" int64_t b2h_gp_layout_check(int n_in, int C, int pos_emb) {
   if (!geo_ok(n_in, C, pos_emb, "b2h_gp_layout_check")) return B2H_ESHAPE;
   Geo g = make_geo(n_in, C, pos_emb);
@@ -315,42 +316,12 @@ extern "C" int b2h_train_forward_backward(const void* x, int x_dtype, const floa
   return launch_reduce(partials, plan.nparts, plan.gp_layout, g, grads_out, loss_partials, loss_out, (cudaStream_t)stream, nullptr, plan.n_loss);
 }
 
-extern "C" int b2h_train_forward_backward_dp(const void* x, int x_dtype, const float* target, const float* conf,
-                                             const int32_t* lengths, const float* params, const void* packed,
-                                             float* sym_grads, float* loss_out, int B, int T, int n_in, int C, int pos_emb,
-                                             int loss_kind, int precision, int64_t* step_dev, int64_t* epoch_dev,
-                                             void* workspace, int64_t workspace_bytes, void* stream) {
-  if (!sym_grads || !loss_out || !step_dev || !epoch_dev) { set_error("b2h_train_forward_backward_dp: null pointer"); return B2H_EINVAL; }
-  Geo g; TrainPlan plan; float *partials, *loss_partials;
-  int rc = train_common(x, x_dtype, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C, pos_emb,
-                        loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
-                        loss_partials, "b2h_train_forward_backward_dp", reinterpret_cast<long long*>(step_dev),
-                        reinterpret_cast<long long*>(epoch_dev));
-  if (rc) return rc;
-  return launch_reduce(partials, plan.nparts, plan.gp_layout, g, sym_grads, loss_partials, loss_out,
-                       (cudaStream_t)stream, reinterpret_cast<const long long*>(epoch_dev), plan.n_loss);
-}
-
-extern "C" int b2h_adam_step_dp(float* params, const void* peer_bufs_dev, int rank, int world, float* exp_avg, float* exp_avg_sq,
-                                int64_t n, double lr, double beta1, double beta2, double eps, const int64_t* step_dev,
-                                const int64_t* epoch_dev, const double* lr_dev, float grad_scale, void* packed, int n_in, int C,
-                                int pos_emb, void* stream) {
-  if (!params || !peer_bufs_dev || !exp_avg || !exp_avg_sq || !step_dev || !epoch_dev) { set_error("b2h_adam_step_dp: null pointer"); return B2H_EINVAL; }
-  if (world < 1 || world > 32 || rank < 0 || rank >= world) { set_error("b2h_adam_step_dp: bad rank/world"); return B2H_EINVAL; }
-  if (!geo_ok(n_in, C, pos_emb, "b2h_adam_step_dp")) return B2H_ESHAPE;
-  Geo g = make_geo(n_in, C, pos_emb);
-  if (g.P != n) { set_error("b2h_adam_step_dp: n=%lld does not match geometry (%d)", (long long)n, g.P); return B2H_ESHAPE; }
-  return launch_adam_dp(params, reinterpret_cast<const float* const*>(peer_bufs_dev), rank, world, exp_avg, exp_avg_sq, n, lr, beta1,
-                        beta2, eps, reinterpret_cast<const long long*>(step_dev), reinterpret_cast<const long long*>(epoch_dev),
-                        lr_dev, grad_scale, packed, g, (cudaStream_t)stream);
-}
-
 extern "C" int64_t b2h_dp_exchange_floats(int n_in, int C, int pos_emb, int world) {
   if (!geo_ok(n_in, C, pos_emb, "b2h_dp_exchange_floats")) return B2H_ESHAPE;
   if (world < 1 || world > 32) { set_error("b2h_dp_exchange_floats: bad world"); return B2H_EINVAL; }
   Geo g = make_geo(n_in, C, pos_emb);
-  // tensor-core path: uint64 words [2][world][slots] (= 4*world*slots floats); the three-launch path needs
-  // [2][P] fp32 + [world] int64 flags, which is smaller
+  // one-launch tile path: 4-byte words [2][world][slots] = 2*world*slots floats (the size returned is twice that); the
+  // three-launch path needs [2][P] fp32 + [world] int64 flags, which is smaller
   return 4 * (int64_t)world * gp_total(g) + 64;
 }
 

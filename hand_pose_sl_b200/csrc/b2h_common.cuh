@@ -85,23 +85,34 @@ __host__ __device__ inline int gp_layer_off(const Geo& g, int l) {
   return o;
 }
 __host__ __device__ inline int gp_total(const Geo& g) { return gp_layer_off(g, 4); }
-// flat parameter index -> index in the GP layout
-__host__ __device__ inline int gp_index_of_flat(const Geo& g, int i) {
+
+// (layer, tap, co, ci) of one parameter; is_bias: co = bias index, k = ci = 0
+struct GpSlot { int l, k, co, ci; bool is_bias; };
+// flat parameter index -> slot
+__host__ __device__ inline GpSlot gp_slot_of_flat(const Geo& g, int i) {
+  GpSlot s;
   int l = 0;
   for (int q = 1; q < 4; ++q)
     if (i >= g.w_off[q]) l = q;
-  const int base = gp_layer_off(g, l);
-  if (i >= g.b_off[l]) return base + B2H_KW * g.cout[l] * g.kp[l] + (i - g.b_off[l]);
+  s.l = l;
+  if (i >= g.b_off[l]) { s.is_bias = true; s.k = 0; s.ci = 0; s.co = i - g.b_off[l]; return s; }
+  s.is_bias = false;
   const int cin = g.cin[l];
   const int rel = i - g.w_off[l];
-  const int co = rel / (cin * B2H_KW);
-  const int rem = rel - co * cin * B2H_KW;
-  const int ci = rem / B2H_KW, k = rem - ci * B2H_KW;
-  return base + ((k * (g.kp[l] >> 2) + (ci >> 2)) * g.cout[l] + co) * 4 + (ci & 3);
+  s.co = rel / (cin * B2H_KW);
+  const int rem = rel - s.co * cin * B2H_KW;
+  s.ci = rem / B2H_KW; s.k = rem - s.ci * B2H_KW;
+  return s;
+}
+// flat parameter index -> index in the GP layout
+__host__ __device__ inline int gp_index_of_flat(const Geo& g, int i) {
+  const GpSlot s = gp_slot_of_flat(g, i);
+  const int l = s.l, base = gp_layer_off(g, l);
+  if (s.is_bias) return base + B2H_KW * g.cout[l] * g.kp[l] + s.co;
+  return base + ((s.k * (g.kp[l] >> 2) + (s.ci >> 2)) * g.cout[l] + s.co) * 4 + (s.ci & 3);
 }
 
-// GP index -> (layer, tap, co, ci); is_bias: co = bias index, k = ci = 0.  Returns false for the padding slots.
-struct GpSlot { int l, k, co, ci; bool is_bias; };
+// GP index -> slot.  Returns false for the padding slots.
 __host__ __device__ inline bool gp_decode(const Geo& g, int j, GpSlot& s) {
   int l = 0, base = 0;
   for (int q = 0; q < 4; ++q) {
@@ -132,38 +143,10 @@ __host__ __device__ inline int flat_index_of_gp(const Geo& g, int j) {
   return gp_decode(g, j, s) ? gp_flat_of_slot(g, s) : -1;
 }
 
-// Scatter one fp32 parameter (flat index i) into the packed operand layouts.
-__device__ __forceinline__ void scatter_packed(const Geo& g, char* packed, int i, float v) {
-  int l = 0;
-#pragma unroll
-  for (int q = 1; q < 4; ++q)
-    if (i >= g.w_off[q]) l = q;
-  if (i >= g.b_off[l]) {        // bias: also kept zero-padded [4][64] for the tensor-core kernels' smem copy
-    if (i - g.b_off[l] < 64) reinterpret_cast<float*>(packed + g.bias_off)[l * 64 + (i - g.b_off[l])] = v;
-    return;
-  }
-  const int cin = g.cin[l], cout = g.cout[l];
-  const int rel = i - g.w_off[l];
-  const int co = rel / (cin * B2H_KW);
-  const int rem = rel - co * cin * B2H_KW;
-  const int ci = rem / B2H_KW, k = rem - ci * B2H_KW;
-  reinterpret_cast<float*>(packed + g.wf_off[l])[(k * cin + ci) * cout + co] = v;
-  const __nv_bfloat16 h = __float2bfloat16_rn(v);
-  const int64_t bo = umma_b_offset(k, ci, co, g.kp[l], g.np_[l]);
-  *reinterpret_cast<__nv_bfloat16*>(packed + g.tf_off[l] + bo) = h;
-  *reinterpret_cast<__nv_bfloat16*>(packed + g.tfl_off[l] + bo) = __float2bfloat16_rn(v - __bfloat162float(h));
-  if (l > 0) {
-    reinterpret_cast<float*>(packed + g.wd_off[l])[((B2H_KW - 1 - k) * cout + co) * cin + ci] = v;
-    *reinterpret_cast<__nv_bfloat16*>(packed + g.td_off[l] +
-                                      umma_b_offset(B2H_KW - 1 - k, co, ci, round_up(cout, 16), round_up(cin, 16))) = h;
-  }
-}
-
-
-// Same scatter from a decoded gradient-partial slot (the fused train kernel decodes its slots before the grid barrier).
-__device__ __forceinline__ void scatter_packed_slot(const Geo& g, char* packed, const GpSlot& s, float v) {
+// Scatter one fp32 parameter into the packed operand layouts (callers holding a flat index decode it with gp_slot_of_flat).
+__device__ __forceinline__ void scatter_packed(const Geo& g, char* packed, const GpSlot& s, float v) {
   const int l = s.l;
-  if (s.is_bias) {
+  if (s.is_bias) {              // bias: also kept zero-padded [4][64] for the tensor-core kernels' smem copy
     if (s.co < 64) reinterpret_cast<float*>(packed + g.bias_off)[l * 64 + s.co] = v;
     return;
   }
@@ -180,6 +163,18 @@ __device__ __forceinline__ void scatter_packed_slot(const Geo& g, char* packed, 
   }
 }
 
+// torch.optim.Adam single-tensor update of one element (defaults: amsgrad=False, weight_decay=0, maximize=False) with the
+// already scaled gradient gr:
+//   m.lerp_(g, 1-b1); v.mul_(b2).addcmul_(g, g, 1-b2);
+//   denom = v.sqrt()/sqrt(1-b2^t) + eps;  p.addcdiv_(m, denom, value=-lr/(1-b1^t))
+// m and v are updated in place; returns the new p.  step_size = lr/(1-b1^t), inv_bc2_sqrt = 1/sqrt(1-b2^t).
+__device__ __forceinline__ float adam_update(float& m, float& v, float p, float gr, float one_minus_b1, float one_minus_b2,
+                                             float beta2, float eps, float step_size, float inv_bc2_sqrt) {
+  m = fmaf(gr - m, one_minus_b1, m);
+  v = fmaf(one_minus_b2 * gr, gr, v * beta2);
+  const float denom = sqrtf(v) * inv_bc2_sqrt + eps;
+  return p - step_size * (m / denom);
+}
 
 // beta^t for an integer step count by binary exponentiation (~2*log2(t) DMULs instead of a double-precision pow())
 __host__ __device__ inline double ipow(double b, long long t) {
@@ -300,7 +295,6 @@ void set_debug_timing(long long* p);
 int launch_tc_bench(long long* out, int M, int N, int reps, int nacc, int mn_major, cudaStream_t stream);
 int launch_format_prediction(const float* pred, float* out, int64_t rows, int mode, cudaStream_t stream);
 int launch_pos_emb_concat(const float* inp, float* out, int B, int Cc, int T, int max_len, cudaStream_t stream);
-int launch_bump_counters(long long* step_dev, long long* epoch_dev, cudaStream_t stream);
 int launch_pack(const float* params, void* packed, const Geo& g, cudaStream_t stream);
 int launch_reduce(const float* partials, int nparts, int gp_layout, const Geo& g, float* grads, const float* loss_partials,
                   float* loss_out, cudaStream_t stream, const long long* epoch_dev = nullptr, int n_loss_parts = -1);

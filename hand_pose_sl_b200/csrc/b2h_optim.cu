@@ -12,7 +12,7 @@ namespace b2h {
 
 __global__ void pack_kernel(const float* __restrict__ params, char* packed, Geo g) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < g.P) scatter_packed(g, packed, i, params[i]);
+  if (i < g.P) scatter_packed(g, packed, gp_slot_of_flat(g, i), params[i]);
 }
 
 // Cross-CTA partial sum, shared by the reduce and the Adam kernel.  A block owns 32 consecutive slots of the
@@ -81,19 +81,26 @@ struct AdamArgs {
   const float* loss_partials; float* loss_out; int n_loss_parts;
 };
 
-// torch.optim.Adam single-tensor update (defaults: amsgrad=False, weight_decay=0, maximize=False):
-//   m.lerp_(g, 1-b1); v.mul_(b2).addcmul_(g, g, 1-b2);
-//   denom = v.sqrt()/sqrt(1-b2^t) + eps;  p.addcdiv_(m, denom, value=-lr/(1-b1^t))
+// Bias corrections step_size = lr/(1-b1^t), inv_bc2_sqrt = 1/sqrt(1-b2^t) from the device-side step counter / learning rate
+// (graph replay), computed by one thread of a block.  Three forms of these coefficients exist, and each stays as it is
+// because switching a path to another form moves its trained weights in the last bits:
+//   - the Adam kernels of this file, when step_dev or lr_dev is given: this function, double precision with ipow;
+//   - launch_adam on the host for calls without step_dev / lr_dev: double-precision pow();
+//   - the fused tail of conv_tc_tile_kernel: fp32 -expm1f(t * log1pf(beta - 1)), because double-precision powers cost
+//     ~5k cycles on B200's few FP64 units inside the one-launch train step.
+__device__ __forceinline__ void adam_bias_corrections(const AdamArgs& a, float& step_size, float& inv_bc2_sqrt) {
+  const long long t = a.step_dev ? *a.step_dev : a.step_host;
+  const double lr = a.lr_dev ? *a.lr_dev : a.lr_d;
+  step_size = (float)(lr / (1.0 - ipow(a.beta1_d, t)));
+  inv_bc2_sqrt = (float)(1.0 / sqrt(1.0 - ipow(a.beta2_d, t)));
+}
+
+// torch.optim.Adam single-tensor update (adam_update) over the flat buffers, 32 slots per block
 __global__ void __launch_bounds__(256) adam_kernel(AdamArgs a) {
   __shared__ float red[8][32];
   __shared__ float s_step_size, s_inv_bc2_sqrt;
-  if (a.step_dev || a.lr_dev) {   // bias corrections from the device-side step counter / learning rate (graph replay)
-    if (threadIdx.x == 0) {
-      const long long t = a.step_dev ? *a.step_dev : a.step_host;
-      const double lr = a.lr_dev ? *a.lr_dev : a.lr_d;
-      s_step_size = (float)(lr / (1.0 - ipow(a.beta1_d, t)));
-      s_inv_bc2_sqrt = (float)(1.0 / sqrt(1.0 - ipow(a.beta2_d, t)));
-    }
+  if (a.step_dev || a.lr_dev) {
+    if (threadIdx.x == 0) adam_bias_corrections(a, s_step_size, s_inv_bc2_sqrt);
     __syncthreads();
     a.step_size = s_step_size;
     a.inv_bc2_sqrt = s_inv_bc2_sqrt;
@@ -109,14 +116,11 @@ __global__ void __launch_bounds__(256) adam_kernel(AdamArgs a) {
   if (threadIdx.x < 32 && j < nj) {
     const int i = a.gp_layout ? flat_index_of_gp(a.g, j) : j;
     if (i >= 0) {
-      gr *= a.grad_scale;
-      float m = a.m[i], v = a.v[i], p = a.params[i];
-      m = fmaf(gr - m, a.one_minus_b1, m);
-      v = fmaf(a.one_minus_b2 * gr, gr, v * a.beta2);
-      const float denom = sqrtf(v) * a.inv_bc2_sqrt + a.eps;
-      p = p - a.step_size * (m / denom);
+      float m = a.m[i], v = a.v[i];
+      const float p = adam_update(m, v, a.params[i], gr * a.grad_scale, a.one_minus_b1, a.one_minus_b2, a.beta2, a.eps,
+                                  a.step_size, a.inv_bc2_sqrt);
       a.m[i] = m; a.v[i] = v; a.params[i] = p;
-      if (a.packed) scatter_packed(a.g, a.packed, i, p);
+      if (a.packed) scatter_packed(a.g, a.packed, gp_slot_of_flat(a.g, i), p);
     }
   }
   loss_partial_sum(a.loss_partials, a.n_loss_parts, a.loss_out);
@@ -136,12 +140,7 @@ __global__ void __launch_bounds__(256) adam_gp_tile_kernel(AdamArgs a) {
   __shared__ float b_s[kAdamCoGroup];
   const Geo& g = a.g;
   if (a.step_dev || a.lr_dev) {
-    if (threadIdx.x == 0) {
-      const long long t = a.step_dev ? *a.step_dev : a.step_host;
-      const double lr = a.lr_dev ? *a.lr_dev : a.lr_d;
-      s_step_size = (float)(lr / (1.0 - ipow(a.beta1_d, t)));
-      s_inv_bc2_sqrt = (float)(1.0 / sqrt(1.0 - ipow(a.beta2_d, t)));
-    }
+    if (threadIdx.x == 0) adam_bias_corrections(a, s_step_size, s_inv_bc2_sqrt);
   } else if (threadIdx.x == 0) {
     s_step_size = a.step_size; s_inv_bc2_sqrt = a.inv_bc2_sqrt;
   }
@@ -186,12 +185,9 @@ __global__ void __launch_bounds__(256) adam_gp_tile_kernel(AdamArgs a) {
   __syncthreads();
   const float step_size = s_step_size, inv_bc2_sqrt = s_inv_bc2_sqrt;
   auto adam1 = [&](int i, float gr) {
-    gr *= a.grad_scale;
-    float m = a.m[i], v = a.v[i], p = a.params[i];
-    m = fmaf(gr - m, a.one_minus_b1, m);
-    v = fmaf(a.one_minus_b2 * gr, gr, v * a.beta2);
-    const float denom = sqrtf(v) * inv_bc2_sqrt + a.eps;
-    p = p - step_size * (m / denom);
+    float m = a.m[i], v = a.v[i];
+    const float p = adam_update(m, v, a.params[i], gr * a.grad_scale, a.one_minus_b1, a.one_minus_b2, a.beta2, a.eps, step_size,
+                                inv_bc2_sqrt);
     a.m[i] = m; a.v[i] = v; a.params[i] = p;
     return p;
   };
@@ -209,7 +205,7 @@ __global__ void __launch_bounds__(256) adam_gp_tile_kernel(AdamArgs a) {
   if (threadIdx.x < kAdamCoGroup && co0 + (int)threadIdx.x < cout) {
     const int co = co0 + threadIdx.x;
     const float p = adam1(g.b_off[l] + co, b_s[threadIdx.x]);
-    if (a.packed && co < 64) reinterpret_cast<float*>(a.packed + g.bias_off)[l * 64 + co] = p;
+    if (a.packed) scatter_packed(g, a.packed, GpSlot{l, 0, co, 0, true}, p);
   }
   __syncthreads();
   // (3) slot order again: scatter the new weights into the packed operand layouts
@@ -218,10 +214,7 @@ __global__ void __launch_bounds__(256) adam_gp_tile_kernel(AdamArgs a) {
       const int e = idx & 3, cl = (idx >> 2) % kAdamCoGroup, r = idx / (4 * kAdamCoGroup);
       const int q = r % q4, k = r / q4;
       const int co = co0 + cl, ci = 4 * q + e;
-      if (co < cout && ci < cin) {
-        GpSlot sl; sl.l = l; sl.k = k; sl.co = co; sl.ci = ci; sl.is_bias = false;
-        scatter_packed_slot(g, a.packed, sl, g_s[(cl * kp + ci) * B2H_KW + k]);
-      }
+      if (co < cout && ci < cin) scatter_packed(g, a.packed, GpSlot{l, k, co, ci, false}, g_s[(cl * kp + ci) * B2H_KW + k]);
     }
   }
   loss_partial_sum(a.loss_partials, a.n_loss_parts, a.loss_out);
@@ -233,12 +226,7 @@ __global__ void __launch_bounds__(256) adam_gp_tile_kernel(AdamArgs a) {
 __global__ void __launch_bounds__(256) adam_gp_wide_kernel(AdamArgs a) {
   __shared__ float s_step_size, s_inv_bc2_sqrt;
   if (a.step_dev || a.lr_dev) {
-    if (threadIdx.x == 0) {
-      const long long t = a.step_dev ? *a.step_dev : a.step_host;
-      const double lr = a.lr_dev ? *a.lr_dev : a.lr_d;
-      s_step_size = (float)(lr / (1.0 - ipow(a.beta1_d, t)));
-      s_inv_bc2_sqrt = (float)(1.0 / sqrt(1.0 - ipow(a.beta2_d, t)));
-    }
+    if (threadIdx.x == 0) adam_bias_corrections(a, s_step_size, s_inv_bc2_sqrt);
     __syncthreads();
     a.step_size = s_step_size;
     a.inv_bc2_sqrt = s_inv_bc2_sqrt;
@@ -251,14 +239,11 @@ __global__ void __launch_bounds__(256) adam_gp_wide_kernel(AdamArgs a) {
     GpSlot sl;
     if (gp_decode(a.g, j, sl)) {
       const int i = gp_flat_of_slot(a.g, sl);
-      gr *= a.grad_scale;
-      float m = a.m[i], v = a.v[i], p = a.params[i];
-      m = fmaf(gr - m, a.one_minus_b1, m);
-      v = fmaf(a.one_minus_b2 * gr, gr, v * a.beta2);
-      const float denom = sqrtf(v) * a.inv_bc2_sqrt + a.eps;
-      p = p - a.step_size * (m / denom);
+      float m = a.m[i], v = a.v[i];
+      const float p = adam_update(m, v, a.params[i], gr * a.grad_scale, a.one_minus_b1, a.one_minus_b2, a.beta2, a.eps,
+                                  a.step_size, a.inv_bc2_sqrt);
       a.m[i] = m; a.v[i] = v; a.params[i] = p;
-      if (a.packed) scatter_packed_slot(a.g, a.packed, sl, p);
+      if (a.packed) scatter_packed(a.g, a.packed, sl, p);
     }
   }
   loss_partial_sum(a.loss_partials, a.n_loss_parts, a.loss_out);
@@ -281,7 +266,9 @@ __global__ void __launch_bounds__(256) reduce_gp_wide_kernel(const float* __rest
 }
 
 // ---- data parallel: gradient exchange over peer (NVLink) memory fused with Adam -------------------------------
-// Every rank owns a symmetric buffer  [2][P] fp32 gradients (double-buffered by epoch parity) + [world] uint64 flags.
+// Three-launch path of b2h_train_step_dp (shapes the one-launch tile kernel does not serve): train kernel, reduce_* into
+// this rank's buffer, adam_dp_kernel.
+// Every rank owns a symmetric buffer  [2][P] fp32 gradients (double-buffered by epoch parity) + [world] int64 flags.
 // Step protocol (one kernel per rank, all ranks run it concurrently on their own GPU):
 //   1. block 0 publishes "my gradients of epoch e are complete" by storing e into flag[rank] of every peer
 //      (the reduce kernel that wrote them is the previous kernel on the stream; __threadfence_system orders it);
@@ -307,10 +294,7 @@ __global__ void __launch_bounds__(256) adam_dp_kernel(AdamDpArgs d) {
   const size_t flag_off = 2 * P;                       // in floats; flags are 8-byte aligned (2P is even)
   __shared__ int s_abort;
   if (threadIdx.x == 0) {
-    const long long t = *a.step_dev;
-    const double lr = a.lr_dev ? *a.lr_dev : a.lr_d;
-    s_step_size = (float)(lr / (1.0 - ipow(a.beta1_d, t)));
-    s_inv_bc2_sqrt = (float)(1.0 / sqrt(1.0 - ipow(a.beta2_d, t)));
+    adam_bias_corrections(a, s_step_size, s_inv_bc2_sqrt);
     s_abort = 0;
   }
   __syncthreads();
@@ -337,28 +321,34 @@ __global__ void __launch_bounds__(256) adam_dp_kernel(AdamDpArgs d) {
     const size_t off = (size_t)(epoch & 1) * P + (size_t)i;
     float gr = 0.f;
     for (int r = 0; r < d.world; ++r) gr += __ldcv(d.peer_bufs[r] + off);
-    gr *= a.grad_scale;
-    float m = a.m[i], v = a.v[i], p = a.params[i];
-    m = fmaf(gr - m, a.one_minus_b1, m);
-    v = fmaf(a.one_minus_b2 * gr, gr, v * a.beta2);
-    const float denom = sqrtf(v) * s_inv_bc2_sqrt + a.eps;
-    p = p - s_step_size * (m / denom);
+    float m = a.m[i], v = a.v[i];
+    const float p = adam_update(m, v, a.params[i], gr * a.grad_scale, a.one_minus_b1, a.one_minus_b2, a.beta2, a.eps, s_step_size,
+                                s_inv_bc2_sqrt);
     a.m[i] = m; a.v[i] = v; a.params[i] = p;
-    if (a.packed) scatter_packed(a.g, a.packed, (int)i, p);
+    if (a.packed) scatter_packed(a.g, a.packed, gp_slot_of_flat(a.g, (int)i), p);
   }
+}
+
+// The AdamArgs fields every Adam launch sets the same way; the caller adds where the gradients come from and the host-side
+// bias corrections.
+static AdamArgs adam_args(float* params, float* m, float* v, int64_t n, double lr, double beta1, double beta2, double eps,
+                          long long step, const long long* step_dev, const double* lr_dev, float grad_scale, void* packed,
+                          const Geo& g) {
+  AdamArgs a{};
+  a.params = params; a.n = n; a.m = m; a.v = v;
+  a.beta1 = (float)beta1; a.beta2 = (float)beta2;
+  a.one_minus_b1 = (float)(1.0 - beta1); a.one_minus_b2 = (float)(1.0 - beta2);
+  a.eps = (float)eps; a.grad_scale = grad_scale;
+  a.packed = reinterpret_cast<char*>(packed); a.g = g;
+  a.lr_d = lr; a.beta1_d = beta1; a.beta2_d = beta2; a.step_dev = step_dev; a.lr_dev = lr_dev; a.step_host = step;
+  return a;
 }
 
 int launch_adam_dp(float* params, const float* const* peer_bufs, int rank, int world, float* m, float* v, int64_t n, double lr,
                    double beta1, double beta2, double eps, const long long* step_dev, const long long* epoch_dev, const double* lr_dev,
                    float grad_scale, void* packed, const Geo& g, cudaStream_t stream) {
   AdamDpArgs d{};
-  AdamArgs& a = d.a;
-  a.params = params; a.grads = nullptr; a.nparts = 1; a.gp_layout = 0; a.n = n; a.m = m; a.v = v;
-  a.beta1 = (float)beta1; a.beta2 = (float)beta2;
-  a.one_minus_b1 = (float)(1.0 - beta1); a.one_minus_b2 = (float)(1.0 - beta2);
-  a.eps = (float)eps; a.grad_scale = grad_scale;
-  a.packed = reinterpret_cast<char*>(packed); a.g = g;
-  a.lr_d = lr; a.beta1_d = beta1; a.beta2_d = beta2; a.step_dev = step_dev; a.lr_dev = lr_dev; a.step_host = 1;
+  d.a = adam_args(params, m, v, n, lr, beta1, beta2, eps, 1, step_dev, lr_dev, grad_scale, packed, g);
   d.peer_bufs = peer_bufs; d.epoch_dev = epoch_dev; d.rank = rank; d.world = world;
   adam_dp_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(d);
   count_launch();
@@ -483,29 +473,20 @@ int launch_format_prediction(const float* pred, float* out, int64_t rows, int mo
   return check_launch("format_prediction_kernel");
 }
 
-// device-side step / exchange-epoch counters for training paths whose kernels do not bump them themselves (wide path)
-__global__ void bump_counters_kernel(long long* step_dev, long long* epoch_dev) {
-  if (threadIdx.x == 0 && blockIdx.x == 0) {
-    if (step_dev) *step_dev += 1;
-    if (epoch_dev) *epoch_dev += 1;
-  }
-}
-int launch_bump_counters(long long* step_dev, long long* epoch_dev, cudaStream_t stream) {
-  bump_counters_kernel<<<1, 32, 0, stream>>>(step_dev, epoch_dev);
-  count_launch();
-  return check_launch("bump_counters_kernel");
-}
-
 int launch_pack(const float* params, void* packed, const Geo& g, cudaStream_t stream) {
   pack_kernel<<<(g.P + 255) / 256, 256, 0, stream>>>(params, reinterpret_cast<char*>(packed), g);
   count_launch();
   return check_launch("pack_kernel");
 }
 
+// Few gradient slices in the slot layout (wide training, small batches of the tile kernel): the reduction and Adam kernels
+// that sum every slice of a slot in one thread, instead of spreading the slices over the 8 warps of a block.
+static bool few_slices(int nparts, int gp_layout) { return gp_layout && nparts <= 64; }
+
 int launch_reduce(const float* partials, int nparts, int gp_layout, const Geo& g, float* grads, const float* loss_partials,
                   float* loss_out, cudaStream_t stream, const long long* epoch_dev, int n_loss_parts) {
   const int nj = gp_layout ? gp_total(g) : g.P;
-  if (gp_layout && nparts <= 64) {                     // few slices (wide training, small batches): one thread per slot
+  if (few_slices(nparts, gp_layout)) {                 // one thread per slot
     reduce_gp_wide_kernel<<<(nj + 255) / 256, 256, 0, stream>>>(partials, nparts, g, grads, loss_partials, loss_out, epoch_dev,
                                                                 n_loss_parts < 0 ? nparts : n_loss_parts);
     count_launch();
@@ -520,25 +501,19 @@ int launch_reduce(const float* partials, int nparts, int gp_layout, const Geo& g
 int launch_adam(float* params, const float* grads, int nparts, int gp_layout, float* m, float* v, int64_t n, double lr, double beta1,
                 double beta2, double eps, int64_t step, const long long* step_dev, const double* lr_dev, float grad_scale, void* packed,
                 const Geo& g, const float* loss_partials, float* loss_out, cudaStream_t stream, int n_loss_parts) {
-  AdamArgs a;
-  a.n_loss_parts = n_loss_parts < 0 ? nparts : n_loss_parts;
-  a.params = params; a.grads = grads; a.nparts = nparts; a.gp_layout = gp_layout; a.n = n; a.m = m; a.v = v;
-  a.beta1 = (float)beta1; a.beta2 = (float)beta2;
-  a.one_minus_b1 = (float)(1.0 - beta1); a.one_minus_b2 = (float)(1.0 - beta2);
+  AdamArgs a = adam_args(params, m, v, n, lr, beta1, beta2, eps, step, step_dev, lr_dev, grad_scale, packed, g);
+  a.grads = grads; a.nparts = nparts; a.gp_layout = gp_layout;
+  a.loss_partials = loss_partials; a.loss_out = loss_out; a.n_loss_parts = n_loss_parts < 0 ? nparts : n_loss_parts;
   const double bc1 = 1.0 - pow(beta1, (double)step), bc2 = 1.0 - pow(beta2, (double)step);
   a.step_size = (float)(lr / bc1);
   a.inv_bc2_sqrt = (float)(1.0 / sqrt(bc2));
-  a.eps = (float)eps; a.grad_scale = grad_scale;
-  a.packed = reinterpret_cast<char*>(packed); a.g = g;
-  a.loss_partials = loss_partials; a.loss_out = loss_out;
-  a.lr_d = lr; a.beta1_d = beta1; a.beta2_d = beta2; a.step_dev = step_dev; a.lr_dev = lr_dev; a.step_host = step;
   const int64_t nj = gp_layout ? (int64_t)gp_total(g) : n;
-  if (gp_layout && nparts <= 64 && nj <= 100000) {     // few slices, small model: one thread per slot
+  if (few_slices(nparts, gp_layout) && nj <= 100000) { // small model: one thread per slot
     adam_gp_wide_kernel<<<(unsigned)((nj + 255) / 256), 256, 0, stream>>>(a);
     count_launch();
     return check_launch("adam_gp_wide_kernel");
   }
-  if (gp_layout && nparts <= 64) {                     // few slices, large model (wide training): coalesced on both sides
+  if (few_slices(nparts, gp_layout)) {                 // large model (wide training): coalesced on both sides
     int blocks = 0, kpmax = 0;
     for (int l = 0; l < 4; ++l) { blocks += (g.cout[l] + kAdamCoGroup - 1) / kAdamCoGroup; kpmax = g.kp[l] > kpmax ? g.kp[l] : kpmax; }
     const size_t smem = (size_t)kAdamCoGroup * kpmax * B2H_KW * sizeof(float);

@@ -68,7 +68,6 @@ constexpr int kAccCol = 0;        // forward / dgrad accumulator: columns [0, 64
 constexpr int kWgPairCols = 5 * 32 + 8;
 constexpr int kGatherDepth = 24; // independent 16-B loads in flight per thread in the cross-CTA gradient gather
 constexpr uint32_t kDpSentinel = 0xFFFFFFFFu;   // "not arrived yet" in the data-parallel exchange buffer (see the train kernel tail)
-constexpr int kDpMaxCta = 160;    // flag slots per rank in the data-parallel exchange buffer (>= CTAs of the train kernel)
 
 struct TileSmem {   // byte offsets into dynamic smem
   int g0, g1, x, a1, a2, a3, ones, lo_off, ys, has_ys, wf[4], wlo_off, wd[4], total;
@@ -197,13 +196,10 @@ __device__ __forceinline__ void grid_barrier_flags(unsigned* hdr, unsigned tok, 
 // torch.optim.Adam single-tensor update on one element whose state (m, v, p) was loaded earlier (before the grid barrier)
 __device__ __forceinline__ void adam_apply(const FuseAdam& f, const Geo& g, const GpSlot& slot, int i, float gr, float m, float v,
                                            float p, float step_size, float inv_bc2_sqrt) {
-  gr *= f.grad_scale;
-  m = fmaf(gr - m, (float)(1.0 - f.beta1), m);
-  v = fmaf((float)(1.0 - f.beta2) * gr, gr, v * (float)f.beta2);
-  const float denom = sqrtf(v) * inv_bc2_sqrt + f.eps;
-  p = p - step_size * (m / denom);
+  p = adam_update(m, v, p, gr * f.grad_scale, (float)(1.0 - f.beta1), (float)(1.0 - f.beta2), (float)f.beta2, f.eps, step_size,
+                  inv_bc2_sqrt);
   f.m[i] = m; f.v[i] = v; f.params[i] = p;
-  if (f.packed) scatter_packed_slot(g, f.packed, slot, p);
+  if (f.packed) scatter_packed(g, f.packed, slot, p);
 }
 
 #define B2H_STAMP() do { if (p.dbg && blockIdx.x == 0 && tid == 0 && dbg_n < 120) p.dbg[dbg_n++] = clock64(); } while (0)

@@ -207,38 +207,31 @@ int b2h_adam_step(float* params, const float* grads, float* exp_avg, float* exp_
                   float grad_scale, void* packed, int n_in, int C, int pos_emb, void* stream);
 
 /* ---- data parallel over peer (NVLink / NVSwitch) memory -----------------------------------------------------
- * The reference is single-process; training shards by batch with ONE gradient exchange per step (SURVEY.md §8e).
- * Every rank owns a symmetric buffer  [2][P] fp32 + [world] int64 flags  (zero-initialised, peer-mapped, e.g.
- * torch.distributed._symmetric_memory).  b2h_train_forward_backward_dp = b2h_train_forward_backward whose reduced
- * flat gradient lands in sym_grads[(epoch & 1) * P ...]; b2h_adam_step_dp = flag exchange with all peers, sum of the
- * peers' gradients in rank order over NVLink and Adam + re-pack, in ONE kernel (no NCCL call on the step path).
- * step_dev / epoch_dev: device int64 counters advanced by the train kernel (epoch_dev is never rewound).
- * peer_bufs_dev: device array [world] of the peers' buffer base pointers, indexed by rank. */
-int b2h_train_forward_backward_dp(const void* x, int x_dtype, const float* target, const float* conf,
-                                  const int32_t* lengths, const float* params, const void* packed, float* sym_grads,
-                                  float* loss_out, int B, int T, int n_in, int C, int pos_emb, int loss_kind,
-                                  int precision, int64_t* step_dev, int64_t* epoch_dev, void* workspace,
-                                  int64_t workspace_bytes, void* stream);
-int b2h_adam_step_dp(float* params, const void* peer_bufs_dev, int rank, int world, float* exp_avg, float* exp_avg_sq,
-                     int64_t n, double lr, double beta1, double beta2, double eps, const int64_t* step_dev,
-                     const int64_t* epoch_dev, const double* lr_dev, float grad_scale, void* packed, int n_in, int C,
-                     int pos_emb, void* stream);
-/* floats a rank's exchange buffer must hold for b2h_train_step_dp / b2h_adam_step_dp */
+ * The reference is single-process; training shards by batch with ONE gradient exchange per step (SURVEY.md §8e) over
+ * peer memory, no NCCL call on the step path.  Every rank owns a symmetric exchange buffer (peer-mapped, e.g.
+ * torch.distributed._symmetric_memory) whose first index is the epoch parity: a rank one step ahead of a peer never
+ * writes words the peer is still reading. */
+/* floats a rank's exchange buffer must hold for b2h_train_step_dp */
 int64_t b2h_dp_exchange_floats(int n_in, int C, int pos_emb, int world);
 /* 32-bit pattern every word of the exchange buffer must be filled with ONCE, before the first step, on every rank:
  * 0xFFFFFFFF for shapes the one-launch tile kernel serves (its exchange words are 4 bytes: the gradient value is its own
  * arrival flag, "not arrived" = this NaN pattern, re-armed by the reader), 0 for the three-launch path (gradients + flags). */
 int64_t b2h_dp_exchange_fill(int T, int n_in, int C, int pos_emb, int precision);
 
-/* The whole data-parallel step as ONE call; in bf16 mode (tensor-core tile kernel) also ONE cooperative kernel
- * launch per rank: forward + loss + backward, grid barrier, cross-CTA reduction, gradient exchange over peer memory
- * (4-byte words pushed into every rank's buffer; the value is its own arrival flag, see b2h_dp_exchange_fill), sum in
- * rank order, Adam + re-pack.
- * multicast_buf (nullable): the multicast (NVLS) address of the ranks' exchange buffers
- * (torch symmetric-memory handle .multicast_ptr): the push is then ONE multimem.st per gradient slot, replicated by
- * the NVSwitch, instead of `world` unicast stores.  lr_dev: see b2h_adam_step.  A wait for a peer that exceeds ~3 s
- * sets the status read by b2h_tc_status / b2h_dp_status and suppresses every parameter update until it is read.
- * Other shapes run the same protocol as three launches. */
+/* The whole data-parallel step as ONE call; every rank sums the ranks' gradients in rank order, so the replicas stay
+ * bit-identical.  Two paths, by shape (b2h_kernel_choice with train = 1):
+ * - B2H_KERNEL_TC_TILE: ONE cooperative launch per rank: forward + loss + backward, grid barrier, cross-CTA reduction,
+ *   exchange, Adam + re-pack.  Buffer: 4-byte words [2][world (source rank)][gradient slots], pushed into every rank's
+ *   buffer; a word is the fp32 gradient and its own arrival flag (see b2h_dp_exchange_fill).  multicast_buf (nullable):
+ *   the multicast (NVLS) address of the buffers (torch symmetric-memory handle .multicast_ptr): ONE multimem.st per slot,
+ *   replicated by the NVSwitch, instead of `world` unicast stores.
+ * - other shapes: three launches: the train kernel, the reduction into this rank's buffer, and a kernel that stores the
+ *   epoch into this rank's flag in every peer's buffer, waits for all flags of its own buffer and sums the peers'
+ *   gradients over NVLink before Adam + re-pack.  Buffer: [2][P] fp32 flat gradients, then [world] int64 flags.
+ * sym_grads: this rank's buffer; peer_bufs_dev: device array [world] of the ranks' buffers, indexed by rank.
+ * step_dev / epoch_dev: device int64 counters advanced by the train kernel (epoch_dev is never rewound).  lr_dev: see
+ * b2h_adam_step.  A wait for a peer that exceeds ~3 s sets the status read by b2h_tc_status / b2h_dp_status and
+ * suppresses every parameter update until it is read. */
 int b2h_train_step_dp(const void* x, int x_dtype, const float* target, const float* conf, const int32_t* lengths,
                       float* params, void* packed, float* exp_avg, float* exp_avg_sq, float* loss_out, int B, int T,
                       int n_in, int C, int pos_emb, int loss_kind, int precision, double lr, double beta1, double beta2,
