@@ -235,14 +235,25 @@ extern "C" int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t
     return B2H_EALIGN;
   }
   Geo g = make_geo(n_in, C, pos_emb);
-  if ((precision != B2H_BF16 && precision != B2H_FP32) || forward_choice(g, T, precision) != B2H_KERNEL_TC_TILE) {
-    set_error("b2h_conv_forward_windows: window views are served by the tcgen05 tile kernel (conv_channels <= 64 in bf16 mode, "
-              "<= 32 in fp32 mode, T <= 256); materialise the windows (b2h_preprocess) for C=%d, T=%d, precision=%d", C, T, precision);
-    return B2H_ESHAPE;
-  }
+  // the tensor-core kernels b2h_conv_forward picks read window views; fp32 mode beyond the tile kernel runs on FFMA, which does not
+  const int choice = (precision == B2H_BF16 || precision == B2H_FP32) ? forward_choice(g, T, precision) : B2H_KERNEL_NONE;
   WindowView wv{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
-  return launch_tc_tile_fwd(frames, x_dtype, params, reinterpret_cast<const char*>(packed), lengths, y, n_win, T, apply_mask, out_scale, g,
-                            (cudaStream_t)stream, &wv, is_split(precision));
+  const char* pk = reinterpret_cast<const char*>(packed);
+  if (choice == B2H_KERNEL_TC_TILE)
+    return launch_tc_tile_fwd(frames, x_dtype, params, pk, lengths, y, n_win, T, apply_mask, out_scale, g, (cudaStream_t)stream, &wv,
+                              is_split(precision));
+  if (choice == B2H_KERNEL_TC_WIDE)
+    return launch_tc_wide_fwd(frames, x_dtype, params, pk, lengths, y, n_win, T, apply_mask, out_scale, g, (cudaStream_t)stream, &wv);
+  if (choice == B2H_KERNEL_TC_ROWSPACE) {
+    TcFwdArgs a{};
+    a.x = frames; a.x_dtype = x_dtype; a.params = params; a.packed = pk; a.lengths = lengths;
+    a.y = y; a.B = n_win; a.T = T; a.apply_mask = apply_mask; a.out_scale = out_scale; a.geo = g; a.wv = wv;
+    return launch_tc_fwd(a, (cudaStream_t)stream);
+  }
+  set_error("b2h_conv_forward_windows: window views are served in bf16 mode for conv_channels <= 64 with T <= 1024 and for "
+            "conv_channels <= 256 with T <= 256, in fp32 mode for conv_channels <= 32 with T <= 256; materialise the windows "
+            "(b2h_preprocess) for C=%d, T=%d, precision=%d", C, T, precision);
+  return B2H_ESHAPE;
 }
 
 static int train_common(const void* x, int x_dtype, const float* target, const float* conf, const float* d_y,

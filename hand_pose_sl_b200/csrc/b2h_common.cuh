@@ -240,6 +240,24 @@ int check_launch(const char* what);
 void count_launch(int n = 1);
 
 
+// Streaming inference (BASELINE config 5): sliding windows read as views of a per-frame stream (n_frames, n_in) instead of
+// materialised (n_win, T, n_in) windows.  win_start == nullptr: the kernel's input is a dense batch of windows.
+struct WindowView { const long long* win_start; const long long* win_end; long long n_frames; int pad_mode; };
+
+// Source row in the stream of (window w, frame t) of a window view; -1 = a zero row.  The crop [start, start + T) is cut at
+// min(win_end[w], n_frames) (win_end nullable), then the dataset's pad rule fills the rest (repeat the crop's first frame:
+// text_pose_dataset.py:511-518; zeros: :614-622) -- the same integer work as K0's windowing (b2h_preprocess.cu), so a view
+// reads exactly the rows K0 would materialise.  The tile kernel keeps the same rule inline (xrow_of, b2h_train_tc.cuh):
+// calling this function there changes the register allocation of its NT = 1 instantiations.
+__device__ __forceinline__ long long window_src_row(const WindowView& v, int w, int t) {
+  const long long start = v.win_start[w];
+  long long cend = v.win_end ? v.win_end[w] : v.n_frames;
+  cend = cend > v.n_frames ? v.n_frames : cend;
+  long long f = start + t;
+  if (f >= cend || f < 0) f = (v.pad_mode == B2H_PAD_REPEAT_FIRST && start >= 0 && start < cend) ? start : -1;
+  return f;
+}
+
 // ---- kernel argument blocks and launchers shared between translation units ----
 struct Fp32Args {
   const void* x; int x_dtype;
@@ -266,6 +284,7 @@ struct TcFwdArgs {
   int B, T, G, NT, RBUF, apply_mask;
   float out_scale;
   Geo geo;
+  WindowView wv;            // win_start set: x is a frame stream and B = the number of windows
 };
 int launch_tc_fwd(TcFwdArgs& p, cudaStream_t stream);
 bool tc_wide_supported(const Geo& g, int T);
@@ -275,7 +294,8 @@ int64_t tc_wide_train_scratch_bytes(const Geo& g, int B, int T);
 int tc_wide_train_loss_parts(const Geo& g, int B, int T);
 int launch_tc_wide_train(const Fp32Args& a, unsigned char* scratch, cudaStream_t stream);
 int launch_tc_wide_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int B, int T, int apply_mask, float out_scale, const Geo& g, cudaStream_t stream);
+                       int B, int T, int apply_mask, float out_scale, const Geo& g, cudaStream_t stream,
+                       const WindowView* wv = nullptr);
 bool tc_fwd_supported(const Geo& g, int T);
 int launch_tc_probe(const void* a, const void* b, float* out, int n, int ksteps, int shift, int variant, cudaStream_t stream);
 int tc_status_and_clear();
@@ -285,7 +305,6 @@ int tc_train_grid(const Geo& g, int B, int T, bool split);
 int tc_train_nsub(int T, bool split);        // sub-windows per window of the tile kernel's training path (1 = whole windows)
 int tc_train_sub_len(bool split);            // their length: 128 frames in fp32 (split) mode, 256 in bf16 mode
 bool tc_tile_ok(const Geo& g, int T, bool train, bool split);   // split = fp32 mode on the tensor pipe (bf16 high/low operand pairs)
-struct WindowView { const long long* win_start; const long long* win_end; long long n_frames; int pad_mode; };
 int launch_tc_tile_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
                        int B, int T, int apply_mask, float out_scale, const Geo& g, cudaStream_t stream, const WindowView* wv = nullptr,
                        bool split = false);

@@ -154,24 +154,28 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_fwd_kernel(TcFwdArgs p)
     for (int i = tid; i < 2 * buf_bytes / 16; i += kTcThreads) z[i] = zero;
   }
   __syncthreads();
-  // stage the input windows: (T, n_in) NWC -> buf0 rows, bf16
+  // stage the input windows: (T, n_in) NWC -> buf0 rows, bf16.  Source row of (window b, frame t): b*T + t, or the window
+  // view's decode (-1: a zero row, left as zeroed above; the pos-emb channel is written for it all the same)
   {
     const int n_in = g.n_in, pe = g.pos_emb;
     const int nwin = (p.B - b0) < G ? (p.B - b0) : G;
+    auto src_row = [&](int b, int t) -> long long { return p.wv.win_start ? window_src_row(p.wv, b, t) : (long long)b * T + t; };
     if (pe == 0 && (n_in & 7) == 0) {
       const int cpr = n_in >> 3;                 // 16-B chunks per row
       for (int i = tid; i < nwin * T * cpr; i += kTcThreads) {
         const int c8 = i % cpr, ft = i / cpr;
         const int gi = ft / T, t = ft - gi * T;
         const int row = 2 + gi * (T + 2) + t;
+        const long long sr = src_row(b0 + gi, t);
+        if (sr < 0) continue;
         float v[8];
         if (p.x_dtype == B2H_DT_F32) {
-          const float4* src = reinterpret_cast<const float4*>(reinterpret_cast<const float*>(p.x) + ((size_t)(b0 + gi) * T + t) * n_in + c8 * 8);
+          const float4* src = reinterpret_cast<const float4*>(reinterpret_cast<const float*>(p.x) + (size_t)sr * n_in + c8 * 8);
           const float4 lo = __ldg(src), hi = __ldg(src + 1);
           v[0] = lo.x; v[1] = lo.y; v[2] = lo.z; v[3] = lo.w; v[4] = hi.x; v[5] = hi.y; v[6] = hi.z; v[7] = hi.w;
           store_row_bf16(buf0, CH, row, c8 * 8, v);
         } else {
-          const uint4 q = __ldg(reinterpret_cast<const uint4*>(reinterpret_cast<const __nv_bfloat16*>(p.x) + ((size_t)(b0 + gi) * T + t) * n_in + c8 * 8));
+          const uint4 q = __ldg(reinterpret_cast<const uint4*>(reinterpret_cast<const __nv_bfloat16*>(p.x) + (size_t)sr * n_in + c8 * 8));
           *reinterpret_cast<uint4*>(buf0 + (size_t)c8 * CH + (size_t)row * 16) = q;
         }
       }
@@ -180,7 +184,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_fwd_kernel(TcFwdArgs p)
         const int c = i % n_in, ft = i / n_in;
         const int gi = ft / T, t = ft - gi * T;
         const int row = 2 + gi * (T + 2) + t;
-        const size_t gidx = ((size_t)(b0 + gi) * T + t) * n_in + c;
+        const long long sr = src_row(b0 + gi, t);
+        if (sr < 0) continue;
+        const size_t gidx = (size_t)sr * n_in + c;
         const float v = (p.x_dtype == B2H_DT_F32) ? __ldg(reinterpret_cast<const float*>(p.x) + gidx)
                                                   : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(p.x)[gidx]);
         const int cc = c + pe;

@@ -49,6 +49,7 @@ struct WideArgs {
   long long act_off[4], dz_off[4];
   float* loss_partials;         // [grid]
   long long* step_dev; long long* epoch_dev;   // MODE 1: device-side step / exchange-epoch counters, bumped by CTA 0 (read by the Adam kernel)
+  WindowView wv;                // MODE 0 only: win_start set = x is a frame stream and B the number of windows viewed in it
 };
 
 constexpr int kWideThreads = 320;
@@ -295,7 +296,18 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
         for (int c8 = ch; c8 < nch0; c8 += 2) {
           uint4 q = make_uint4(0, 0, 0, 0);
           if (rc.valid) {
-            const size_t base = ((size_t)rc.gw * T + rc.t) * n_in;
+            size_t base = ((size_t)rc.gw * T + rc.t) * n_in;
+            if constexpr (MODE == 0) {
+              if (p.wv.win_start) {                  // window view: the source row in the frame stream
+                const long long f = window_src_row(p.wv, rc.gw, rc.t);
+                if (f < 0) {                         // a zero row: no keypoints, the pos-emb channel as in a padded window
+                  if (pe && c8 == 0) q.x = pack_bf16x2(__fdiv_rn((float)rc.t, (float)g.pe_len), 0.0f);
+                  *reinterpret_cast<uint4*>(A + (size_t)c8 * CH + (size_t)rc.row * 16) = q;
+                  continue;
+                }
+                base = (size_t)f * n_in;
+              }
+            }
             if (vec_in && c8 * 8 < n_in) {
               if (p.x_dtype == B2H_DT_F32) {
                 const float4* src = reinterpret_cast<const float4*>(reinterpret_cast<const float*>(p.x) + base) + 2 * c8;
@@ -758,10 +770,11 @@ static void wide_forward_stages(WideArgs& p, const Geo& g) {
 }
 
 int launch_tc_wide_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int B, int T, int apply_mask, float out_scale, const Geo& g, cudaStream_t stream) {
+                       int B, int T, int apply_mask, float out_scale, const Geo& g, cudaStream_t stream, const WindowView* wv) {
   WideArgs p{};
   p.x = x; p.x_dtype = x_dtype; p.params = params; p.packed = packed; p.lengths = lengths; p.y = y;
   p.apply_mask = apply_mask; p.out_scale = out_scale;
+  if (wv) p.wv = *wv;
   size_t smem; int grid;
   if (int rc = wide_common(p, g, B, T, smem, grid)) return rc;
   wide_forward_stages(p, g);

@@ -148,7 +148,9 @@ int b2h_conv_forward(const void* x, int x_dtype, const float* params, const void
  * covering the clip); window w, frame t reads row win_start[w] + t, cut at win_end[w] (nullable: n_frames) and padded by
  * `pad_mode` exactly like b2h_preprocess pads a crop (dataloaders/text_pose_dataset.py:52-68, 511-518, 614-622) -- the
  * same result as materialising the (n_win, T, n_in) windows first, without writing or re-reading them (stride 16 = 4x
- * overlap).  y (n_win, T, 42) fp32.  bf16 mode, conv_channels <= 64, T <= 256 (B2H_ESHAPE otherwise). */
+ * overlap).  y (n_win, T, 42) fp32.  Served by the tensor-core kernels b2h_conv_forward runs: bf16 mode with
+ * conv_channels <= 64 and T <= 1024 or conv_channels <= 256 and T <= 256, fp32 mode with conv_channels <= 32 and T <= 256
+ * (B2H_ESHAPE otherwise, including every shape b2h_conv_forward runs on the FFMA kernel). */
 int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t n_frames, const int64_t* win_start, const int64_t* win_end,
                              int pad_mode, const float* params, const void* packed, const int32_t* lengths, float* y, int n_win,
                              int T, int n_in, int C, int pos_emb, int precision, int apply_mask, float out_scale, void* stream);
