@@ -29,37 +29,44 @@ int check_launch(const char* what) {
 }
 void count_launch(int n) { g_launches.fetch_add(n); }
 
-static bool geo_ok(int n_in, int C, int pos_emb, const char* who) {
-  if (n_in < 1 || n_in > 64 || C < 1 || C > B2H_MAX_C || pos_emb < 0 || pos_emb > 65536) {
-    set_error("%s: unsupported geometry n_in=%d C=%d pos_emb=%d", who, n_in, C, pos_emb);
-    return false;
-  }
-  return true;
+// who == nullptr: a query, which leaves the error string alone
+static bool geo_ok(int n_in, int C, int pos_emb, const char* who = nullptr) {
+  if (n_in >= 1 && n_in <= 64 && C >= 1 && C <= B2H_MAX_C && pos_emb >= 0 && pos_emb <= 65536) return true;
+  if (who) set_error("%s: unsupported geometry n_in=%d C=%d pos_emb=%d", who, n_in, C, pos_emb);
+  return false;
 }
 
 // precision -> is it a tensor-core mode, and with bf16 high/low operand pairs (fp32 mode) or plain bf16 operands
 static bool is_split(int precision) { return precision == B2H_FP32; }
 static bool prec_ok(int precision) { return precision == B2H_FP32 || precision == B2H_BF16 || precision == B2H_FP32_FFMA; }
-static bool use_tc_train(const Geo& g, int T, int precision) {
-  return (precision == B2H_BF16 || precision == B2H_FP32) && tc_tile_ok(g, T, true, is_split(precision));
-}
 
-// Which kernel b2h_conv_forward launches (the ONE place that decides; b2h_kernel_choice reports it).
-static int forward_choice(const Geo& g, int T, int precision) {
-  const int ffma = fp32_smem_bytes(g, T, false) <= (size_t)226 * 1024 ? B2H_KERNEL_FFMA : B2H_KERNEL_NONE;
-  if (precision == B2H_FP32_FFMA) return ffma;
-  if (precision == B2H_FP32) return tc_tile_ok(g, T, false, true) ? B2H_KERNEL_TC_TILE : ffma;   // split tile kernel: C <= 32, T <= 256
-  if (precision != B2H_BF16) return B2H_KERNEL_NONE;
-  if (tc_tile_ok(g, T, false, false)) return B2H_KERNEL_TC_TILE; // independent 128/256-row tiles (T <= 256, C <= 64)
-  if (tc_fwd_supported(g, T)) return B2H_KERNEL_TC_ROWSPACE;     // long windows (T <= 1024, C <= 64): layer-major row space
-  if (tc_wide_supported(g, T)) return B2H_KERNEL_TC_WIDE;        // wide models (C <= 256, T <= 256): streamed weights
-  return B2H_KERNEL_NONE;
+// Which kernel b2h_conv_forward launches and how (the ONE place that decides; b2h_kernel_choice reports it).
+struct ForwardPlan {
+  int kernel;
+  TilePlan tile; RowspacePlan rowspace; WidePlan wide; FfmaPlan ffma;
+};
+static ForwardPlan forward_plan(const Geo& g, int B, int T, int precision) {
+  ForwardPlan f{};
+  f.tile = plan_tile(g, B, T, false, is_split(precision));   // independent 64/128/256-row tiles (T <= 256)
+  f.rowspace = plan_rowspace(g, B, T);                         // long windows (T <= 1024): layer-major row space
+  f.wide = plan_wide(g, B, T);                                 // wide models (C <= 256, T <= 256): streamed weights
+  f.ffma = plan_ffma(g, B, T, false);
+  f.kernel = B2H_KERNEL_NONE;
+  if (precision == B2H_FP32_FFMA) {
+    if (f.ffma.ok) f.kernel = B2H_KERNEL_FFMA;
+  } else if (precision == B2H_FP32) {
+    f.kernel = f.tile.ok ? B2H_KERNEL_TC_TILE : f.ffma.ok ? B2H_KERNEL_FFMA : B2H_KERNEL_NONE;
+  } else if (precision == B2H_BF16) {
+    f.kernel = f.tile.ok ? B2H_KERNEL_TC_TILE : f.rowspace.ok ? B2H_KERNEL_TC_ROWSPACE : f.wide.ok ? B2H_KERNEL_TC_WIDE : B2H_KERNEL_NONE;
+  }
+  return f;
 }
 
 // Which training path serves (B, T, C, precision) and how its workspace is laid out: the ONE place that decides.
 //   [header B2H_WS_HEADER][gradient partials: nparts x stride floats][loss partials: n_loss floats][scratch (wide path)]
 struct TrainPlan {
   int kernel;            // B2H_KERNEL_TC_TILE | B2H_KERNEL_TC_WIDE_TRAIN | B2H_KERNEL_FFMA | B2H_KERNEL_NONE
+  TilePlan tile; WidePlan wide; FfmaPlan ffma;
   int nparts, gp_layout, n_loss;
   int64_t stride, scratch_off, total;
 };
@@ -67,15 +74,16 @@ static TrainPlan train_plan(const Geo& g, int B, int T, int precision) {
   TrainPlan t{};
   t.kernel = B2H_KERNEL_NONE;
   int64_t scratch = 0;
-  if (use_tc_train(g, T, precision)) {
-    t.kernel = B2H_KERNEL_TC_TILE; t.nparts = tc_train_grid(g, B, T, is_split(precision)); t.stride = gp_total(g); t.gp_layout = 1; t.n_loss = t.nparts;
-  } else if (precision == B2H_BF16 && tc_wide_supported(g, T)) {
-    // 32 < conv_channels <= 256: forward+criterion / dgrad chain / split-K wgrad kernels over scratch dumps
-    t.kernel = B2H_KERNEL_TC_WIDE_TRAIN; t.nparts = tc_wide_train_ksplit(g, B, T); t.stride = gp_total(g); t.gp_layout = 1;
-    t.n_loss = tc_wide_train_loss_parts(g, B, T);
-    scratch = tc_wide_train_scratch_bytes(g, B, T);
-  } else if (fp32_smem_bytes(g, T, true) <= (size_t)226 * 1024) {
-    t.kernel = B2H_KERNEL_FFMA; t.nparts = fp32_train_grid(g, B, T); t.stride = g.P; t.gp_layout = 0; t.n_loss = t.nparts;
+  if (precision == B2H_BF16 || precision == B2H_FP32) t.tile = plan_tile(g, B, T, true, is_split(precision));
+  if (precision == B2H_BF16) t.wide = plan_wide(g, B, T);   // 32 < conv_channels <= 256: forward+criterion / dgrad chain / split-K wgrad
+  t.ffma = plan_ffma(g, B, T, true);
+  if (t.tile.ok) {
+    t.kernel = B2H_KERNEL_TC_TILE; t.nparts = t.tile.grid; t.stride = gp_total(g); t.gp_layout = 1; t.n_loss = t.nparts;
+  } else if (t.wide.ok) {
+    t.kernel = B2H_KERNEL_TC_WIDE_TRAIN; t.nparts = t.wide.ksplit; t.stride = gp_total(g); t.gp_layout = 1; t.n_loss = t.wide.n_loss;
+    scratch = t.wide.scratch_bytes;
+  } else if (t.ffma.ok) {
+    t.kernel = B2H_KERNEL_FFMA; t.nparts = t.ffma.grid; t.stride = g.P; t.gp_layout = 0; t.n_loss = t.nparts;
   }
   int64_t o = B2H_WS_HEADER + ((int64_t)t.nparts * t.stride + t.n_loss) * 4;
   o = (o + 255) / 256 * 256;
@@ -137,19 +145,18 @@ extern "C" int64_t b2h_packed_bytes(int n_in, int C, int pos_emb) {
   return make_geo(n_in, C, pos_emb).packed_bytes;
 }
 extern "C" int b2h_supported(int T, int n_in, int C, int pos_emb, int precision) {
-  if (n_in < 1 || n_in > 64 || C < 1 || C > B2H_MAX_C || T < 1 || pos_emb < 0 || pos_emb > 65536) return 0;
+  if (!geo_ok(n_in, C, pos_emb) || T < 1 || !prec_ok(precision)) return 0;
   Geo g = make_geo(n_in, C, pos_emb);
-  if (!prec_ok(precision)) return 0;
-  return (forward_choice(g, T, precision) != B2H_KERNEL_NONE && train_plan(g, 1, T, precision).kernel != B2H_KERNEL_NONE) ? 1 : 0;
+  return (forward_plan(g, 1, T, precision).kernel != B2H_KERNEL_NONE && train_plan(g, 1, T, precision).kernel != B2H_KERNEL_NONE) ? 1 : 0;
 }
 extern "C" int b2h_forward_supported(int T, int n_in, int C, int pos_emb, int precision) {
-  if (n_in < 1 || n_in > 64 || C < 1 || C > B2H_MAX_C || T < 1 || pos_emb < 0 || pos_emb > 65536) return 0;
-  return forward_choice(make_geo(n_in, C, pos_emb), T, precision) != B2H_KERNEL_NONE ? 1 : 0;
+  if (!geo_ok(n_in, C, pos_emb) || T < 1) return 0;
+  return forward_plan(make_geo(n_in, C, pos_emb), 1, T, precision).kernel != B2H_KERNEL_NONE ? 1 : 0;
 }
 extern "C" int b2h_kernel_choice(int T, int n_in, int C, int pos_emb, int precision, int train) {
-  if (n_in < 1 || n_in > 64 || C < 1 || C > B2H_MAX_C || T < 1 || pos_emb < 0 || pos_emb > 65536) return B2H_KERNEL_NONE;
+  if (!geo_ok(n_in, C, pos_emb) || T < 1) return B2H_KERNEL_NONE;
   Geo g = make_geo(n_in, C, pos_emb);
-  if (!train) return forward_choice(g, T, precision);
+  if (!train) return forward_plan(g, 1, T, precision).kernel;
   if (!prec_ok(precision)) return B2H_KERNEL_NONE;
   return train_plan(g, 1, T, precision).kernel;
 }
@@ -158,16 +165,13 @@ extern "C" int b2h_kernel_choice(int T, int n_in, int C, int pos_emb, int precis
 extern "C" int b2h_train_subwindows(int T, int n_in, int C, int pos_emb, int precision, int i, int* out4) {
   if (!geo_ok(n_in, C, pos_emb, "b2h_train_subwindows")) return B2H_ESHAPE;
   if (T < 1) { set_error("b2h_train_subwindows: bad T"); return B2H_ESHAPE; }
-  Geo g = make_geo(n_in, C, pos_emb);
-  const int n = use_tc_train(g, T, precision) ? tc_train_nsub(T, is_split(precision)) : 1;
+  const TrainPlan t = train_plan(make_geo(n_in, C, pos_emb), 1, T, precision);
+  const bool tile = t.kernel == B2H_KERNEL_TC_TILE;
+  const int n = tile ? t.tile.n_sub : 1, Ts = tile ? t.tile.T : T;
   if (out4) {
     if (i < 0 || i >= n) { set_error("b2h_train_subwindows: sub-window %d of %d", i, n); return B2H_EINVAL; }
-    if (n == 1) { out4[0] = 0; out4[1] = 0; out4[2] = T; out4[3] = T; }
-    else {
-      const int Ts = tc_train_sub_len(is_split(precision));
-      const SubWindow s = sub_window(T, Ts, n, i);
-      out4[0] = s.start; out4[1] = s.clo; out4[2] = s.chi; out4[3] = Ts;
-    }
+    const SubWindow s = sub_window(T, Ts, n, i);
+    out4[0] = s.start; out4[1] = s.clo; out4[2] = s.chi; out4[3] = Ts;
   }
   return n;
 }
@@ -184,76 +188,66 @@ extern "C" int b2h_pack_weights(const float* params, void* packed, int n_in, int
   return launch_pack(params, packed, make_geo(n_in, C, pos_emb), (cudaStream_t)stream);
 }
 
+// The forward of B dense windows x (wv == nullptr) or of B windows viewed in the frame stream x.  Window views are read by
+// the tensor-core kernels only: fp32 mode beyond the tile kernel runs on FFMA, which reads dense windows.
+static int conv_forward(const void* x, int x_dtype, const WindowView* wv, const float* params, const void* packed,
+                        const int32_t* lengths, float* y, int B, int T, int n_in, int C, int pos_emb, int precision,
+                        int apply_mask, float out_scale, cudaStream_t stream, const char* who) {
+  if (!x || (wv && !wv->win_start) || !params || !packed || !y) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  if (x_dtype != B2H_DT_F32 && x_dtype != B2H_DT_BF16) { set_error("%s: bad x_dtype %d", who, x_dtype); return B2H_EINVAL; }
+  if (wv && wv->pad_mode != B2H_PAD_REPEAT_FIRST && wv->pad_mode != B2H_PAD_ZEROS) { set_error("%s: bad pad_mode %d", who, wv->pad_mode); return B2H_EINVAL; }
+  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
+  if (B < 0 || T < 1 || (wv && wv->n_frames < 0)) { set_error("%s: bad B=%d T=%d", who, B, T); return B2H_ESHAPE; }
+  if (apply_mask && !lengths) { set_error("%s: apply_mask needs lengths", who); return B2H_EINVAL; }
+  if (B == 0) return B2H_OK;
+  if ((reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(y) & 15) || (reinterpret_cast<uintptr_t>(packed) & 15)) {
+    set_error("%s: %s, y and packed must be 16-byte aligned", who, wv ? "frames" : "x");
+    return B2H_EALIGN;
+  }
+  if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
+  const Geo g = make_geo(n_in, C, pos_emb);
+  const ForwardPlan f = forward_plan(g, B, T, precision);
+  const char* pk = reinterpret_cast<const char*>(packed);
+  if (f.kernel == B2H_KERNEL_TC_TILE) return launch_tc_tile_fwd(x, x_dtype, params, pk, lengths, y, apply_mask, out_scale, g, f.tile, stream, wv);
+  if (f.kernel == B2H_KERNEL_TC_WIDE) return launch_tc_wide_fwd(x, x_dtype, params, pk, lengths, y, B, T, apply_mask, out_scale, g, f.wide, stream, wv);
+  if (f.kernel == B2H_KERNEL_TC_ROWSPACE) {
+    TcFwdArgs a{};
+    a.x = x; a.x_dtype = x_dtype; a.params = params; a.packed = pk; a.lengths = lengths;
+    a.y = y; a.B = B; a.T = T; a.apply_mask = apply_mask; a.out_scale = out_scale; a.geo = g;
+    if (wv) a.wv = *wv;
+    return launch_tc_fwd(a, f.rowspace, stream);
+  }
+  if (f.kernel == B2H_KERNEL_FFMA && !wv) {
+    Fp32Args a{};
+    a.x = x; a.x_dtype = x_dtype; a.lengths = lengths; a.params = params; a.packed = pk;
+    a.y = y; a.B = B; a.T = T; a.apply_mask = apply_mask; a.mode = 0; a.out_scale = out_scale; a.geo = g;
+    return launch_fp32(a, f.ffma, stream);
+  }
+  if (wv)
+    set_error("%s: window views are served in bf16 mode for conv_channels <= 256 with T <= 256, <= 48 with T <= 640 and <= 32 "
+              "with T <= 1024 (the last two with at most 32 input channels), in fp32 mode for conv_channels <= 32 with T <= 256; "
+              "materialise the windows (b2h_preprocess) for C=%d, T=%d, precision=%d", who, C, T, precision);
+  else
+    set_error("%s: no kernel for C=%d, T=%d, precision=%d (tensor cores: bf16 conv_channels <= 256 with T <= 256, <= 48 with "
+              "T <= 640 and <= 32 with T <= 1024 at up to 32 input channels, fp32 conv_channels <= 32 with T <= 256; the FFMA "
+              "kernel would need %zu B of its 226 KB of shared memory)", who, C, T, precision, f.ffma.smem);
+  return B2H_ESHAPE;
+}
+
 extern "C" int b2h_conv_forward(const void* x, int x_dtype, const float* params, const void* packed, const int32_t* lengths,
                                 float* y, int B, int T, int n_in, int C, int pos_emb, int precision, int apply_mask,
                                 float out_scale, void* stream) {
-  if (!x || !params || !packed || !y) { set_error("b2h_conv_forward: null pointer"); return B2H_EINVAL; }
-  if (x_dtype != B2H_DT_F32 && x_dtype != B2H_DT_BF16) { set_error("b2h_conv_forward: bad x_dtype %d", x_dtype); return B2H_EINVAL; }
-  if (!geo_ok(n_in, C, pos_emb, "b2h_conv_forward")) return B2H_ESHAPE;
-  if (B < 0 || T < 1) { set_error("b2h_conv_forward: bad B=%d T=%d", B, T); return B2H_ESHAPE; }
-  if (apply_mask && !lengths) { set_error("b2h_conv_forward: apply_mask needs lengths"); return B2H_EINVAL; }
-  if (B == 0) return B2H_OK;
-  if ((reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(y) & 15) || (reinterpret_cast<uintptr_t>(packed) & 15)) {
-    set_error("b2h_conv_forward: x, y and packed must be 16-byte aligned");
-    return B2H_EALIGN;
-  }
-  Geo g = make_geo(n_in, C, pos_emb);
-  if (!prec_ok(precision)) { set_error("b2h_conv_forward: bad precision %d", precision); return B2H_EINVAL; }
-  const int choice = forward_choice(g, T, precision);
-  if (precision == B2H_FP32_FFMA || (precision == B2H_FP32 && choice != B2H_KERNEL_TC_TILE)) {
-    Fp32Args a{};
-    a.x = x; a.x_dtype = x_dtype; a.lengths = lengths; a.params = params; a.packed = reinterpret_cast<const char*>(packed);
-    a.y = y; a.B = B; a.T = T; a.apply_mask = apply_mask; a.mode = 0; a.out_scale = out_scale; a.geo = g;
-    return launch_fp32(a, false, (cudaStream_t)stream, 0);
-  } else {
-    if (choice == B2H_KERNEL_TC_TILE)
-      return launch_tc_tile_fwd(x, x_dtype, params, reinterpret_cast<const char*>(packed), lengths, y, B, T, apply_mask, out_scale, g,
-                                (cudaStream_t)stream, nullptr, is_split(precision));
-    if (choice == B2H_KERNEL_TC_WIDE)
-      return launch_tc_wide_fwd(x, x_dtype, params, reinterpret_cast<const char*>(packed), lengths, y, B, T, apply_mask, out_scale, g,
-                                (cudaStream_t)stream);
-    TcFwdArgs a{};                 // long windows: layer-major row-space kernel (reports the limits itself when unsupported)
-    a.x = x; a.x_dtype = x_dtype; a.params = params; a.packed = reinterpret_cast<const char*>(packed); a.lengths = lengths;
-    a.y = y; a.B = B; a.T = T; a.apply_mask = apply_mask; a.out_scale = out_scale; a.geo = g;
-    return launch_tc_fwd(a, (cudaStream_t)stream);
-  }
+  return conv_forward(x, x_dtype, nullptr, params, packed, lengths, y, B, T, n_in, C, pos_emb, precision, apply_mask, out_scale,
+                      (cudaStream_t)stream, "b2h_conv_forward");
 }
 
 extern "C" int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t n_frames, const int64_t* win_start,
                                         const int64_t* win_end, int pad_mode, const float* params, const void* packed,
                                         const int32_t* lengths, float* y, int n_win, int T, int n_in, int C, int pos_emb,
                                         int precision, int apply_mask, float out_scale, void* stream) {
-  if (!frames || !win_start || !params || !packed || !y) { set_error("b2h_conv_forward_windows: null pointer"); return B2H_EINVAL; }
-  if (x_dtype != B2H_DT_F32 && x_dtype != B2H_DT_BF16) { set_error("b2h_conv_forward_windows: bad x_dtype %d", x_dtype); return B2H_EINVAL; }
-  if (pad_mode != B2H_PAD_REPEAT_FIRST && pad_mode != B2H_PAD_ZEROS) { set_error("b2h_conv_forward_windows: bad pad_mode %d", pad_mode); return B2H_EINVAL; }
-  if (!geo_ok(n_in, C, pos_emb, "b2h_conv_forward_windows")) return B2H_ESHAPE;
-  if (n_win < 0 || T < 1 || n_frames < 0) { set_error("b2h_conv_forward_windows: bad n_win=%d T=%d", n_win, T); return B2H_ESHAPE; }
-  if (apply_mask && !lengths) { set_error("b2h_conv_forward_windows: apply_mask needs lengths"); return B2H_EINVAL; }
-  if (n_win == 0) return B2H_OK;
-  if ((reinterpret_cast<uintptr_t>(frames) & 15) || (reinterpret_cast<uintptr_t>(y) & 15) || (reinterpret_cast<uintptr_t>(packed) & 15)) {
-    set_error("b2h_conv_forward_windows: frames, y and packed must be 16-byte aligned");
-    return B2H_EALIGN;
-  }
-  Geo g = make_geo(n_in, C, pos_emb);
-  // the tensor-core kernels b2h_conv_forward picks read window views; fp32 mode beyond the tile kernel runs on FFMA, which does not
-  const int choice = (precision == B2H_BF16 || precision == B2H_FP32) ? forward_choice(g, T, precision) : B2H_KERNEL_NONE;
-  WindowView wv{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
-  const char* pk = reinterpret_cast<const char*>(packed);
-  if (choice == B2H_KERNEL_TC_TILE)
-    return launch_tc_tile_fwd(frames, x_dtype, params, pk, lengths, y, n_win, T, apply_mask, out_scale, g, (cudaStream_t)stream, &wv,
-                              is_split(precision));
-  if (choice == B2H_KERNEL_TC_WIDE)
-    return launch_tc_wide_fwd(frames, x_dtype, params, pk, lengths, y, n_win, T, apply_mask, out_scale, g, (cudaStream_t)stream, &wv);
-  if (choice == B2H_KERNEL_TC_ROWSPACE) {
-    TcFwdArgs a{};
-    a.x = frames; a.x_dtype = x_dtype; a.params = params; a.packed = pk; a.lengths = lengths;
-    a.y = y; a.B = n_win; a.T = T; a.apply_mask = apply_mask; a.out_scale = out_scale; a.geo = g; a.wv = wv;
-    return launch_tc_fwd(a, (cudaStream_t)stream);
-  }
-  set_error("b2h_conv_forward_windows: window views are served in bf16 mode for conv_channels <= 64 with T <= 1024 and for "
-            "conv_channels <= 256 with T <= 256, in fp32 mode for conv_channels <= 32 with T <= 256; materialise the windows "
-            "(b2h_preprocess) for C=%d, T=%d, precision=%d", C, T, precision);
-  return B2H_ESHAPE;
+  const WindowView wv{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
+  return conv_forward(frames, x_dtype, &wv, params, packed, lengths, y, n_win, T, n_in, C, pos_emb, precision, apply_mask,
+                      out_scale, (cudaStream_t)stream, "b2h_conv_forward_windows");
 }
 
 static int train_common(const void* x, int x_dtype, const float* target, const float* conf, const float* d_y,
@@ -281,7 +275,7 @@ static int train_common(const void* x, int x_dtype, const float* target, const f
   if (plan.kernel == B2H_KERNEL_NONE) {
     set_error("%s: no training kernel for conv_channels=%d, T=%d, precision=%d (tcgen05 training: C <= 32 in the one-launch tile "
               "kernel, C <= 256 in bf16 mode through the wide kernels, T <= 256; the FFMA kernel would need %zu B of shared memory)",
-              who, C, T, precision, fp32_smem_bytes(g, T, true));
+              who, C, T, precision, plan.ffma.smem);
     return B2H_ESHAPE;
   }
   const int nparts = plan.nparts;
@@ -304,13 +298,13 @@ static int train_common(const void* x, int x_dtype, const float* target, const f
       fuse->hdr = reinterpret_cast<unsigned*>(workspace);
       a.fuse = *fuse;
     }
-    return launch_tc_tile_train(a, stream, is_split(precision));
+    return launch_tc_tile_train(a, plan.tile, stream);
   }
   if (plan.kernel == B2H_KERNEL_TC_WIDE_TRAIN) {
     // (the forward+criterion kernel's CTA 0 bumps the device-side step / epoch counters the Adam kernels read)
-    return launch_tc_wide_train(a, reinterpret_cast<unsigned char*>(workspace) + plan.scratch_off, stream);
+    return launch_tc_wide_train(a, plan.wide, reinterpret_cast<unsigned char*>(workspace) + plan.scratch_off, stream);
   }
-  return launch_fp32(a, true, stream, nparts);
+  return launch_fp32(a, plan.ffma, stream);
 }
 
 extern "C" int b2h_train_forward_backward(const void* x, int x_dtype, const float* target, const float* conf,

@@ -258,6 +258,50 @@ __device__ __forceinline__ long long window_src_row(const WindowView& v, int w, 
   return f;
 }
 
+// ---- launch plans: for each kernel family, one host function (in the file that owns the kernel) decides whether a
+// shape fits and how it launches.  The C-ABI queries, the workspace layout and the launchers all read the same plan, so
+// the number of gradient / loss partial slices a launch writes is the number the workspace was sized for. ----
+
+// Tile kernel (b2h_train_tc.cuh): weights resident in shared memory, independent 64/128/256-row tiles.
+struct TilePlan {
+  bool ok, train, split;    // split = fp32 mode on the tensor pipe (bf16 high/low operand pairs)
+  int n_sub;                // training sub-windows per window (1 = whole windows; see TcTileArgs)
+  int B, T;                 // launch batch and window length: B * n_sub sub-windows of T = 128 (split) / 256 frames if n_sub > 1
+  int nhalf, MB, NT, HR, gh, n_tiles;
+  size_t smem;
+  int grid;                 // CTAs = gradient and loss partial slices of a training launch
+};
+TilePlan plan_tile(const Geo& g, int B, int T, bool train, bool split);
+
+// Row-space forward (b2h_conv_tc.cu): G windows per CTA in one layer-major row space of NT 128-row tiles.
+struct RowspacePlan {
+  bool ok;                  // one window per CTA fits: support does not depend on B
+  int G, NT, RBUF;
+  size_t smem;
+  int grid;
+};
+RowspacePlan plan_rowspace(const Geo& g, int B, int T);
+
+// Wide kernels (b2h_wide_tc.cuh): weights streamed through a ring of nstage stages; training adds split-K wgrad.
+struct WidePlan {
+  bool ok;
+  int gh, n_tiles, a_bytes, nstage;
+  size_t smem;
+  int grid;
+  int ksplit;               // training: gradient partial slices written by the wgrad kernel
+  int n_loss;               // training: loss partials (one per CTA of the forward+criterion kernel)
+  int64_t scratch_bytes;    // training: per-tile operand dumps
+};
+WidePlan plan_wide(const Geo& g, int B, int T);
+
+// FFMA kernel (b2h_conv_fp32.cu): one window per CTA iteration, fp32 activations in shared memory.
+struct FfmaPlan {
+  bool ok, train;
+  size_t smem;
+  int grid;                 // training: CTAs = gradient and loss partial slices
+};
+FfmaPlan plan_ffma(const Geo& g, int B, int T, bool train);
+
 // ---- kernel argument blocks and launchers shared between translation units ----
 struct Fp32Args {
   const void* x; int x_dtype;
@@ -273,9 +317,7 @@ struct Fp32Args {
   float out_scale;
   Geo geo;
 };
-int launch_fp32(Fp32Args& p, bool train, cudaStream_t stream, int grid_override);
-int fp32_train_grid(const Geo& g, int B, int T);
-size_t fp32_smem_bytes(const Geo& g, int T, bool train);
+int launch_fp32(Fp32Args& p, const FfmaPlan& plan, cudaStream_t stream);
 
 struct TcFwdArgs {
   const void* x; int x_dtype;
@@ -286,29 +328,19 @@ struct TcFwdArgs {
   Geo geo;
   WindowView wv;            // win_start set: x is a frame stream and B = the number of windows
 };
-int launch_tc_fwd(TcFwdArgs& p, cudaStream_t stream);
-bool tc_wide_supported(const Geo& g, int T);
+int launch_tc_fwd(TcFwdArgs& p, const RowspacePlan& plan, cudaStream_t stream);
 // wide training (32 < conv_channels <= 256, bf16 mode): forward+criterion / dgrad chain / split-K wgrad over scratch dumps
-int tc_wide_train_ksplit(const Geo& g, int B, int T);          // gradient-partial slices written (= nparts of the reduction)
-int64_t tc_wide_train_scratch_bytes(const Geo& g, int B, int T);
-int tc_wide_train_loss_parts(const Geo& g, int B, int T);
-int launch_tc_wide_train(const Fp32Args& a, unsigned char* scratch, cudaStream_t stream);
+int launch_tc_wide_train(const Fp32Args& a, const WidePlan& plan, unsigned char* scratch, cudaStream_t stream);
 int launch_tc_wide_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int B, int T, int apply_mask, float out_scale, const Geo& g, cudaStream_t stream,
-                       const WindowView* wv = nullptr);
-bool tc_fwd_supported(const Geo& g, int T);
+                       int B, int T, int apply_mask, float out_scale, const Geo& g, const WidePlan& plan, cudaStream_t stream,
+                       const WindowView* wv);
 int launch_tc_probe(const void* a, const void* b, float* out, int n, int ksteps, int shift, int variant, cudaStream_t stream);
 int tc_status_and_clear();
 
-struct TcTileArgs;
-int tc_train_grid(const Geo& g, int B, int T, bool split);
-int tc_train_nsub(int T, bool split);        // sub-windows per window of the tile kernel's training path (1 = whole windows)
-int tc_train_sub_len(bool split);            // their length: 128 frames in fp32 (split) mode, 256 in bf16 mode
-bool tc_tile_ok(const Geo& g, int T, bool train, bool split);   // split = fp32 mode on the tensor pipe (bf16 high/low operand pairs)
+// the tile launchers take the launch batch and window length from the plan
 int launch_tc_tile_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int B, int T, int apply_mask, float out_scale, const Geo& g, cudaStream_t stream, const WindowView* wv = nullptr,
-                       bool split = false);
-int launch_tc_tile_train(const Fp32Args& a, cudaStream_t stream, bool split = false);
+                       int apply_mask, float out_scale, const Geo& g, const TilePlan& plan, cudaStream_t stream, const WindowView* wv);
+int launch_tc_tile_train(const Fp32Args& a, const TilePlan& plan, cudaStream_t stream);
 
 void set_debug_timing(long long* p);
 int launch_tc_bench(long long* out, int M, int N, int reps, int nacc, int mn_major, cudaStream_t stream);

@@ -297,42 +297,33 @@ __global__ void __launch_bounds__(kThreads) conv_fp32_kernel(Fp32Args p) {
 }
 
 
-size_t fp32_smem_bytes(const Geo& g, int T, bool train) {
+FfmaPlan plan_ffma(const Geo& g, int B, int T, bool train) {
+  FfmaPlan p{};
+  p.train = train;
   const int TR = round_up(T, 8) + 4;
   const int ld0 = round_up(g.cin[0], 4), ldc = round_up(g.C, 4), ldg = round_up(g.C > B2H_COUT ? g.C : B2H_COUT, 4);
   size_t fl = train ? (size_t)TR * (ld0 + 3 * ldc + 2 * ldg) : (size_t)TR * (ld0 + 2 * ldc);
-  return fl * 4;
-}
-
-int fp32_train_grid(const Geo& g, int B, int T) {
-  size_t smem = fp32_smem_bytes(g, T, true);
-  int per_sm = (int)((size_t)220 * 1024 / (smem + 1024));
-  if (per_sm < 1) per_sm = 1;
-  if (per_sm > 2) per_sm = 2;
-  int grid = num_sms() * per_sm;
-  return B < grid ? B : grid;
-}
-
-int launch_fp32(Fp32Args& p, bool train, cudaStream_t stream, int grid_override) {
-  const size_t smem = fp32_smem_bytes(p.geo, p.T, train);
-  if (smem > (size_t)226 * 1024) {
-    set_error("fp32 path: window of T=%d, C=%d needs %zu B of shared memory (> 227 KB)", p.T, p.geo.C, smem);
-    return B2H_ESHAPE;
-  }
-  // opt in to > 48 KB of dynamic shared memory (dynamic + static must stay <= 227 KB)
-  if (int rc = ensure_dyn_smem(train ? reinterpret_cast<const void*>(conv_fp32_kernel<true>) : reinterpret_cast<const void*>(conv_fp32_kernel<false>), smem))
-    return rc;
-  int grid;
+  p.smem = fl * 4;
+  p.ok = p.smem <= (size_t)226 * 1024;   // dynamic + static shared memory must stay <= 227 KB
+  int per_sm = 8;
   if (train) {
-    grid = grid_override > 0 ? grid_override : fp32_train_grid(p.geo, p.B, p.T);
-    conv_fp32_kernel<true><<<grid, kThreads, smem, stream>>>(p);
-  } else {
-    int cap = num_sms() * 8;
-    grid = p.B < cap ? p.B : cap;
-    conv_fp32_kernel<false><<<grid, kThreads, smem, stream>>>(p);
+    per_sm = (int)((size_t)220 * 1024 / (p.smem + 1024));
+    if (per_sm < 1) per_sm = 1;
+    if (per_sm > 2) per_sm = 2;
   }
+  const int cap = num_sms() * per_sm;
+  p.grid = B < cap ? B : cap;
+  return p;
+}
+
+int launch_fp32(Fp32Args& p, const FfmaPlan& plan, cudaStream_t stream) {
+  const void* fn = plan.train ? reinterpret_cast<const void*>(conv_fp32_kernel<true>) : reinterpret_cast<const void*>(conv_fp32_kernel<false>);
+  // opt in to > 48 KB of dynamic shared memory
+  if (int rc = ensure_dyn_smem(fn, plan.smem)) return rc;
+  if (plan.train) conv_fp32_kernel<true><<<plan.grid, kThreads, plan.smem, stream>>>(p);
+  else conv_fp32_kernel<false><<<plan.grid, kThreads, plan.smem, stream>>>(p);
   count_launch();
-  return check_launch(train ? "conv_fp32_kernel<train>" : "conv_fp32_kernel<fwd>");
+  return check_launch(plan.train ? "conv_fp32_kernel<train>" : "conv_fp32_kernel<fwd>");
 }
 
 }  // namespace b2h

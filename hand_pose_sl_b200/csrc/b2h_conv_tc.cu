@@ -283,41 +283,36 @@ __global__ void __launch_bounds__(kTcThreads, 1) conv_tc_fwd_kernel(TcFwdArgs p)
 }
 
 
-bool tc_fwd_supported(const Geo& g, int T) {
-  if (g.C > 64 || g.cin[0] > 64) return false;
-  // one window must fit the row space of a CTA (<= 8 tiles of 128 rows)
-  return (T + 2) - 2 <= 8 * 128 && T >= 1;
-}
-
-static void tc_plan(const Geo& g, int B, int T, int& G, int& NT, int& RBUF, size_t& smem) {
-  const int sms = num_sms();
-  G = (B + sms - 1) / sms;
-  if (G < 1) G = 1;
-  const int gmax = (8 * 128 + 2) / (T + 2);
-  if (G > gmax) G = gmax;
-  if (G < 1) G = 1;
-  NT = (G * (T + 2) - 2 + 127) / 128;
-  RBUF = 128 * NT + 8;
+// G = enough windows per CTA to cover B with one CTA per SM, capped by the row space (<= 8 tiles of 128 rows) and by the
+// 225 KB of shared memory that hold all four layers' weights and two activation buffers of RBUF rows.
+RowspacePlan plan_rowspace(const Geo& g, int B, int T) {
+  RowspacePlan p{};
   int wtot = 0;
   for (int l = 0; l < 4; ++l) wtot += B2H_KW * g.kp[l] * g.np_[l] * 2;
   const int KPmax = g.kp[0] > g.kp[1] ? g.kp[0] : g.kp[1];
-  smem = (size_t)((wtot + 127) / 128) * 128 + (size_t)2 * (KPmax / 8) * RBUF * 16;
+  auto geometry = [&](int G) {
+    p.G = G;
+    p.NT = (G * (T + 2) - 2 + 127) / 128;
+    p.RBUF = 128 * p.NT + 8;
+    p.smem = (size_t)((wtot + 127) / 128) * 128 + (size_t)2 * (KPmax / 8) * p.RBUF * 16;
+  };
+  if (g.C > 64 || g.cin[0] > 64 || T < 1 || T > 8 * 128) return p;
+  const int sms = num_sms();
+  int G = (B + sms - 1) / sms;
+  const int gmax = (8 * 128 + 2) / (T + 2);
+  if (G > gmax) G = gmax;
+  if (G < 1) G = 1;
+  geometry(G);
+  while (p.G > 1 && p.smem > (size_t)225 * 1024) geometry(p.G - 1);
+  p.ok = p.smem <= (size_t)225 * 1024;
+  p.grid = (B + p.G - 1) / p.G;
+  return p;
 }
 
-int launch_tc_fwd(TcFwdArgs& p, cudaStream_t stream) {
-  if (!tc_fwd_supported(p.geo, p.T)) {
-    set_error("bf16 tensor-core forward supports C <= 64 and T <= 1024 (got C=%d, T=%d)", p.geo.C, p.T);
-    return B2H_ESHAPE;
-  }
-  size_t smem;
-  tc_plan(p.geo, p.B, p.T, p.G, p.NT, p.RBUF, smem);
-  if (smem > (size_t)225 * 1024) {
-    set_error("bf16 forward: T=%d C=%d needs %zu B shared memory", p.T, p.geo.C, smem);
-    return B2H_ESHAPE;
-  }
-  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_fwd_kernel), smem)) return rc;
-  const int grid = (p.B + p.G - 1) / p.G;
-  conv_tc_fwd_kernel<<<grid, kTcThreads, smem, stream>>>(p);
+int launch_tc_fwd(TcFwdArgs& p, const RowspacePlan& plan, cudaStream_t stream) {
+  p.G = plan.G; p.NT = plan.NT; p.RBUF = plan.RBUF;
+  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_fwd_kernel), plan.smem)) return rc;
+  conv_tc_fwd_kernel<<<plan.grid, kTcThreads, plan.smem, stream>>>(p);
   count_launch();
   return check_launch("conv_tc_fwd_kernel");
 }

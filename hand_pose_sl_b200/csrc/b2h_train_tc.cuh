@@ -1017,61 +1017,46 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
 }
 
 // ---- host side ----
-inline size_t tc_tile_smem(const Geo& g, int T, bool train, bool split) {
-  const int MB = T <= 64 ? 64 : (T > 128 ? 256 : 128), nhalf = T <= 64 ? 2 : 1;
-  return (size_t)tile_smem_layout(g, nhalf * (MB + 8), train, split).total;
-}
-
 // Training of windows longer than one tile segment (128 frames in fp32 mode, 256 in bf16 mode): n_sub overlapping
 // sub-windows of Ts frames (see TcTileArgs), every cut with >= 16 real frames of context on both sides: the two edge
 // sub-windows carry up to Ts - 16 core frames, the interior ones Ts - 32.
 constexpr int kTileMaxTrainT = 4096;
-inline int tc_tile_sub_len(bool split) { return split ? 128 : 256; }
-inline int tc_tile_nsub(int T, bool train, bool split) {
-  const int Ts = tc_tile_sub_len(split);
-  if (!train || T <= Ts) return 1;
-  int n = 2;
-  while (2 * (Ts - 16) + (n - 2) * (Ts - 32) < T) ++n;
-  return n;
-}
 
-inline bool tc_tile_supported(const Geo& g, int T, bool train, bool split) {
-  if (T < 1 || T > (train ? kTileMaxTrainT : 256)) return false;
-  if ((g.kp[0] > 32 || g.kp[1] > 32) && (train || split || g.kp[0] > 64 || g.kp[1] > 64)) return false;
-  const int Tk = tc_tile_nsub(T, train, split) > 1 ? tc_tile_sub_len(split) : T;
-  return tc_tile_smem(g, Tk, train, split) <= (size_t)225 * 1024;
-}
-
-inline void tc_tile_plan(const Geo& g, int B, int T, bool train, bool split, TcTileArgs& p, size_t& smem, int& grid) {
-  if (T <= 64) { p.nhalf = 2; p.MB = 64; p.NT = 1; }
-  else { p.nhalf = 1; p.NT = (T > 128) ? 2 : 1; p.MB = 128 * p.NT; }
+TilePlan plan_tile(const Geo& g, int B, int T, bool train, bool split) {
+  TilePlan p{};
+  p.train = train; p.split = split;
+  if (T < 1 || T > (train ? kTileMaxTrainT : 256)) return p;
+  if ((g.kp[0] > 32 || g.kp[1] > 32) && (train || split || g.kp[0] > 64 || g.kp[1] > 64)) return p;
+  p.n_sub = 1;
+  const int Ts = split ? 128 : 256;
+  if (train && T > Ts) {
+    p.n_sub = 2;
+    while (2 * (Ts - 16) + (p.n_sub - 2) * (Ts - 32) < T) ++p.n_sub;
+  }
+  p.B = B * p.n_sub;
+  p.T = p.n_sub > 1 ? Ts : T;
+  if (p.T <= 64) { p.nhalf = 2; p.MB = 64; p.NT = 1; }
+  else { p.nhalf = 1; p.NT = (p.T > 128) ? 2 : 1; p.MB = 128 * p.NT; }
   p.HR = p.MB + 8;
-  p.gh = (p.MB + 2) / (T + 2);
+  p.gh = (p.MB + 2) / (p.T + 2);
   const int wpt = p.nhalf * p.gh;
-  p.n_tiles = (B + wpt - 1) / wpt;
-  smem = (size_t)tile_smem_layout(g, p.nhalf * p.HR, train, split).total;
-  int per_sm = train ? 1 : (int)((size_t)220 * 1024 / (smem + 2048));
+  p.n_tiles = (p.B + wpt - 1) / wpt;
+  p.smem = (size_t)tile_smem_layout(g, p.nhalf * p.HR, train, split).total;
+  p.ok = p.smem <= (size_t)225 * 1024;
+  int per_sm = train ? 1 : (int)((size_t)220 * 1024 / (p.smem + 2048));
   if (per_sm < 1) per_sm = 1;
   if (per_sm > 4) per_sm = 4;
-  grid = num_sms() * per_sm;
-  if (grid > p.n_tiles) grid = p.n_tiles;
+  p.grid = num_sms() * per_sm;
+  if (p.grid > p.n_tiles) p.grid = p.n_tiles;
+  return p;
 }
 
-int tc_train_nsub(int T, bool split) { return tc_tile_nsub(T, true, split); }
-int tc_train_sub_len(bool split) { return tc_tile_sub_len(split); }
-
-int tc_train_grid(const Geo& g, int B, int T, bool split) {
-  TcTileArgs p{};
-  size_t smem; int grid;
-  const int ns = tc_tile_nsub(T, true, split);
-  tc_tile_plan(g, ns > 1 ? B * ns : B, ns > 1 ? tc_tile_sub_len(split) : T, true, split, p, smem, grid);
-  return grid;
-}
-
-int launch_tc_tile(TcTileArgs& p, bool train, bool split, cudaStream_t stream) {
-  size_t smem; int grid;
-  tc_tile_plan(p.geo, p.B, p.T, train, split, p, smem, grid);
-  if (smem > (size_t)225 * 1024) { set_error("tensor-core tile kernel: %zu B shared memory needed", smem); return B2H_ESHAPE; }
+static int launch_tc_tile(TcTileArgs& p, const TilePlan& plan, cudaStream_t stream) {
+  p.B = plan.B; p.T = plan.T;
+  p.nhalf = plan.nhalf; p.MB = plan.MB; p.NT = plan.NT; p.HR = plan.HR; p.gh = plan.gh; p.n_tiles = plan.n_tiles;
+  const bool train = plan.train, split = plan.split;
+  const size_t smem = plan.smem;
+  const int grid = plan.grid;
   // eight instantiations: {forward, train} x {NT = 1, 2} x {bf16 operands, bf16 high/low pairs (fp32 mode)}
   const int nt2 = p.NT == 2 ? 1 : 0;
   const void* fns[2][2][2] = {
@@ -1119,29 +1104,26 @@ int launch_tc_tile(TcTileArgs& p, bool train, bool split, cudaStream_t stream) {
 static long long* g_dbg_timing = nullptr;
 void set_debug_timing(long long* p) { g_dbg_timing = p; }
 
-bool tc_tile_ok(const Geo& g, int T, bool train, bool split) { return tc_tile_supported(g, T, train, split); }
-
 int launch_tc_tile_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int B, int T, int apply_mask, float out_scale, const Geo& g, cudaStream_t stream, const WindowView* wv, bool split) {
+                       int apply_mask, float out_scale, const Geo& g, const TilePlan& plan, cudaStream_t stream, const WindowView* wv) {
   TcTileArgs p{};
   p.x = x; p.x_dtype = x_dtype; p.params = params; p.packed = packed; p.lengths = lengths; p.y = y;
-  p.B = B; p.T = T; p.apply_mask = apply_mask; p.mode = 0; p.out_scale = out_scale; p.geo = g;
+  p.apply_mask = apply_mask; p.mode = 0; p.out_scale = out_scale; p.geo = g;
   if (wv) { p.win_start = wv->win_start; p.win_end = wv->win_end; p.n_frames = wv->n_frames; p.pad_mode = wv->pad_mode; }
   p.dbg = g_dbg_timing;
-  return launch_tc_tile(p, false, split, stream);
+  return launch_tc_tile(p, plan, stream);
 }
 
-int launch_tc_tile_train(const Fp32Args& a, cudaStream_t stream, bool split) {
+int launch_tc_tile_train(const Fp32Args& a, const TilePlan& plan, cudaStream_t stream) {
   TcTileArgs p{};
   p.x = a.x; p.x_dtype = a.x_dtype; p.target = a.target; p.conf = a.conf; p.d_y = a.d_y; p.lengths = a.lengths;
   p.params = a.params; p.packed = a.packed; p.y = a.y; p.partials = a.partials; p.loss_partials = a.loss_partials;
-  p.step_dev = a.step_dev; p.epoch_dev = a.epoch_dev; p.B = a.B; p.T = a.T; p.loss_kind = a.loss_kind; p.apply_mask = 1; p.mode = a.mode;
+  p.step_dev = a.step_dev; p.epoch_dev = a.epoch_dev; p.loss_kind = a.loss_kind; p.apply_mask = 1; p.mode = a.mode;
   p.out_scale = 1.0f; p.geo = a.geo;
   p.fuse = a.fuse;
   p.dbg = g_dbg_timing;
-  p.loss_B = a.B; p.T_orig = a.T; p.n_sub = tc_tile_nsub(a.T, true, split);
-  if (p.n_sub > 1) { p.B = a.B * p.n_sub; p.T = tc_tile_sub_len(split); }
-  return launch_tc_tile(p, true, split, stream);
+  p.loss_B = a.B; p.T_orig = a.T; p.n_sub = plan.n_sub;
+  return launch_tc_tile(p, plan, stream);
 }
 
 }  // namespace b2h

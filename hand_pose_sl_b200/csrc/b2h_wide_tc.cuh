@@ -709,16 +709,46 @@ __global__ void __launch_bounds__(kWgThreads, 1) conv_tc_wide_wgrad_kernel(Wgrad
 }
 
 // ---- host side ----
-inline int wide_a_bytes(const Geo& g) {
+static int wide_wgrad_items(const Geo& g, WgradItem* items) {
+  int n = 0;
+  for (int l = 0; l < 4; ++l) {
+    const int M = g.np_[l] <= 64 ? 64 : 128;
+    for (int m0 = 0; m0 < g.np_[l]; m0 += M)
+      for (int n0 = 0; n0 < g.kp[l]; n0 += 64) {
+        if (n >= kWgMaxItems) return -1;
+        const int N = g.kp[l] - n0 < 64 ? g.kp[l] - n0 : 64;
+        items[n++] = WgradItem{l, m0, M, n0, N, n0 == 0 ? 1 : 0};
+      }
+  }
+  return n;
+}
+
+// 220 KB hold the activation buffer and a ring of 3..16 weight stages; a tile holds gh whole windows; training splits
+// the weight-gradient GEMMs K-wise over the tiles so that items x ksplit CTAs about fill the SMs.
+WidePlan plan_wide(const Geo& g, int B, int T) {
+  WidePlan p{};
+  if (T < 1 || T > 256 || g.C > 256 || g.cin[0] > 64) return p;
   int kmax = g.kp[0];
   for (int l = 1; l < 4; ++l) kmax = kmax > g.kp[l] ? kmax : g.kp[l];
   for (int l = 0; l < 4; ++l) kmax = kmax > g.np_[l] ? kmax : g.np_[l];
-  return (kmax / 8) * kWideRows * 16;
-}
-
-bool tc_wide_supported(const Geo& g, int T) {
-  if (T < 1 || T > 256 || g.C > 256 || g.cin[0] > 64) return false;
-  return (size_t)wide_a_bytes(g) + 3 * kWideStage <= (size_t)220 * 1024;
+  p.a_bytes = (kmax / 8) * kWideRows * 16;
+  int S = (int)(((size_t)220 * 1024 - p.a_bytes) / kWideStage);
+  if (S > kWideMaxStages) S = kWideMaxStages;
+  p.ok = S >= 3;
+  p.nstage = S;
+  p.smem = (size_t)p.a_bytes + (size_t)S * kWideStage;
+  p.gh = 258 / (T + 2);
+  p.n_tiles = (B + p.gh - 1) / p.gh;
+  const int sms = num_sms();
+  p.grid = sms < p.n_tiles ? sms : p.n_tiles;
+  p.n_loss = p.grid;
+  p.scratch_bytes = (int64_t)p.n_tiles * wide_scratch(g).tile_bytes;
+  WgradItem items[kWgMaxItems];
+  const int n = wide_wgrad_items(g, items);
+  p.ksplit = n > 0 ? sms / n : 1;
+  if (p.ksplit < 1) p.ksplit = 1;
+  if (p.ksplit > p.n_tiles) p.ksplit = p.n_tiles;
+  return p;
 }
 
 // tensor map over a run of packed UMMA weight sections viewed as rows of 64 bf16 (128 B), box = 128 rows (one ring stage)
@@ -745,23 +775,13 @@ static int wide_weight_map(const char* base, int64_t bytes, CUtensorMap* out, in
   return B2H_OK;
 }
 
-static int wide_common(WideArgs& p, const Geo& g, int B, int T, size_t& smem, int& grid) {
+static void wide_common(WideArgs& p, const Geo& g, const WidePlan& plan, int B, int T) {
   p.B = B; p.T = T; p.geo = g;
   p.dbg = g_dbg_timing;
-  p.gh = 258 / (T + 2);
-  p.n_tiles = (B + p.gh - 1) / p.gh;
-  p.a_bytes = wide_a_bytes(g);
-  int S = (int)(((size_t)220 * 1024 - p.a_bytes) / kWideStage);
-  if (S > kWideMaxStages) S = kWideMaxStages;
-  if (S < 3) { set_error("wide tensor-core kernel: C=%d leaves no room for the weight ring", g.C); return B2H_ESHAPE; }
-  p.nstage = S;
-  smem = (size_t)p.a_bytes + (size_t)S * kWideStage;
-  grid = num_sms();
-  if (grid > p.n_tiles) grid = p.n_tiles;
+  p.gh = plan.gh; p.n_tiles = plan.n_tiles; p.a_bytes = plan.a_bytes; p.nstage = plan.nstage;
   const WideScratch ws = wide_scratch(g);
   p.tile_bytes = ws.tile_bytes;
   for (int l = 0; l < 4; ++l) { p.act_off[l] = ws.act_off[l]; p.dz_off[l] = ws.dz_off[l]; }
-  return B2H_OK;
 }
 
 static void wide_forward_stages(WideArgs& p, const Geo& g) {
@@ -770,60 +790,24 @@ static void wide_forward_stages(WideArgs& p, const Geo& g) {
 }
 
 int launch_tc_wide_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int B, int T, int apply_mask, float out_scale, const Geo& g, cudaStream_t stream, const WindowView* wv) {
+                       int B, int T, int apply_mask, float out_scale, const Geo& g, const WidePlan& plan, cudaStream_t stream,
+                       const WindowView* wv) {
   WideArgs p{};
   p.x = x; p.x_dtype = x_dtype; p.params = params; p.packed = packed; p.lengths = lengths; p.y = y;
   p.apply_mask = apply_mask; p.out_scale = out_scale;
   if (wv) p.wv = *wv;
-  size_t smem; int grid;
-  if (int rc = wide_common(p, g, B, T, smem, grid)) return rc;
+  wide_common(p, g, plan, B, T);
   wide_forward_stages(p, g);
-  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_wide_kernel<0>), smem)) return rc;
+  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_wide_kernel<0>), plan.smem)) return rc;
   CUtensorMap wmap;
   if (int rc = wide_weight_map(packed + g.tf_off[0], g.td_off[0] - g.tf_off[0], &wmap)) return rc;
-  conv_tc_wide_kernel<0><<<grid, kWideThreads, smem, stream>>>(p, wmap);
+  conv_tc_wide_kernel<0><<<plan.grid, kWideThreads, plan.smem, stream>>>(p, wmap);
   count_launch();
   return check_launch("conv_tc_wide_kernel<fwd>");
 }
 
 // ---- wide training: forward+criterion (saves layer inputs), dgrad chain, split-K wgrad; the caller reduces + applies Adam ----
-static int wide_wgrad_items(const Geo& g, WgradItem* items) {
-  int n = 0;
-  for (int l = 0; l < 4; ++l) {
-    const int M = g.np_[l] <= 64 ? 64 : 128;
-    for (int m0 = 0; m0 < g.np_[l]; m0 += M)
-      for (int n0 = 0; n0 < g.kp[l]; n0 += 64) {
-        if (n >= kWgMaxItems) return -1;
-        const int N = g.kp[l] - n0 < 64 ? g.kp[l] - n0 : 64;
-        items[n++] = WgradItem{l, m0, M, n0, N, n0 == 0 ? 1 : 0};
-      }
-  }
-  return n;
-}
-
-int tc_wide_train_ksplit(const Geo& g, int B, int T) {
-  WgradItem items[kWgMaxItems];
-  const int n = wide_wgrad_items(g, items);
-  if (n <= 0) return 1;
-  const int gh = 258 / (T + 2), n_tiles = (B + gh - 1) / gh;
-  int ks = num_sms() / n;
-  if (ks < 1) ks = 1;
-  if (ks > n_tiles) ks = n_tiles;
-  return ks;
-}
-
-int64_t tc_wide_train_scratch_bytes(const Geo& g, int B, int T) {
-  const int gh = 258 / (T + 2), n_tiles = (B + gh - 1) / gh;
-  return (int64_t)n_tiles * wide_scratch(g).tile_bytes;
-}
-
-int tc_wide_train_loss_parts(const Geo& g, int B, int T) {
-  const int gh = 258 / (T + 2), n_tiles = (B + gh - 1) / gh;
-  const int sms = num_sms();
-  return n_tiles < sms ? n_tiles : sms;
-}
-
-int launch_tc_wide_train(const Fp32Args& a, unsigned char* scratch, cudaStream_t stream) {
+int launch_tc_wide_train(const Fp32Args& a, const WidePlan& plan, unsigned char* scratch, cudaStream_t stream) {
   const Geo& g = a.geo;
   WideArgs p{};
   p.x = a.x; p.x_dtype = a.x_dtype; p.params = a.params; p.packed = a.packed; p.lengths = a.lengths; p.y = a.y;
@@ -831,8 +815,9 @@ int launch_tc_wide_train(const Fp32Args& a, unsigned char* scratch, cudaStream_t
   p.target = a.target; p.conf = a.conf; p.d_y = a.d_y; p.loss_kind = a.loss_kind; p.train_mode = a.mode;
   p.scratch = scratch; p.loss_partials = a.loss_partials;
   p.step_dev = a.step_dev; p.epoch_dev = a.epoch_dev;
-  size_t smem; int grid;
-  if (int rc = wide_common(p, g, a.B, a.T, smem, grid)) return rc;
+  wide_common(p, g, plan, a.B, a.T);
+  const size_t smem = plan.smem;
+  const int grid = plan.grid;
   // ---- 1. forward + criterion ----
   wide_forward_stages(p, g);
   if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_wide_kernel<1>), smem)) return rc;
@@ -859,7 +844,7 @@ int launch_tc_wide_train(const Fp32Args& a, unsigned char* scratch, cudaStream_t
   w.n_tiles = p.n_tiles; w.partials = a.partials; w.geo = g;
   w.n_items = wide_wgrad_items(g, w.items);
   if (w.n_items <= 0) { set_error("wide wgrad: too many work items"); return B2H_ESHAPE; }
-  w.ksplit = tc_wide_train_ksplit(g, a.B, a.T);
+  w.ksplit = plan.ksplit;
   const size_t wsmem = (size_t)2 * kWgStageBytes + 2 * kWgChunkB;
   if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_wide_wgrad_kernel), wsmem)) return rc;
   CUtensorMap smap;

@@ -268,8 +268,9 @@ class ConvModel(nn.Module):
         [win_start[w], win_start[w] + T) cut at win_end[w] (default F) and padded by the dataset's rule
         (text_pose_dataset.py:511-518 repeat-first / :614-622 zeros).  Returns (W, T, 21, 2), identical to
         `predict` on the materialised (W, T, K, 2) windows.  Every shape `predict` runs on the tensor cores: bf16 mode with
-        conv_channels <= 64 and T <= 1024 or conv_channels <= 256 and T <= 256, fp32 mode with conv_channels <= 32 and
-        T <= 256; other shapes raise B2HError."""
+        conv_channels <= 256 and T <= 256, conv_channels <= 48 and T <= 640 or conv_channels <= 32 and T <= 1024 (the
+        last two with at most 32 input channels), fp32 mode with conv_channels <= 32 and T <= 256, at any number of
+        windows; other shapes raise B2HError."""
         if not self._is_flat():
             self._flatten()
         _lib.require_device(frames, "frames")

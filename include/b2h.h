@@ -88,7 +88,8 @@ int b2h_forward_supported(int T, int n_in, int C, int pos_emb, int precision);
 #define B2H_KERNEL_FFMA 1        /* fp32-accumulate FFMA kernel (B2H_FP32_FFMA; shapes beyond the tile kernel) */
 #define B2H_KERNEL_TC_TILE 2     /* tcgen05 tile kernel, weights resident in shared memory (bf16: C <= 64 fwd / 32 train;
                                     fp32 mode = bf16 high/low pairs: C <= 32; T <= 256) */
-#define B2H_KERNEL_TC_ROWSPACE 3 /* tcgen05 layer-major row-space forward (C <= 64, T <= 1024) */
+#define B2H_KERNEL_TC_ROWSPACE 3 /* tcgen05 layer-major row-space forward (C <= 32 up to T = 1024, C <= 48 up to T = 640,
+                                    with up to 32 input channels; at any batch) */
 #define B2H_KERNEL_TC_WIDE 4     /* tcgen05 streamed-weight forward (C <= 256, T <= 256) */
 #define B2H_KERNEL_TC_WIDE_TRAIN 5 /* tcgen05 wide training (32 < C <= 256, T <= 256, bf16 mode): streamed-weight forward that
                                     saves the layer inputs + criterion, dgrad chain with the transposed blocks, split-K
@@ -149,8 +150,9 @@ int b2h_conv_forward(const void* x, int x_dtype, const float* params, const void
  * `pad_mode` exactly like b2h_preprocess pads a crop (dataloaders/text_pose_dataset.py:52-68, 511-518, 614-622) -- the
  * same result as materialising the (n_win, T, n_in) windows first, without writing or re-reading them (stride 16 = 4x
  * overlap).  y (n_win, T, 42) fp32.  Served by the tensor-core kernels b2h_conv_forward runs: bf16 mode with
- * conv_channels <= 64 and T <= 1024 or conv_channels <= 256 and T <= 256, fp32 mode with conv_channels <= 32 and T <= 256
- * (B2H_ESHAPE otherwise, including every shape b2h_conv_forward runs on the FFMA kernel). */
+ * conv_channels <= 256 and T <= 256, conv_channels <= 48 and T <= 640 or conv_channels <= 32 and T <= 1024 (the last two
+ * with up to 32 input channels), fp32 mode with conv_channels <= 32 and T <= 256, at any n_win (B2H_ESHAPE otherwise,
+ * including every shape b2h_conv_forward runs on the FFMA kernel). */
 int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t n_frames, const int64_t* win_start, const int64_t* win_end,
                              int pad_mode, const float* params, const void* packed, const int32_t* lengths, float* y, int n_win,
                              int T, int n_in, int C, int pos_emb, int precision, int apply_mask, float out_scale, void* stream);

@@ -87,6 +87,10 @@ def test_kernel_choice_pins_the_tensor_core_paths():
     assert fwd(64, 64, _lib.BF16) == TILE and trn(64, 64, _lib.BF16) == WIDE_TRAIN          # C > 32 trains on the wide tcgen05 kernels
     assert fwd(200, 64, _lib.BF16) == ROWSPACE                                              # tile does not fit smem
     assert fwd(257, 30, _lib.BF16) == ROWSPACE and fwd(1000, 30, _lib.BF16) == ROWSPACE
+    # row space beyond 256 frames: C <= 48 up to T = 640, C <= 32 up to T = 1024, at any batch; beyond that one window's
+    # buffers and the weights do not fit in shared memory
+    assert fwd(640, 48, _lib.BF16) == ROWSPACE and fwd(1024, 30, _lib.BF16) == ROWSPACE
+    assert fwd(257, 64, _lib.BF16) == NONE and fwd(641, 48, _lib.BF16) == NONE
     assert trn(257, 30, _lib.BF16) == TILE and trn(1000, 30, _lib.BF16) == TILE and trn(300, 30, _lib.FP32) == TILE   # sub-windows
     for C in (80, 96, 128, 256):
         for T in (64, 126, 200, 256):

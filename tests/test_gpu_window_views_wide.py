@@ -207,8 +207,7 @@ def test_wide_views_graph_capture():
 @pytest.mark.parametrize("T", [64, 256, 257, 1024, 1025])
 def test_view_dispatch_rule(T, C, prec):
     """predict_windows serves exactly the shapes predict runs on a tensor-core kernel: it raises B2HError when
-    b2h_kernel_choice is not the tile, row-space or wide kernel, and otherwise returns what predict returns (or raises
-    what predict raises: the row-space kernel does not fit C > 48 beyond 256 frames in shared memory)."""
+    b2h_kernel_choice is not the tile, row-space or wide kernel, and otherwise returns what predict returns."""
     choice = _lib.load().b2h_kernel_choice(T, 24, C, 0, _lib.PRECISIONS[prec], 0)
     m = _model(C, prec, seed=2)
     F = 1200
@@ -222,12 +221,39 @@ def test_view_dispatch_rule(T, C, prec):
         return
     mat = pre(*t, starts, T)
     x = mat["input_kp_bf16"] if prec == "bf16" else mat["input_kp"]
-    try:
-        y_mat = m.predict(x)
-    except _lib.B2HError:
-        with pytest.raises(_lib.B2HError):
-            m.predict_windows(frames, starts, T)
-        return
+    y_mat = m.predict(x)
     _tc_clean()
     assert torch.equal(m.predict_windows(frames, starts, T), y_mat)
     _tc_clean()
+
+
+@pytest.mark.parametrize("B", [1, 297, 600])
+@pytest.mark.parametrize("C,T", [(48, 257), (48, 400), (48, 640), (40, 641), (64, 257), (30, 1024)])
+def test_rowspace_limits_hold_at_every_batch(C, T, B):
+    """The row-space kernel packs more windows into a CTA as the batch grows, but never more than fit in shared memory, so
+    a shape b2h_forward_supported reports runs at every batch: predict and predict_windows equal predict over chunks of at
+    most 100 windows bit for bit (each row accumulates the same taps and k-steps whichever tile holds it) and the oracle
+    within 2e-2.  Where not even one window fits, both raise."""
+    m = _model(C, seed=C + T)
+    F = 4000
+    t, pre, s16, _, (pose, lh, rh) = _clip(F, "repeat_first")
+    starts = (np.arange(B, dtype=np.int64) * 37) % (F - T)
+    if not _lib.load().b2h_forward_supported(T, 24, C, 0, _lib.PRECISIONS["bf16"]):
+        x = torch.zeros((B, T, 12, 2), dtype=torch.bfloat16, device=DEV)
+        with pytest.raises(_lib.B2HError):
+            m.predict(x)
+        with pytest.raises(_lib.B2HError):
+            m.predict_windows(s16, starts, T)
+        return
+    x = pre(*t, starts, T)["input_kp_bf16"]
+    y = m.predict(x)
+    _tc_clean()
+    y_view = m.predict_windows(s16, starts, T)
+    _tc_clean()
+    y_chunks = torch.cat([m.predict(x[i:i + 100]) for i in range(0, B, 100)])
+    _tc_clean()
+    assert torch.equal(y, y_chunks) and torch.equal(y_view, y_chunks)
+    sd = oracle.init_params(C, False, seed=C + T)
+    want = oracle.preprocess_windows(pose, lh, rh, starts, T)
+    ref = oracle.conv_model_forward(sd, torch.from_numpy(want["input_kp"])).contiguous().numpy()
+    assert oracle.rel_err(y.cpu().numpy(), ref) <= 2e-2

@@ -14,7 +14,7 @@ from hand_pose_sl_b200 import synthetic
 
 
 def plan(T, wide):
-    """(segment rows MB, segments per tile, windows per segment) as tc_tile_plan / launch_tc_wide_fwd choose them."""
+    """(segment rows MB, segments per tile, windows per segment) as plan_tile / plan_wide choose them."""
     if wide:
         return 256, 1, 258 // (T + 2)
     if T <= 64:
