@@ -438,12 +438,12 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
               }
               const uint4 q0 = pack8(f0), q1 = pack8(f1);
               const size_t o0 = (size_t)((c0 >> 3) + i) * CH + (size_t)rc0.row * 16, o1 = (size_t)((c0 >> 3) + i) * CH + (size_t)rc1.row * 16;
-              *reinterpret_cast<uint4*>(A + o0) = q0;
-              *reinterpret_cast<uint4*>(A + o1) = q1;
-              if (dd) {
-                *reinterpret_cast<uint4*>(dd + o0) = q0;
-                *reinterpret_cast<uint4*>(dd + o1) = q1;
-              }
+              // MODE 2, last stage: dZ_0 goes to the dump only.  The buffer already belongs to the CTA's next tile: epilogue
+              // threads that finish first copy that tile's dZ_4 into it (stage_inputs below, with no barrier in between),
+              // and a late store of dZ_0 here would overwrite it.
+              unsigned char* out = dd ? dd : A;
+              *reinterpret_cast<uint4*>(out + o0) = q0;
+              *reinterpret_cast<uint4*>(out + o1) = q1;
             }
           }
         } else if (MODE == 0) {

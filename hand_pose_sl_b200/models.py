@@ -248,6 +248,10 @@ class ConvModel(nn.Module):
         view of a (B,42,T) tensor; this returns the same values contiguous.)"""
         if not self._is_flat():
             self._flatten()
+        if torch.is_grad_enabled() and inp.requires_grad:
+            # the kernels compute parameter gradients only: a trainable module in front of this one would silently get none
+            raise RuntimeError("ConvModel computes no input gradient: its input must not require grad "
+                               "(detach it, or run the modules in front of ConvModel without autograd)")
         if torch.is_grad_enabled() and any(p.requires_grad for p in self._ordered_params()):
             return _ConvForward.apply(inp, self, *self._ordered_params())
         return self._forward_impl(inp)

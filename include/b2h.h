@@ -77,7 +77,8 @@ int b2h_train_subwindows(int T, int n_in, int C, int pos_emb, int precision, int
 /* bytes of scratch the train entry points need (1-KB header of the fused kernel's grid barrier + per-CTA gradient
  * partials for a deterministic two-stage reduction + loss partials); 16-byte aligned, zeroed once at allocation */
 int64_t b2h_workspace_bytes(int B, int T, int n_in, int C, int pos_emb, int precision);
-/* 1 if (T, C) is supported by the given precision's kernels (forward AND training) on this build, else 0 */
+/* 1 if (T, C) is supported by the given precision's kernels (forward AND training) on this build, else 0.  A bf16-mode
+ * shape counts as supported when its training runs on the FFMA kernel (see B2H_KERNEL_FFMA). */
 int b2h_supported(int T, int n_in, int C, int pos_emb, int precision);
 /* 1 if b2h_conv_forward alone covers (T, C) in the given precision -- wider than b2h_supported: bf16 inference runs
  * conv_channels up to 256 (streamed-weight tensor-core kernel) -- else 0 */
@@ -85,7 +86,10 @@ int b2h_forward_supported(int T, int n_in, int C, int pos_emb, int precision);
 /* Which kernel the forward (train = 0) or the train step (train = 1) runs for this shape -- the dispatch itself uses
  * this function, so a test can pin "the tensor-core path is the one that runs" without a GPU. */
 #define B2H_KERNEL_NONE 0        /* unsupported: the entry point returns B2H_ESHAPE */
-#define B2H_KERNEL_FFMA 1        /* fp32-accumulate FFMA kernel (B2H_FP32_FFMA; shapes beyond the tile kernel) */
+#define B2H_KERNEL_FFMA 1        /* fp32-accumulate FFMA kernel (B2H_FP32_FFMA; B2H_FP32 beyond the tile kernel; and B2H_BF16
+                                    TRAINING where no tensor-core training kernel fits but FFMA's shared memory does: 16 input
+                                    channels, no pos_emb, C = 33..36, T = 257..264 -- those steps run with unrounded fp32
+                                    operands) */
 #define B2H_KERNEL_TC_TILE 2     /* tcgen05 tile kernel, weights resident in shared memory (bf16: C <= 64 fwd / 32 train;
                                     fp32 mode = bf16 high/low pairs: C <= 32; T <= 256) */
 #define B2H_KERNEL_TC_ROWSPACE 3 /* tcgen05 layer-major row-space forward (C <= 32 up to T = 1024, C <= 48 up to T = 640,

@@ -100,6 +100,13 @@ def test_kernel_choice_pins_the_tensor_core_paths():
         for T in (9, 64, 126, 200, 256):
             assert trn(T, C, _lib.BF16) == WIDE_TRAIN, (T, C)
     assert trn(300, 256, _lib.BF16) == NONE and trn(64, 256, _lib.FP32) == NONE             # fp32 mode: 396 KB of activations
+    # bf16 training falls back to FFMA (unrounded fp32 operands) exactly where no tensor-core training kernel fits and FFMA's
+    # shared memory does: 16 input channels, no positional row, C = 33..36, T = 257..264 (include/b2h.h, DESIGN §1)
+    on_ffma = {(n_in, pe, C, T) for n_in in (16, 24) for pe in (0, 1) for C in range(30, 50) for T in range(250, 272)
+               if lib.b2h_kernel_choice(T, n_in, C, pe, _lib.BF16, 1) == FFMA}
+    assert on_ffma == {(16, 0, C, T) for C in range(33, 37) for T in range(257, 265)}
+    assert all(lib.b2h_supported(T, 16, C, 0, _lib.BF16) == 1 for C in (33, 36) for T in (257, 264))
+    assert lib.b2h_kernel_choice(257, 24, 33, 0, _lib.BF16, 1) == NONE and lib.b2h_kernel_choice(265, 16, 33, 0, _lib.BF16, 1) == NONE
     assert fwd(64, 256, _lib.FP32) == FFMA
     assert lib.b2h_kernel_choice(64, 24, 30, 0, 7, 0) == NONE                                # bad precision
     for T, C in ((64, 30), (200, 30), (64, 256), (300, 256)):
