@@ -49,6 +49,9 @@ _SIGNATURES = {
     "b2h_train_forward_backward": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                            c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p,
                                            c_void_p, c_int64, c_void_p]),
+    "b2h_train_forward_backward_windows": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int,
+                                                   c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                                   c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int64, c_void_p]),
     "b2h_conv_backward": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                   c_int, c_int, c_void_p, c_int64, c_void_p]),
     "b2h_mask_output": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
@@ -59,6 +62,10 @@ _SIGNATURES = {
     "b2h_train_step": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_double, c_double, c_double,
                                c_double, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    "b2h_train_step_windows": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_void_p,
+                                       c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
+                                       c_int, c_int, c_double, c_double, c_double, c_double, c_int64, c_void_p, c_void_p,
+                                       c_void_p, c_int64, c_void_p]),
     "b2h_train_step_dp": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_double, c_double, c_double,
                                   c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_float,

@@ -250,28 +250,43 @@ extern "C" int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t
                       out_scale, (cudaStream_t)stream, "b2h_conv_forward_windows");
 }
 
-static int train_common(const void* x, int x_dtype, const float* target, const float* conf, const float* d_y,
-                        const int32_t* lengths, const float* params, const void* packed, float* pred_out, int B, int T,
-                        int n_in, int C, int pos_emb, int loss_kind, int precision, int mode, void* workspace,
+// The training forward + criterion + backward of B dense windows (wv == nullptr) or of B windows viewed in the frame
+// streams x / target / conf (mode 1 only; the tensor-core kernels only: the FFMA kernel reads dense windows).
+static int train_common(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
+                        const float* d_y, const int32_t* lengths, const float* params, const void* packed, float* pred_out,
+                        int B, int T, int n_in, int C, int pos_emb, int loss_kind, int precision, int mode, void* workspace,
                         int64_t workspace_bytes, cudaStream_t stream, Geo& g, TrainPlan& plan, float*& partials,
                         float*& loss_partials, const char* who, long long* step_dev = nullptr, long long* epoch_dev = nullptr,
                         FuseAdam* fuse = nullptr) {
-  if (!x || !params || !packed || !workspace) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  if (!x || (wv && !wv->win_start) || !params || !packed || !workspace) { set_error("%s: null pointer", who); return B2H_EINVAL; }
   if (x_dtype != B2H_DT_F32 && x_dtype != B2H_DT_BF16) { set_error("%s: bad x_dtype %d", who, x_dtype); return B2H_EINVAL; }
+  if (wv && wv->pad_mode != B2H_PAD_REPEAT_FIRST && wv->pad_mode != B2H_PAD_ZEROS) { set_error("%s: bad pad_mode %d", who, wv->pad_mode); return B2H_EINVAL; }
   if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
-  if (B < 1 || T < 1) { set_error("%s: bad B=%d T=%d", who, B, T); return B2H_ESHAPE; }
+  if (B < 1 || T < 1 || (wv && wv->n_frames < 0)) { set_error("%s: bad B=%d T=%d", who, B, T); return B2H_ESHAPE; }
   if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
   if (mode == 1) {
     if (!target || !lengths) { set_error("%s: null target/lengths", who); return B2H_EINVAL; }
     if (loss_kind != B2H_LOSS_L1 && loss_kind != B2H_LOSS_CONFL1) { set_error("%s: bad loss_kind %d", who, loss_kind); return B2H_EINVAL; }
     if (loss_kind == B2H_LOSS_CONFL1 && !conf) { set_error("%s: confL1 needs scores", who); return B2H_EINVAL; }
   } else if (!d_y) { set_error("%s: null d_y", who); return B2H_EINVAL; }
-  if ((reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(target) & 15) || (reinterpret_cast<uintptr_t>(packed) & 15)) {
-    set_error("%s: x, target and packed must be 16-byte aligned", who);
+  // A stream's target row (168 B) and confidence row (84 B) start 8 / 4 bytes past a 16-B boundary at odd frames: the
+  // kernels read them with float2 / float loads and use a bulk copy only where the address allows it.
+  const uintptr_t talign = wv ? 7 : 15, calign = wv ? 3 : 0;
+  if ((reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(target) & talign) ||
+      (reinterpret_cast<uintptr_t>(conf) & calign) || (reinterpret_cast<uintptr_t>(packed) & 15)) {
+    if (wv) set_error("%s: frames and packed must be 16-byte aligned, target_frames 8-byte and conf_frames 4-byte aligned", who);
+    else set_error("%s: x, target and packed must be 16-byte aligned", who);
     return B2H_EALIGN;
   }
   g = make_geo(n_in, C, pos_emb);
   plan = train_plan(g, B, T, precision);
+  if (wv && plan.kernel != B2H_KERNEL_TC_TILE && plan.kernel != B2H_KERNEL_TC_WIDE_TRAIN) {
+    set_error("%s: window views are trained on the tensor cores: in bf16 mode for conv_channels <= 32 with at most 32 input "
+              "channels and T <= 4096, and for conv_channels <= 256 with T <= 256; in fp32 mode for conv_channels <= 32 with at "
+              "most 32 input channels and T <= 4096; materialise the windows (b2h_preprocess) for C=%d, T=%d, precision=%d",
+              who, C, T, precision);
+    return B2H_ESHAPE;
+  }
   if (plan.kernel == B2H_KERNEL_NONE) {
     set_error("%s: no training kernel for conv_channels=%d, T=%d, precision=%d (tcgen05 training: C <= 32 in the one-launch tile "
               "kernel, C <= 256 in bf16 mode through the wide kernels, T <= 256; the FFMA kernel would need %zu B of shared memory)",
@@ -291,6 +306,7 @@ static int train_common(const void* x, int x_dtype, const float* target, const f
   a.B = B; a.T = T; a.loss_kind = loss_kind; a.apply_mask = 1; a.mode = mode; a.out_scale = 1.0f; a.geo = g;
   a.step_dev = step_dev;
   a.epoch_dev = epoch_dev;
+  if (wv) a.wv = *wv;
   if (plan.kernel == B2H_KERNEL_TC_TILE) {
     if (fuse) {
       if (nparts > B2H_WS_MAX_CTA) { set_error("%s: %d CTAs exceed the %d arrival flags of the workspace header", who, nparts, B2H_WS_MAX_CTA); return B2H_ESHAPE; }
@@ -307,18 +323,41 @@ static int train_common(const void* x, int x_dtype, const float* target, const f
   return launch_fp32(a, plan.ffma, stream);
 }
 
+static int train_forward_backward(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
+                                  const int32_t* lengths, const float* params, const void* packed, float* grads_out,
+                                  float* loss_out, float* pred_out, int B, int T, int n_in, int C, int pos_emb, int loss_kind,
+                                  int precision, int64_t* step_dev, void* workspace, int64_t workspace_bytes, void* stream,
+                                  const char* who) {
+  if (grads_out && !loss_out) { set_error("%s: null loss_out", who); return B2H_EINVAL; }
+  Geo g; TrainPlan plan; float *partials, *loss_partials;
+  int rc = train_common(x, x_dtype, wv, target, conf, nullptr, lengths, params, packed, pred_out, B, T, n_in, C, pos_emb,
+                        loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
+                        loss_partials, who, reinterpret_cast<long long*>(step_dev));
+  if (rc || !grads_out) return rc;   // grads_out == NULL: only the fused kernel runs, partials stay in the workspace
+  return launch_reduce(partials, plan.nparts, plan.gp_layout, g, grads_out, loss_partials, loss_out, (cudaStream_t)stream, nullptr, plan.n_loss);
+}
+
 extern "C" int b2h_train_forward_backward(const void* x, int x_dtype, const float* target, const float* conf,
                                           const int32_t* lengths, const float* params, const void* packed,
                                           float* grads_out, float* loss_out, float* pred_out, int B, int T, int n_in,
                                           int C, int pos_emb, int loss_kind, int precision, int64_t* step_dev,
                                           void* workspace, int64_t workspace_bytes, void* stream) {
-  if (grads_out && !loss_out) { set_error("b2h_train_forward_backward: null loss_out"); return B2H_EINVAL; }
-  Geo g; TrainPlan plan; float *partials, *loss_partials;
-  int rc = train_common(x, x_dtype, target, conf, nullptr, lengths, params, packed, pred_out, B, T, n_in, C, pos_emb,
-                        loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
-                        loss_partials, "b2h_train_forward_backward", reinterpret_cast<long long*>(step_dev));
-  if (rc || !grads_out) return rc;   // grads_out == NULL: only the fused kernel runs, partials stay in the workspace
-  return launch_reduce(partials, plan.nparts, plan.gp_layout, g, grads_out, loss_partials, loss_out, (cudaStream_t)stream, nullptr, plan.n_loss);
+  return train_forward_backward(x, x_dtype, nullptr, target, conf, lengths, params, packed, grads_out, loss_out, pred_out, B, T,
+                                n_in, C, pos_emb, loss_kind, precision, step_dev, workspace, workspace_bytes, stream,
+                                "b2h_train_forward_backward");
+}
+
+extern "C" int b2h_train_forward_backward_windows(const void* frames, int x_dtype, const float* target_frames,
+                                                  const float* conf_frames, int64_t n_frames, const int64_t* win_start,
+                                                  const int64_t* win_end, int pad_mode, const int32_t* lengths,
+                                                  const float* params, const void* packed, float* grads_out, float* loss_out,
+                                                  float* pred_out, int n_win, int T, int n_in, int C, int pos_emb,
+                                                  int loss_kind, int precision, int64_t* step_dev, void* workspace,
+                                                  int64_t workspace_bytes, void* stream) {
+  const WindowView wv{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
+  return train_forward_backward(frames, x_dtype, &wv, target_frames, conf_frames, lengths, params, packed, grads_out, loss_out,
+                                pred_out, n_win, T, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace,
+                                workspace_bytes, stream, "b2h_train_forward_backward_windows");
 }
 
 extern "C" int64_t b2h_dp_exchange_floats(int n_in, int C, int pos_emb, int world) {
@@ -343,20 +382,20 @@ extern "C" int b2h_conv_backward(const void* x, int x_dtype, const float* d_y, c
                                  void* workspace, int64_t workspace_bytes, void* stream) {
   if (!grads_out) { set_error("b2h_conv_backward: null output"); return B2H_EINVAL; }
   Geo g; TrainPlan plan; float *partials, *loss_partials;
-  int rc = train_common(x, x_dtype, nullptr, nullptr, d_y, nullptr, params, packed, nullptr, B, T, n_in, C, pos_emb, 0,
+  int rc = train_common(x, x_dtype, nullptr, nullptr, nullptr, d_y, nullptr, params, packed, nullptr, B, T, n_in, C, pos_emb, 0,
                         precision, 2, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
                         loss_partials, "b2h_conv_backward");
   if (rc) return rc;
   return launch_reduce(partials, plan.nparts, plan.gp_layout, g, grads_out, nullptr, nullptr, (cudaStream_t)stream, nullptr, plan.n_loss);
 }
 
-extern "C" int b2h_train_step(const void* x, int x_dtype, const float* target, const float* conf, const int32_t* lengths,
-                              float* params, void* packed, float* exp_avg, float* exp_avg_sq, float* loss_out, int B,
-                              int T, int n_in, int C, int pos_emb, int loss_kind, int precision, double lr, double beta1,
-                              double beta2, double eps, int64_t step, int64_t* step_dev, const double* lr_dev, void* workspace,
-                              int64_t workspace_bytes, void* stream) {
-  if (!exp_avg || !exp_avg_sq || !loss_out) { set_error("b2h_train_step: null pointer"); return B2H_EINVAL; }
-  if (step < 1 && !step_dev) { set_error("b2h_train_step: step must be >= 1"); return B2H_EINVAL; }
+static int train_step(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
+                      const int32_t* lengths, float* params, void* packed, float* exp_avg, float* exp_avg_sq, float* loss_out,
+                      int B, int T, int n_in, int C, int pos_emb, int loss_kind, int precision, double lr, double beta1,
+                      double beta2, double eps, int64_t step, int64_t* step_dev, const double* lr_dev, void* workspace,
+                      int64_t workspace_bytes, void* stream, const char* who) {
+  if (!exp_avg || !exp_avg_sq || !loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  if (step < 1 && !step_dev) { set_error("%s: step must be >= 1", who); return B2H_EINVAL; }
   Geo g; TrainPlan plan; float *partials, *loss_partials;
   // bf16 tile kernel + device-side step counter: ONE cooperative launch (reduction + Adam + re-pack in its tail)
   FuseAdam fuse{};
@@ -364,15 +403,38 @@ extern "C" int b2h_train_step(const void* x, int x_dtype, const float* target, c
   fuse.lr = lr; fuse.beta1 = beta1; fuse.beta2 = beta2; fuse.eps = (float)eps; fuse.grad_scale = 1.0f;
   fuse.lr_dev = lr_dev;
   fuse.step_dev = reinterpret_cast<const long long*>(step_dev); fuse.loss_out = loss_out; fuse.world = 1;
-  int rc = train_common(x, x_dtype, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C, pos_emb,
+  int rc = train_common(x, x_dtype, wv, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C, pos_emb,
                         loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
-                        loss_partials, "b2h_train_step", reinterpret_cast<long long*>(step_dev), nullptr,
+                        loss_partials, who, reinterpret_cast<long long*>(step_dev), nullptr,
                         step_dev ? &fuse : nullptr);
   if (rc) return rc;
   if (step_dev && plan.kernel == B2H_KERNEL_TC_TILE) return B2H_OK;
   return launch_adam(params, partials, plan.nparts, plan.gp_layout, exp_avg, exp_avg_sq, g.P, lr, beta1, beta2, eps, step < 1 ? 1 : step,
                      reinterpret_cast<const long long*>(step_dev), lr_dev, 1.0f, packed, g,
                      loss_partials, loss_out, (cudaStream_t)stream, plan.n_loss);
+}
+
+extern "C" int b2h_train_step(const void* x, int x_dtype, const float* target, const float* conf, const int32_t* lengths,
+                              float* params, void* packed, float* exp_avg, float* exp_avg_sq, float* loss_out, int B,
+                              int T, int n_in, int C, int pos_emb, int loss_kind, int precision, double lr, double beta1,
+                              double beta2, double eps, int64_t step, int64_t* step_dev, const double* lr_dev, void* workspace,
+                              int64_t workspace_bytes, void* stream) {
+  return train_step(x, x_dtype, nullptr, target, conf, lengths, params, packed, exp_avg, exp_avg_sq, loss_out, B, T, n_in, C,
+                    pos_emb, loss_kind, precision, lr, beta1, beta2, eps, step, step_dev, lr_dev, workspace, workspace_bytes,
+                    stream, "b2h_train_step");
+}
+
+extern "C" int b2h_train_step_windows(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
+                                      int64_t n_frames, const int64_t* win_start, const int64_t* win_end, int pad_mode,
+                                      const int32_t* lengths, float* params, void* packed, float* exp_avg, float* exp_avg_sq,
+                                      float* loss_out, int n_win, int T, int n_in, int C, int pos_emb, int loss_kind,
+                                      int precision, double lr, double beta1, double beta2, double eps, int64_t step,
+                                      int64_t* step_dev, const double* lr_dev, void* workspace, int64_t workspace_bytes,
+                                      void* stream) {
+  const WindowView wv{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
+  return train_step(frames, x_dtype, &wv, target_frames, conf_frames, lengths, params, packed, exp_avg, exp_avg_sq, loss_out,
+                    n_win, T, n_in, C, pos_emb, loss_kind, precision, lr, beta1, beta2, eps, step, step_dev, lr_dev, workspace,
+                    workspace_bytes, stream, "b2h_train_step_windows");
 }
 
 extern "C" int b2h_train_step_dp(const void* x, int x_dtype, const float* target, const float* conf, const int32_t* lengths,
@@ -395,7 +457,7 @@ extern "C" int b2h_train_step_dp(const void* x, int x_dtype, const float* target
   fuse.peer_bufs = reinterpret_cast<const float* const*>(peer_bufs_dev); fuse.sym_grads = sym_grads;
   fuse.mc_buf = reinterpret_cast<unsigned long long*>(multicast_buf);
   fuse.epoch_dev = reinterpret_cast<const long long*>(epoch_dev); fuse.rank = rank; fuse.world = world;
-  int rc = train_common(x, x_dtype, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C, pos_emb,
+  int rc = train_common(x, x_dtype, nullptr, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C, pos_emb,
                         loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
                         loss_partials, "b2h_train_step_dp", reinterpret_cast<long long*>(step_dev),
                         reinterpret_cast<long long*>(epoch_dev), &fuse);

@@ -240,8 +240,9 @@ int check_launch(const char* what);
 void count_launch(int n = 1);
 
 
-// Streaming inference (BASELINE config 5): sliding windows read as views of a per-frame stream (n_frames, n_in) instead of
-// materialised (n_win, T, n_in) windows.  win_start == nullptr: the kernel's input is a dense batch of windows.
+// Streaming inference (BASELINE config 5) and training from device-resident streams: sliding windows read as views of a
+// per-frame stream (n_frames, n_in) -- and, in training, of the target (n_frames, 42) and confidence (n_frames, 21) streams
+// at the same rows -- instead of materialised (n_win, T, .) windows.  win_start == nullptr: the kernel's inputs are dense.
 struct WindowView { const long long* win_start; const long long* win_end; long long n_frames; int pad_mode; };
 
 // Source row in the stream of (window w, frame t) of a window view; -1 = a zero row.  The crop [start, start + T) is cut at
@@ -316,6 +317,7 @@ struct Fp32Args {
   int B, T, loss_kind, apply_mask, mode;   // mode 0 = forward, 1 = train (loss inside), 2 = backward of given d_y
   float out_scale;
   Geo geo;
+  WindowView wv;            // tensor-core training only: win_start set = x / target / conf are frame streams, B = windows
 };
 int launch_fp32(Fp32Args& p, const FfmaPlan& plan, cudaStream_t stream);
 

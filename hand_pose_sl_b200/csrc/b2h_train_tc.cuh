@@ -46,9 +46,10 @@ struct TcTileArgs {
   long long* epoch_dev;
   long long* dbg;         // nullable: CTA 0 / thread 0 writes clock64() phase stamps here (b2h_debug_timing)
   FuseAdam fuse;
-  // Streaming inference (BASELINE config 5): when win_start is set, x is a per-frame stream (n_frames, n_in) and window
-  // w, frame t reads row win_start[w] + t of it (cut at win_end[w] / n_frames, then the dataset's pad rule) -- overlapping
-  // windows are views of the stream, nothing is re-materialised.
+  // Window views (streaming inference; training from device-resident streams): when win_start is set, x is a per-frame
+  // stream (n_frames, n_in) and window w, frame t reads row win_start[w] + t of it (cut at win_end[w] / n_frames, then the
+  // dataset's pad rule) -- overlapping windows are views of the stream, nothing is re-materialised.  Training reads the
+  // target (n_frames, 42) and confidence (n_frames, 21) rows at the same stream row; the prediction stays dense.
   const long long* win_start; const long long* win_end; long long n_frames; int pad_mode;
   // Sub-window training (n_sub > 1: T_orig > 128 in fp32 mode, > 256 in bf16 mode): a tile segment holds 128 (doubled
   // operand buffers) / 256 frames, so every window is processed as n_sub overlapping sub-windows that read REAL neighbouring frames
@@ -211,7 +212,10 @@ __device__ __forceinline__ long long global_ns() { long long t; asm volatile("mo
 // NT (128-row MMA tiles per segment) is a compile-time constant: with it at run time the per-row loops and the row
 // context inside them cost the T <= 128 shapes ~6 % (27.4 -> 29.1 us per train step, 10.5 -> 11.3 us forward).
 // SPLIT = fp32 mode: bf16 high/low operand pairs, three MMAs per product term group (see tile_smem_layout).
-template <bool TRAIN, int NT, bool SPLIT>
+// VIEW (training only) = window views of frame streams: target / confidence rows through the view, per-window staging of
+// the target tile.  A separate instantiation: the same code behind a run-time test made the dense 256x64 step 1.9 us
+// slower (27.4 -> 29.3 us) with the same register count.  The forward kernel tests p.win_start at run time.
+template <bool TRAIN, int NT, bool SPLIT, bool VIEW = false>
 __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArgs p) {
   int dbg_n = 0;
   extern __shared__ __align__(128) unsigned char smem[];
@@ -292,14 +296,28 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
     const SubW sw = subw(gw);
     return (long long)sw.b * p.T_orig + sw.start + tt;
   };
+  // row of (window / sub-window gw, frame tt) in p.x -- and in training also in p.target / p.conf
   auto xrow_of = [&](int gw, int tt) -> long long {
     if (!p.win_start) return dense_row(gw, tt);
+    if (VIEW && p.n_sub > 1) {           // sub-window -> frame of its window's crop: context frames past win_end are pad
+      const SubW sw = subw(gw);
+      gw = sw.b; tt += sw.start;
+    }
     const long long start = p.win_start[gw];
     long long cend = p.win_end ? p.win_end[gw] : p.n_frames;
     cend = cend > p.n_frames ? p.n_frames : cend;
     long long f = start + tt;
     if (f >= cend || f < 0) f = (p.pad_mode == B2H_PAD_REPEAT_FIRST && start >= 0 && start < cend) ? start : -1;
     return f;
+  };
+  // A viewed window's T target rows go to the staging tile as one bulk copy only when they are one contiguous run (the
+  // crop is neither cut nor padded) starting at a 16-B aligned address: a row is 168 B, so odd stream rows sit 8 B off a
+  // 16-B boundary (and the base pointer itself need only be 8-B aligned).  Other windows are staged row by row.
+  auto view_bulk = [&](int gw) -> bool {
+    const long long start = p.win_start[gw];
+    long long cend = p.win_end ? p.win_end[gw] : p.n_frames;
+    cend = cend > p.n_frames ? p.n_frames : cend;
+    return start >= 0 && start + T <= cend && (reinterpret_cast<uintptr_t>(p.target + start * B2H_COUT) & 15) == 0;
   };
   // ---- input prefetch registers (one tile ahead) ----
   float4 xf[8];
@@ -454,11 +472,23 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
       if (tgt_smem) {                             // target rows of this tile's windows -> staging tile (TMA bulk loads)
         int nw = p.B - wbase; nw = nw > wpt ? wpt : nw;
         fence_proxy_async_smem();
-        mbar_arrive_expect_tx(&tbar, (uint32_t)nw * T * B2H_COUT * 4);
-        for (int w = 0; w < nw; ++w) {
-          const int h = w / gh, j = w - h * gh;
-          bulk_g2s(YS + (size_t)(h * MB + j * (T + 2)) * B2H_COUT, p.target + (size_t)(wbase + w) * T * B2H_COUT,
-                   (uint32_t)T * B2H_COUT * 4, &tbar);
+        if (!VIEW) {
+          mbar_arrive_expect_tx(&tbar, (uint32_t)nw * T * B2H_COUT * 4);
+          for (int w = 0; w < nw; ++w) {
+            const int h = w / gh, j = w - h * gh;
+            bulk_g2s(YS + (size_t)(h * MB + j * (T + 2)) * B2H_COUT, p.target + (size_t)(wbase + w) * T * B2H_COUT,
+                     (uint32_t)T * B2H_COUT * 4, &tbar);
+          }
+        } else {                                  // window views: the bulk-eligible windows only (view_bulk)
+          int nb = 0;
+          for (int w = 0; w < nw; ++w) nb += view_bulk(wbase + w) ? 1 : 0;
+          mbar_arrive_expect_tx(&tbar, (uint32_t)nb * T * B2H_COUT * 4);
+          for (int w = 0; w < nw; ++w) {
+            if (!view_bulk(wbase + w)) continue;
+            const int h = w / gh, j = w - h * gh;
+            bulk_g2s(YS + (size_t)(h * MB + j * (T + 2)) * B2H_COUT, p.target + (size_t)p.win_start[wbase + w] * B2H_COUT,
+                     (uint32_t)T * B2H_COUT * 4, &tbar);
+          }
         }
       }
     }
@@ -510,6 +540,14 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
           *reinterpret_cast<uint4*>(X + (size_t)c8 * CH + (size_t)row * 16) = zero;
           if (SPLIT) *reinterpret_cast<uint4*>(X + LO + (size_t)c8 * CH + (size_t)row * 16) = zero;
         }
+      }
+      if (VIEW && tgt_smem && rc.valid && !view_bulk(rc.gw)) {
+        // viewed window staged row by row: this thread's half of its row's 21 float2 (8-B aligned in any stream row), or
+        // a zero row; read after the barrier below
+        const long long tr = xrow_of(rc.gw, rc.t);
+        const float2* src = reinterpret_cast<const float2*>(p.target + (tr < 0 ? 0 : tr) * B2H_COUT);
+        float2* dst = reinterpret_cast<float2*>(YS + (size_t)srow * B2H_COUT);
+        for (int q = ch * 11; q < (ch ? B2H_COUT / 2 : 11); ++q) dst[q] = tr < 0 ? make_float2(0.f, 0.f) : __ldg(src + q);
       }
       if (TRAIN && ch == 0) {   // ones column (B operand of the bias-gradient GEMM): 1 on real frames
         uint4 o = make_uint4(0, 0, 0, 0);
@@ -571,7 +609,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
         float n_el = 0.f, scale = 0.f;
         const float* tg = nullptr; const float* cf = nullptr; const float* dy = nullptr;
         const size_t drow = valid ? (size_t)dense_row(gw, t) : 0;       // row of this frame in the dense (B, T, .) arrays
-        bool in_core = true;
+        bool in_core = true, zrow = false;
         if (TRAIN && valid) {
           n_el = (float)len * (float)B2H_COUT;                      // (sub-window mode: len = the WINDOW's sequence length)
           scale = (p.loss_kind == B2H_LOSS_L1) ? (1.0f / (float)p.loss_B) / n_el : 1.0f / n_el;
@@ -580,9 +618,15 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
             in_core = t >= sw.clo && t < sw.chi;
             len -= sw.start;
           }
-          if (p.mode == 1) {
-            tg = p.target + drow * B2H_COUT;                        // global copy (used when the tile is not staged)
-            cf = p.conf ? p.conf + drow * (B2H_COUT / 2) : nullptr;
+          if (p.mode == 1) {                                        // global copy (used when the tile is not staged)
+            long long trow = (long long)drow;
+            if (VIEW) {                                             // window view: the stream row; a zero row reads as zeros
+              trow = xrow_of(gw, t);
+              zrow = trow < 0;
+              trow = zrow ? 0 : trow;
+            }
+            tg = p.target + trow * B2H_COUT;
+            cf = p.conf ? p.conf + trow * (B2H_COUT / 2) : nullptr;
           } else {
             dy = p.d_y + drow * B2H_COUT;
           }
@@ -666,6 +710,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
                 if (p.mode == 1) tv2 = tgt_smem ? *reinterpret_cast<const float2*>(ys_row + c0 + q) : __ldg(reinterpret_cast<const float2*>(tg + c0 + q));
                 else tv2 = __ldg(reinterpret_cast<const float2*>(dy + c0 + q));
                 if (cf && p.loss_kind == B2H_LOSS_CONFL1) sv = __ldg(cf + ((c0 + q) >> 1));
+                if (VIEW && zrow) { tv2 = make_float2(0.f, 0.f); sv = (cf && p.loss_kind == B2H_LOSS_CONFL1) ? 0.f : 1.0f; }
               }
               tvals[q] = tv2.x; tvals[q + 1] = tv2.y; svals[q] = sv; svals[q + 1] = sv;
             }
@@ -1057,14 +1102,18 @@ static int launch_tc_tile(TcTileArgs& p, const TilePlan& plan, cudaStream_t stre
   const bool train = plan.train, split = plan.split;
   const size_t smem = plan.smem;
   const int grid = plan.grid;
-  // eight instantiations: {forward, train} x {NT = 1, 2} x {bf16 operands, bf16 high/low pairs (fp32 mode)}
+  // twelve instantiations: {forward, train, train over window views} x {NT = 1, 2} x {bf16 operands, bf16 high/low pairs
+  // (fp32 mode)}
   const int nt2 = p.NT == 2 ? 1 : 0;
-  const void* fns[2][2][2] = {
+  const int kind = !train ? 0 : p.win_start ? 2 : 1;
+  const void* fns[3][2][2] = {
       {{(const void*)conv_tc_tile_kernel<false, 1, false>, (const void*)conv_tc_tile_kernel<false, 1, true>},
        {(const void*)conv_tc_tile_kernel<false, 2, false>, (const void*)conv_tc_tile_kernel<false, 2, true>}},
       {{(const void*)conv_tc_tile_kernel<true, 1, false>, (const void*)conv_tc_tile_kernel<true, 1, true>},
-       {(const void*)conv_tc_tile_kernel<true, 2, false>, (const void*)conv_tc_tile_kernel<true, 2, true>}}};
-  const void* fn = fns[train ? 1 : 0][nt2][split ? 1 : 0];
+       {(const void*)conv_tc_tile_kernel<true, 2, false>, (const void*)conv_tc_tile_kernel<true, 2, true>}},
+      {{(const void*)conv_tc_tile_kernel<true, 1, false, true>, (const void*)conv_tc_tile_kernel<true, 1, true, true>},
+       {(const void*)conv_tc_tile_kernel<true, 2, false, true>, (const void*)conv_tc_tile_kernel<true, 2, true, true>}}};
+  const void* fn = fns[kind][nt2][split ? 1 : 0];
   if (int rc = ensure_dyn_smem(fn, smem)) return rc;
   void* kargs[] = {&p};
   cudaError_t le;
@@ -1123,6 +1172,7 @@ int launch_tc_tile_train(const Fp32Args& a, const TilePlan& plan, cudaStream_t s
   p.fuse = a.fuse;
   p.dbg = g_dbg_timing;
   p.loss_B = a.B; p.T_orig = a.T; p.n_sub = plan.n_sub;
+  p.win_start = a.wv.win_start; p.win_end = a.wv.win_end; p.n_frames = a.wv.n_frames; p.pad_mode = a.wv.pad_mode;
   return launch_tc_tile(p, plan, stream);
 }
 

@@ -49,7 +49,7 @@ struct WideArgs {
   long long act_off[4], dz_off[4];
   float* loss_partials;         // [grid]
   long long* step_dev; long long* epoch_dev;   // MODE 1: device-side step / exchange-epoch counters, bumped by CTA 0 (read by the Adam kernel)
-  WindowView wv;                // MODE 0 only: win_start set = x is a frame stream and B the number of windows viewed in it
+  WindowView wv;                // MODE 0 / 1: win_start set = x (and target / conf) are frame streams, B = windows viewed in them
 };
 
 constexpr int kWideThreads = 320;
@@ -115,7 +115,9 @@ __device__ __forceinline__ bool wait_addr(uint32_t bar, uint32_t parity, int sit
 // MODE 2: dgrad chain: DZ[3] -> DZ[2] -> DZ[1] -> DZ[0] with the transposed weight blocks; epilogue = ReLU mask on the
 //         saved activation (loss.backward(), steps/traintest.py:120).  The weight gradients are a separate split-K GEMM
 //         over the dumps (conv_tc_wide_wgrad_kernel).
-template <int MODE>
+// VIEW (MODE 1 only): training over window views, a separate instantiation so that the dense training forward keeps its
+// code (the run-time test cost the C = 256 step ~0.6 %).  MODE 0 tests p.wv.win_start at run time.
+template <int MODE, bool VIEW = false>
 __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs p, const __grid_constant__ CUtensorMap wmap) {
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) uint64_t full_bar[kWideMaxStages];    // stage landed (TMA complete_tx)
@@ -297,7 +299,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
           uint4 q = make_uint4(0, 0, 0, 0);
           if (rc.valid) {
             size_t base = ((size_t)rc.gw * T + rc.t) * n_in;
-            if constexpr (MODE == 0) {
+            if constexpr (MODE == 0 || VIEW) {
               if (p.wv.win_start) {                  // window view: the source row in the frame stream
                 const long long f = window_src_row(p.wv, rc.gw, rc.t);
                 if (f < 0) {                         // a zero row: no keypoints, the pos-emb channel as in a padded window
@@ -486,8 +488,15 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
             const float n_el = (float)len * (float)B2H_COUT;
             const float scale = !live ? 0.f : ((p.loss_kind == B2H_LOSS_L1) ? (1.0f / (float)p.B) / n_el : 1.0f / n_el);
             const size_t ro = rc.valid ? ((size_t)rc.gw * T + rc.t) : 0;
-            const float* tg = p.train_mode == 1 ? p.target + ro * B2H_COUT : p.d_y + ro * B2H_COUT;
-            const float* cf = (p.conf && p.loss_kind == B2H_LOSS_CONFL1) ? p.conf + ro * (B2H_COUT / 2) : nullptr;
+            size_t tro = ro;                         // row of the target / confidences: a stream row for a window view
+            bool zrow = false;                       // ... or a zero row (its target and confidences read as zeros)
+            if (VIEW && rc.valid) {
+              const long long f = window_src_row(p.wv, rc.gw, rc.t);
+              zrow = f < 0;
+              tro = zrow ? 0 : (size_t)f;
+            }
+            const float* tg = p.train_mode == 1 ? p.target + tro * B2H_COUT : p.d_y + ro * B2H_COUT;
+            const float* cf = (p.conf && p.loss_kind == B2H_LOSS_CONFL1) ? p.conf + tro * (B2H_COUT / 2) : nullptr;
             float* yrow = (rc.valid && p.y) ? p.y + ro * B2H_COUT : nullptr;
             float sum = 0.f;
             for (int c0 = 16 * ch; c0 < N; c0 += 32) {
@@ -504,6 +513,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
                 if (on) {
                   tv = __ldg(reinterpret_cast<const float2*>(tg + c));
                   if (cf) sv = __ldg(cf + (c >> 1));
+                  if (VIEW && zrow) { tv = make_float2(0.f, 0.f); sv = cf ? 0.f : 1.0f; }
                 }
                 const float a0 = on ? __uint_as_float(v[q]) + bias_s[3][c < 255 ? c : 255] : 0.0f;
                 const float a1 = on ? __uint_as_float(v[q + 1]) + bias_s[3][c < 254 ? c + 1 : 255] : 0.0f;
@@ -815,15 +825,17 @@ int launch_tc_wide_train(const Fp32Args& a, const WidePlan& plan, unsigned char*
   p.target = a.target; p.conf = a.conf; p.d_y = a.d_y; p.loss_kind = a.loss_kind; p.train_mode = a.mode;
   p.scratch = scratch; p.loss_partials = a.loss_partials;
   p.step_dev = a.step_dev; p.epoch_dev = a.epoch_dev;
+  p.wv = a.wv;
   wide_common(p, g, plan, a.B, a.T);
   const size_t smem = plan.smem;
   const int grid = plan.grid;
   // ---- 1. forward + criterion ----
   wide_forward_stages(p, g);
-  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_wide_kernel<1>), smem)) return rc;
+  auto* fwd = p.wv.win_start ? conv_tc_wide_kernel<1, true> : conv_tc_wide_kernel<1>;
+  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fwd), smem)) return rc;
   CUtensorMap fmap, bmap;
   if (int rc = wide_weight_map(a.packed + g.tf_off[0], g.td_off[0] - g.tf_off[0], &fmap)) return rc;
-  conv_tc_wide_kernel<1><<<grid, kWideThreads, smem, stream>>>(p, fmap);
+  fwd<<<grid, kWideThreads, smem, stream>>>(p, fmap);
   count_launch();
   if (int rc = check_launch("conv_tc_wide_kernel<train fwd>")) return rc;
   // ---- 2. dgrad chain: layers 4, 3, 2 with the transposed blocks (td sections are contiguous from td_off[1]) ----

@@ -97,6 +97,7 @@ class GpuPoseDataset(Dataset):
         self.lh = torch.from_numpy(packed.hand_left).to(self.device)
         self.rh = torch.from_numpy(packed.hand_right).to(self.device)
         self.pre = PreprocessRightHand(factor=factor, dif_encoding=dif_encoding, normalize=normalize, pad_mode="repeat_first")
+        self._streams = {}
 
     def __len__(self):
         return len(self.packed)
@@ -106,14 +107,34 @@ class GpuPoseDataset(Dataset):
         start, stop = select_window(hi - lo, self.max_frames, self.selection, self.rng)     # :52-68
         return lo + start, lo + stop, start
 
+    def _draw(self, indices):
+        """Crop draws (in index order) and sequence lengths of one batch: shared by `batch()` and `crops()`."""
+        starts, ends, rel = zip(*(self._crop(int(i)) for i in indices))
+        nf = [min(int(self.packed.n_frames_meta[int(i)]), self.max_frames) for i in indices]           # :447
+        return starts, ends, rel, nf
+
+    def crops(self, indices):
+        """The crop list of a training step over `training_streams()`: {win_start, win_end, n_frames} as CPU int64 (B,)
+        tensors -- the same `select_window` draws (one per index, in order) and the same n_frames rule as `batch()`."""
+        starts, ends, _, nf = self._draw(indices)
+        return {"win_start": torch.tensor(starts, dtype=torch.int64), "win_end": torch.tensor(ends, dtype=torch.int64),
+                "n_frames": torch.tensor(nf, dtype=torch.int64)}
+
+    def training_streams(self, dtype=torch.bfloat16):
+        """Per-frame training data of ALL packed frames, built once per dtype and cached ({input_kp, target_kp,
+        target_conf}, `PreprocessRightHand.training_stream`).  Per-frame preprocessing does not depend on the window, so the
+        windows of `crops()` over these streams equal the windows `batch()` materialises with the same draws."""
+        if dtype not in self._streams:
+            self._streams[dtype] = self.pre.training_stream(self.pose, self.lh, self.rh, dtype=dtype)
+        return self._streams[dtype]
+
     def batch(self, indices):
         """Stacked item dict for several utterances with ONE preprocessing launch (what DataLoader + default_collate
         produce, traintest.py:87): tensors (B,T,...) on the device, n_frames (B,) CPU int64 like the reference
         (traintest.py:91), text / json_paths / utt_id as python lists (collate_function, steps/utils.py:383-396)."""
-        starts, ends, rel = zip(*(self._crop(int(i)) for i in indices))
+        starts, ends, rel, nf = self._draw(indices)
         out = self.pre(self.pose, self.lh, self.rh, np.asarray(starts, dtype=np.int64), self.max_frames,
                        win_end=np.asarray(ends, dtype=np.int64))
-        nf = [min(int(self.packed.n_frames_meta[int(i)]), self.max_frames) for i in indices]           # :447
         out["n_frames"] = torch.tensor(nf, dtype=torch.int64)
         out["text"] = [self.packed.texts[int(i)] for i in indices]
         out["utt_id"] = [self.packed.utt_ids[int(i)] for i in indices]

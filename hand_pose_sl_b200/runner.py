@@ -5,6 +5,7 @@ what a training / serving loop uses once shapes are fixed (SURVEY.md §0.7: laun
 tensor pipe or HBM, bounds every BASELINE config).
 
 Input staging: every slot is ONE contiguous device buffer  [input_kp | target_kp | target_conf? | n_frames(int32)]
+(WindowTrainStepRunner, over frame streams resident on the device: [win_start | win_end | n_frames])
 and `host_stage(batch)` builds the same layout in pinned host memory, so a step's inputs travel with ONE
 cudaMemcpyAsync (`load_staged`).  With `x_dtype=torch.bfloat16` the keypoint input is shipped as bf16 -- the bf16
 kernels round it to bf16 on the way into shared memory anyway (cvt.rn == torch's CPU rounding), so the result is
@@ -23,9 +24,25 @@ def _align(n, a=256):
 
 
 class _StepBuffers:
-    """Static per-slot buffers shared by TrainStepRunner and parallel.DataParallelTrainer."""
+    """Static per-slot buffers shared by TrainStepRunner, WindowTrainStepRunner and parallel.DataParallelTrainer."""
 
     def _init_buffers(self, model: ConvModel, optimizer: FusedAdam, B: int, T: int, loss: str, n_slots: int, x_dtype):
+        x_dtype = x_dtype or torch.float32
+        if x_dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError("x_dtype must be torch.float32 or torch.bfloat16")
+        if x_dtype == torch.bfloat16 and model.precision != "bf16":
+            raise ValueError("bf16 inputs are only bit-identical to fp32 inputs in bf16 mode")
+        self.x_dtype = x_dtype
+        K = model.n_in // 2
+        conf = _lib.LOSSES[loss] == _lib.LOSS_CONFL1
+        self._init_common(model, optimizer, B, T, loss, n_slots, (
+            ("x", "input_kp", x_dtype, (B, T, K, 2)), ("target", "target_kp", torch.float32, (B, T, 21, 2)),
+            ("conf", "target_conf", torch.float32, (B, T, 21) if conf else None), ("lengths", "n_frames", torch.int32, (B,))))
+        self.lengths.fill_(T)
+
+    def _init_common(self, model, optimizer, B, T, loss, n_slots, fields):
+        """`fields`: (attribute, batch key, dtype, shape per slot or None) of every section of a slot.  A slot is ONE
+        contiguous device buffer (every section 256-B aligned); `host_stage` builds the same layout in pinned host memory."""
         self.model, self.opt, self.B, self.T = model, optimizer, B, T
         self.loss_name = loss
         self.kind = _lib.LOSSES[loss]
@@ -38,34 +55,20 @@ class _StepBuffers:
         if optimizer._owner(group) is not model:
             raise RuntimeError(f"{type(self).__name__} needs FusedAdam(model.parameters()) over exactly this model")
         self.state = optimizer._group_state(0, group, model)
-        K = model.n_in // 2
         self.n_slots = n_slots
-        x_dtype = x_dtype or torch.float32
-        if x_dtype not in (torch.float32, torch.bfloat16):
-            raise ValueError("x_dtype must be torch.float32 or torch.bfloat16")
-        if x_dtype == torch.bfloat16 and model.precision != "bf16":
-            raise ValueError("bf16 inputs are only bit-identical to fp32 inputs in bf16 mode")
-        self.x_dtype = x_dtype
-        esz = 2 if x_dtype == torch.bfloat16 else 4
+        self._fields = [(name, key, dtype) for name, key, dtype, shape in fields if shape is not None]
         # byte layout of one slot (every section 256-B aligned)
         self._sec = {}
         off = 0
-        for name, nbytes in (("x", B * T * K * 2 * esz), ("target", B * T * 42 * 4),
-                             ("conf", B * T * 21 * 4 if self.kind == _lib.LOSS_CONFL1 else 0), ("lengths", B * 4)):
+        for name, _, dtype, shape in fields:
+            nbytes = 0 if shape is None else torch.Size(shape).numel() * dtype.itemsize
             self._sec[name] = (off, nbytes)
             off = _align(off + nbytes)
         self.slot_bytes = off
         self.stage = torch.zeros((n_slots, self.slot_bytes), dtype=torch.uint8, device=dev)
-
-        def view(name, dtype, shape):
+        for name, _, dtype, shape in fields:
             o, n = self._sec[name]
-            return self.stage[:, o:o + n].view(dtype).view((n_slots,) + shape)
-
-        self.x = view("x", x_dtype, (B, T, K, 2))
-        self.target = view("target", torch.float32, (B, T, 21, 2))
-        self.conf = view("conf", torch.float32, (B, T, 21)) if self.kind == _lib.LOSS_CONFL1 else None
-        self.lengths = view("lengths", torch.int32, (B,))
-        self.lengths.fill_(T)
+            setattr(self, name, None if shape is None else self.stage[:, o:o + n].view(dtype).view((n_slots,) + tuple(shape)))
         self.loss = torch.zeros((n_slots,), dtype=torch.float32, device=dev)
         # Pinned, device-mapped host words: with step(..., to_host=True) the kernel stores the step's loss straight into host
         # memory (a 4-byte posted write over PCIe) -- a cudaMemcpy D2H of the loss queues behind the NEXT batch's 3.5 MB
@@ -91,29 +94,19 @@ class _StepBuffers:
 
     # ------------------------------------------------------------------ inputs
     def load(self, batch, slot=0, non_blocking=True):
-        """Copy one reference-style batch dict (CPU pinned or device tensors) into slot `slot` (one copy per tensor;
-        `load_staged` moves the same bytes with a single copy)."""
-        self.x[slot].copy_(batch["input_kp"], non_blocking=non_blocking)
-        self.target[slot].copy_(batch["target_kp"], non_blocking=non_blocking)
-        if self.conf is not None:
-            self.conf[slot].copy_(batch["target_conf"], non_blocking=non_blocking)
-        self.lengths[slot].copy_(batch["n_frames"], non_blocking=non_blocking)
+        """Copy one batch dict (CPU pinned or device tensors) into slot `slot` (one copy per tensor; `load_staged` moves
+        the same bytes with a single copy)."""
+        for name, key, _ in self._fields:
+            getattr(self, name)[slot].copy_(torch.as_tensor(batch[key]), non_blocking=non_blocking)
 
     def host_stage(self, batch, out=None):
-        """Pack a reference-style batch dict (CPU tensors) into ONE pinned host buffer with the slot's byte layout
-        (the collate step of a data loader).  Returns the uint8 tensor `load_staged` takes."""
+        """Pack a batch dict (CPU tensors) into ONE pinned host buffer with the slot's byte layout (the collate step of a
+        data loader).  Returns the uint8 tensor `load_staged` takes."""
         if out is None:
             out = torch.zeros(self.slot_bytes, dtype=torch.uint8).pin_memory()
-
-        def put(name, t, dtype):
+        for name, key, dtype in self._fields:
             o, n = self._sec[name]
-            out[o:o + n].view(dtype).copy_(t.reshape(-1))
-
-        put("x", batch["input_kp"], self.x_dtype)
-        put("target", batch["target_kp"], torch.float32)
-        if self.conf is not None:
-            put("conf", batch["target_conf"], torch.float32)
-        put("lengths", torch.as_tensor(batch["n_frames"]), torch.int32)
+            out[o:o + n].view(dtype).copy_(torch.as_tensor(batch[key]).reshape(-1))
         return out
 
     def load_staged(self, staged, slot=0, non_blocking=True):
@@ -213,10 +206,51 @@ class TrainStepRunner(_StepBuffers):
         return loss[0]
 
 
+class WindowTrainStepRunner(_StepBuffers):
+    """TrainStepRunner over window views of device-resident frame streams (`PreprocessRightHand.training_stream`,
+    `GpuPoseDataset.training_streams`): a slot holds only the step's crop list, ONE buffer
+    [win_start int64 | win_end int64 | lengths int32] (20 B per window: 5 KB at B = 256 instead of a 3.54 MB batch),
+    loaded from a dict {win_start, win_end, n_frames} (`GpuPoseDataset.crops`) by `load` / `host_stage` + `load_staged`.
+    Steps, capture, replay and finish behave as TrainStepRunner's; the results are bit-identical to TrainStepRunner on the
+    windows K0 materialises.  `streams` stay referenced by the runner (a captured graph reads them by address)."""
+
+    def __init__(self, model: ConvModel, optimizer: FusedAdam, streams, B: int, T: int, loss: str = "L1", n_slots: int = 1,
+                 pad_mode: str = "repeat_first"):
+        x = streams["input_kp"]
+        if x.dtype == torch.bfloat16 and model.precision != "bf16":
+            raise ValueError("bf16 inputs are only bit-identical to fp32 inputs in bf16 mode")
+        self._init_common(model, optimizer, B, T, loss, n_slots, (
+            ("win_start", "win_start", torch.int64, (B,)), ("win_end", "win_end", torch.int64, (B,)),
+            ("lengths", "n_frames", torch.int32, (B,))))
+        from .steps import _window_args
+        # stream arguments, validated and converted once: (x, x_dtype, target, conf, n_frames)
+        self._streams = _window_args(model, streams, self.win_start[0], T, self.lengths[0], None, pad_mode, loss)[0][:5]
+        self.pad_mode = {"repeat_first": _lib.PAD_REPEAT_FIRST, "zeros": _lib.PAD_ZEROS}[pad_mode]
+        self.win_end.fill_(self._streams[4])
+        self.lengths.fill_(T)
+
+    def step(self, slot=0, to_host=False):
+        """Enqueue one training step over the crops in slot `slot`; returns the loss as TrainStepRunner.step does."""
+        self._sync_host_state()
+        m, g = self.model, self.opt.param_groups[0]
+        n_in, C, pe = m._geometry()
+        b1, b2 = g["betas"]
+        x, dt, tgt, conf, F = self._streams
+        loss = (self.loss_host if to_host else self.loss)[slot:slot + 1]
+        _lib.check(self.lib.b2h_train_step_windows(
+            _lib.ptr(x), dt, _lib.ptr(tgt), _lib.ptr(conf), F, _lib.ptr(self.win_start[slot]), _lib.ptr(self.win_end[slot]),
+            self.pad_mode, _lib.ptr(self.lengths[slot]), _lib.ptr(m._flat), _lib.ptr(self.packed), _lib.ptr(self.state["m"]),
+            _lib.ptr(self.state["v"]), _lib.ptr(loss), self.B, self.T, n_in, C, pe, self.kind, _lib.PRECISIONS[m.precision],
+            float(g["lr"]), b1, b2, g["eps"], 0, _lib.ptr(self.step_dev), _lib.ptr(self.lr_dev), _lib.ptr(self.ws),
+            self.ws.numel(), _lib.stream_ptr(self.dev)))
+        self._advance(1)
+        return loss[0]
+
+
 def pipelined_steps(runner, batches, status_every=0, copy_streams=1):
     """Training loop with a double-buffered input pipeline (what a DataLoader with prefetch gives the reference loop,
     steps/traintest.py:87-123): while step i runs, batch i+1 travels host -> device on copy stream(s) into the other
-    slot.  `runner` is a TrainStepRunner or parallel.DataParallelTrainer with n_slots >= 2; `batches` yields either
+    slot.  `runner` is a TrainStepRunner, WindowTrainStepRunner or parallel.DataParallelTrainer with n_slots >= 2; `batches` yields either
     `runner.host_stage(...)` buffers or reference-style batch dicts in pinned host memory.  A staged buffer can be moved as
     `copy_streams` contiguous pieces on as many streams: in isolation two halves in parallel reach 49 GB/s against
     42 GB/s for one 3.5 MB copy on B200, but inside this loop the extra per-step host calls cost more than the copy
@@ -225,7 +259,7 @@ def pipelined_steps(runner, batches, status_every=0, copy_streams=1):
     after step i+1 has been enqueued (one step of lag), which keeps the GPU fed."""
     if runner.n_slots < 2:
         raise RuntimeError("pipelined_steps needs a runner with n_slots >= 2")
-    dev = runner.x.device
+    dev = runner.dev if hasattr(runner, "dev") else runner.x.device     # (a runner without its own device attribute)
     main = torch.cuda.current_stream(dev)
     ncs = max(1, int(copy_streams))
     cstreams = [torch.cuda.Stream(dev) for _ in range(ncs)]

@@ -308,6 +308,89 @@ def forward_backward(model: ConvModel, batch, loss="L1", want_pred=False):
     return (loss_out, grads, pred) if want_pred else (loss_out, grads)
 
 
+def _window_args(model: ConvModel, streams, win_start, T, lengths, win_end, pad_mode, loss):
+    """Device arguments of the *_windows calls: the three frame streams, the crop list and the lengths."""
+    x = streams["input_kp"]
+    _lib.require_device(x, "input_kp stream")
+    _lib.require_sm100(x.device)
+    if x.dim() != 3 or x.shape[1] * x.shape[2] != model.n_in:
+        raise RuntimeError(f"expected an input_kp stream (F, {model.n_in // 2}, 2), got {tuple(x.shape)}")
+    if x.dtype not in (torch.float32, torch.bfloat16):
+        raise RuntimeError(f"the input_kp stream must be float32 or bfloat16, got {x.dtype}")
+    if model.pos_emb is not None and T != model.pos_emb.max_len and not model.pos_emb_any_length:
+        raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {model.pos_emb.max_len}, got {T}")
+    dev, F = x.device, x.shape[0]
+    kind = _lib.LOSSES[loss]
+    tgt = streams["target_kp"].to(device=dev, dtype=torch.float32).contiguous()
+    if tgt.numel() != F * 42:
+        raise RuntimeError(f"target_kp stream has {tgt.numel()} values for {F} frames (expected (F, 21, 2))")
+    conf = None
+    if kind == _lib.LOSS_CONFL1:
+        conf = streams["target_conf"].to(device=dev, dtype=torch.float32).contiguous()
+        if conf.numel() != F * 21:
+            raise RuntimeError(f"target_conf stream has {conf.numel()} values for {F} frames (expected (F, 21))")
+    ws = torch.as_tensor(win_start).to(device=dev, dtype=torch.int64).contiguous()
+    W = ws.numel()
+    we = None if win_end is None else torch.as_tensor(win_end).to(device=dev, dtype=torch.int64).contiguous()
+    if we is not None and we.numel() != W:
+        raise RuntimeError("win_end must have one entry per window")
+    pm = {"repeat_first": _lib.PAD_REPEAT_FIRST, "zeros": _lib.PAD_ZEROS}[pad_mode]
+    len32 = _lengths_i32(lengths, dev, W)
+    dt = _lib.DT_BF16 if x.dtype == torch.bfloat16 else _lib.DT_F32
+    return (x.contiguous(), dt, tgt, conf, F, ws, we, pm, len32), W, kind, dev
+
+
+def _window_ptrs(args):
+    x, dt, tgt, conf, F, ws, we, pm, len32 = args
+    return (_lib.ptr(x), dt, _lib.ptr(tgt), _lib.ptr(conf), F, _lib.ptr(ws), _lib.ptr(we), pm, _lib.ptr(len32))
+
+
+def fused_train_step_windows(model: ConvModel, streams, win_start, T, lengths, optimizer: FusedAdam, win_end=None,
+                             pad_mode="repeat_first", loss="L1"):
+    """`fused_train_step` on window views of device-resident frame streams: `streams` = {input_kp (F, K, 2) fp32 / bf16,
+    target_kp (F, 21, 2), target_conf (F, 21) for confL1} (`PreprocessRightHand.training_stream`); window w covers frames
+    [win_start[w], win_start[w] + T) cut at win_end[w] (default F) and padded by the dataset's rule, in all three streams.
+    `lengths` = the windows' n_frames.  Bit-identical to `fused_train_step` on the windows K0 materialises; served where
+    the tensor cores train (b2h_kernel_choice tile / wide), B2HError otherwise.  Returns the 0-dim device loss."""
+    args, W, kind, dev = _window_args(model, streams, win_start, T, lengths, win_end, pad_mode, loss)
+    group = optimizer.param_groups[0]
+    if optimizer._owner(group) is not model:
+        raise RuntimeError("fused_train_step_windows needs FusedAdam(model.parameters()) over exactly this model")
+    st = optimizer._group_state(0, group, model)
+    st["step"] += 1
+    n_in, C, pe = model._geometry()
+    packed = model.packed_weights()
+    ws = model.workspace(W, T)
+    flat = model.flat_parameters()
+    loss_out = torch.empty((), dtype=torch.float32, device=dev)
+    b1, b2 = group["betas"]
+    _lib.check(_lib.load().b2h_train_step_windows(
+        *_window_ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(st["m"]), _lib.ptr(st["v"]), _lib.ptr(loss_out), W, T,
+        n_in, C, pe, kind, _lib.PRECISIONS[model.precision], float(group["lr"]), b1, b2, group["eps"], st["step"], None, None,
+        _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
+    model.packed_weights(fresh_from_kernel=True)
+    st["step_t"].fill_(float(st["step"]))
+    return loss_out
+
+
+def forward_backward_windows(model: ConvModel, streams, win_start, T, lengths, win_end=None, pad_mode="repeat_first",
+                             loss="L1", want_pred=False):
+    """`forward_backward` on window views of frame streams (see `fused_train_step_windows`): returns (loss, flat gradients
+    [, masked prediction (W, T, 21, 2)]), bit-identical to `forward_backward` on the materialised windows."""
+    args, W, kind, dev = _window_args(model, streams, win_start, T, lengths, win_end, pad_mode, loss)
+    n_in, C, pe = model._geometry()
+    packed = model.packed_weights()
+    ws = model.workspace(W, T)
+    flat = model.flat_parameters()
+    grads = torch.empty_like(flat)
+    loss_out = torch.empty((), dtype=torch.float32, device=dev)
+    pred = torch.empty((W, T, 21, 2), dtype=torch.float32, device=dev) if want_pred else None
+    _lib.check(_lib.load().b2h_train_forward_backward_windows(
+        *_window_ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(grads), _lib.ptr(loss_out), _lib.ptr(pred), W, T,
+        n_in, C, pe, kind, _lib.PRECISIONS[model.precision], None, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
+    return (loss_out, grads, pred) if want_pred else (loss_out, grads)
+
+
 @torch.no_grad()
 def validate_batch(model: ConvModel, batch, loss="L1"):
     """validate() body, traintest.py:174-207, for one batch: forward + mask_output + criterion."""

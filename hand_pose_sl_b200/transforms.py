@@ -114,6 +114,33 @@ class PreprocessRightHand:
                                               f32, None, None, None, None, None, None, b16, _lib.stream_ptr(dev)))
         return out
 
+    def training_stream(self, pose25, hand_left, hand_right, dtype=torch.bfloat16):
+        """Training from device-resident frames: the per-frame preprocessed training data of a whole clip, from ONE K0
+        launch (one window covering the clip) -- {input_kp (F, 12, 2) in `dtype`, target_kp (F, 21, 2) fp32,
+        target_conf (F, 21) fp32}, 300 B per frame in bf16.  Per-frame preprocessing does not depend on the window, so
+        the crops of `steps.fused_train_step_windows` / `runner.WindowTrainStepRunner` over these streams are exactly
+        the windows `__call__` materialises.  (H5 rows: `from_h5_rows(rows, [0], F)` with the window axis dropped.)"""
+        _lib.require_device(pose25, "pose25")
+        _lib.require_sm100(pose25.device)
+        dev = pose25.device
+        F = pose25.shape[0]
+        if tuple(pose25.shape[1:]) != (25, 3) or tuple(hand_left.shape) != (F, 21, 3) or tuple(hand_right.shape) != (F, 21, 3):
+            raise RuntimeError("expected pose25 (F,25,3), hand_left (F,21,3), hand_right (F,21,3)")
+        if dtype not in (torch.bfloat16, torch.float32):
+            raise ValueError("dtype must be torch.bfloat16 or torch.float32")
+        pose25, hand_left, hand_right = (_dev_f32(a, dev) for a in (pose25, hand_left, hand_right))
+        f32 = dict(dtype=torch.float32, device=dev)
+        out = {"input_kp": torch.empty((F, 12, 2), dtype=dtype, device=dev), "target_kp": torch.empty((F, 21, 2), **f32),
+               "target_conf": torch.empty((F, 21), **f32)}
+        x32 = _lib.ptr(out["input_kp"]) if dtype == torch.float32 else None
+        x16 = _lib.ptr(out["input_kp"]) if dtype == torch.bfloat16 else None
+        start = torch.zeros(1, dtype=torch.int64, device=dev)
+        _lib.check(_lib.load().b2h_preprocess(_lib.ptr(pose25), _lib.ptr(hand_left), _lib.ptr(hand_right), F, _lib.ptr(start), None,
+                                              1, F, self.pad_mode, self.factor, int(self.dif_encoding), int(self.normalize), x32,
+                                              None, _lib.ptr(out["target_kp"]), _lib.ptr(out["target_conf"]), None, None, None,
+                                              x16, _lib.stream_ptr(dev)))
+        return out
+
     def from_h5_rows(self, rows150, win_start, T, win_end=None):
         """Packed rows of TextPoseH5Dataset.array2item (text_pose_dataset.py:587-612): (F,150) =
         [x0..x49|y0..y49|c0..c49]; body = 8 keypoints."""

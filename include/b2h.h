@@ -180,6 +180,23 @@ int b2h_train_forward_backward(const void* x, int x_dtype, const float* target, 
                                int pos_emb, int loss_kind, int precision, int64_t* step_dev, void* workspace,
                                int64_t workspace_bytes, void* stream);
 
+/* b2h_train_forward_backward over WINDOW VIEWS of device-resident frame streams: training from a preprocessed set kept in
+ * device memory, where a step needs only its crop list (win_start, win_end, lengths: 20 B per window) instead of a
+ * materialised (n_win, T, .) batch.  frames (n_frames, n_in) fp32 or bf16 (16-byte aligned), target_frames
+ * (n_frames, 42) fp32 (8-byte aligned), conf_frames (n_frames, 21) fp32 (4-byte aligned, B2H_LOSS_CONFL1 only): window w,
+ * frame t reads the SAME row of all three streams, the crop [win_start[w], win_start[w] + T) cut at min(win_end[w],
+ * n_frames) (win_end nullable) and padded by `pad_mode` exactly like b2h_preprocess; a padded row of B2H_PAD_ZEROS is a
+ * zero row in all three.  lengths (n_win) as in the dense call (the reference takes them from the metadata, not the
+ * crop); pred_out stays dense (n_win, T, 42).  Bit-identical to b2h_train_forward_backward on the windows b2h_preprocess
+ * materialises.  Workspace: b2h_workspace_bytes(n_win, T, ...).  Served where b2h_kernel_choice(T, ..., train = 1) is
+ * B2H_KERNEL_TC_TILE or B2H_KERNEL_TC_WIDE_TRAIN; B2H_ESHAPE on every FFMA shape. */
+int b2h_train_forward_backward_windows(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
+                                       int64_t n_frames, const int64_t* win_start, const int64_t* win_end, int pad_mode,
+                                       const int32_t* lengths, const float* params, const void* packed, float* grads_out,
+                                       float* loss_out, float* pred_out, int n_win, int T, int n_in, int C, int pos_emb,
+                                       int loss_kind, int precision, int64_t* step_dev, void* workspace,
+                                       int64_t workspace_bytes, void* stream);
+
 /* Backward of ConvModel.forward alone for the modular autograd path (what loss.backward() does
  * below the criterion, steps/traintest.py:120): d_y (B,T,42) fp32 -> flat parameter gradients
  * (activations are recomputed in shared memory, nothing was saved by the forward). */
@@ -261,6 +278,16 @@ int b2h_train_step(const void* x, int x_dtype, const float* target, const float*
                    int n_in, int C, int pos_emb, int loss_kind, int precision, double lr, double beta1,
                    double beta2, double eps, int64_t step, int64_t* step_dev, const double* lr_dev, void* workspace,
                    int64_t workspace_bytes, void* stream);
+
+/* b2h_train_step over window views of frame streams (the streams, crop rule, alignment and served shapes of
+ * b2h_train_forward_backward_windows; every other argument as in b2h_train_step).  Bit-identical to b2h_train_step on the
+ * materialised windows: loss, params, exp_avg, exp_avg_sq and the packed buffer. */
+int b2h_train_step_windows(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
+                           int64_t n_frames, const int64_t* win_start, const int64_t* win_end, int pad_mode,
+                           const int32_t* lengths, float* params, void* packed, float* exp_avg, float* exp_avg_sq,
+                           float* loss_out, int n_win, int T, int n_in, int C, int pos_emb, int loss_kind, int precision,
+                           double lr, double beta1, double beta2, double eps, int64_t step, int64_t* step_dev,
+                           const double* lr_dev, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* tcgen05 / TMEM / descriptor self-test (tests/test_tc_probe.py): D = A·B^T for one 128xNx(16*ksteps)
  * bf16 tile staged in the no-swizzle K-major layout the conv kernels use, A rows shifted by `shift`
