@@ -20,6 +20,12 @@ PAD_REPEAT_FIRST, PAD_ZEROS = 0, 1
 DT_F32, DT_BF16 = 0, 1
 PRECISIONS = {"fp32": FP32, "bf16": BF16, "fp32-ffma": FP32_FFMA}
 LOSSES = {"L1": LOSS_L1, "confL1": LOSS_CONFL1}
+PAD_MODES = {"repeat_first": PAD_REPEAT_FIRST, "zeros": PAD_ZEROS}
+
+
+def dtype_code(dtype):
+    """The C-ABI `x_dtype` of a float32 / bfloat16 keypoint input."""
+    return DT_BF16 if dtype == torch.bfloat16 else DT_F32
 
 _SIGNATURES = {
     "b2h_last_error": (c_char_p, []),
@@ -137,6 +143,19 @@ def require_sm100(device):
 
 def ptr(t):
     return None if t is None else c_void_p(t.data_ptr())
+
+
+def ptrs(args):
+    """C arguments: every tensor of `args` replaced by its pointer."""
+    return tuple(ptr(a) if isinstance(a, torch.Tensor) else a for a in args)
+
+
+def lengths_i32(lengths, device, B):
+    """`lengths` is `batch["n_frames"]`, a CPU int64 tensor in the reference (traintest.py:91)."""
+    t = torch.as_tensor(lengths)
+    if t.numel() != B:
+        raise RuntimeError(f"lengths has {t.numel()} entries for a batch of {B}")
+    return t.to(device=device, dtype=torch.int32, non_blocking=True).contiguous()
 
 
 def stream_ptr(device=None):

@@ -188,41 +188,48 @@ extern "C" int b2h_pack_weights(const float* params, void* packed, int n_in, int
   return launch_pack(params, packed, make_geo(n_in, C, pos_emb), (cudaStream_t)stream);
 }
 
+// The window view of the *_windows entry points.
+static WindowView window_view(const int64_t* win_start, const int64_t* win_end, int64_t n_frames, int pad_mode) {
+  return WindowView{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
+}
+
+// The checks every forward and training entry point makes first, in this order: pointers (`out` = y in the forward, the
+// workspace in training), x_dtype, pad_mode, geometry, shape (B >= B_min).
+static int check_common(const void* x, int x_dtype, const WindowView* wv, const float* params, const void* packed,
+                        const void* out, int B, int B_min, int T, int n_in, int C, int pos_emb, const char* who) {
+  if (!x || (wv && !wv->win_start) || !params || !packed || !out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  if (x_dtype != B2H_DT_F32 && x_dtype != B2H_DT_BF16) { set_error("%s: bad x_dtype %d", who, x_dtype); return B2H_EINVAL; }
+  if (wv && wv->pad_mode != B2H_PAD_REPEAT_FIRST && wv->pad_mode != B2H_PAD_ZEROS) { set_error("%s: bad pad_mode %d", who, wv->pad_mode); return B2H_EINVAL; }
+  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
+  if (B < B_min || T < 1 || (wv && wv->n_frames < 0)) { set_error("%s: bad B=%d T=%d", who, B, T); return B2H_ESHAPE; }
+  return B2H_OK;
+}
+
+static bool misaligned(const void* p, uintptr_t mask) { return reinterpret_cast<uintptr_t>(p) & mask; }
+
 // The forward of B dense windows x (wv == nullptr) or of B windows viewed in the frame stream x.  Window views are read by
 // the tensor-core kernels only: fp32 mode beyond the tile kernel runs on FFMA, which reads dense windows.
 static int conv_forward(const void* x, int x_dtype, const WindowView* wv, const float* params, const void* packed,
                         const int32_t* lengths, float* y, int B, int T, int n_in, int C, int pos_emb, int precision,
                         int apply_mask, float out_scale, cudaStream_t stream, const char* who) {
-  if (!x || (wv && !wv->win_start) || !params || !packed || !y) { set_error("%s: null pointer", who); return B2H_EINVAL; }
-  if (x_dtype != B2H_DT_F32 && x_dtype != B2H_DT_BF16) { set_error("%s: bad x_dtype %d", who, x_dtype); return B2H_EINVAL; }
-  if (wv && wv->pad_mode != B2H_PAD_REPEAT_FIRST && wv->pad_mode != B2H_PAD_ZEROS) { set_error("%s: bad pad_mode %d", who, wv->pad_mode); return B2H_EINVAL; }
-  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
-  if (B < 0 || T < 1 || (wv && wv->n_frames < 0)) { set_error("%s: bad B=%d T=%d", who, B, T); return B2H_ESHAPE; }
+  if (int rc = check_common(x, x_dtype, wv, params, packed, y, B, 0, T, n_in, C, pos_emb, who)) return rc;
   if (apply_mask && !lengths) { set_error("%s: apply_mask needs lengths", who); return B2H_EINVAL; }
   if (B == 0) return B2H_OK;
-  if ((reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(y) & 15) || (reinterpret_cast<uintptr_t>(packed) & 15)) {
+  if (misaligned(x, 15) || misaligned(y, 15) || misaligned(packed, 15)) {
     set_error("%s: %s, y and packed must be 16-byte aligned", who, wv ? "frames" : "x");
     return B2H_EALIGN;
   }
   if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
-  const Geo g = make_geo(n_in, C, pos_emb);
-  const ForwardPlan f = forward_plan(g, B, T, precision);
-  const char* pk = reinterpret_cast<const char*>(packed);
-  if (f.kernel == B2H_KERNEL_TC_TILE) return launch_tc_tile_fwd(x, x_dtype, params, pk, lengths, y, apply_mask, out_scale, g, f.tile, stream, wv);
-  if (f.kernel == B2H_KERNEL_TC_WIDE) return launch_tc_wide_fwd(x, x_dtype, params, pk, lengths, y, B, T, apply_mask, out_scale, g, f.wide, stream, wv);
-  if (f.kernel == B2H_KERNEL_TC_ROWSPACE) {
-    TcFwdArgs a{};
-    a.x = x; a.x_dtype = x_dtype; a.params = params; a.packed = pk; a.lengths = lengths;
-    a.y = y; a.B = B; a.T = T; a.apply_mask = apply_mask; a.out_scale = out_scale; a.geo = g;
-    if (wv) a.wv = *wv;
-    return launch_tc_fwd(a, f.rowspace, stream);
-  }
-  if (f.kernel == B2H_KERNEL_FFMA && !wv) {
-    Fp32Args a{};
-    a.x = x; a.x_dtype = x_dtype; a.lengths = lengths; a.params = params; a.packed = pk;
-    a.y = y; a.B = B; a.T = T; a.apply_mask = apply_mask; a.mode = 0; a.out_scale = out_scale; a.geo = g;
-    return launch_fp32(a, f.ffma, stream);
-  }
+  ConvArgs a{};
+  a.x = x; a.x_dtype = x_dtype; a.lengths = lengths; a.params = params; a.packed = reinterpret_cast<const char*>(packed);
+  a.y = y; a.B = B; a.T = T; a.apply_mask = apply_mask; a.mode = 0; a.out_scale = out_scale;
+  a.geo = make_geo(n_in, C, pos_emb);
+  if (wv) a.wv = *wv;
+  const ForwardPlan f = forward_plan(a.geo, B, T, precision);
+  if (f.kernel == B2H_KERNEL_TC_TILE) return launch_tc_tile(a, f.tile, stream);
+  if (f.kernel == B2H_KERNEL_TC_WIDE) return launch_tc_wide_fwd(a, f.wide, stream);
+  if (f.kernel == B2H_KERNEL_TC_ROWSPACE) return launch_tc_fwd(a, f.rowspace, stream);
+  if (f.kernel == B2H_KERNEL_FFMA && !wv) return launch_fp32(a, f.ffma, stream);
   if (wv)
     set_error("%s: window views are served in bf16 mode for conv_channels <= 256 with T <= 256, <= 48 with T <= 640 and <= 32 "
               "with T <= 1024 (the last two with at most 32 input channels), in fp32 mode for conv_channels <= 32 with T <= 256; "
@@ -245,82 +252,85 @@ extern "C" int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t
                                         const int64_t* win_end, int pad_mode, const float* params, const void* packed,
                                         const int32_t* lengths, float* y, int n_win, int T, int n_in, int C, int pos_emb,
                                         int precision, int apply_mask, float out_scale, void* stream) {
-  const WindowView wv{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
+  const WindowView wv = window_view(win_start, win_end, n_frames, pad_mode);
   return conv_forward(frames, x_dtype, &wv, params, packed, lengths, y, n_win, T, n_in, C, pos_emb, precision, apply_mask,
                       out_scale, (cudaStream_t)stream, "b2h_conv_forward_windows");
 }
 
+// What a training launch left for the reduction / Adam launches that follow it (rc != B2H_OK: nothing was launched).
+struct TrainResult {
+  int rc;
+  Geo g;
+  TrainPlan plan;
+  float* partials;        // gradient partials in the workspace: plan.nparts slices of plan.stride floats
+  float* loss_partials;   // plan.n_loss floats
+};
+
 // The training forward + criterion + backward of B dense windows (wv == nullptr) or of B windows viewed in the frame
-// streams x / target / conf (mode 1 only; the tensor-core kernels only: the FFMA kernel reads dense windows).
-static int train_common(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
-                        const float* d_y, const int32_t* lengths, const float* params, const void* packed, float* pred_out,
-                        int B, int T, int n_in, int C, int pos_emb, int loss_kind, int precision, int mode, void* workspace,
-                        int64_t workspace_bytes, cudaStream_t stream, Geo& g, TrainPlan& plan, float*& partials,
-                        float*& loss_partials, const char* who, long long* step_dev = nullptr, long long* epoch_dev = nullptr,
-                        FuseAdam* fuse = nullptr) {
-  if (!x || (wv && !wv->win_start) || !params || !packed || !workspace) { set_error("%s: null pointer", who); return B2H_EINVAL; }
-  if (x_dtype != B2H_DT_F32 && x_dtype != B2H_DT_BF16) { set_error("%s: bad x_dtype %d", who, x_dtype); return B2H_EINVAL; }
-  if (wv && wv->pad_mode != B2H_PAD_REPEAT_FIRST && wv->pad_mode != B2H_PAD_ZEROS) { set_error("%s: bad pad_mode %d", who, wv->pad_mode); return B2H_EINVAL; }
-  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
-  if (B < 1 || T < 1 || (wv && wv->n_frames < 0)) { set_error("%s: bad B=%d T=%d", who, B, T); return B2H_ESHAPE; }
-  if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
+// streams x / target / conf (mode 1 only; the tensor-core kernels only: the FFMA kernel reads dense windows).  fuse != nullptr
+// asks the tile kernel to reduce and apply Adam in the same launch.
+static TrainResult train_common(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
+                                const float* d_y, const int32_t* lengths, const float* params, const void* packed,
+                                float* pred_out, int B, int T, int n_in, int C, int pos_emb, int loss_kind, int precision,
+                                int mode, void* workspace, int64_t workspace_bytes, cudaStream_t stream, const char* who,
+                                long long* step_dev, long long* epoch_dev, const FuseAdam* fuse) {
+  TrainResult r{};
+  auto result = [&r](int rc) { r.rc = rc; return r; };
+  if (int rc = check_common(x, x_dtype, wv, params, packed, workspace, B, 1, T, n_in, C, pos_emb, who)) return result(rc);
+  if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return result(B2H_EINVAL); }
   if (mode == 1) {
-    if (!target || !lengths) { set_error("%s: null target/lengths", who); return B2H_EINVAL; }
-    if (loss_kind != B2H_LOSS_L1 && loss_kind != B2H_LOSS_CONFL1) { set_error("%s: bad loss_kind %d", who, loss_kind); return B2H_EINVAL; }
-    if (loss_kind == B2H_LOSS_CONFL1 && !conf) { set_error("%s: confL1 needs scores", who); return B2H_EINVAL; }
-  } else if (!d_y) { set_error("%s: null d_y", who); return B2H_EINVAL; }
+    if (!target || !lengths) { set_error("%s: null target/lengths", who); return result(B2H_EINVAL); }
+    if (loss_kind != B2H_LOSS_L1 && loss_kind != B2H_LOSS_CONFL1) { set_error("%s: bad loss_kind %d", who, loss_kind); return result(B2H_EINVAL); }
+    if (loss_kind == B2H_LOSS_CONFL1 && !conf) { set_error("%s: confL1 needs scores", who); return result(B2H_EINVAL); }
+  } else if (!d_y) { set_error("%s: null d_y", who); return result(B2H_EINVAL); }
   // A stream's target row (168 B) and confidence row (84 B) start 8 / 4 bytes past a 16-B boundary at odd frames: the
   // kernels read them with float2 / float loads and use a bulk copy only where the address allows it.
-  const uintptr_t talign = wv ? 7 : 15, calign = wv ? 3 : 0;
-  if ((reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(target) & talign) ||
-      (reinterpret_cast<uintptr_t>(conf) & calign) || (reinterpret_cast<uintptr_t>(packed) & 15)) {
+  if (misaligned(x, 15) || misaligned(target, wv ? 7 : 15) || misaligned(conf, wv ? 3 : 0) || misaligned(packed, 15)) {
     if (wv) set_error("%s: frames and packed must be 16-byte aligned, target_frames 8-byte and conf_frames 4-byte aligned", who);
     else set_error("%s: x, target and packed must be 16-byte aligned", who);
-    return B2H_EALIGN;
+    return result(B2H_EALIGN);
   }
-  g = make_geo(n_in, C, pos_emb);
-  plan = train_plan(g, B, T, precision);
+  r.g = make_geo(n_in, C, pos_emb);
+  const TrainPlan& plan = r.plan = train_plan(r.g, B, T, precision);
   if (wv && plan.kernel != B2H_KERNEL_TC_TILE && plan.kernel != B2H_KERNEL_TC_WIDE_TRAIN) {
     set_error("%s: window views are trained on the tensor cores: in bf16 mode for conv_channels <= 32 with at most 32 input "
               "channels and T <= 4096, and for conv_channels <= 256 with T <= 256; in fp32 mode for conv_channels <= 32 with at "
               "most 32 input channels and T <= 4096; materialise the windows (b2h_preprocess) for C=%d, T=%d, precision=%d",
               who, C, T, precision);
-    return B2H_ESHAPE;
+    return result(B2H_ESHAPE);
   }
   if (plan.kernel == B2H_KERNEL_NONE) {
     set_error("%s: no training kernel for conv_channels=%d, T=%d, precision=%d (tcgen05 training: C <= 32 in the one-launch tile "
               "kernel, C <= 256 in bf16 mode through the wide kernels, T <= 256; the FFMA kernel would need %zu B of shared memory)",
               who, C, T, precision, plan.ffma.smem);
-    return B2H_ESHAPE;
+    return result(B2H_ESHAPE);
   }
-  const int nparts = plan.nparts;
-  const int64_t stride = plan.stride;
-  if (workspace_bytes < plan.total - 256) { set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.total); return B2H_EWORKSPACE; }
-  if (reinterpret_cast<uintptr_t>(workspace) & 15) { set_error("%s: workspace must be 16-byte aligned", who); return B2H_EALIGN; }
+  if (workspace_bytes < plan.total - 256) { set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.total); return result(B2H_EWORKSPACE); }
+  if (misaligned(workspace, 15)) { set_error("%s: workspace must be 16-byte aligned", who); return result(B2H_EALIGN); }
   // [header: launch sequence + per-CTA arrival flags of the fused kernel, FIXED offset][gradient partials][loss partials][scratch]
-  partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + B2H_WS_HEADER);
-  loss_partials = partials + (size_t)nparts * stride;
-  Fp32Args a{};
+  r.partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + B2H_WS_HEADER);
+  r.loss_partials = r.partials + (size_t)plan.nparts * plan.stride;
+  ConvArgs a{};
   a.x = x; a.x_dtype = x_dtype; a.target = target; a.conf = conf; a.d_y = d_y; a.lengths = lengths; a.params = params;
-  a.packed = reinterpret_cast<const char*>(packed); a.y = pred_out; a.partials = partials; a.loss_partials = loss_partials;
-  a.B = B; a.T = T; a.loss_kind = loss_kind; a.apply_mask = 1; a.mode = mode; a.out_scale = 1.0f; a.geo = g;
+  a.packed = reinterpret_cast<const char*>(packed); a.y = pred_out; a.partials = r.partials; a.loss_partials = r.loss_partials;
+  a.B = B; a.T = T; a.loss_kind = loss_kind; a.apply_mask = 1; a.mode = mode; a.out_scale = 1.0f; a.geo = r.g;
   a.step_dev = step_dev;
   a.epoch_dev = epoch_dev;
   if (wv) a.wv = *wv;
   if (plan.kernel == B2H_KERNEL_TC_TILE) {
     if (fuse) {
-      if (nparts > B2H_WS_MAX_CTA) { set_error("%s: %d CTAs exceed the %d arrival flags of the workspace header", who, nparts, B2H_WS_MAX_CTA); return B2H_ESHAPE; }
-      fuse->enabled = 1;
-      fuse->hdr = reinterpret_cast<unsigned*>(workspace);
+      if (plan.nparts > B2H_WS_MAX_CTA) { set_error("%s: %d CTAs exceed the %d arrival flags of the workspace header", who, plan.nparts, B2H_WS_MAX_CTA); return result(B2H_ESHAPE); }
       a.fuse = *fuse;
+      a.fuse.enabled = 1;
+      a.fuse.hdr = reinterpret_cast<unsigned*>(workspace);
     }
-    return launch_tc_tile_train(a, plan.tile, stream);
+    return result(launch_tc_tile(a, plan.tile, stream));
   }
   if (plan.kernel == B2H_KERNEL_TC_WIDE_TRAIN) {
     // (the forward+criterion kernel's CTA 0 bumps the device-side step / epoch counters the Adam kernels read)
-    return launch_tc_wide_train(a, plan.wide, reinterpret_cast<unsigned char*>(workspace) + plan.scratch_off, stream);
+    return result(launch_tc_wide_train(a, plan.wide, reinterpret_cast<unsigned char*>(workspace) + plan.scratch_off, stream));
   }
-  return launch_fp32(a, plan.ffma, stream);
+  return result(launch_fp32(a, plan.ffma, stream));
 }
 
 static int train_forward_backward(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
@@ -329,12 +339,12 @@ static int train_forward_backward(const void* x, int x_dtype, const WindowView* 
                                   int precision, int64_t* step_dev, void* workspace, int64_t workspace_bytes, void* stream,
                                   const char* who) {
   if (grads_out && !loss_out) { set_error("%s: null loss_out", who); return B2H_EINVAL; }
-  Geo g; TrainPlan plan; float *partials, *loss_partials;
-  int rc = train_common(x, x_dtype, wv, target, conf, nullptr, lengths, params, packed, pred_out, B, T, n_in, C, pos_emb,
-                        loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
-                        loss_partials, who, reinterpret_cast<long long*>(step_dev));
-  if (rc || !grads_out) return rc;   // grads_out == NULL: only the fused kernel runs, partials stay in the workspace
-  return launch_reduce(partials, plan.nparts, plan.gp_layout, g, grads_out, loss_partials, loss_out, (cudaStream_t)stream, nullptr, plan.n_loss);
+  const TrainResult r = train_common(x, x_dtype, wv, target, conf, nullptr, lengths, params, packed, pred_out, B, T, n_in, C,
+                                     pos_emb, loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, who,
+                                     reinterpret_cast<long long*>(step_dev), nullptr, nullptr);
+  if (r.rc || !grads_out) return r.rc;   // grads_out == NULL: only the fused kernel runs, partials stay in the workspace
+  return launch_reduce(r.partials, r.plan.nparts, r.plan.gp_layout, r.g, grads_out, r.loss_partials, loss_out,
+                       (cudaStream_t)stream, nullptr, r.plan.n_loss);
 }
 
 extern "C" int b2h_train_forward_backward(const void* x, int x_dtype, const float* target, const float* conf,
@@ -354,7 +364,7 @@ extern "C" int b2h_train_forward_backward_windows(const void* frames, int x_dtyp
                                                   float* pred_out, int n_win, int T, int n_in, int C, int pos_emb,
                                                   int loss_kind, int precision, int64_t* step_dev, void* workspace,
                                                   int64_t workspace_bytes, void* stream) {
-  const WindowView wv{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
+  const WindowView wv = window_view(win_start, win_end, n_frames, pad_mode);
   return train_forward_backward(frames, x_dtype, &wv, target_frames, conf_frames, lengths, params, packed, grads_out, loss_out,
                                 pred_out, n_win, T, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace,
                                 workspace_bytes, stream, "b2h_train_forward_backward_windows");
@@ -381,12 +391,23 @@ extern "C" int b2h_conv_backward(const void* x, int x_dtype, const float* d_y, c
                                  float* grads_out, int B, int T, int n_in, int C, int pos_emb, int precision,
                                  void* workspace, int64_t workspace_bytes, void* stream) {
   if (!grads_out) { set_error("b2h_conv_backward: null output"); return B2H_EINVAL; }
-  Geo g; TrainPlan plan; float *partials, *loss_partials;
-  int rc = train_common(x, x_dtype, nullptr, nullptr, nullptr, d_y, nullptr, params, packed, nullptr, B, T, n_in, C, pos_emb, 0,
-                        precision, 2, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
-                        loss_partials, "b2h_conv_backward");
-  if (rc) return rc;
-  return launch_reduce(partials, plan.nparts, plan.gp_layout, g, grads_out, nullptr, nullptr, (cudaStream_t)stream, nullptr, plan.n_loss);
+  const TrainResult r = train_common(x, x_dtype, nullptr, nullptr, nullptr, d_y, nullptr, params, packed, nullptr, B, T, n_in, C,
+                                     pos_emb, 0, precision, 2, workspace, workspace_bytes, (cudaStream_t)stream,
+                                     "b2h_conv_backward", nullptr, nullptr, nullptr);
+  if (r.rc) return r.rc;
+  return launch_reduce(r.partials, r.plan.nparts, r.plan.gp_layout, r.g, grads_out, nullptr, nullptr, (cudaStream_t)stream,
+                       nullptr, r.plan.n_loss);
+}
+
+// The Adam tail of the fused tile kernel (train_common enables it and points it at the workspace header).
+static FuseAdam fuse_adam(float* params, void* packed, float* exp_avg, float* exp_avg_sq, float* loss_out, double lr,
+                          double beta1, double beta2, double eps, float grad_scale, int64_t* step_dev, const double* lr_dev) {
+  FuseAdam f{};
+  f.params = params; f.m = exp_avg; f.v = exp_avg_sq; f.packed = reinterpret_cast<char*>(packed);
+  f.lr = lr; f.beta1 = beta1; f.beta2 = beta2; f.eps = (float)eps; f.grad_scale = grad_scale;
+  f.lr_dev = lr_dev;
+  f.step_dev = reinterpret_cast<const long long*>(step_dev); f.loss_out = loss_out; f.world = 1;
+  return f;
 }
 
 static int train_step(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
@@ -396,22 +417,16 @@ static int train_step(const void* x, int x_dtype, const WindowView* wv, const fl
                       int64_t workspace_bytes, void* stream, const char* who) {
   if (!exp_avg || !exp_avg_sq || !loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
   if (step < 1 && !step_dev) { set_error("%s: step must be >= 1", who); return B2H_EINVAL; }
-  Geo g; TrainPlan plan; float *partials, *loss_partials;
-  // bf16 tile kernel + device-side step counter: ONE cooperative launch (reduction + Adam + re-pack in its tail)
-  FuseAdam fuse{};
-  fuse.params = params; fuse.m = exp_avg; fuse.v = exp_avg_sq; fuse.packed = reinterpret_cast<char*>(packed);
-  fuse.lr = lr; fuse.beta1 = beta1; fuse.beta2 = beta2; fuse.eps = (float)eps; fuse.grad_scale = 1.0f;
-  fuse.lr_dev = lr_dev;
-  fuse.step_dev = reinterpret_cast<const long long*>(step_dev); fuse.loss_out = loss_out; fuse.world = 1;
-  int rc = train_common(x, x_dtype, wv, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C, pos_emb,
-                        loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
-                        loss_partials, who, reinterpret_cast<long long*>(step_dev), nullptr,
-                        step_dev ? &fuse : nullptr);
-  if (rc) return rc;
-  if (step_dev && plan.kernel == B2H_KERNEL_TC_TILE) return B2H_OK;
-  return launch_adam(params, partials, plan.nparts, plan.gp_layout, exp_avg, exp_avg_sq, g.P, lr, beta1, beta2, eps, step < 1 ? 1 : step,
-                     reinterpret_cast<const long long*>(step_dev), lr_dev, 1.0f, packed, g,
-                     loss_partials, loss_out, (cudaStream_t)stream, plan.n_loss);
+  // tile kernel + device-side step counter: ONE cooperative launch (reduction + Adam + re-pack in its tail)
+  const FuseAdam fuse = fuse_adam(params, packed, exp_avg, exp_avg_sq, loss_out, lr, beta1, beta2, eps, 1.0f, step_dev, lr_dev);
+  const TrainResult r = train_common(x, x_dtype, wv, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C,
+                                     pos_emb, loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, who,
+                                     reinterpret_cast<long long*>(step_dev), nullptr, step_dev ? &fuse : nullptr);
+  if (r.rc) return r.rc;
+  if (step_dev && r.plan.kernel == B2H_KERNEL_TC_TILE) return B2H_OK;
+  return launch_adam(params, r.partials, r.plan.nparts, r.plan.gp_layout, exp_avg, exp_avg_sq, r.g.P, lr, beta1, beta2, eps,
+                     step < 1 ? 1 : step, reinterpret_cast<const long long*>(step_dev), lr_dev, 1.0f, packed, r.g,
+                     r.loss_partials, loss_out, (cudaStream_t)stream, r.plan.n_loss);
 }
 
 extern "C" int b2h_train_step(const void* x, int x_dtype, const float* target, const float* conf, const int32_t* lengths,
@@ -431,7 +446,7 @@ extern "C" int b2h_train_step_windows(const void* frames, int x_dtype, const flo
                                       int precision, double lr, double beta1, double beta2, double eps, int64_t step,
                                       int64_t* step_dev, const double* lr_dev, void* workspace, int64_t workspace_bytes,
                                       void* stream) {
-  const WindowView wv{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
+  const WindowView wv = window_view(win_start, win_end, n_frames, pad_mode);
   return train_step(frames, x_dtype, &wv, target_frames, conf_frames, lengths, params, packed, exp_avg, exp_avg_sq, loss_out,
                     n_win, T, n_in, C, pos_emb, loss_kind, precision, lr, beta1, beta2, eps, step, step_dev, lr_dev, workspace,
                     workspace_bytes, stream, "b2h_train_step_windows");
@@ -448,27 +463,22 @@ extern "C" int b2h_train_step_dp(const void* x, int x_dtype, const float* target
     return B2H_EINVAL;
   }
   if (world < 1 || world > 32 || rank < 0 || rank >= world) { set_error("b2h_train_step_dp: bad rank/world"); return B2H_EINVAL; }
-  Geo g; TrainPlan plan; float *partials, *loss_partials;
-  FuseAdam fuse{};
-  fuse.params = params; fuse.m = exp_avg; fuse.v = exp_avg_sq; fuse.packed = reinterpret_cast<char*>(packed);
-  fuse.lr = lr; fuse.beta1 = beta1; fuse.beta2 = beta2; fuse.eps = (float)eps; fuse.grad_scale = grad_scale;
-  fuse.lr_dev = lr_dev;
-  fuse.step_dev = reinterpret_cast<const long long*>(step_dev); fuse.loss_out = loss_out;
+  FuseAdam fuse = fuse_adam(params, packed, exp_avg, exp_avg_sq, loss_out, lr, beta1, beta2, eps, grad_scale, step_dev, lr_dev);
   fuse.peer_bufs = reinterpret_cast<const float* const*>(peer_bufs_dev); fuse.sym_grads = sym_grads;
   fuse.mc_buf = reinterpret_cast<unsigned long long*>(multicast_buf);
   fuse.epoch_dev = reinterpret_cast<const long long*>(epoch_dev); fuse.rank = rank; fuse.world = world;
-  int rc = train_common(x, x_dtype, nullptr, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C, pos_emb,
-                        loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, g, plan, partials,
-                        loss_partials, "b2h_train_step_dp", reinterpret_cast<long long*>(step_dev),
-                        reinterpret_cast<long long*>(epoch_dev), &fuse);
-  if (rc) return rc;
-  if (plan.kernel == B2H_KERNEL_TC_TILE) return B2H_OK;    // everything happened inside the one cooperative launch
-  rc = launch_reduce(partials, plan.nparts, plan.gp_layout, g, sym_grads, loss_partials, loss_out, (cudaStream_t)stream,
-                     reinterpret_cast<const long long*>(epoch_dev), plan.n_loss);
-  if (rc) return rc;
-  return launch_adam_dp(params, reinterpret_cast<const float* const*>(peer_bufs_dev), rank, world, exp_avg, exp_avg_sq, g.P, lr,
+  const TrainResult r = train_common(x, x_dtype, nullptr, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C,
+                                     pos_emb, loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream,
+                                     "b2h_train_step_dp", reinterpret_cast<long long*>(step_dev),
+                                     reinterpret_cast<long long*>(epoch_dev), &fuse);
+  if (r.rc) return r.rc;
+  if (r.plan.kernel == B2H_KERNEL_TC_TILE) return B2H_OK;    // everything happened inside the one cooperative launch
+  if (int rc = launch_reduce(r.partials, r.plan.nparts, r.plan.gp_layout, r.g, sym_grads, r.loss_partials, loss_out,
+                             (cudaStream_t)stream, reinterpret_cast<const long long*>(epoch_dev), r.plan.n_loss))
+    return rc;
+  return launch_adam_dp(params, reinterpret_cast<const float* const*>(peer_bufs_dev), rank, world, exp_avg, exp_avg_sq, r.g.P, lr,
                         beta1, beta2, eps, reinterpret_cast<const long long*>(step_dev),
-                        reinterpret_cast<const long long*>(epoch_dev), lr_dev, grad_scale, packed, g, (cudaStream_t)stream);
+                        reinterpret_cast<const long long*>(epoch_dev), lr_dev, grad_scale, packed, r.g, (cudaStream_t)stream);
 }
 
 extern "C" int b2h_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, double lr,

@@ -303,8 +303,10 @@ struct FfmaPlan {
 };
 FfmaPlan plan_ffma(const Geo& g, int B, int T, bool train);
 
-// ---- kernel argument blocks and launchers shared between translation units ----
-struct Fp32Args {
+// ---- the request block of every forward / training launch, and the launchers ----
+// Filled once by the C-ABI entry points; each launcher copies what its kernel needs into that kernel's own parameter
+// block.  Its layout is also conv_fp32_kernel's parameter block.
+struct ConvArgs {
   const void* x; int x_dtype;
   const float* target; const float* conf; const float* d_y; const int32_t* lengths;
   const float* params; const char* packed;
@@ -317,32 +319,18 @@ struct Fp32Args {
   int B, T, loss_kind, apply_mask, mode;   // mode 0 = forward, 1 = train (loss inside), 2 = backward of given d_y
   float out_scale;
   Geo geo;
-  WindowView wv;            // tensor-core training only: win_start set = x / target / conf are frame streams, B = windows
+  WindowView wv;            // tensor-core kernels only: win_start set = x (and target / conf) are frame streams, B = windows
 };
-int launch_fp32(Fp32Args& p, const FfmaPlan& plan, cudaStream_t stream);
-
-struct TcFwdArgs {
-  const void* x; int x_dtype;
-  const float* params; const char* packed; const int32_t* lengths;
-  float* y;
-  int B, T, G, NT, RBUF, apply_mask;
-  float out_scale;
-  Geo geo;
-  WindowView wv;            // win_start set: x is a frame stream and B = the number of windows
-};
-int launch_tc_fwd(TcFwdArgs& p, const RowspacePlan& plan, cudaStream_t stream);
-// wide training (32 < conv_channels <= 256, bf16 mode): forward+criterion / dgrad chain / split-K wgrad over scratch dumps
-int launch_tc_wide_train(const Fp32Args& a, const WidePlan& plan, unsigned char* scratch, cudaStream_t stream);
-int launch_tc_wide_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int B, int T, int apply_mask, float out_scale, const Geo& g, const WidePlan& plan, cudaStream_t stream,
-                       const WindowView* wv);
+int launch_fp32(const ConvArgs& a, const FfmaPlan& plan, cudaStream_t stream);
+int launch_tc_fwd(const ConvArgs& a, const RowspacePlan& plan, cudaStream_t stream);
+// forward (mode 0) or training; the tile kernel takes its launch batch and window length from the plan
+int launch_tc_tile(const ConvArgs& a, const TilePlan& plan, cudaStream_t stream);
+int launch_tc_wide_fwd(const ConvArgs& a, const WidePlan& plan, cudaStream_t stream);
+// wide training (32 < conv_channels <= 256, bf16 mode): forward+criterion / dgrad chain / split-K wgrad over the per-tile
+// operand dumps in `scratch` (workspace past the partials, TrainPlan::scratch_off)
+int launch_tc_wide_train(const ConvArgs& a, const WidePlan& plan, unsigned char* scratch, cudaStream_t stream);
 int launch_tc_probe(const void* a, const void* b, float* out, int n, int ksteps, int shift, int variant, cudaStream_t stream);
 int tc_status_and_clear();
-
-// the tile launchers take the launch batch and window length from the plan
-int launch_tc_tile_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int apply_mask, float out_scale, const Geo& g, const TilePlan& plan, cudaStream_t stream, const WindowView* wv);
-int launch_tc_tile_train(const Fp32Args& a, const TilePlan& plan, cudaStream_t stream);
 
 void set_debug_timing(long long* p);
 int launch_tc_bench(long long* out, int M, int N, int reps, int nacc, int mn_major, cudaStream_t stream);

@@ -122,7 +122,7 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
 }
 
 template <bool TRAIN>
-__global__ void __launch_bounds__(kThreads) conv_fp32_kernel(Fp32Args p) {
+__global__ void __launch_bounds__(kThreads) conv_fp32_kernel(ConvArgs p) {
   extern __shared__ __align__(16) float smem[];
   __shared__ float red[kWarps];
   const Geo& g = p.geo;
@@ -316,12 +316,12 @@ FfmaPlan plan_ffma(const Geo& g, int B, int T, bool train) {
   return p;
 }
 
-int launch_fp32(Fp32Args& p, const FfmaPlan& plan, cudaStream_t stream) {
+int launch_fp32(const ConvArgs& a, const FfmaPlan& plan, cudaStream_t stream) {
   const void* fn = plan.train ? reinterpret_cast<const void*>(conv_fp32_kernel<true>) : reinterpret_cast<const void*>(conv_fp32_kernel<false>);
   // opt in to > 48 KB of dynamic shared memory
   if (int rc = ensure_dyn_smem(fn, plan.smem)) return rc;
-  if (plan.train) conv_fp32_kernel<true><<<plan.grid, kThreads, plan.smem, stream>>>(p);
-  else conv_fp32_kernel<false><<<plan.grid, kThreads, plan.smem, stream>>>(p);
+  if (plan.train) conv_fp32_kernel<true><<<plan.grid, kThreads, plan.smem, stream>>>(a);
+  else conv_fp32_kernel<false><<<plan.grid, kThreads, plan.smem, stream>>>(a);
   count_launch();
   return check_launch(plan.train ? "conv_fp32_kernel<train>" : "conv_fp32_kernel<fwd>");
 }

@@ -107,6 +107,16 @@ __global__ void __launch_bounds__(128) tc_probe_kernel(const __nv_bfloat16* __re
 constexpr int kTcThreads = 128;
 constexpr int kTileCols = 64;   // TMEM column stride between the accumulators of consecutive tiles
 
+struct TcFwdArgs {
+  const void* x; int x_dtype;
+  const float* params; const char* packed; const int32_t* lengths;
+  float* y;
+  int B, T, G, NT, RBUF, apply_mask;
+  float out_scale;
+  Geo geo;
+  WindowView wv;            // win_start set: x is a frame stream and B = the number of windows
+};
+
 __device__ __forceinline__ void store_row_bf16(unsigned char* buf, int chunk_stride, int row, int c0, const float* v8) {
   uint4 q;
   q.x = pack_bf16x2(v8[0], v8[1]); q.y = pack_bf16x2(v8[2], v8[3]);
@@ -309,7 +319,10 @@ RowspacePlan plan_rowspace(const Geo& g, int B, int T) {
   return p;
 }
 
-int launch_tc_fwd(TcFwdArgs& p, const RowspacePlan& plan, cudaStream_t stream) {
+int launch_tc_fwd(const ConvArgs& a, const RowspacePlan& plan, cudaStream_t stream) {
+  TcFwdArgs p{};
+  p.x = a.x; p.x_dtype = a.x_dtype; p.params = a.params; p.packed = a.packed; p.lengths = a.lengths;
+  p.y = a.y; p.B = a.B; p.T = a.T; p.apply_mask = a.apply_mask; p.out_scale = a.out_scale; p.geo = a.geo; p.wv = a.wv;
   p.G = plan.G; p.NT = plan.NT; p.RBUF = plan.RBUF;
   if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_fwd_kernel), plan.smem)) return rc;
   conv_tc_fwd_kernel<<<plan.grid, kTcThreads, plan.smem, stream>>>(p);

@@ -1096,7 +1096,19 @@ TilePlan plan_tile(const Geo& g, int B, int T, bool train, bool split) {
   return p;
 }
 
-static int launch_tc_tile(TcTileArgs& p, const TilePlan& plan, cudaStream_t stream) {
+static long long* g_dbg_timing = nullptr;
+void set_debug_timing(long long* p) { g_dbg_timing = p; }
+
+// Forward (plan.train false) and training: in the forward, the fields only training sets stay zero in `a`, and the
+// sub-window fields (n_sub = 1, T_orig = T) select whole windows exactly as zero would.
+int launch_tc_tile(const ConvArgs& a, const TilePlan& plan, cudaStream_t stream) {
+  TcTileArgs p{};
+  p.x = a.x; p.x_dtype = a.x_dtype; p.target = a.target; p.conf = a.conf; p.d_y = a.d_y; p.lengths = a.lengths;
+  p.params = a.params; p.packed = a.packed; p.y = a.y; p.partials = a.partials; p.loss_partials = a.loss_partials;
+  p.step_dev = a.step_dev; p.epoch_dev = a.epoch_dev; p.dbg = g_dbg_timing; p.fuse = a.fuse;
+  p.win_start = a.wv.win_start; p.win_end = a.wv.win_end; p.n_frames = a.wv.n_frames; p.pad_mode = a.wv.pad_mode;
+  p.T_orig = a.T; p.n_sub = plan.n_sub; p.loss_B = a.B;
+  p.loss_kind = a.loss_kind; p.apply_mask = a.apply_mask; p.mode = a.mode; p.out_scale = a.out_scale; p.geo = a.geo;
   p.B = plan.B; p.T = plan.T;
   p.nhalf = plan.nhalf; p.MB = plan.MB; p.NT = plan.NT; p.HR = plan.HR; p.gh = plan.gh; p.n_tiles = plan.n_tiles;
   const bool train = plan.train, split = plan.split;
@@ -1148,32 +1160,6 @@ static int launch_tc_tile(TcTileArgs& p, const TilePlan& plan, cudaStream_t stre
   if (le != cudaSuccess) { cudaGetLastError(); set_error("tile kernel launch: %s", cudaGetErrorString(le)); return B2H_ECUDA; }
   count_launch();
   return check_launch(train ? "conv_tc_tile_kernel<train>" : "conv_tc_tile_kernel<fwd>");
-}
-
-static long long* g_dbg_timing = nullptr;
-void set_debug_timing(long long* p) { g_dbg_timing = p; }
-
-int launch_tc_tile_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int apply_mask, float out_scale, const Geo& g, const TilePlan& plan, cudaStream_t stream, const WindowView* wv) {
-  TcTileArgs p{};
-  p.x = x; p.x_dtype = x_dtype; p.params = params; p.packed = packed; p.lengths = lengths; p.y = y;
-  p.apply_mask = apply_mask; p.mode = 0; p.out_scale = out_scale; p.geo = g;
-  if (wv) { p.win_start = wv->win_start; p.win_end = wv->win_end; p.n_frames = wv->n_frames; p.pad_mode = wv->pad_mode; }
-  p.dbg = g_dbg_timing;
-  return launch_tc_tile(p, plan, stream);
-}
-
-int launch_tc_tile_train(const Fp32Args& a, const TilePlan& plan, cudaStream_t stream) {
-  TcTileArgs p{};
-  p.x = a.x; p.x_dtype = a.x_dtype; p.target = a.target; p.conf = a.conf; p.d_y = a.d_y; p.lengths = a.lengths;
-  p.params = a.params; p.packed = a.packed; p.y = a.y; p.partials = a.partials; p.loss_partials = a.loss_partials;
-  p.step_dev = a.step_dev; p.epoch_dev = a.epoch_dev; p.loss_kind = a.loss_kind; p.apply_mask = 1; p.mode = a.mode;
-  p.out_scale = 1.0f; p.geo = a.geo;
-  p.fuse = a.fuse;
-  p.dbg = g_dbg_timing;
-  p.loss_B = a.B; p.T_orig = a.T; p.n_sub = plan.n_sub;
-  p.win_start = a.wv.win_start; p.win_end = a.wv.win_end; p.n_frames = a.wv.n_frames; p.pad_mode = a.wv.pad_mode;
-  return launch_tc_tile(p, plan, stream);
 }
 
 }  // namespace b2h

@@ -785,52 +785,46 @@ static int wide_weight_map(const char* base, int64_t bytes, CUtensorMap* out, in
   return B2H_OK;
 }
 
-static void wide_common(WideArgs& p, const Geo& g, const WidePlan& plan, int B, int T) {
-  p.B = B; p.T = T; p.geo = g;
+// The forward's and the training forward's arguments (mode 0: the training fields stay zero in `a`), with the four
+// forward conv stages.
+static WideArgs wide_args(const ConvArgs& a, const WidePlan& plan) {
+  const Geo& g = a.geo;
+  WideArgs p{};
+  p.x = a.x; p.x_dtype = a.x_dtype; p.params = a.params; p.packed = a.packed; p.lengths = a.lengths; p.y = a.y;
+  p.apply_mask = a.apply_mask; p.out_scale = a.out_scale;
+  p.target = a.target; p.conf = a.conf; p.d_y = a.d_y; p.loss_kind = a.loss_kind; p.train_mode = a.mode;
+  p.loss_partials = a.loss_partials; p.step_dev = a.step_dev; p.epoch_dev = a.epoch_dev;
+  p.wv = a.wv;
+  p.B = a.B; p.T = a.T; p.geo = g;
   p.dbg = g_dbg_timing;
   p.gh = plan.gh; p.n_tiles = plan.n_tiles; p.a_bytes = plan.a_bytes; p.nstage = plan.nstage;
   const WideScratch ws = wide_scratch(g);
   p.tile_bytes = ws.tile_bytes;
   for (int l = 0; l < 4; ++l) { p.act_off[l] = ws.act_off[l]; p.dz_off[l] = ws.dz_off[l]; }
-}
-
-static void wide_forward_stages(WideArgs& p, const Geo& g) {
   p.n_stages = 4;
   for (int l = 0; l < 4; ++l) { p.st[l].KS = g.kp[l] >> 4; p.st[l].N = g.np_[l]; p.st[l].row0 = (int)((g.tf_off[l] - g.tf_off[0]) >> 7); p.st[l].layer = l; }
+  return p;
 }
 
-int launch_tc_wide_fwd(const void* x, int x_dtype, const float* params, const char* packed, const int32_t* lengths, float* y,
-                       int B, int T, int apply_mask, float out_scale, const Geo& g, const WidePlan& plan, cudaStream_t stream,
-                       const WindowView* wv) {
-  WideArgs p{};
-  p.x = x; p.x_dtype = x_dtype; p.params = params; p.packed = packed; p.lengths = lengths; p.y = y;
-  p.apply_mask = apply_mask; p.out_scale = out_scale;
-  if (wv) p.wv = *wv;
-  wide_common(p, g, plan, B, T);
-  wide_forward_stages(p, g);
+int launch_tc_wide_fwd(const ConvArgs& a, const WidePlan& plan, cudaStream_t stream) {
+  const Geo& g = a.geo;
+  const WideArgs p = wide_args(a, plan);
   if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_wide_kernel<0>), plan.smem)) return rc;
   CUtensorMap wmap;
-  if (int rc = wide_weight_map(packed + g.tf_off[0], g.td_off[0] - g.tf_off[0], &wmap)) return rc;
+  if (int rc = wide_weight_map(a.packed + g.tf_off[0], g.td_off[0] - g.tf_off[0], &wmap)) return rc;
   conv_tc_wide_kernel<0><<<plan.grid, kWideThreads, plan.smem, stream>>>(p, wmap);
   count_launch();
   return check_launch("conv_tc_wide_kernel<fwd>");
 }
 
 // ---- wide training: forward+criterion (saves layer inputs), dgrad chain, split-K wgrad; the caller reduces + applies Adam ----
-int launch_tc_wide_train(const Fp32Args& a, const WidePlan& plan, unsigned char* scratch, cudaStream_t stream) {
+int launch_tc_wide_train(const ConvArgs& a, const WidePlan& plan, unsigned char* scratch, cudaStream_t stream) {
   const Geo& g = a.geo;
-  WideArgs p{};
-  p.x = a.x; p.x_dtype = a.x_dtype; p.params = a.params; p.packed = a.packed; p.lengths = a.lengths; p.y = a.y;
-  p.apply_mask = 1; p.out_scale = 1.0f;
-  p.target = a.target; p.conf = a.conf; p.d_y = a.d_y; p.loss_kind = a.loss_kind; p.train_mode = a.mode;
-  p.scratch = scratch; p.loss_partials = a.loss_partials;
-  p.step_dev = a.step_dev; p.epoch_dev = a.epoch_dev;
-  p.wv = a.wv;
-  wide_common(p, g, plan, a.B, a.T);
+  WideArgs p = wide_args(a, plan);
+  p.scratch = scratch;
   const size_t smem = plan.smem;
   const int grid = plan.grid;
   // ---- 1. forward + criterion ----
-  wide_forward_stages(p, g);
   auto* fwd = p.wv.win_start ? conv_tc_wide_kernel<1, true> : conv_tc_wide_kernel<1>;
   if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fwd), smem)) return rc;
   CUtensorMap fmap, bmap;

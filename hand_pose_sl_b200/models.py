@@ -190,23 +190,28 @@ class ConvModel(nn.Module):
         return self._workspace
 
     # ------------------------------------------------------------------ kernels
-    def _check_input(self, inp):
-        _lib.require_device(inp, "ConvModel input")
-        _lib.require_sm100(inp.device)
-        if inp.dim() != 4:
-            raise RuntimeError(f"ConvModel expects (B, T, K, 2), got {tuple(inp.shape)}")
-        B, T, K, D = inp.shape
-        if K * D != self.n_in:
+    def _check_input(self, x, T=None):
+        """The model-level checks of every entry point, on windows x (B, T, K, 2) or, with T given, on a frame stream
+        x (F, K, 2) read as windows of T frames: a CUDA tensor on an sm_100 device and on the model's device, K * 2 =
+        n_in channels, float32 / bfloat16, and the pos_emb window length.  Returns (B or F, T)."""
+        stream = T is not None
+        _lib.require_device(x, "frame stream" if stream else "ConvModel input")
+        _lib.require_sm100(x.device)
+        if x.dim() != (3 if stream else 4):
+            raise RuntimeError(f"ConvModel expects {'a frame stream (F, K, 2)' if stream else '(B, T, K, 2)'}, "
+                               f"got {tuple(x.shape)}")
+        if x.shape[-2] * x.shape[-1] != self.n_in:
             # the reference fails inside conv1 with a channel-mismatch RuntimeError (SURVEY.md §0.4)
-            raise RuntimeError(f"expected input with {self.n_in} channels (K*2), got {K * D} channels instead")
+            raise RuntimeError(f"expected input with {self.n_in} channels (K*2), got {x.shape[-2] * x.shape[-1]} channels instead")
+        T = T if stream else x.shape[1]
         if self.pos_emb is not None and T != self.pos_emb.max_len and not self.pos_emb_any_length:
             # torch.cat in LinearPositionalEmbedding.forward fails unless T == max_len (HandPoseModels.py:82)
             raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {self.pos_emb.max_len}, got {T}")
-        if inp.dtype not in (torch.float32, torch.bfloat16):
-            raise RuntimeError(f"ConvModel input must be float32 or bfloat16, got {inp.dtype}")
-        if self._flat.device != inp.device:
-            raise RuntimeError(f"input is on {inp.device} but the model is on {self._flat.device}")
-        return B, T
+        if x.dtype not in (torch.float32, torch.bfloat16):
+            raise RuntimeError(f"ConvModel input must be float32 or bfloat16, got {x.dtype}")
+        if self._flat.device != x.device:
+            raise RuntimeError(f"input is on {x.device} but the model is on {self._flat.device}")
+        return x.shape[0], T
 
     def _forward_impl(self, inp, lengths=None, out_scale=1.0):
         B, T = self._check_input(inp)
@@ -214,14 +219,11 @@ class ConvModel(nn.Module):
         n_in, C, pe = self._geometry()
         packed = self.packed_weights()
         y = torch.empty((B, T, 21, 2), dtype=torch.float32, device=x.device)
-        lib = _lib.load()
-        len32 = None
-        if lengths is not None:
-            len32 = torch.as_tensor(lengths).to(device=x.device, dtype=torch.int32, non_blocking=True).contiguous()
-        _lib.check(lib.b2h_conv_forward(_lib.ptr(x), _lib.DT_BF16 if x.dtype == torch.bfloat16 else _lib.DT_F32,
-                                        _lib.ptr(self._flat), _lib.ptr(packed), _lib.ptr(len32), _lib.ptr(y), B, T,
-                                        n_in, C, pe, _lib.PRECISIONS[self.precision], 1 if len32 is not None else 0,
-                                        float(out_scale), _lib.stream_ptr(x.device)))
+        len32 = None if lengths is None else _lib.lengths_i32(lengths, x.device, B)
+        _lib.check(_lib.load().b2h_conv_forward(_lib.ptr(x), _lib.dtype_code(x.dtype), _lib.ptr(self._flat), _lib.ptr(packed),
+                                                _lib.ptr(len32), _lib.ptr(y), B, T, n_in, C, pe,
+                                                _lib.PRECISIONS[self.precision], 1 if len32 is not None else 0,
+                                                float(out_scale), _lib.stream_ptr(x.device)))
         return y
 
     def _backward_impl(self, x, grad_y):
@@ -233,7 +235,7 @@ class ConvModel(nn.Module):
         ws = self.workspace(B, T)
         grads = torch.empty_like(self._flat)
         lib = _lib.load()
-        _lib.check(lib.b2h_conv_backward(_lib.ptr(xc), _lib.DT_BF16 if xc.dtype == torch.bfloat16 else _lib.DT_F32,
+        _lib.check(lib.b2h_conv_backward(_lib.ptr(xc), _lib.dtype_code(xc.dtype),
                                          _lib.ptr(gy), _lib.ptr(self._flat), _lib.ptr(packed), _lib.ptr(grads), B, T,
                                          n_in, C, pe, _lib.PRECISIONS[self.precision], _lib.ptr(ws), ws.numel(),
                                          _lib.stream_ptr(xc.device)))
@@ -277,25 +279,17 @@ class ConvModel(nn.Module):
         windows; other shapes raise B2HError."""
         if not self._is_flat():
             self._flatten()
-        _lib.require_device(frames, "frames")
-        _lib.require_sm100(frames.device)
-        if frames.dim() != 3 or frames.shape[1] * frames.shape[2] != self.n_in:
-            raise RuntimeError(f"expected frames (F, {self.n_in // 2}, 2), got {tuple(frames.shape)}")
-        if frames.dtype not in (torch.float32, torch.bfloat16):
-            raise RuntimeError(f"frames must be float32 or bfloat16, got {frames.dtype}")
-        if self.pos_emb is not None and T != self.pos_emb.max_len and not self.pos_emb_any_length:
-            raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {self.pos_emb.max_len}, got {T}")
+        F, T = self._check_input(frames, T)
         dev = frames.device
         x = frames.contiguous()
         ws = torch.as_tensor(win_start).to(device=dev, dtype=torch.int64).contiguous()
         we = None if win_end is None else torch.as_tensor(win_end).to(device=dev, dtype=torch.int64).contiguous()
         W = ws.numel()
-        pm = {"repeat_first": _lib.PAD_REPEAT_FIRST, "zeros": _lib.PAD_ZEROS}[pad_mode]
-        len32 = None if lengths is None else torch.as_tensor(lengths).to(device=dev, dtype=torch.int32).contiguous()
+        len32 = None if lengths is None else _lib.lengths_i32(lengths, dev, W)
         n_in, C, pe = self._geometry()
         y = out if out is not None else torch.empty((W, T, 21, 2), dtype=torch.float32, device=dev)
         _lib.check(_lib.load().b2h_conv_forward_windows(
-            _lib.ptr(x), _lib.DT_BF16 if x.dtype == torch.bfloat16 else _lib.DT_F32, x.shape[0], _lib.ptr(ws), _lib.ptr(we), pm,
+            _lib.ptr(x), _lib.dtype_code(x.dtype), F, _lib.ptr(ws), _lib.ptr(we), _lib.PAD_MODES[pad_mode],
             _lib.ptr(self._flat), _lib.ptr(self.packed_weights()), _lib.ptr(len32), _lib.ptr(y), W, T, n_in, C, pe,
             _lib.PRECISIONS[self.precision], 1 if len32 is not None else 0, 1.0 if denormalize is None else float(denormalize),
             _lib.stream_ptr(dev)))

@@ -14,7 +14,7 @@ import torch.distributed as dist
 from . import _lib
 from .models import ConvModel
 from .runner import _StepBuffers
-from .steps import FusedAdam
+from .steps import FusedAdam, _dense_inputs
 
 
 def shard_range(n_items: int, rank: int, world: int):
@@ -123,30 +123,25 @@ class DataParallelTrainer(_StepBuffers):
                     raise
                 import warnings
                 warnings.warn(f"symmetric-memory gradient exchange unavailable ({type(e).__name__}: {e}); using NCCL all-reduce")
+        tail = None                # exchange="nccl": step() below runs forward_backward + all-reduce + the Adam kernel
+        if self.exchange == "p2p":  # b2h_train_step_dp's arguments after eps
+            tail = (_lib.ptr(self.step_dev), _lib.ptr(self.epoch_dev), _lib.ptr(self.lr_dev), _lib.ptr(self.sym),
+                    _lib.ptr(self.peer_ptrs), (self.mc_ptr or None), self.rank, self.world,
+                    grad_scale_for(self.loss_name, self.world), _lib.ptr(self.ws), self.ws.numel())
+        self._bind(self.lib.b2h_train_step_dp, lambda batch: _dense_inputs(model, batch, loss), tail)
 
     def step(self, slot=0, to_host=False):
+        if self.exchange == "p2p":
+            return super().step(slot, to_host)
         self._sync_host_state()
         m, g = self.model, self.opt.param_groups[0]
         n_in, C, pe = m._geometry()
         b1, b2 = g["betas"]
-        conf = None if self.conf is None else self.conf[slot]
         sp = _lib.stream_ptr(self.dev)
         loss = (self.loss_host if to_host else self.loss)[slot:slot + 1]
-        if self.exchange == "p2p":
-            _lib.check(self.lib.b2h_train_step_dp(
-                _lib.ptr(self.x[slot]), self._x_dt(), _lib.ptr(self.target[slot]), _lib.ptr(conf), _lib.ptr(self.lengths[slot]),
-                _lib.ptr(m._flat), _lib.ptr(self.packed), _lib.ptr(self.state["m"]), _lib.ptr(self.state["v"]),
-                _lib.ptr(loss), self.B, self.T, n_in, C, pe, self.kind, _lib.PRECISIONS[m.precision],
-                float(g["lr"]), b1, b2, g["eps"], _lib.ptr(self.step_dev), _lib.ptr(self.epoch_dev), _lib.ptr(self.lr_dev),
-                _lib.ptr(self.sym), _lib.ptr(self.peer_ptrs), (self.mc_ptr or None), self.rank, self.world,
-                grad_scale_for(self.loss_name, self.world), _lib.ptr(self.ws), self.ws.numel(), sp))
-            self._advance(1)
-            return loss[0]
         _lib.check(self.lib.b2h_train_forward_backward(
-            _lib.ptr(self.x[slot]), self._x_dt(), _lib.ptr(self.target[slot]), _lib.ptr(conf), _lib.ptr(self.lengths[slot]),
-            _lib.ptr(m._flat), _lib.ptr(self.packed), _lib.ptr(self.grads), _lib.ptr(loss), None,
-            self.B, self.T, n_in, C, pe, self.kind, _lib.PRECISIONS[m.precision], _lib.ptr(self.step_dev),
-            _lib.ptr(self.ws), self.ws.numel(), sp))
+            *self._inputs[slot], _lib.ptr(m._flat), _lib.ptr(self.packed), _lib.ptr(self.grads), _lib.ptr(loss), None,
+            *self._shape, _lib.ptr(self.step_dev), _lib.ptr(self.ws), self.ws.numel(), sp))
         allreduce_flat(self.grads, self.group)
         _lib.check(self.lib.b2h_adam_step(
             _lib.ptr(m._flat), _lib.ptr(self.grads), _lib.ptr(self.state["m"]), _lib.ptr(self.state["v"]), m._flat.numel(),

@@ -16,11 +16,16 @@ import torch
 
 from . import _lib
 from .models import ConvModel
-from .steps import FusedAdam
+from .steps import FusedAdam, _dense_inputs, _view_inputs
 
 
 def _align(n, a=256):
     return (n + a - 1) // a * a
+
+
+def _check_x_dtype(model, x_dtype):
+    if x_dtype == torch.bfloat16 and model.precision != "bf16":
+        raise ValueError("bf16 inputs are only bit-identical to fp32 inputs in bf16 mode")
 
 
 class _StepBuffers:
@@ -30,8 +35,7 @@ class _StepBuffers:
         x_dtype = x_dtype or torch.float32
         if x_dtype not in (torch.float32, torch.bfloat16):
             raise ValueError("x_dtype must be torch.float32 or torch.bfloat16")
-        if x_dtype == torch.bfloat16 and model.precision != "bf16":
-            raise ValueError("bf16 inputs are only bit-identical to fp32 inputs in bf16 mode")
+        _check_x_dtype(model, x_dtype)
         self.x_dtype = x_dtype
         K = model.n_in // 2
         conf = _lib.LOSSES[loss] == _lib.LOSS_CONFL1
@@ -129,7 +133,33 @@ class _StepBuffers:
         self.packed = self.model.packed_weights()        # cheap version compare; re-packs after load_state_dict etc.
 
     def _x_dt(self):
-        return _lib.DT_BF16 if self.x_dtype == torch.bfloat16 else _lib.DT_F32
+        return _lib.dtype_code(self.x_dtype)
+
+    def _bind(self, entry, decode, tail=None):
+        """Pre-binds the C arguments of step(): `decode(batch)` (steps._dense_inputs / _view_inputs) gives the leading
+        arguments of a slot's batch dict {key: slot tensor}; `tail` the arguments after eps (default: b2h_train_step's)."""
+        self._entry = entry
+        self._decoded = [decode({key: getattr(self, name)[s] for name, key, _ in self._fields})[0] for s in range(self.n_slots)]
+        self._inputs = [_lib.ptrs(args) for args in self._decoded]
+        n_in, C, pe = self.model._geometry()
+        self._shape = (self.B, self.T, n_in, C, pe, self.kind, _lib.PRECISIONS[self.model.precision])
+        self._tail = tail or (0, _lib.ptr(self.step_dev), _lib.ptr(self.lr_dev), _lib.ptr(self.ws), self.ws.numel())
+
+    def _model_args(self, loss):
+        """The model and optimiser arguments shared by every training entry point, from params through eps, read fresh."""
+        g = self.opt.param_groups[0]
+        b1, b2 = g["betas"]
+        return (_lib.ptr(self.model._flat), _lib.ptr(self.packed), _lib.ptr(self.state["m"]), _lib.ptr(self.state["v"]),
+                _lib.ptr(loss), *self._shape, float(g["lr"]), b1, b2, g["eps"])
+
+    def step(self, slot=0, to_host=False):
+        """Enqueue one training step on the batch in slot `slot` on the current stream; returns the 0-dim loss tensor: on
+        the device, or (to_host=True) the pinned host word the kernel writes -- valid once the stream has been synchronised."""
+        self._sync_host_state()
+        loss = (self.loss_host if to_host else self.loss)[slot:slot + 1]
+        _lib.check(self._entry(*self._inputs[slot], *self._model_args(loss), *self._tail, _lib.stream_ptr(self.dev)))
+        self._advance(1)
+        return loss[0]
 
     def check_status(self):
         """Raise if a device-side wait gave up (grid barrier, MMA completion, data-parallel peer wait).  Synchronises."""
@@ -186,24 +216,7 @@ class TrainStepRunner(_StepBuffers):
 
     def __init__(self, model: ConvModel, optimizer: FusedAdam, B: int, T: int, loss: str = "L1", n_slots: int = 1, x_dtype=None):
         self._init_buffers(model, optimizer, B, T, loss, n_slots, x_dtype)
-
-    def step(self, slot=0, to_host=False):
-        """Enqueue one training step on the current stream; returns the 0-dim loss tensor: on the device, or (to_host=True)
-        the pinned host word the kernel writes -- valid once the stream has been synchronised."""
-        self._sync_host_state()
-        m, g = self.model, self.opt.param_groups[0]
-        n_in, C, pe = m._geometry()
-        b1, b2 = g["betas"]
-        conf = None if self.conf is None else self.conf[slot]
-        loss = (self.loss_host if to_host else self.loss)[slot:slot + 1]
-        _lib.check(self.lib.b2h_train_step(
-            _lib.ptr(self.x[slot]), self._x_dt(), _lib.ptr(self.target[slot]), _lib.ptr(conf), _lib.ptr(self.lengths[slot]),
-            _lib.ptr(m._flat), _lib.ptr(self.packed), _lib.ptr(self.state["m"]), _lib.ptr(self.state["v"]),
-            _lib.ptr(loss), self.B, self.T, n_in, C, pe, self.kind, _lib.PRECISIONS[m.precision],
-            float(g["lr"]), b1, b2, g["eps"], 0, _lib.ptr(self.step_dev), _lib.ptr(self.lr_dev), _lib.ptr(self.ws),
-            self.ws.numel(), _lib.stream_ptr(self.dev)))
-        self._advance(1)
-        return loss[0]
+        self._bind(self.lib.b2h_train_step, lambda batch: _dense_inputs(model, batch, loss))
 
 
 class WindowTrainStepRunner(_StepBuffers):
@@ -216,35 +229,14 @@ class WindowTrainStepRunner(_StepBuffers):
 
     def __init__(self, model: ConvModel, optimizer: FusedAdam, streams, B: int, T: int, loss: str = "L1", n_slots: int = 1,
                  pad_mode: str = "repeat_first"):
-        x = streams["input_kp"]
-        if x.dtype == torch.bfloat16 and model.precision != "bf16":
-            raise ValueError("bf16 inputs are only bit-identical to fp32 inputs in bf16 mode")
+        _check_x_dtype(model, streams["input_kp"].dtype)
         self._init_common(model, optimizer, B, T, loss, n_slots, (
             ("win_start", "win_start", torch.int64, (B,)), ("win_end", "win_end", torch.int64, (B,)),
             ("lengths", "n_frames", torch.int32, (B,))))
-        from .steps import _window_args
-        # stream arguments, validated and converted once: (x, x_dtype, target, conf, n_frames)
-        self._streams = _window_args(model, streams, self.win_start[0], T, self.lengths[0], None, pad_mode, loss)[0][:5]
-        self.pad_mode = {"repeat_first": _lib.PAD_REPEAT_FIRST, "zeros": _lib.PAD_ZEROS}[pad_mode]
-        self.win_end.fill_(self._streams[4])
+        self._bind(self.lib.b2h_train_step_windows, lambda crops: _view_inputs(
+            model, streams, crops["win_start"], T, crops["n_frames"], crops["win_end"], pad_mode, loss))
+        self.win_end.fill_(streams["input_kp"].shape[0])
         self.lengths.fill_(T)
-
-    def step(self, slot=0, to_host=False):
-        """Enqueue one training step over the crops in slot `slot`; returns the loss as TrainStepRunner.step does."""
-        self._sync_host_state()
-        m, g = self.model, self.opt.param_groups[0]
-        n_in, C, pe = m._geometry()
-        b1, b2 = g["betas"]
-        x, dt, tgt, conf, F = self._streams
-        loss = (self.loss_host if to_host else self.loss)[slot:slot + 1]
-        _lib.check(self.lib.b2h_train_step_windows(
-            _lib.ptr(x), dt, _lib.ptr(tgt), _lib.ptr(conf), F, _lib.ptr(self.win_start[slot]), _lib.ptr(self.win_end[slot]),
-            self.pad_mode, _lib.ptr(self.lengths[slot]), _lib.ptr(m._flat), _lib.ptr(self.packed), _lib.ptr(self.state["m"]),
-            _lib.ptr(self.state["v"]), _lib.ptr(loss), self.B, self.T, n_in, C, pe, self.kind, _lib.PRECISIONS[m.precision],
-            float(g["lr"]), b1, b2, g["eps"], 0, _lib.ptr(self.step_dev), _lib.ptr(self.lr_dev), _lib.ptr(self.ws),
-            self.ws.numel(), _lib.stream_ptr(self.dev)))
-        self._advance(1)
-        return loss[0]
 
 
 def pipelined_steps(runner, batches, status_every=0, copy_streams=1):
@@ -354,7 +346,7 @@ class ForwardRunner:
             self.packed = m.packed_weights()             # follows load_state_dict / optimiser updates (version compare)
         n_in, C, pe = m._geometry()
         _lib.check(self.lib.b2h_conv_forward(
-            _lib.ptr(self.x[slot]), _lib.DT_BF16 if self.x.dtype == torch.bfloat16 else _lib.DT_F32, _lib.ptr(m._flat),
+            _lib.ptr(self.x[slot]), _lib.dtype_code(self.x.dtype), _lib.ptr(m._flat),
             _lib.ptr(self.packed), None, _lib.ptr(self.y[slot]), self.B, self.T, n_in, C, pe, _lib.PRECISIONS[m.precision], 0,
             self.out_scale, _lib.stream_ptr(self.dev)))
         return self.y[slot]

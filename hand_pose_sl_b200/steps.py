@@ -11,14 +11,6 @@ from . import _lib
 from .models import ConvModel, owner_of
 
 
-def _lengths_i32(lengths, device, B):
-    """`lengths` is `batch["n_frames"]`, a CPU int64 tensor in the reference (traintest.py:91)."""
-    t = torch.as_tensor(lengths)
-    if t.numel() != B:
-        raise RuntimeError(f"lengths has {t.numel()} entries for a batch of {B}")
-    return t.to(device=device, dtype=torch.int32, non_blocking=True).contiguous()
-
-
 class _MaskOutput(torch.autograd.Function):
     @staticmethod
     def forward(ctx, output, len32):
@@ -46,7 +38,7 @@ def mask_output(output, lengths):
     _lib.require_device(output, "mask_output input")
     if output.dtype != torch.float32 or not output.is_contiguous():
         raise RuntimeError("mask_output expects a contiguous float32 tensor (ConvModel's output is)")
-    len32 = _lengths_i32(lengths, output.device, output.shape[0])
+    len32 = _lib.lengths_i32(lengths, output.device, output.shape[0])
     return _MaskOutput.apply(output, len32)
 
 
@@ -90,7 +82,7 @@ class maskedPoseL1(nn.Module):
 
     def forward(self, prediction, target, lengths):
         _criterion_checks(prediction, target)
-        len32 = _lengths_i32(lengths, prediction.device, prediction.shape[0])
+        len32 = _lib.lengths_i32(lengths, prediction.device, prediction.shape[0])
         return _PoseL1.apply(prediction, target, len32, None, _lib.LOSS_L1)
 
 
@@ -99,7 +91,7 @@ class poderatedPoseL1(nn.Module):
 
     def forward(self, prediction, target, lengths, scores):
         _criterion_checks(prediction, target)
-        len32 = _lengths_i32(lengths, prediction.device, prediction.shape[0])
+        len32 = _lib.lengths_i32(lengths, prediction.device, prediction.shape[0])
         return _PoseL1.apply(prediction, target, len32, scores, _lib.LOSS_CONFL1)
 
 
@@ -245,87 +237,28 @@ class FusedAdam(torch.optim.Optimizer):
         return loss
 
 
-def fused_train_step(model: ConvModel, batch, optimizer: FusedAdam, loss="L1"):
-    """The body of the reference's hot loop, traintest.py:94-121, as two launches:
-    forward + mask_output + criterion + backward (one kernel), cross-CTA gradient reduction + Adam +
-    weight re-pack (one kernel).  `batch` is the reference's batch dict (input_kp, target_kp, n_frames
-    [, target_conf]) with tensors already on the model's device.  Returns the loss as a 0-dim device
-    tensor (no host sync; call .item() only when you log it, cf. traintest.py:123)."""
+def _dense_inputs(model: ConvModel, batch, loss):
+    """The C arguments in front of `params` of the dense training entry points (x, x_dtype, target, conf, lengths; tensors
+    stay tensors), and the batch size, window length and device."""
     x = batch["input_kp"]
     B, T = model._check_input(x)
-    x = x.contiguous()
     dev = x.device
     tgt = batch["target_kp"].to(device=dev, dtype=torch.float32).contiguous()
-    kind = _lib.LOSSES[loss]
-    conf = batch["target_conf"].to(device=dev, dtype=torch.float32).contiguous() if kind == _lib.LOSS_CONFL1 else None
-    len32 = _lengths_i32(batch["n_frames"], dev, B)
-    group = optimizer.param_groups[0]
-    if optimizer._owner(group) is not model:
-        raise RuntimeError("fused_train_step needs FusedAdam(model.parameters()) over exactly this model")
-    st = optimizer._group_state(0, group, model)
-    st["step"] += 1
-    n_in, C, pe = model._geometry()
-    packed = model.packed_weights()
-    ws = model.workspace(B, T)
-    flat = model.flat_parameters()
-    loss_out = torch.empty((), dtype=torch.float32, device=dev)
-    b1, b2 = group["betas"]
-    lib = _lib.load()
-    _lib.check(lib.b2h_train_step(_lib.ptr(x), _lib.DT_BF16 if x.dtype == torch.bfloat16 else _lib.DT_F32, _lib.ptr(tgt),
-                                  _lib.ptr(conf), _lib.ptr(len32), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(st["m"]),
-                                  _lib.ptr(st["v"]), _lib.ptr(loss_out), B, T, n_in, C, pe, kind,
-                                  _lib.PRECISIONS[model.precision], float(group["lr"]), b1, b2, group["eps"], st["step"],
-                                  None, None, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
-    model.packed_weights(fresh_from_kernel=True)
-    st["step_t"].fill_(float(st["step"]))
-    return loss_out
+    conf = batch["target_conf"].to(device=dev, dtype=torch.float32).contiguous() if _lib.LOSSES[loss] == _lib.LOSS_CONFL1 else None
+    return (x.contiguous(), _lib.dtype_code(x.dtype), tgt, conf, _lib.lengths_i32(batch["n_frames"], dev, B)), B, T, dev
 
 
-def forward_backward(model: ConvModel, batch, loss="L1", want_pred=False):
-    """traintest.py:94-120 without the optimiser: returns (loss 0-dim tensor, flat gradient tensor
-    [, masked prediction]).  Used by the data-parallel trainer (all-reduce between this and Adam)."""
-    x = batch["input_kp"]
-    B, T = model._check_input(x)
-    x = x.contiguous()
-    dev = x.device
-    tgt = batch["target_kp"].to(device=dev, dtype=torch.float32).contiguous()
-    kind = _lib.LOSSES[loss]
-    conf = batch["target_conf"].to(device=dev, dtype=torch.float32).contiguous() if kind == _lib.LOSS_CONFL1 else None
-    len32 = _lengths_i32(batch["n_frames"], dev, B)
-    n_in, C, pe = model._geometry()
-    packed = model.packed_weights()
-    ws = model.workspace(B, T)
-    flat = model.flat_parameters()
-    grads = torch.empty_like(flat)
-    loss_out = torch.empty((), dtype=torch.float32, device=dev)
-    pred = torch.empty((B, T, 21, 2), dtype=torch.float32, device=dev) if want_pred else None
-    lib = _lib.load()
-    _lib.check(lib.b2h_train_forward_backward(_lib.ptr(x), _lib.DT_BF16 if x.dtype == torch.bfloat16 else _lib.DT_F32,
-                                              _lib.ptr(tgt), _lib.ptr(conf), _lib.ptr(len32), _lib.ptr(flat),
-                                              _lib.ptr(packed), _lib.ptr(grads), _lib.ptr(loss_out), _lib.ptr(pred), B, T,
-                                              n_in, C, pe, kind, _lib.PRECISIONS[model.precision], None,
-                                              _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
-    return (loss_out, grads, pred) if want_pred else (loss_out, grads)
-
-
-def _window_args(model: ConvModel, streams, win_start, T, lengths, win_end, pad_mode, loss):
-    """Device arguments of the *_windows calls: the three frame streams, the crop list and the lengths."""
+def _view_inputs(model: ConvModel, streams, win_start, T, lengths, win_end, pad_mode, loss):
+    """`_dense_inputs` of the *_windows entry points: (frames, x_dtype, target_frames, conf_frames, n_frames, win_start,
+    win_end, pad_mode, lengths), and the number of windows, T and the device."""
     x = streams["input_kp"]
-    _lib.require_device(x, "input_kp stream")
-    _lib.require_sm100(x.device)
-    if x.dim() != 3 or x.shape[1] * x.shape[2] != model.n_in:
-        raise RuntimeError(f"expected an input_kp stream (F, {model.n_in // 2}, 2), got {tuple(x.shape)}")
-    if x.dtype not in (torch.float32, torch.bfloat16):
-        raise RuntimeError(f"the input_kp stream must be float32 or bfloat16, got {x.dtype}")
-    if model.pos_emb is not None and T != model.pos_emb.max_len and not model.pos_emb_any_length:
-        raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {model.pos_emb.max_len}, got {T}")
-    dev, F = x.device, x.shape[0]
-    kind = _lib.LOSSES[loss]
+    F, T = model._check_input(x, T)
+    dev = x.device
     tgt = streams["target_kp"].to(device=dev, dtype=torch.float32).contiguous()
     if tgt.numel() != F * 42:
         raise RuntimeError(f"target_kp stream has {tgt.numel()} values for {F} frames (expected (F, 21, 2))")
     conf = None
-    if kind == _lib.LOSS_CONFL1:
+    if _lib.LOSSES[loss] == _lib.LOSS_CONFL1:
         conf = streams["target_conf"].to(device=dev, dtype=torch.float32).contiguous()
         if conf.numel() != F * 21:
             raise RuntimeError(f"target_conf stream has {conf.numel()} values for {F} frames (expected (F, 21))")
@@ -334,15 +267,63 @@ def _window_args(model: ConvModel, streams, win_start, T, lengths, win_end, pad_
     we = None if win_end is None else torch.as_tensor(win_end).to(device=dev, dtype=torch.int64).contiguous()
     if we is not None and we.numel() != W:
         raise RuntimeError("win_end must have one entry per window")
-    pm = {"repeat_first": _lib.PAD_REPEAT_FIRST, "zeros": _lib.PAD_ZEROS}[pad_mode]
-    len32 = _lengths_i32(lengths, dev, W)
-    dt = _lib.DT_BF16 if x.dtype == torch.bfloat16 else _lib.DT_F32
-    return (x.contiguous(), dt, tgt, conf, F, ws, we, pm, len32), W, kind, dev
+    return (x.contiguous(), _lib.dtype_code(x.dtype), tgt, conf, F, ws, we, _lib.PAD_MODES[pad_mode],
+            _lib.lengths_i32(lengths, dev, W)), W, T, dev
 
 
-def _window_ptrs(args):
-    x, dt, tgt, conf, F, ws, we, pm, len32 = args
-    return (_lib.ptr(x), dt, _lib.ptr(tgt), _lib.ptr(conf), F, _lib.ptr(ws), _lib.ptr(we), pm, _lib.ptr(len32))
+def _train_step(entry, model, optimizer, inputs, loss, who):
+    """forward + criterion + backward + reduction + Adam + re-pack through C entry point `entry` (b2h_train_step[_windows])."""
+    args, W, T, dev = inputs
+    group = optimizer.param_groups[0]
+    if optimizer._owner(group) is not model:
+        raise RuntimeError(f"{who} needs FusedAdam(model.parameters()) over exactly this model")
+    st = optimizer._group_state(0, group, model)
+    st["step"] += 1
+    n_in, C, pe = model._geometry()
+    packed = model.packed_weights()
+    ws = model.workspace(W, T)
+    flat = model.flat_parameters()
+    loss_out = torch.empty((), dtype=torch.float32, device=dev)
+    b1, b2 = group["betas"]
+    _lib.check(getattr(_lib.load(), entry)(
+        *_lib.ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(st["m"]), _lib.ptr(st["v"]), _lib.ptr(loss_out), W, T,
+        n_in, C, pe, _lib.LOSSES[loss], _lib.PRECISIONS[model.precision], float(group["lr"]), b1, b2, group["eps"], st["step"],
+        None, None, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
+    model.packed_weights(fresh_from_kernel=True)
+    st["step_t"].fill_(float(st["step"]))
+    return loss_out
+
+
+def _forward_backward(entry, model, inputs, loss, want_pred):
+    """forward + criterion + backward and the gradient reduction through C entry point `entry`
+    (b2h_train_forward_backward[_windows])."""
+    args, W, T, dev = inputs
+    n_in, C, pe = model._geometry()
+    packed = model.packed_weights()
+    ws = model.workspace(W, T)
+    flat = model.flat_parameters()
+    grads = torch.empty_like(flat)
+    loss_out = torch.empty((), dtype=torch.float32, device=dev)
+    pred = torch.empty((W, T, 21, 2), dtype=torch.float32, device=dev) if want_pred else None
+    _lib.check(getattr(_lib.load(), entry)(
+        *_lib.ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(grads), _lib.ptr(loss_out), _lib.ptr(pred), W, T,
+        n_in, C, pe, _lib.LOSSES[loss], _lib.PRECISIONS[model.precision], None, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
+    return (loss_out, grads, pred) if want_pred else (loss_out, grads)
+
+
+def fused_train_step(model: ConvModel, batch, optimizer: FusedAdam, loss="L1"):
+    """The body of the reference's hot loop, traintest.py:94-121, as two launches:
+    forward + mask_output + criterion + backward (one kernel), cross-CTA gradient reduction + Adam +
+    weight re-pack (one kernel).  `batch` is the reference's batch dict (input_kp, target_kp, n_frames
+    [, target_conf]) with tensors already on the model's device.  Returns the loss as a 0-dim device
+    tensor (no host sync; call .item() only when you log it, cf. traintest.py:123)."""
+    return _train_step("b2h_train_step", model, optimizer, _dense_inputs(model, batch, loss), loss, "fused_train_step")
+
+
+def forward_backward(model: ConvModel, batch, loss="L1", want_pred=False):
+    """traintest.py:94-120 without the optimiser: returns (loss 0-dim tensor, flat gradient tensor
+    [, masked prediction]).  Used by the data-parallel trainer (all-reduce between this and Adam)."""
+    return _forward_backward("b2h_train_forward_backward", model, _dense_inputs(model, batch, loss), loss, want_pred)
 
 
 def fused_train_step_windows(model: ConvModel, streams, win_start, T, lengths, optimizer: FusedAdam, win_end=None,
@@ -352,43 +333,16 @@ def fused_train_step_windows(model: ConvModel, streams, win_start, T, lengths, o
     [win_start[w], win_start[w] + T) cut at win_end[w] (default F) and padded by the dataset's rule, in all three streams.
     `lengths` = the windows' n_frames.  Bit-identical to `fused_train_step` on the windows K0 materialises; served where
     the tensor cores train (b2h_kernel_choice tile / wide), B2HError otherwise.  Returns the 0-dim device loss."""
-    args, W, kind, dev = _window_args(model, streams, win_start, T, lengths, win_end, pad_mode, loss)
-    group = optimizer.param_groups[0]
-    if optimizer._owner(group) is not model:
-        raise RuntimeError("fused_train_step_windows needs FusedAdam(model.parameters()) over exactly this model")
-    st = optimizer._group_state(0, group, model)
-    st["step"] += 1
-    n_in, C, pe = model._geometry()
-    packed = model.packed_weights()
-    ws = model.workspace(W, T)
-    flat = model.flat_parameters()
-    loss_out = torch.empty((), dtype=torch.float32, device=dev)
-    b1, b2 = group["betas"]
-    _lib.check(_lib.load().b2h_train_step_windows(
-        *_window_ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(st["m"]), _lib.ptr(st["v"]), _lib.ptr(loss_out), W, T,
-        n_in, C, pe, kind, _lib.PRECISIONS[model.precision], float(group["lr"]), b1, b2, group["eps"], st["step"], None, None,
-        _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
-    model.packed_weights(fresh_from_kernel=True)
-    st["step_t"].fill_(float(st["step"]))
-    return loss_out
+    inputs = _view_inputs(model, streams, win_start, T, lengths, win_end, pad_mode, loss)
+    return _train_step("b2h_train_step_windows", model, optimizer, inputs, loss, "fused_train_step_windows")
 
 
 def forward_backward_windows(model: ConvModel, streams, win_start, T, lengths, win_end=None, pad_mode="repeat_first",
                              loss="L1", want_pred=False):
     """`forward_backward` on window views of frame streams (see `fused_train_step_windows`): returns (loss, flat gradients
     [, masked prediction (W, T, 21, 2)]), bit-identical to `forward_backward` on the materialised windows."""
-    args, W, kind, dev = _window_args(model, streams, win_start, T, lengths, win_end, pad_mode, loss)
-    n_in, C, pe = model._geometry()
-    packed = model.packed_weights()
-    ws = model.workspace(W, T)
-    flat = model.flat_parameters()
-    grads = torch.empty_like(flat)
-    loss_out = torch.empty((), dtype=torch.float32, device=dev)
-    pred = torch.empty((W, T, 21, 2), dtype=torch.float32, device=dev) if want_pred else None
-    _lib.check(_lib.load().b2h_train_forward_backward_windows(
-        *_window_ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(grads), _lib.ptr(loss_out), _lib.ptr(pred), W, T,
-        n_in, C, pe, kind, _lib.PRECISIONS[model.precision], None, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
-    return (loss_out, grads, pred) if want_pred else (loss_out, grads)
+    inputs = _view_inputs(model, streams, win_start, T, lengths, win_end, pad_mode, loss)
+    return _forward_backward("b2h_train_forward_backward_windows", model, inputs, loss, want_pred)
 
 
 @torch.no_grad()

@@ -120,6 +120,119 @@ def test_kernel_choice_pins_the_tensor_core_paths():
     assert rc == -2 and "no training kernel for conv_channels=256" in _lib.last_error()
 
 
+# Argument names of the entry points whose checks the table below pins, in C-ABI order (include/b2h.h).
+_ABI_ARGS = {
+    "b2h_conv_forward": "x x_dtype params packed lengths y B T n_in C pos_emb precision apply_mask out_scale stream",
+    "b2h_conv_forward_windows": "x x_dtype n_frames win_start win_end pad_mode params packed lengths y B T n_in C pos_emb "
+                                "precision apply_mask out_scale stream",
+    "b2h_train_forward_backward": "x x_dtype target conf lengths params packed grads loss pred B T n_in C pos_emb loss_kind "
+                                  "precision step_dev ws ws_bytes stream",
+    "b2h_train_forward_backward_windows": "x x_dtype target conf n_frames win_start win_end pad_mode lengths params packed "
+                                          "grads loss pred B T n_in C pos_emb loss_kind precision step_dev ws ws_bytes stream",
+    "b2h_conv_backward": "x x_dtype d_y params packed grads B T n_in C pos_emb precision ws ws_bytes stream",
+    "b2h_train_step": "x x_dtype target conf lengths params packed m v loss B T n_in C pos_emb loss_kind precision lr b1 b2 "
+                      "eps step step_dev lr_dev ws ws_bytes stream",
+    "b2h_train_step_windows": "x x_dtype target conf n_frames win_start win_end pad_mode lengths params packed m v loss B T "
+                              "n_in C pos_emb loss_kind precision lr b1 b2 eps step step_dev lr_dev ws ws_bytes stream",
+    "b2h_train_step_dp": "x x_dtype target conf lengths params packed m v loss B T n_in C pos_emb loss_kind precision lr b1 "
+                         "b2 eps step_dev epoch_dev lr_dev sym peers mc rank world grad_scale ws ws_bytes stream",
+}
+_FWD = ("b2h_conv_forward", "b2h_conv_forward_windows")
+_VIEWS = ("b2h_conv_forward_windows", "b2h_train_forward_backward_windows", "b2h_train_step_windows")
+_TRAIN = tuple(n for n in _ABI_ARGS if n not in _FWD)
+_LOSS = tuple(n for n in _TRAIN if n != "b2h_conv_backward")      # the entry points that compute the criterion
+_ALL = tuple(_ABI_ARGS)
+OK, EINVAL, ESHAPE, EALIGN, EWORKSPACE = 0, -1, -2, -3, -6
+
+# (entry points, overrides of the defaults, expected code, fragment of b2h_last_error()).  Every case is refused (or, for
+# B == 0 in the forward, accepted) before anything is launched, so host buffers stand in for device memory.  Cases that
+# are bad in two ways pin the order of the checks.
+_ARG_CASES = [
+    (_ALL, dict(x=None), EINVAL, "null pointer"),
+    (_ALL, dict(params=None), EINVAL, "null pointer"),
+    (_ALL, dict(packed=None), EINVAL, "null pointer"),
+    (_FWD, dict(y=None), EINVAL, "null pointer"),
+    (_TRAIN, dict(ws=None), EINVAL, "null pointer"),
+    (_VIEWS, dict(win_start=None), EINVAL, "null pointer"),
+    (("b2h_train_step", "b2h_train_step_windows", "b2h_train_step_dp"), dict(m=None), EINVAL, "null pointer"),
+    (("b2h_train_step_dp",), dict(step_dev=None), EINVAL, "null pointer"),
+    (("b2h_train_step_dp",), dict(peers=None), EINVAL, "null pointer"),
+    (("b2h_train_step_dp",), dict(rank=2), EINVAL, "bad rank/world"),
+    (("b2h_conv_backward",), dict(grads=None), EINVAL, "null output"),
+    (("b2h_conv_backward",), dict(d_y=None), EINVAL, "null d_y"),
+    (("b2h_train_forward_backward", "b2h_train_forward_backward_windows"), dict(loss=None), EINVAL, "null loss_out"),
+    (("b2h_train_step", "b2h_train_step_windows"), dict(step=0), EINVAL, "step must be >= 1"),
+    (_ALL, dict(x_dtype=5), EINVAL, "bad x_dtype 5"),
+    (_ALL, dict(x_dtype=5, C=100000), EINVAL, "bad x_dtype 5"),
+    (_VIEWS, dict(pad_mode=7), EINVAL, "bad pad_mode 7"),
+    (_VIEWS, dict(pad_mode=7, x_dtype=5), EINVAL, "bad x_dtype 5"),
+    (_ALL, dict(C=100000), ESHAPE, "unsupported geometry n_in=24 C=100000"),
+    (_ALL, dict(n_in=0, B=-1), ESHAPE, "unsupported geometry"),
+    (_ALL, dict(B=-1), ESHAPE, "bad B=-1 T=64"),
+    (_ALL, dict(T=0), ESHAPE, "bad B=2 T=0"),
+    (_TRAIN, dict(B=0), ESHAPE, "bad B=0 T=64"),
+    (_VIEWS, dict(n_frames=-1), ESHAPE, "bad B=2 T=64"),
+    (_FWD, dict(B=0, x=1), OK, None),                     # an empty forward succeeds before the alignment test
+    (_FWD, dict(apply_mask=1, lengths=None), EINVAL, "apply_mask needs lengths"),
+    (_LOSS, dict(target=None), EINVAL, "null target/lengths"),
+    (_LOSS, dict(lengths=None), EINVAL, "null target/lengths"),
+    (_LOSS, dict(loss_kind=3), EINVAL, "bad loss_kind 3"),
+    (_LOSS, dict(loss_kind=1), EINVAL, "confL1 needs scores"),
+    (_ALL, dict(x=8), EALIGN, "16-byte aligned"),
+    (_FWD, dict(y=8), EALIGN, "16-byte aligned"),
+    (_ALL, dict(packed=8), EALIGN, "16-byte aligned"),
+    (tuple(n for n in _LOSS if n not in _VIEWS), dict(target=8), EALIGN, "x, target and packed must be 16-byte aligned"),
+    (tuple(n for n in _TRAIN if n in _VIEWS), dict(target=4), EALIGN, "target_frames 8-byte"),
+    (tuple(n for n in _TRAIN if n in _VIEWS), dict(target=8, conf=4, loss_kind=1, C=256, T=300), ESHAPE,
+     "window views are trained on the tensor cores"),
+    (("b2h_train_forward_backward_windows",), dict(conf=2, loss_kind=1), EALIGN, "conf_frames 4-byte"),
+    (_FWD, dict(x=8, y=None), EINVAL, "null pointer"),
+    (_ALL, dict(precision=7), EINVAL, "bad precision 7"),
+    (_FWD, dict(precision=7, x=8), EALIGN, "16-byte aligned"),              # forward: alignment before precision
+    (_TRAIN, dict(precision=7, x=8), EINVAL, "bad precision 7"),            # training: precision before alignment
+    (_LOSS, dict(precision=7, loss_kind=3), EINVAL, "bad precision 7"),
+    (("b2h_conv_forward",), dict(C=256, T=300), ESHAPE, "no kernel for C=256, T=300, precision=1"),
+    (("b2h_conv_forward_windows",), dict(C=256, T=300), ESHAPE, "window views are served in bf16 mode"),
+    (("b2h_conv_forward_windows",), dict(C=64, precision=2), ESHAPE, "materialise the windows"),
+    (tuple(n for n in _TRAIN if n not in _VIEWS), dict(C=256, T=300), ESHAPE, "no training kernel for conv_channels=256, T=300"),
+    (tuple(n for n in _TRAIN if n in _VIEWS), dict(C=256, T=300), ESHAPE, "window views are trained on the tensor cores"),
+    (tuple(n for n in _TRAIN if n in _VIEWS), dict(C=30, precision=2), ESHAPE, "precision=2"),
+    (_TRAIN, dict(ws_bytes=64), EWORKSPACE, "workspace 64 B <"),
+    (_TRAIN, dict(ws=8), EALIGN, "workspace must be 16-byte aligned"),
+    (_TRAIN, dict(ws=8, ws_bytes=64), EWORKSPACE, "workspace 64 B <"),
+]
+
+
+def _abi_call(lib, keep, name, over):
+    """Calls entry point `name` with a well-formed bf16 C=30 T=64 batch of 2 (host buffers), changed by `over`.  A pointer
+    override is None or a byte offset into its aligned buffer."""
+    assert set(over) <= set(_ABI_ARGS[name].split()), (name, over)
+    v = ctypes.c_void_p
+    bufs = {}
+
+    def buf(key, off=0):
+        if key not in bufs:
+            keep.append(np.zeros(1 << 16, dtype=np.uint8))
+            a = keep[-1].ctypes.data
+            bufs[key] = a + (-a) % 256
+        return v(bufs[key] + off)
+
+    scalars = dict(x_dtype=_lib.DT_BF16, n_frames=100, pad_mode=_lib.PAD_REPEAT_FIRST, B=2, T=64, n_in=24, C=30, pos_emb=0,
+                   precision=_lib.BF16, apply_mask=0, out_scale=1.0, loss_kind=_lib.LOSS_L1, ws_bytes=1 << 30, lr=1e-3,
+                   b1=0.9, b2=0.999, eps=1e-8, step=1, rank=0, world=2, grad_scale=0.5)
+    nulls = ("conf", "win_end", "stream", "mc", "step_dev", "lr_dev", "pred") if name != "b2h_train_step_dp" else \
+        ("conf", "win_end", "stream", "mc", "lr_dev")
+    args = []
+    for a in _ABI_ARGS[name].split():
+        if a in scalars:
+            args.append(over.get(a, scalars[a]))
+        elif a in over:
+            args.append(None if over[a] is None else buf(a, over[a]))
+        else:
+            args.append(None if a in nulls else buf(a))
+    return getattr(lib, name)(*args)
+
+
 def test_null_and_bad_arguments_return_error_codes():
     lib = _lib.load()
     assert lib.b2h_conv_forward(None, 0, None, None, None, None, 1, 64, 24, 30, 0, 0, 0, 1.0, None) == -1
@@ -128,6 +241,15 @@ def test_null_and_bad_arguments_return_error_codes():
                               None, None, None) == -1
     assert lib.b2h_pack_weights(None, None, 24, 30, 0, None) == -1
     assert lib.b2h_adam_step(None, None, None, None, 10, 1e-3, 0.9, 0.999, 1e-8, 1, None, None, 1.0, None, 0, 0, 0, None) == -1
+    # the argument checks of every forward / training entry point: code and message, case by case
+    keep = []
+    for names, over, code, fragment in _ARG_CASES:
+        for name in names:
+            rc = _abi_call(lib, keep, name, over)
+            assert rc == code, (name, over, rc, _lib.last_error())
+            if fragment is not None:
+                msg = _lib.last_error()
+                assert msg.startswith(name + ":") and fragment in msg, (name, over, msg)
 
 
 def test_convmodel_is_a_drop_in_on_the_host_side():
