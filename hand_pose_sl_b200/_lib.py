@@ -84,7 +84,6 @@ _SIGNATURES = {
     "b2h_tc_probe": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "b2h_tc_status": (c_int, []),
     "b2h_debug_timing": (None, [c_void_p]),
-    "b2h_tc_bench": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "b2h_launch_count": (c_int64, []),
 }
 

@@ -534,11 +534,6 @@ extern "C" int b2h_tc_probe(const void* a_bf16, const void* b_bf16, float* out, 
   return launch_tc_probe(a_bf16, b_bf16, out, n, ksteps, shift, variant, (cudaStream_t)stream);
 }
 
-extern "C" int b2h_tc_bench(void* out_i64x2, int M, int N, int reps, int nacc, int mn_major, void* stream) {
-  if (!out_i64x2) { set_error("b2h_tc_bench: null pointer"); return B2H_EINVAL; }
-  return launch_tc_bench(reinterpret_cast<long long*>(out_i64x2), M, N, reps, nacc, mn_major, (cudaStream_t)stream);
-}
-
 extern "C" void b2h_debug_timing(void* dev_i64x1024) { set_debug_timing(reinterpret_cast<long long*>(dev_i64x1024)); }
 
 extern "C" int b2h_tc_status(void) { return tc_status_and_clear(); }

@@ -333,7 +333,6 @@ int launch_tc_probe(const void* a, const void* b, float* out, int n, int ksteps,
 int tc_status_and_clear();
 
 void set_debug_timing(long long* p);
-int launch_tc_bench(long long* out, int M, int N, int reps, int nacc, int mn_major, cudaStream_t stream);
 int launch_format_prediction(const float* pred, float* out, int64_t rows, int mode, cudaStream_t stream);
 int launch_pos_emb_concat(const float* inp, float* out, int B, int Cc, int T, int max_len, cudaStream_t stream);
 int launch_pack(const float* params, void* packed, const Geo& g, cudaStream_t stream);

@@ -358,130 +358,5 @@ int tc_status_and_clear() {
 
 }  // namespace b2h
 
-namespace b2h {
-using namespace tc;
-// ------------------------------------------------------------------------------------------------
-// Microbenchmark (bring-up aid): cycles per tcgen05.mma for a given shape, issued back to back by one
-// thread, rotating over `nacc` accumulators.  out[0] = cycles from first issue to completion,
-// out[1] = cycles spent in the issue loop alone.
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) tc_bench_kernel(long long* out, int M, int N, int reps, int nacc, int mn_major, int rows) {
-  extern __shared__ __align__(128) unsigned char bsm[];
-  __shared__ __align__(8) uint64_t bar;
-  __shared__ uint32_t tmem_slot;
-  const int tid = threadIdx.x;
-  const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
-  __shared__ __align__(8) uint64_t bar2;
-  const bool rnd = (mn_major >> 4) & 1;          // non-zero operand bits (values in [1, 2)): data-dependent pacing / power
-  for (int i = tid; i < 64 * 1024 / 16; i += 128) {
-    uint32_t h = (uint32_t)i * 2654435761u + blockIdx.x * 40503u;
-    const uint32_t w0 = rnd ? (0x3F803F80u | (h & 0x007F007Fu)) : 0u, w1 = rnd ? (0x3F803F80u | ((h >> 7) & 0x007F007Fu)) : 0u;
-    reinterpret_cast<uint4*>(bsm)[i] = make_uint4(w0, w1, w0 ^ (rnd ? 0x00150015u : 0u), w1 ^ (rnd ? 0x002A002Au : 0u));
-  }
-  if (warp == 0) tmem_alloc(&tmem_slot, 512);
-  fence_proxy_async_smem();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tbase = tmem_slot;
-  long long t0 = 0, t1 = 0;
-  const int nissue = nacc >> 8;          // upper bits: number of issuing warps (each with its own accumulators)
-  nacc &= 255;
-  if (tid == 0) { mbar_init(&bar, nissue > 0 ? nissue : 1); mbar_init(&bar2, 1u << 20); fence_barrier_init(); }
-  __syncthreads();
-  if (warp < (nissue > 0 ? nissue : 1)) {
-    if (elect_one()) {
-      const uint32_t a0 = smem_u32(bsm), b0 = smem_u32(bsm + 32 * 1024);
-      const uint32_t CH = rows * 16;
-      const int vary = (mn_major >> 2) & 1;    // walk A rows and B blocks like a streamed-weight main loop
-      const int commit2 = (mn_major >> 3) & 1; // tcgen05.commit after every second MMA (ring-stage release)
-      const int sw128 = (mn_major >> 1) & 1;   // timing-only variant: 128-byte-swizzle K-major descriptors (SBO = 1024 B)
-      mn_major &= 1;
-      uint64_t ad = mn_major ? make_smem_desc(a0, 128, CH) : make_smem_desc(a0, CH, 128);
-      uint64_t bd = mn_major ? make_smem_desc(b0, 128, CH) : make_smem_desc(b0, CH, 128);
-      if ((mn_major >> 5) & 1) bd = make_smem_desc(b0, 4096, 128);   // B chunk stride = even multiple of 128 B
-      if ((mn_major >> 6) & 1) ad = make_smem_desc(a0, 4096, 128);   // A chunk stride likewise
-      if ((mn_major >> 7) & 1) bd = make_smem_desc(b0, 4096 + 128, 128);
-      if (sw128) {
-        ad = make_smem_desc(a0, 16, 1024) | (2ull << 61);
-        bd = make_smem_desc(b0, 16, 1024) | (2ull << 61);
-      }
-      const uint32_t idesc = make_idesc_bf16(M, N, mn_major, mn_major);
-      const uint32_t dbase = tbase + warp * nacc * N;
-      t0 = clock64();
-      if (!vary && !commit2) {
-        for (int r = 0; r < reps; ++r) umma_bf16(dbase + (r % nacc) * N, ad + (uint64_t)(sw128 ? 2 * (r & 3) : (r & 3)), bd, idesc, 1);
-      } else {
-        for (int r = 0; r < reps; ++r) {
-          const uint64_t aoff = vary ? (uint64_t)(((r >> 1) * 7) & 63) + (uint64_t)((r & 1) * 128) : (uint64_t)(r & 3);
-          const uint64_t boff = vary ? (uint64_t)(((r >> 1) & 3) * 256) : 0ull;      // 4-KB steps
-          umma_bf16(dbase + (r % nacc) * N, ad + aoff, bd + boff, idesc, 1);
-          if (commit2 && (r & 1)) umma_commit(&bar2);
-        }
-      }
-      t1 = clock64();
-      umma_commit(&bar);
-    }
-    __syncwarp();
-  }
-  mbar_wait(&bar, 0, 40);
-  const long long t2 = clock64();
-  if (warp == 0 && t0 != 0 && blockIdx.x == 0) { out[0] = t2 - t0; out[1] = t1 - t0; }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tbase, 512);
-}
-
-// Bring-up microbenchmark (M == 1 in b2h_tc_bench): steady-state global(L2) -> shared throughput of 1-D bulk copies.
-// A ring of `depth` 8-KB stages is kept full by one warp; every stage is fetched as 8192/copy_bytes copies issued by
-// consecutive lanes.  out[0] = cycles, out[1] = bytes moved (CTA 0).
-__device__ unsigned char g_tma_src[1 << 20];
-__global__ void __launch_bounds__(32) tma_bench_kernel(long long* out, int copy_bytes, int rounds, int depth) {
-  extern __shared__ __align__(128) unsigned char bsm[];
-  __shared__ __align__(8) uint64_t full[16];
-  const int lane = threadIdx.x;
-  if (lane == 0) { for (int s = 0; s < depth; ++s) mbar_init(&full[s], 1); fence_barrier_init(); }
-  __syncwarp();
-  const int ncopy = 8192 / copy_bytes;
-  auto issue = [&](int s, int blk) {
-    if (lane == 0) mbar_arrive_expect_tx(&full[s], 8192);
-    __syncwarp();
-    for (int c = lane; c < ncopy; c += 32)
-      bulk_g2s(bsm + s * 8192 + c * copy_bytes, g_tma_src + (size_t)(blk & 127) * 8192 + c * copy_bytes, copy_bytes, &full[s]);
-  };
-  int blk = 0;
-  for (int s = 0; s < depth; ++s) issue(s, blk++);
-  const long long t0 = clock64();
-  for (int r = 0; r < rounds; ++r)
-    for (int s = 0; s < depth; ++s) {
-      mbar_wait(&full[s], r & 1, 41);
-      __syncwarp();
-      issue(s, blk++);
-    }
-  const long long t1 = clock64();
-  for (int s = 0; s < depth; ++s) mbar_wait(&full[s], rounds & 1, 42);
-  if (lane == 0 && blockIdx.x == 0) { out[0] = t1 - t0; out[1] = (long long)rounds * depth * 8192; }
-}
-
-int launch_tc_bench(long long* out, int M, int N, int reps, int nacc, int mn_major, cudaStream_t stream) {
-  if (M == 1) {   // TMA bulk-copy throughput: N = bytes per copy, reps = rounds, nacc = ring depth, mn_major = CTAs
-    if (N < 16 || N > 8192 || (8192 % N) || nacc < 1 || nacc > 16 || reps < 1 || mn_major < 1) { set_error("b2h_tc_bench(tma): bad arguments"); return B2H_EINVAL; }
-    if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(tma_bench_kernel), 128 * 1024)) return rc;
-    tma_bench_kernel<<<mn_major, 32, 128 * 1024, stream>>>(out, N, reps, nacc);
-    count_launch();
-    return check_launch("tma_bench_kernel");
-  }
-  if ((M != 64 && M != 128) || N < 8 || N > 256 || (N % (M == 64 ? 8 : 16)) || reps < 1 || (nacc & 255) < 1 || (nacc & 255) * N * ((nacc >> 8) > 0 ? (nacc >> 8) : 1) > 512 || (nacc >> 8) > 4) {
-    set_error("b2h_tc_bench: bad arguments");
-    return B2H_EINVAL;
-  }
-  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(tc_bench_kernel), 64 * 1024)) return rc;
-  const int grid = (mn_major >> 8) > 0 ? (mn_major >> 8) : 1;     // bits 8..: CTAs (all SMs busy -> chip-level pacing)
-  tc_bench_kernel<<<grid, 128, 64 * 1024, stream>>>(out, M, N, reps, nacc, mn_major & 255, 136);
-  count_launch();
-  return check_launch("tc_bench_kernel");
-}
-}  // namespace b2h
-
 #include "b2h_train_tc.cuh"
 #include "b2h_wide_tc.cuh"

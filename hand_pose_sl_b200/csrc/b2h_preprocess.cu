@@ -443,13 +443,12 @@ static int launch_pre(PreArgs& p, cudaStream_t stream) {
   // Resident CTAs, grid-stride beyond that.  Measured on B200 (profiles/r2_k0_residency.txt): while the launch's bytes fit
   // the 126 MB L2 with room to spare, 4 CTAs/SM (24 warps) are fastest (1 h clip: 28.1 vs 31.0 us); once reads and writes
   // both stream through DRAM, 2 CTAs/SM keep fewer DRAM pages open at a time and win (2 h: 56.8 vs 60.6 us, 8 h: 209 vs
-  // 236 us = 0.92 of the measured copy peak).  B2H_K0_CTAS (measurement aid, read once) forces a residency.
-  static const int forced = [] { const char* e = getenv("B2H_K0_CTAS"); const int v = e ? atoi(e) : 0; return v >= 1 && v <= kBlocksPerSM ? v : 0; }();
+  // 236 us = 0.92 of the measured copy peak).
   using F = Fmt<FMT>;
   const int out_floats[6] = {F::kBody * 2, F::kBody, 42, 21, 42, 21};
   int64_t bytes_per_slot = (FMT == 0 ? 804 : 600) + (p.input_bf16 ? F::kBody * 4 : 0);
   for (int a = 0; a < 6; ++a) bytes_per_slot += p.out[a] ? out_floats[a] * 4 : 0;
-  const int per_sm = forced ? forced : (S * bytes_per_slot > (int64_t)190 * 1000 * 1000 ? 2 : kBlocksPerSM);
+  const int per_sm = S * bytes_per_slot > (int64_t)190 * 1000 * 1000 ? 2 : kBlocksPerSM;
   int64_t cap = (int64_t)num_sms() * per_sm;
   if (blocks > cap) blocks = cap;
   preprocess_kernel<FMT><<<(unsigned)blocks, kWarpsPerBlock * 32, 0, stream>>>(p);

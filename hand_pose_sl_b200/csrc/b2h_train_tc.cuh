@@ -357,8 +357,8 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
     const uint4 zero = make_uint4(0, 0, 0, 0);
     for (int i = tid; i < act_bytes / 16; i += kTileThreads) z[i] = zero;
   };
-  // forward launches are programmatic by default: zero before the wait (under the predecessor); the train step is a
-  // normal launch unless B2H_PDL=2 (the wait is then a no-op) and zeroes under its own loads in flight instead
+  // forward launches are programmatic: zero before the wait (under the predecessor); the train step is a normal launch
+  // (the wait is then a no-op) and zeroes under its own loads in flight instead
   if (!TRAIN) zero_buffers();
   // ---- part 2: the previous kernel has completed and its writes (weights, Adam state, counters, inputs) are visible ----
   griddep_wait();
@@ -1129,28 +1129,23 @@ int launch_tc_tile(const ConvArgs& a, const TilePlan& plan, cudaStream_t stream)
   if (int rc = ensure_dyn_smem(fn, smem)) return rc;
   void* kargs[] = {&p};
   cudaError_t le;
-  // Grid barrier inside: a cooperative launch guarantees that all CTAs (<= 1 per SM) are co-resident.  B2H_NONCOOP=1
-  // (measurement aid, read once) uses a plain launch of the same grid: identical residency on an otherwise idle GPU,
-  // but nothing guarantees it when other kernels share the device.
-  // Programmatic dependent launch: the kernel may start while its predecessor on the stream is still running; it
-  // allocates TMEM, initialises its barriers and zeroes its shared memory, then blocks in griddepcontrol.wait until the
-  // predecessor has completed (conv_tc_tile_kernel, part 1 / part 2).  Measured on B200 (profiles/r2_pdl.txt): forward
-  // B=512x64 10.7 -> 9.2 us per batch, B=1 latency 8.7 -> 7.3 us; the train step gains 0.3 us of 27.4 (its 128 CTAs hold
-  // one SM each, so only 20 of the next step's CTAs find a free SM early, and the wait releases no sooner than a normal
-  // launch would start).  B2H_PDL (read once): unset / 1 = forward launches only, 2 = train steps too, 0 = none.
-  static const bool noncoop = [] { const char* e = getenv("B2H_NONCOOP"); return e && e[0] == '1'; }();
-  static const int pdl_mode = [] { const char* e = getenv("B2H_PDL"); return e && e[0] >= '0' && e[0] <= '2' ? e[0] - '0' : 1; }();
-  const bool coop = train && p.fuse.enabled && !noncoop;
-  const bool pdl = train ? pdl_mode == 2 : pdl_mode >= 1;
+  // The fused train step has a grid barrier inside: a cooperative launch guarantees that all its CTAs (<= 1 per SM)
+  // are co-resident, also when other kernels share the device.
+  // Forward launches are programmatic dependent launches: the kernel may start while its predecessor on the stream is
+  // still running; it allocates TMEM, initialises its barriers and zeroes its shared memory, then blocks in
+  // griddepcontrol.wait until the predecessor has completed (conv_tc_tile_kernel, part 1 / part 2).  Measured on B200
+  // (profiles/r2_pdl.txt): forward B=512x64 10.7 -> 9.2 us per batch, B=1 latency 8.7 -> 7.3 us.  Train steps are
+  // normal launches: PDL gained them only 0.3 us of 27.4 (their 128 CTAs hold one SM each, so only 20 of the next
+  // step's CTAs find a free SM early, and the wait releases no sooner than a normal launch would start).
+  const bool coop = train && p.fuse.enabled;
+  const bool pdl = !train;
   if (pdl) {
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kTileThreads); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute at[2];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    at[1].id = cudaLaunchAttributeCooperative;
-    at[1].val.cooperative = 1;
-    cfg.attrs = at; cfg.numAttrs = coop ? 2 : 1;
+    cudaLaunchAttribute at;
+    at.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at.val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = &at; cfg.numAttrs = 1;
     le = cudaLaunchKernelExC(&cfg, fn, kargs);
   } else if (coop) {
     le = cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kTileThreads), kargs, smem, stream);

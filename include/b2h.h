@@ -299,16 +299,6 @@ int b2h_tc_probe(const void* a_bf16, const void* b_bf16, float* out, int n, int 
  * gave up (the kernels never spin forever); reading clears it.  Synchronises the device. */
 int b2h_tc_status(void);
 
-/* Bring-up aid (microbenchmarks behind DESIGN.md's pacing numbers; tools/tc_bench*.py, tools/tma_bench.py).
- * M = 64 | 128: cycles for `reps` back-to-back tcgen05.mma (bf16, K=16) of shape MxN rotating over `nacc & 255`
- *   accumulators, issued from `nacc >> 8` warps (0 = 1); out[0] = issue-to-completion cycles, out[1] = issue-loop cycles.
- *   `mn_major` bit 0: MN-major operands; bit 1: 128B-swizzle descriptors (timing only); bit 2: walk A rows / B blocks;
- *   bit 3: tcgen05.commit after every second MMA; bit 4: non-zero operand data; bits 5-7: chunk-stride variants;
- *   bits 8..: number of CTAs (0 = 1).
- * M = 1: steady-state L2 -> shared throughput of 1-D cp.async.bulk copies: N = bytes per copy (divides 8192),
- *   reps = rounds, nacc = ring depth in 8-KB stages (<= 16), mn_major = CTAs; out[0] = cycles, out[1] = bytes. */
-int b2h_tc_bench(void* out_i64x2, int M, int N, int reps, int nacc, int mn_major, void* stream);
-
 /* Bring-up aid: when set to a device buffer of 1024 int64, CTA 0 of the tile kernels stamps clock64() at every
  * phase boundary (setup, staging, per-layer issue / ready / epilogue) into words [0, 128), and every CTA c of the fused
  * train kernel writes %globaltimer (ns) at its start / barrier arrival / barrier exit / end into words

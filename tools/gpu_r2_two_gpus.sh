@@ -1,12 +1,11 @@
 #!/bin/bash
-# round 2, run B (2+ GPUs): train tests, phase stamps (coop / non-coop), DP tests, DP stamps (multicast on/off), bench N=1,2
+# round 2, run B (2+ GPUs): train tests, phase stamps, DP tests, DP stamps (multicast on/off), bench N=1,2
 N=${1:-2}
 mkdir -p gpurun_out; rm -f gpurun_out/summary.txt
 S=gpurun_out/summary.txt
 timeout 900 python -m pytest tests/test_gpu_train.py tests/test_gpu_forward.py -q -m gpu --tb=short -x > gpurun_out/pytest_train.log 2>&1; echo "train tests exit $?" >> $S
 tail -5 gpurun_out/pytest_train.log >> $S
 timeout 200 python tools/phase_timing.py > gpurun_out/phase_n1.log 2>&1; echo "phase n1 exit $?" >> $S; grep -E "steady state \(graph replay, rep 2\)|us/step|   setup" gpurun_out/phase_n1.log | tail -4 >> $S
-B2H_NONCOOP=1 timeout 200 python tools/phase_timing.py > gpurun_out/phase_n1_noncoop.log 2>&1; echo "phase n1 noncoop exit $?" >> $S; grep -E "us/step" gpurun_out/phase_n1_noncoop.log >> $S
 timeout 600 python -m pytest tests/test_gpu_dp.py -q -m gpu --tb=short -x > gpurun_out/test_gpu_dp.log 2>&1; echo "dp tests exit $?" >> $S
 tail -8 gpurun_out/test_gpu_dp.log >> $S
 for MC in 1 0; do

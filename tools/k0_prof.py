@@ -39,7 +39,7 @@ if sys.argv[1:2] == ["time"]:
         e1.record()
         torch.cuda.synchronize()
         us = e0.elapsed_time(e1) / 40 * 1e3
-        print(f"K0 {F} frames: {us:.2f} us/launch (graph replay), {F * 1452 / us / 1e6:.3f} TB/s, env B2H_K0_CTAS={os.environ.get('B2H_K0_CTAS')}")
+        print(f"K0 {F} frames: {us:.2f} us/launch (graph replay), {F * 1452 / us / 1e6:.3f} TB/s")
         del tp, tl, tr, out, g
 else:
     F = int(sys.argv[1]) if len(sys.argv) > 1 else 108000
