@@ -63,12 +63,12 @@ static ForwardPlan forward_plan(const Geo& g, int B, int T, int precision) {
 }
 
 // Which training path serves (B, T, C, precision) and how its workspace is laid out: the ONE place that decides.
-//   [header B2H_WS_HEADER][gradient partials: nparts x stride floats][loss partials: n_loss floats][scratch (wide path)]
+//   [header B2H_WS_HEADER][gradient partials: nparts x gp_total floats][loss partials: n_loss floats][scratch (wide path)]
 struct TrainPlan {
   int kernel;            // B2H_KERNEL_TC_TILE | B2H_KERNEL_TC_WIDE_TRAIN | B2H_KERNEL_FFMA | B2H_KERNEL_NONE
   TilePlan tile; WidePlan wide; FfmaPlan ffma;
-  int nparts, gp_layout, n_loss;
-  int64_t stride, scratch_off, total;
+  int nparts, n_loss;
+  int64_t scratch_off, total;
 };
 static TrainPlan train_plan(const Geo& g, int B, int T, int precision) {
   TrainPlan t{};
@@ -78,14 +78,14 @@ static TrainPlan train_plan(const Geo& g, int B, int T, int precision) {
   if (precision == B2H_BF16) t.wide = plan_wide(g, B, T);   // 32 < conv_channels <= 256: forward+criterion / dgrad chain / split-K wgrad
   t.ffma = plan_ffma(g, B, T, true);
   if (t.tile.ok) {
-    t.kernel = B2H_KERNEL_TC_TILE; t.nparts = t.tile.grid; t.stride = gp_total(g); t.gp_layout = 1; t.n_loss = t.nparts;
+    t.kernel = B2H_KERNEL_TC_TILE; t.nparts = t.tile.grid; t.n_loss = t.nparts;
   } else if (t.wide.ok) {
-    t.kernel = B2H_KERNEL_TC_WIDE_TRAIN; t.nparts = t.wide.ksplit; t.stride = gp_total(g); t.gp_layout = 1; t.n_loss = t.wide.n_loss;
+    t.kernel = B2H_KERNEL_TC_WIDE_TRAIN; t.nparts = t.wide.ksplit; t.n_loss = t.wide.n_loss;
     scratch = t.wide.scratch_bytes;
   } else if (t.ffma.ok) {
-    t.kernel = B2H_KERNEL_FFMA; t.nparts = t.ffma.grid; t.stride = g.P; t.gp_layout = 0; t.n_loss = t.nparts;
+    t.kernel = B2H_KERNEL_FFMA; t.nparts = t.ffma.grid; t.n_loss = t.nparts;
   }
-  int64_t o = B2H_WS_HEADER + ((int64_t)t.nparts * t.stride + t.n_loss) * 4;
+  int64_t o = B2H_WS_HEADER + ((int64_t)t.nparts * gp_total(g) + t.n_loss) * 4;
   o = (o + 255) / 256 * 256;
   t.scratch_off = o;
   t.total = o + scratch + 256;
@@ -117,9 +117,10 @@ extern "C" int64_t b2h_param_offset(int n_in, int C, int pos_emb, int layer, int
   Geo g = make_geo(n_in, C, pos_emb);
   return is_bias ? g.b_off[layer - 1] : g.w_off[layer - 1];
 }
-/* Host-side self-check of the gradient-partial slot layout (no GPU): every flat parameter index maps to a distinct
- * slot and back, every other slot decodes as padding.  gp_index_of_flat goes through gp_slot_of_flat, the decode the
- * packed-weight scatter uses.  Returns the number of violations (0 = consistent). */
+/* Host-side self-check of the gradient-partial slot layout every training kernel writes (no GPU): every flat parameter
+ * index maps to a distinct slot and back, every other slot decodes as padding.  gp_index_of_flat goes through
+ * gp_slot_of_flat, the decode the packed-weight scatter uses, and gp_slot_in_layer, the slot the FFMA kernel writes.
+ * Returns the number of violations (0 = consistent). */
 extern "C" int64_t b2h_gp_layout_check(int n_in, int C, int pos_emb) {
   if (!geo_ok(n_in, C, pos_emb, "b2h_gp_layout_check")) return B2H_ESHAPE;
   Geo g = make_geo(n_in, C, pos_emb);
@@ -262,7 +263,7 @@ struct TrainResult {
   int rc;
   Geo g;
   TrainPlan plan;
-  float* partials;        // gradient partials in the workspace: plan.nparts slices of plan.stride floats
+  float* partials;        // gradient partials in the workspace: plan.nparts slices of gp_total(g) floats
   float* loss_partials;   // plan.n_loss floats
 };
 
@@ -309,7 +310,7 @@ static TrainResult train_common(const void* x, int x_dtype, const WindowView* wv
   if (misaligned(workspace, 15)) { set_error("%s: workspace must be 16-byte aligned", who); return result(B2H_EALIGN); }
   // [header: launch sequence + per-CTA arrival flags of the fused kernel, FIXED offset][gradient partials][loss partials][scratch]
   r.partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + B2H_WS_HEADER);
-  r.loss_partials = r.partials + (size_t)plan.nparts * plan.stride;
+  r.loss_partials = r.partials + (size_t)plan.nparts * gp_total(r.g);
   ConvArgs a{};
   a.x = x; a.x_dtype = x_dtype; a.target = target; a.conf = conf; a.d_y = d_y; a.lengths = lengths; a.params = params;
   a.packed = reinterpret_cast<const char*>(packed); a.y = pred_out; a.partials = r.partials; a.loss_partials = r.loss_partials;
@@ -343,8 +344,8 @@ static int train_forward_backward(const void* x, int x_dtype, const WindowView* 
                                      pos_emb, loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, who,
                                      reinterpret_cast<long long*>(step_dev), nullptr, nullptr);
   if (r.rc || !grads_out) return r.rc;   // grads_out == NULL: only the fused kernel runs, partials stay in the workspace
-  return launch_reduce(r.partials, r.plan.nparts, r.plan.gp_layout, r.g, grads_out, r.loss_partials, loss_out,
-                       (cudaStream_t)stream, nullptr, r.plan.n_loss);
+  return launch_reduce(r.partials, r.plan.nparts, r.g, grads_out, r.loss_partials, r.plan.n_loss, loss_out, nullptr,
+                       (cudaStream_t)stream);
 }
 
 extern "C" int b2h_train_forward_backward(const void* x, int x_dtype, const float* target, const float* conf,
@@ -395,8 +396,7 @@ extern "C" int b2h_conv_backward(const void* x, int x_dtype, const float* d_y, c
                                      pos_emb, 0, precision, 2, workspace, workspace_bytes, (cudaStream_t)stream,
                                      "b2h_conv_backward", nullptr, nullptr, nullptr);
   if (r.rc) return r.rc;
-  return launch_reduce(r.partials, r.plan.nparts, r.plan.gp_layout, r.g, grads_out, nullptr, nullptr, (cudaStream_t)stream,
-                       nullptr, r.plan.n_loss);
+  return launch_reduce(r.partials, r.plan.nparts, r.g, grads_out, nullptr, r.plan.n_loss, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 // The Adam tail of the fused tile kernel (train_common enables it and points it at the workspace header).
@@ -424,9 +424,9 @@ static int train_step(const void* x, int x_dtype, const WindowView* wv, const fl
                                      reinterpret_cast<long long*>(step_dev), nullptr, step_dev ? &fuse : nullptr);
   if (r.rc) return r.rc;
   if (step_dev && r.plan.kernel == B2H_KERNEL_TC_TILE) return B2H_OK;
-  return launch_adam(params, r.partials, r.plan.nparts, r.plan.gp_layout, exp_avg, exp_avg_sq, r.g.P, lr, beta1, beta2, eps,
-                     step < 1 ? 1 : step, reinterpret_cast<const long long*>(step_dev), lr_dev, 1.0f, packed, r.g,
-                     r.loss_partials, loss_out, (cudaStream_t)stream, r.plan.n_loss);
+  return launch_adam_partials(params, r.partials, r.plan.nparts, exp_avg, exp_avg_sq, lr, beta1, beta2, eps, step < 1 ? 1 : step,
+                              reinterpret_cast<const long long*>(step_dev), lr_dev, packed, r.g, r.loss_partials, r.plan.n_loss,
+                              loss_out, (cudaStream_t)stream);
 }
 
 extern "C" int b2h_train_step(const void* x, int x_dtype, const float* target, const float* conf, const int32_t* lengths,
@@ -473,8 +473,8 @@ extern "C" int b2h_train_step_dp(const void* x, int x_dtype, const float* target
                                      reinterpret_cast<long long*>(epoch_dev), &fuse);
   if (r.rc) return r.rc;
   if (r.plan.kernel == B2H_KERNEL_TC_TILE) return B2H_OK;    // everything happened inside the one cooperative launch
-  if (int rc = launch_reduce(r.partials, r.plan.nparts, r.plan.gp_layout, r.g, sym_grads, r.loss_partials, loss_out,
-                             (cudaStream_t)stream, reinterpret_cast<const long long*>(epoch_dev), r.plan.n_loss))
+  if (int rc = launch_reduce(r.partials, r.plan.nparts, r.g, sym_grads, r.loss_partials, r.plan.n_loss, loss_out,
+                             reinterpret_cast<const long long*>(epoch_dev), (cudaStream_t)stream))
     return rc;
   return launch_adam_dp(params, reinterpret_cast<const float* const*>(peer_bufs_dev), rank, world, exp_avg, exp_avg_sq, r.g.P, lr,
                         beta1, beta2, eps, reinterpret_cast<const long long*>(step_dev),
@@ -493,8 +493,8 @@ extern "C" int b2h_adam_step(float* params, const float* grads, float* exp_avg, 
     if (g.P != n) { set_error("b2h_adam_step: n=%lld does not match geometry (%d)", (long long)n, g.P); return B2H_ESHAPE; }
   }
   if (n == 0) return B2H_OK;
-  return launch_adam(params, grads, 1, 0, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, step < 1 ? 1 : step,
-                     reinterpret_cast<const long long*>(step_dev), lr_dev, grad_scale, packed, g, nullptr, nullptr, (cudaStream_t)stream);
+  return launch_adam_flat(params, grads, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, step < 1 ? 1 : step,
+                          reinterpret_cast<const long long*>(step_dev), lr_dev, grad_scale, packed, g, (cudaStream_t)stream);
 }
 
 extern "C" int b2h_mask_output(float* y, const int32_t* lengths, int B, int T, int row_elems, void* stream) {

@@ -73,11 +73,14 @@ __host__ __device__ inline int64_t umma_b_offset(int k, int kk, int n, int KP, i
   return q * ((int64_t)N * 32) + (int64_t)chunk * (N * 16) + (int64_t)n * 16 + within * 2;
 }
 
-// Gradient-partial layout written by the tensor-core train kernel.  The TMEM read-out has lane = output channel
-// and 32 consecutive columns = input channels, so the W part is stored [k][ci/4][co][4 ci]: for a fixed (k, ci/4)
-// the lanes of a warp store consecutive float4s (coalesced; the [k][co][ci] order of round 1 made every lane of a
-// store instruction hit its own 128-B line: ~6k cycles of read-out per CTA).
+// Gradient-partial layout written by every training kernel (tile, wide wgrad, FFMA).  The TMEM read-out has lane =
+// output channel and 32 consecutive columns = input channels, so the W part is stored [k][ci/4][co][4 ci]: for a fixed
+// (k, ci/4) the lanes of a warp store consecutive float4s (coalesced; the [k][co][ci] order of round 1 made every lane
+// of a store instruction hit its own 128-B line: ~6k cycles of read-out per CTA).  The FFMA kernel's lanes are output
+// channels too: for a fixed (k, ci) its stores are 16 B apart.
 //   per layer l: W part [k][kp_l/4][cout_l][4] then bias part [cout_l] (padded to a multiple of 4)
+// The slots with ci >= cin and the bias padding carry no parameter: writers may leave them unwritten, readers decode
+// them as padding (gp_decode / flat_index_of_gp) and never apply them.
 __host__ __device__ inline int gp_layer_size(const Geo& g, int l) { return B2H_KW * g.cout[l] * g.kp[l] + round_up(g.cout[l], 4); }
 __host__ __device__ inline int gp_layer_off(const Geo& g, int l) {
   int o = 0;
@@ -88,6 +91,12 @@ __host__ __device__ inline int gp_total(const Geo& g) { return gp_layer_off(g, 4
 
 // (layer, tap, co, ci) of one parameter; is_bias: co = bias index, k = ci = 0
 struct GpSlot { int l, k, co, ci; bool is_bias; };
+// slot of weight (s.l, s.k, s.ci, s.co) or of bias (s.l, s.co) inside layer s.l's part of a slice (add gp_layer_off)
+__host__ __device__ inline int gp_slot_in_layer(const Geo& g, const GpSlot& s) {
+  const int l = s.l;
+  if (s.is_bias) return B2H_KW * g.cout[l] * g.kp[l] + s.co;
+  return ((s.k * (g.kp[l] >> 2) + (s.ci >> 2)) * g.cout[l] + s.co) * 4 + (s.ci & 3);
+}
 // flat parameter index -> slot
 __host__ __device__ inline GpSlot gp_slot_of_flat(const Geo& g, int i) {
   GpSlot s;
@@ -107,9 +116,7 @@ __host__ __device__ inline GpSlot gp_slot_of_flat(const Geo& g, int i) {
 // flat parameter index -> index in the GP layout
 __host__ __device__ inline int gp_index_of_flat(const Geo& g, int i) {
   const GpSlot s = gp_slot_of_flat(g, i);
-  const int l = s.l, base = gp_layer_off(g, l);
-  if (s.is_bias) return base + B2H_KW * g.cout[l] * g.kp[l] + s.co;
-  return base + ((s.k * (g.kp[l] >> 2) + (s.ci >> 2)) * g.cout[l] + s.co) * 4 + (s.ci & 3);
+  return gp_layer_off(g, s.l) + gp_slot_in_layer(g, s);
 }
 
 // GP index -> slot.  Returns false for the padding slots.
@@ -311,7 +318,7 @@ struct ConvArgs {
   const float* target; const float* conf; const float* d_y; const int32_t* lengths;
   const float* params; const char* packed;
   float* y;                 // forward output / masked prediction (nullable in train mode)
-  float* partials;          // [grid][P]
+  float* partials;          // [grid][gp_total]
   float* loss_partials;     // [grid]
   long long* step_dev;      // nullable: device step counter, incremented by block 0 (read by the Adam kernel)
   long long* epoch_dev;     // nullable: data-parallel exchange epoch, incremented the same way (never rewound)
@@ -336,15 +343,21 @@ void set_debug_timing(long long* p);
 int launch_format_prediction(const float* pred, float* out, int64_t rows, int mode, cudaStream_t stream);
 int launch_pos_emb_concat(const float* inp, float* out, int B, int Cc, int T, int max_len, cudaStream_t stream);
 int launch_pack(const float* params, void* packed, const Geo& g, cudaStream_t stream);
-int launch_reduce(const float* partials, int nparts, int gp_layout, const Geo& g, float* grads, const float* loss_partials,
-                  float* loss_out, cudaStream_t stream, const long long* epoch_dev = nullptr, int n_loss_parts = -1);
+// grads (flat parameter order) = sum of the nparts gradient-partial slices; *loss_out = sum of the n_loss loss partials
+int launch_reduce(const float* partials, int nparts, const Geo& g, float* grads, const float* loss_partials, int n_loss,
+                  float* loss_out, const long long* epoch_dev, cudaStream_t stream);
 int launch_adam_dp(float* params, const float* const* peer_bufs, int rank, int world, float* m, float* v, int64_t n, double lr,
                    double beta1, double beta2, double eps, const long long* step_dev, const long long* epoch_dev, const double* lr_dev,
                    float grad_scale, void* packed, const Geo& g, cudaStream_t stream);
 int dp_status_and_clear();
-int launch_adam(float* params, const float* grads, int nparts, int gp_layout, float* m, float* v, int64_t n, double lr, double beta1, double beta2,
-                double eps, int64_t step, const long long* step_dev, const double* lr_dev, float grad_scale, void* packed, const Geo& g,
-                const float* loss_partials, float* loss_out, cudaStream_t stream, int n_loss_parts = -1);
+// Adam on the sum of the nparts gradient-partial slices a training launch left in the workspace (+ the loss sum)
+int launch_adam_partials(float* params, const float* partials, int nparts, float* m, float* v, double lr, double beta1,
+                         double beta2, double eps, int64_t step, const long long* step_dev, const double* lr_dev, void* packed,
+                         const Geo& g, const float* loss_partials, int n_loss, float* loss_out, cudaStream_t stream);
+// Adam on an already-reduced gradient of n parameters in flat order (b2h_adam_step); packed == nullptr: no re-pack
+int launch_adam_flat(float* params, const float* grads, float* m, float* v, int64_t n, double lr, double beta1, double beta2,
+                     double eps, int64_t step, const long long* step_dev, const double* lr_dev, float grad_scale, void* packed,
+                     const Geo& g, cudaStream_t stream);
 int launch_mask_output(float* y, const int32_t* lengths, int B, int T, int row, cudaStream_t stream);
 int launch_pose_l1(const float* pred, const float* target, const float* scores, const int32_t* lengths, int B, int T, int row,
                    int loss_kind, float* loss_out, float* d_pred, float* row_scratch, cudaStream_t stream);

@@ -14,7 +14,8 @@
 // and behind (the conv's zero padding), so tap k of output frame t reads row t+k.  lane -> output
 // channel (coalesced tap-major weights Wf[k][ci][co] through the read-only path, conflict-free smem
 // writes), each warp register-blocks 8 frames.  Gradients: every CTA owns one slice of the
-// partials workspace (no atomics, deterministic); b2h_optim.cu reduces the slices.
+// partials workspace (no atomics, deterministic), in the gradient-partial slot layout every training
+// kernel writes (b2h_common.cuh gp_*); b2h_optim.cu reduces the slices.
 #include "b2h_common.cuh"
 
 namespace b2h {
@@ -69,11 +70,12 @@ __device__ __forceinline__ void conv_rows(const float* __restrict__ in, int ldi,
   }
 }
 
-// dW[co][ci][k] (+)= sum_t g[t][co] * a[t+k-2][ci];  db[co] (+)= sum_t g[t][co]
-__device__ __forceinline__ void wgrad_rows(const float* __restrict__ g, int ldg, int Cout, const float* __restrict__ a,
-                                           int lda, int Cin, float* __restrict__ pW, float* __restrict__ pB, int T,
-                                           bool first) {
+// dW[co][ci][k] (+)= sum_t g[t][co] * a[t+k-2][ci];  db[co] (+)= sum_t g[t][co]  of layer l, at their slots of the
+// gradient-partial layout in pl = this CTA's slice + gp_layer_off(geo, l) (the padding slots are left unwritten)
+__device__ __forceinline__ void wgrad_rows(const Geo& geo, int l, const float* __restrict__ g, int ldg,
+                                           const float* __restrict__ a, int lda, float* __restrict__ pl, int T, bool first) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int Cout = geo.cout[l], Cin = geo.cin[l];
   const int nCG = (Cout + 31) >> 5;
   const int ntask = (Cin + 1) * nCG;          // the extra "ci" row is the bias gradient
   for (int task = warp; task < ntask; task += kWarps) {
@@ -96,14 +98,19 @@ __device__ __forceinline__ void wgrad_rows(const float* __restrict__ g, int ldg,
         a0 = a1; a1 = a2; a2 = a3; a3 = a4;
       }
       if (active) {
-        float* dst = pW + ((size_t)co * Cin + ci) * B2H_KW;
 #pragma unroll
-        for (int k = 0; k < B2H_KW; ++k) dst[k] = first ? acc[k] : dst[k] + acc[k];
+        for (int k = 0; k < B2H_KW; ++k) {
+          float* dst = pl + gp_slot_in_layer(geo, GpSlot{l, k, co, ci, false});
+          *dst = first ? acc[k] : *dst + acc[k];
+        }
       }
     } else {
       float s = 0.f;
       for (int t = 0; t < T; ++t) s += gp[t * ldg];
-      if (active) pB[co] = first ? s : pB[co] + s;
+      if (active) {
+        float* dst = pl + gp_slot_in_layer(geo, GpSlot{l, 0, co, 0, true});
+        *dst = first ? s : *dst + s;
+      }
     }
   }
 }
@@ -150,7 +157,7 @@ __global__ void __launch_bounds__(kThreads) conv_fp32_kernel(ConvArgs p) {
   }
   if (TRAIN && p.step_dev && blockIdx.x == 0 && threadIdx.x == 0) *p.step_dev += 1;
   if (TRAIN && p.epoch_dev && blockIdx.x == 0 && threadIdx.x == 0) *p.epoch_dev += 1;
-  float* part = TRAIN ? p.partials + (size_t)blockIdx.x * g.P : nullptr;
+  float* part = TRAIN ? p.partials + (size_t)blockIdx.x * gp_total(g) : nullptr;
   float loss_acc = 0.0f;
   bool first = true;
 
@@ -277,16 +284,16 @@ __global__ void __launch_bounds__(kThreads) conv_fp32_kernel(ConvArgs p) {
     }
     __syncthreads();
     // layer 4: wgrad(dY, a3), dgrad -> dZ3 = (W4^T * dY) . (a3 > 0)
-    wgrad_rows(G0, ldg, g.cout[3], A3, ldc, g.cin[3], part + g.w_off[3], part + g.b_off[3], T, first);
+    wgrad_rows(g, 3, G0, ldg, A3, ldc, part + gp_layer_off(g, 3), T, first);
     conv_rows<2>(G0, ldg, g.cout[3], Wd[3], g.cin[3], nullptr, G1, ldg, A3, ldc, T);
     __syncthreads();
-    wgrad_rows(G1, ldg, g.cout[2], A2, ldc, g.cin[2], part + g.w_off[2], part + g.b_off[2], T, first);
+    wgrad_rows(g, 2, G1, ldg, A2, ldc, part + gp_layer_off(g, 2), T, first);
     conv_rows<2>(G1, ldg, g.cout[2], Wd[2], g.cin[2], nullptr, G0, ldg, A2, ldc, T);
     __syncthreads();
-    wgrad_rows(G0, ldg, g.cout[1], A1, ldc, g.cin[1], part + g.w_off[1], part + g.b_off[1], T, first);
+    wgrad_rows(g, 1, G0, ldg, A1, ldc, part + gp_layer_off(g, 1), T, first);
     conv_rows<2>(G0, ldg, g.cout[1], Wd[1], g.cin[1], nullptr, G1, ldg, A1, ldc, T);
     __syncthreads();
-    wgrad_rows(G1, ldg, g.cout[0], X, ld0, g.cin[0], part + g.w_off[0], part + g.b_off[0], T, first);
+    wgrad_rows(g, 0, G1, ldg, X, ld0, part + gp_layer_off(g, 0), T, first);
     __syncthreads();
     first = false;
   }

@@ -53,24 +53,24 @@ __device__ __forceinline__ void loss_partial_sum(const float* __restrict__ loss_
 }
 
 // grads[i] = sum_c partials[c][slot(i)];  loss = sum_c loss_partials[c]
-__global__ void __launch_bounds__(256) reduce_partials_kernel(const float* __restrict__ partials, int nparts, int gp_layout, Geo g,
+__global__ void __launch_bounds__(256) reduce_partials_kernel(const float* __restrict__ partials, int nparts, Geo g,
                                                               float* __restrict__ grads, const float* __restrict__ loss_partials,
                                                               float* __restrict__ loss_out, const long long* __restrict__ epoch_dev,
                                                               int n_loss_parts) {
   __shared__ float red[8][32];
   if (epoch_dev) grads += (size_t)(*epoch_dev & 1) * g.P;      // data parallel: double-buffered exchange slot
-  const int nj = gp_layout ? gp_total(g) : g.P;
+  const int nj = gp_total(g);
   const int j = blockIdx.x * 32 + (threadIdx.x & 31);
   const float s = block_partial_sum(partials, nparts, (size_t)nj, j, nj, red);
   if (threadIdx.x < 32 && j < nj) {
-    const int i = gp_layout ? flat_index_of_gp(g, j) : j;
+    const int i = flat_index_of_gp(g, j);
     if (i >= 0) grads[i] = s;
   }
   loss_partial_sum(loss_partials, n_loss_parts, loss_out);
 }
 
 struct AdamArgs {
-  float* params; const float* grads; int nparts; int gp_layout; int64_t n;
+  float* params; const float* grads; int nparts; int64_t n;   // grads: nparts partial slices, or a flat gradient of n
   float* m; float* v;
   float beta1, beta2, one_minus_b1, one_minus_b2, step_size, inv_bc2_sqrt, eps, grad_scale;
   double lr_d, beta1_d, beta2_d;
@@ -85,7 +85,7 @@ struct AdamArgs {
 // (graph replay), computed by one thread of a block.  Three forms of these coefficients exist, and each stays as it is
 // because switching a path to another form moves its trained weights in the last bits:
 //   - the Adam kernels of this file, when step_dev or lr_dev is given: this function, double precision with ipow;
-//   - launch_adam on the host for calls without step_dev / lr_dev: double-precision pow();
+//   - adam_args on the host for calls without step_dev / lr_dev: double-precision pow();
 //   - the fused tail of conv_tc_tile_kernel: fp32 -expm1f(t * log1pf(beta - 1)), because double-precision powers cost
 //     ~5k cycles on B200's few FP64 units inside the one-launch train step.
 __device__ __forceinline__ void adam_bias_corrections(const AdamArgs& a, float& step_size, float& inv_bc2_sqrt) {
@@ -95,7 +95,7 @@ __device__ __forceinline__ void adam_bias_corrections(const AdamArgs& a, float& 
   inv_bc2_sqrt = (float)(1.0 / sqrt(1.0 - ipow(a.beta2_d, t)));
 }
 
-// torch.optim.Adam single-tensor update (adam_update) over the flat buffers, 32 slots per block
+// torch.optim.Adam single-tensor update (adam_update) on the sum of many gradient-partial slices, 32 slots per block
 __global__ void __launch_bounds__(256) adam_kernel(AdamArgs a) {
   __shared__ float red[8][32];
   __shared__ float s_step_size, s_inv_bc2_sqrt;
@@ -105,16 +105,11 @@ __global__ void __launch_bounds__(256) adam_kernel(AdamArgs a) {
     a.step_size = s_step_size;
     a.inv_bc2_sqrt = s_inv_bc2_sqrt;
   }
-  const int nj = a.gp_layout ? gp_total(a.g) : (int)a.n;
+  const int nj = gp_total(a.g);
   const int j = blockIdx.x * 32 + (threadIdx.x & 31);
-  float gr;
-  if (a.nparts == 1) {            // already-reduced flat gradient (modular / data-parallel path)
-    gr = (j < nj && threadIdx.x < 32) ? a.grads[j] : 0.f;
-  } else {
-    gr = block_partial_sum(a.grads, a.nparts, (size_t)nj, j, nj, red);
-  }
+  const float gr = block_partial_sum(a.grads, a.nparts, (size_t)nj, j, nj, red);
   if (threadIdx.x < 32 && j < nj) {
-    const int i = a.gp_layout ? flat_index_of_gp(a.g, j) : j;
+    const int i = flat_index_of_gp(a.g, j);
     if (i >= 0) {
       float m = a.m[i], v = a.v[i];
       const float p = adam_update(m, v, a.params[i], gr * a.grad_scale, a.one_minus_b1, a.one_minus_b2, a.beta2, a.eps,
@@ -126,13 +121,33 @@ __global__ void __launch_bounds__(256) adam_kernel(AdamArgs a) {
   loss_partial_sum(a.loss_partials, a.n_loss_parts, a.loss_out);
 }
 
-// Few gradient slices (wide training: split-K factor 6..37; small batches of the tile kernel): Adam with BOTH sides coalesced.
-// The gradient slices are in slot order [k][ci/4][co][4] (what the TMEM read-out writes), the parameters / moments in the
-// reference's (co, ci, k) order: one thread per slot made every m / v / p access and most packed-operand stores hit their
-// own 32-byte sector (ncu at C = 256: 302 MB of DRAM writes for 3 MB of parameters, 87 us).  Here a block owns 2 output
-// channels of one layer: (1) sum the slices in slot order (32-B runs) into shared memory [co][ci][k], (2) walk the flat
-// order -- cin*5 contiguous floats per output channel -- for the Adam update, (3) scatter the new weights into the packed
-// operand layouts in slot order, where their stores coalesce.  Fixed summation order -> deterministic.
+// The same update on an already-reduced gradient in flat parameter order (b2h_adam_step), one thread per parameter
+__global__ void __launch_bounds__(256) adam_flat_kernel(AdamArgs a) {
+  __shared__ float s_step_size, s_inv_bc2_sqrt;
+  if (a.step_dev || a.lr_dev) {
+    if (threadIdx.x == 0) adam_bias_corrections(a, s_step_size, s_inv_bc2_sqrt);
+    __syncthreads();
+    a.step_size = s_step_size;
+    a.inv_bc2_sqrt = s_inv_bc2_sqrt;
+  }
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < a.n) {
+    float m = a.m[i], v = a.v[i];
+    const float p = adam_update(m, v, a.params[i], a.grads[i] * a.grad_scale, a.one_minus_b1, a.one_minus_b2, a.beta2, a.eps,
+                                a.step_size, a.inv_bc2_sqrt);
+    a.m[i] = m; a.v[i] = v; a.params[i] = p;
+    if (a.packed) scatter_packed(a.g, a.packed, gp_slot_of_flat(a.g, (int)i), p);
+  }
+}
+
+// Few gradient slices (wide training: split-K factor 6..37; small batches of the tile and FFMA kernels): Adam with BOTH
+// sides coalesced.  The gradient slices are in slot order [k][ci/4][co][4] (what the training kernels write), the
+// parameters / moments in the reference's (co, ci, k) order: one thread per slot made every m / v / p access and most
+// packed-operand stores hit their own 32-byte sector (ncu at C = 256: 302 MB of DRAM writes for 3 MB of parameters,
+// 87 us).  Here a block owns 2 output channels of one layer: (1) sum the slices in slot order (32-B runs) into shared
+// memory [co][ci][k], (2) walk the flat order -- cin*5 contiguous floats per output channel -- for the Adam update,
+// (3) scatter the new weights into the packed operand layouts in slot order, where their stores coalesce.  Fixed
+// summation order -> deterministic.
 constexpr int kAdamCoGroup = 2;   // output channels per block: 406 blocks at C = 256 (latency-bound kernel: many small blocks)
 __global__ void __launch_bounds__(256) adam_gp_tile_kernel(AdamArgs a) {
   extern __shared__ float g_s[];                      // [kAdamCoGroup][kp][5] gradient sums, then the new weights
@@ -329,8 +344,8 @@ __global__ void __launch_bounds__(256) adam_dp_kernel(AdamDpArgs d) {
   }
 }
 
-// The AdamArgs fields every Adam launch sets the same way; the caller adds where the gradients come from and the host-side
-// bias corrections.
+// The AdamArgs fields every Adam launch sets the same way, with the host-side bias corrections (the kernels replace them
+// when step_dev or lr_dev is given); the caller adds where the gradients come from.
 static AdamArgs adam_args(float* params, float* m, float* v, int64_t n, double lr, double beta1, double beta2, double eps,
                           long long step, const long long* step_dev, const double* lr_dev, float grad_scale, void* packed,
                           const Geo& g) {
@@ -341,6 +356,9 @@ static AdamArgs adam_args(float* params, float* m, float* v, int64_t n, double l
   a.eps = (float)eps; a.grad_scale = grad_scale;
   a.packed = reinterpret_cast<char*>(packed); a.g = g;
   a.lr_d = lr; a.beta1_d = beta1; a.beta2_d = beta2; a.step_dev = step_dev; a.lr_dev = lr_dev; a.step_host = step;
+  const double bc1 = 1.0 - pow(beta1, (double)step), bc2 = 1.0 - pow(beta2, (double)step);
+  a.step_size = (float)(lr / bc1);
+  a.inv_bc2_sqrt = (float)(1.0 / sqrt(bc2));
   return a;
 }
 
@@ -479,41 +497,38 @@ int launch_pack(const float* params, void* packed, const Geo& g, cudaStream_t st
   return check_launch("pack_kernel");
 }
 
-// Few gradient slices in the slot layout (wide training, small batches of the tile kernel): the reduction and Adam kernels
-// that sum every slice of a slot in one thread, instead of spreading the slices over the 8 warps of a block.
-static bool few_slices(int nparts, int gp_layout) { return gp_layout && nparts <= 64; }
+// Few gradient slices (wide training, small batches of the tile and FFMA kernels): the reduction and Adam kernels that sum
+// every slice of a slot in one thread, instead of spreading the slices over the 8 warps of a block.
+static bool few_slices(int nparts) { return nparts <= 64; }
 
-int launch_reduce(const float* partials, int nparts, int gp_layout, const Geo& g, float* grads, const float* loss_partials,
-                  float* loss_out, cudaStream_t stream, const long long* epoch_dev, int n_loss_parts) {
-  const int nj = gp_layout ? gp_total(g) : g.P;
-  if (few_slices(nparts, gp_layout)) {                 // one thread per slot
+int launch_reduce(const float* partials, int nparts, const Geo& g, float* grads, const float* loss_partials, int n_loss,
+                  float* loss_out, const long long* epoch_dev, cudaStream_t stream) {
+  const int nj = gp_total(g);
+  if (few_slices(nparts)) {                            // one thread per slot
     reduce_gp_wide_kernel<<<(nj + 255) / 256, 256, 0, stream>>>(partials, nparts, g, grads, loss_partials, loss_out, epoch_dev,
-                                                                n_loss_parts < 0 ? nparts : n_loss_parts);
+                                                                n_loss);
     count_launch();
     return check_launch("reduce_gp_wide_kernel");
   }
-  reduce_partials_kernel<<<(nj + 31) / 32, 256, 0, stream>>>(partials, nparts, gp_layout, g, grads, loss_partials, loss_out, epoch_dev,
-                                                             n_loss_parts < 0 ? nparts : n_loss_parts);
+  reduce_partials_kernel<<<(nj + 31) / 32, 256, 0, stream>>>(partials, nparts, g, grads, loss_partials, loss_out, epoch_dev,
+                                                             n_loss);
   count_launch();
   return check_launch("reduce_partials_kernel");
 }
 
-int launch_adam(float* params, const float* grads, int nparts, int gp_layout, float* m, float* v, int64_t n, double lr, double beta1,
-                double beta2, double eps, int64_t step, const long long* step_dev, const double* lr_dev, float grad_scale, void* packed,
-                const Geo& g, const float* loss_partials, float* loss_out, cudaStream_t stream, int n_loss_parts) {
-  AdamArgs a = adam_args(params, m, v, n, lr, beta1, beta2, eps, step, step_dev, lr_dev, grad_scale, packed, g);
-  a.grads = grads; a.nparts = nparts; a.gp_layout = gp_layout;
-  a.loss_partials = loss_partials; a.loss_out = loss_out; a.n_loss_parts = n_loss_parts < 0 ? nparts : n_loss_parts;
-  const double bc1 = 1.0 - pow(beta1, (double)step), bc2 = 1.0 - pow(beta2, (double)step);
-  a.step_size = (float)(lr / bc1);
-  a.inv_bc2_sqrt = (float)(1.0 / sqrt(bc2));
-  const int64_t nj = gp_layout ? (int64_t)gp_total(g) : n;
-  if (few_slices(nparts, gp_layout) && nj <= 100000) { // small model: one thread per slot
+int launch_adam_partials(float* params, const float* partials, int nparts, float* m, float* v, double lr, double beta1,
+                         double beta2, double eps, int64_t step, const long long* step_dev, const double* lr_dev, void* packed,
+                         const Geo& g, const float* loss_partials, int n_loss, float* loss_out, cudaStream_t stream) {
+  AdamArgs a = adam_args(params, m, v, g.P, lr, beta1, beta2, eps, step, step_dev, lr_dev, 1.0f, packed, g);
+  a.grads = partials; a.nparts = nparts;
+  a.loss_partials = loss_partials; a.loss_out = loss_out; a.n_loss_parts = n_loss;
+  const int nj = gp_total(g);
+  if (few_slices(nparts) && nj <= 100000) {           // small model: one thread per slot
     adam_gp_wide_kernel<<<(unsigned)((nj + 255) / 256), 256, 0, stream>>>(a);
     count_launch();
     return check_launch("adam_gp_wide_kernel");
   }
-  if (few_slices(nparts, gp_layout)) {                 // large model (wide training): coalesced on both sides
+  if (few_slices(nparts)) {                            // large model: coalesced on both sides
     int blocks = 0, kpmax = 0;
     for (int l = 0; l < 4; ++l) { blocks += (g.cout[l] + kAdamCoGroup - 1) / kAdamCoGroup; kpmax = g.kp[l] > kpmax ? g.kp[l] : kpmax; }
     const size_t smem = (size_t)kAdamCoGroup * kpmax * B2H_KW * sizeof(float);
@@ -521,10 +536,19 @@ int launch_adam(float* params, const float* grads, int nparts, int gp_layout, fl
     count_launch();
     return check_launch("adam_gp_tile_kernel");
   }
-  if (nparts == 1) adam_kernel<<<(unsigned)((nj + 31) / 32), 32, 0, stream>>>(a);
-  else adam_kernel<<<(unsigned)((nj + 31) / 32), 256, 0, stream>>>(a);
+  adam_kernel<<<(unsigned)((nj + 31) / 32), 256, 0, stream>>>(a);
   count_launch();
   return check_launch("adam_kernel");
+}
+
+int launch_adam_flat(float* params, const float* grads, float* m, float* v, int64_t n, double lr, double beta1, double beta2,
+                     double eps, int64_t step, const long long* step_dev, const double* lr_dev, float grad_scale, void* packed,
+                     const Geo& g, cudaStream_t stream) {
+  AdamArgs a = adam_args(params, m, v, n, lr, beta1, beta2, eps, step, step_dev, lr_dev, grad_scale, packed, g);
+  a.grads = grads;
+  adam_flat_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(a);
+  count_launch();
+  return check_launch("adam_flat_kernel");
 }
 
 int launch_mask_output(float* y, const int32_t* lengths, int B, int T, int row, cudaStream_t stream) {

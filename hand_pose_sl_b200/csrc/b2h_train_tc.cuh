@@ -442,7 +442,8 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
 #pragma unroll
       for (int k = 0; k < 3; ++k) {
         if (k >= nk) continue;
-        // slot layout [k][ci/4][co][4]: for a fixed (k, q) the 16 lanes of a layer store 16 consecutive float4s
+        // slot layout [k][ci/4][co][4] (gp_slot_in_layer, b2h_common.cuh) as float4s: for a fixed (k, q) the 16 lanes
+        // of a layer store 16 consecutive float4s
         float4* dst = lp4 + (size_t)(k0 + k) * q4 * cout_l + co;
 #pragma unroll
         for (int q = 0; q < 8; ++q)

@@ -63,7 +63,7 @@ int64_t b2h_param_count(int n_in, int C, int pos_emb);
 int64_t b2h_param_offset(int n_in, int C, int pos_emb, int layer, int is_bias);
 /* bytes of the extension-owned packed weight buffer (fp32 tap-major + bf16 UMMA operand layouts) */
 int64_t b2h_packed_bytes(int n_in, int C, int pos_emb);
-/* Host-only self-check of the internal gradient-partial slot layout of the tensor-core train kernel (flat parameter
+/* Host-only self-check of the internal gradient-partial slot layout that every training kernel writes (flat parameter
  * index <-> slot bijection, padding slots, float4 alignment); returns the number of violations, 0 = consistent. */
 int64_t b2h_gp_layout_check(int n_in, int C, int pos_emb);
 /* Host-only query of the training path's window decomposition: returns the number of sub-windows a window of T frames is

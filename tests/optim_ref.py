@@ -128,10 +128,11 @@ def _prec(prec):
     return _lib.PRECISIONS[prec] if isinstance(prec, str) else int(prec)
 
 
-def tile_nparts(B, T, n_in, C, pe, prec):
-    """Gradient-partial slices (= CTAs) of the tile kernel's training path for this shape, from b2h_workspace_bytes:
-    roundup256(1024 + 4 * nparts * (gp_total + 1)) + 256.  The rounding slack is smaller than one slice."""
+def train_nparts(B, T, n_in, C, pe, prec):
+    """Gradient-partial slices (= CTAs) of the tile or the FFMA kernel's training path for this shape, from
+    b2h_workspace_bytes: roundup256(1024 + 4 * nparts * (gp_total + 1)) + 256.  The rounding slack is smaller than one
+    slice."""
     lib = _lib.load()
-    assert lib.b2h_kernel_choice(T, n_in, C, int(pe), _prec(prec), 1) == 2, "not a tile-kernel training shape"
+    assert lib.b2h_kernel_choice(T, n_in, C, int(pe), _prec(prec), 1) in (1, 2), "not a tile- or FFMA-kernel training shape"
     ws = _lib.workspace_bytes(B, T, n_in, C, pe, _prec(prec))
     return (ws - 256 - 1024) // (4 * (gp_total(n_in, C, pe) + 1))

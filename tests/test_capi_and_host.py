@@ -14,6 +14,7 @@ from hypothesis import given, settings, strategies as st
 import b2h_oracle as oracle
 import hand_pose_sl_b200 as b2h
 from hand_pose_sl_b200 import _lib
+from optim_ref import gp_total
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -58,13 +59,19 @@ def test_geometry_queries():
 
 
 def test_gradient_partial_slot_layout_is_a_bijection():
-    """The tensor-core train kernel reads its weight-gradient accumulators out as [k][ci/4][co][4] slots (coalesced
-    stores); the Adam tail maps slots back to flat parameter indices.  Host-side check of that map for every geometry
-    the kernel serves (incl. pos_emb's 25 input channels and C = 32 where cin == the padded reduction)."""
+    """Every train kernel writes its weight-gradient partials as [k][ci/4][co][4] slots (coalesced stores); the
+    reduction and Adam kernels map slots back to flat parameter indices.  Host-side check of that map for every geometry
+    the kernels serve (incl. pos_emb's 25 input channels and C = 32 where cin == the padded reduction)."""
     lib = _lib.load()
     for n_in, C, pe in ((24, 30, 0), (24, 30, 1), (24, 32, 0), (24, 16, 0), (16, 30, 0), (24, 64, 0), (24, 256, 0), (24, 1, 0)):
         assert lib.b2h_gp_layout_check(n_in, C, pe) == 0, (n_in, C, pe)
     assert lib.b2h_workspace_bytes(256, 64, 24, 30, 0, _lib.BF16) > 1024 + 128 * 19032 * 4
+    # the FFMA kernel's slices are slot-layout slices too: B = 4 windows run as 4 CTAs on any GPU, so the workspace is
+    # [1 KB header][4 slices of gp_total floats][4 loss partials], rounded up to 256 B, + 256 B
+    for C, prec in ((30, _lib.FP32_FFMA), (64, _lib.FP32), (128, _lib.FP32_FFMA)):
+        assert lib.b2h_kernel_choice(64, 24, C, 0, prec, 1) == 1, (C, prec)
+        want = (1024 + 4 * (4 * gp_total(24, C, 0) + 4) + 255) // 256 * 256 + 256
+        assert lib.b2h_workspace_bytes(4, 64, 24, C, 0, prec) == want, (C, prec)
 
 
 def test_kernel_choice_pins_the_tensor_core_paths():

@@ -2,8 +2,8 @@
 numpy restatement of its layout, byte for byte.
 
 Which kernel applies Adam depends on the entry point, the precision, the batch and conv_channels: adam_gp_wide_kernel,
-adam_kernel (slot or flat layout, many slices or one), adam_gp_tile_kernel, adam_dp_kernel, or the fused tail of the
-tile train kernel (one pass or several per CTA).  The bias corrections come in three forms: host pow(), device ipow and
+adam_kernel (more than 64 slices), adam_gp_tile_kernel, adam_flat_kernel (an already-reduced gradient), adam_dp_kernel,
+or the fused tail of the tile train kernel (one pass or several per CTA).  The bias corrections come in three forms: host pow(), device ipow and
 the tail's fp32 expm1f.  Each case pins its path (kernel choice, slice count, slot count) and then checks two
 consecutive steps, each from its own snapshot:
   m within 1e-5 * rms_l, v within 1e-5 relative, p within one fp32 ulp + 1e-4 * lr / (1 - b1^t),
@@ -17,7 +17,7 @@ import torch
 import b2h_oracle as oracle
 import hand_pose_sl_b200 as b2h
 from hand_pose_sl_b200 import _lib, synthetic
-from optim_ref import adam_step_f64, gp_total, pack_reference, tile_nparts
+from optim_ref import adam_step_f64, gp_total, pack_reference, train_nparts
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -45,9 +45,12 @@ CASES = [
     _case("fused-tile-bf16-C30-B130", "fused", "bf16", 30, 130, 0, loss="confL1", path="many"),
     _case("fused-tile-fp32-C30-B256", "fused", "fp32", 30, 256, 99999, path="many"),
     _case("fused-tile-bf16-C30-B256", "fused", "bf16", 30, 256, 9, path="many"),
-    # fused_train_step, fp32-ffma: adam_kernel on the flat layout, one slice per CTA, host pow()
-    _case("fused-ffma-C30-B8", "fused", "fp32-ffma", 30, 8, 9, loss="confL1"),
-    _case("fused-ffma-C64-B4", "fused", "fp32-ffma", 64, 4, 999),
+    # fused_train_step, fp32-ffma, one slice per CTA: <= 64 slices: adam_gp_wide_kernel up to 100 000 slots,
+    # adam_gp_tile_kernel above; > 64 slices: adam_kernel; host pow()
+    _case("fused-ffma-C30-B8", "fused", "fp32-ffma", 30, 8, 9, loss="confL1", path="few"),
+    _case("fused-ffma-C64-B4", "fused", "fp32-ffma", 64, 4, 999, path="few"),
+    _case("fused-ffma-C128-B4", "fused", "fp32-ffma", 128, 4, 0, path="few-slots>1e5"),
+    _case("fused-ffma-C30-B130", "fused", "fp32-ffma", 30, 130, 99999, path="many"),
     # fused_train_step, wide kernels (bf16): adam_gp_wide_kernel up to 100 000 slots, adam_gp_tile_kernel above
     _case("fused-wide-C64-B6", "fused", "bf16", 64, 6, 0, path="slots<=1e5"),
     _case("fused-wide-C80-B5-betas0.8-eps", "fused", "bf16", 80, 5, 9, betas=(0.8, 0.99), eps="rms", path="slots<=1e5"),
@@ -69,13 +72,13 @@ CASES = [
     _case("runner-tile-fp32-T200-B48", "runner", "fp32", 30, 48, 9, T=200, path="one-pass"),
     # TrainStepRunner, separate Adam launch with the device-side step counter and learning rate (device ipow)
     _case("runner-wide-C96-B6-lr-change", "runner", "bf16", 96, 6, 9, lr2=2e-4, path="slots>1e5"),
-    _case("runner-ffma-C64-B4", "runner", "fp32-ffma", 64, 4, 0, loss="confL1"),
-    # DataParallelTrainer without a process group: reduction, then adam_kernel on one flat slice, device ipow
+    _case("runner-ffma-C64-B4", "runner", "fp32-ffma", 64, 4, 0, loss="confL1", path="few"),
+    # DataParallelTrainer without a process group: reduction, then adam_flat_kernel on the reduced gradient, device ipow
     _case("dptrainer-bf16-C30-B16", "dptrainer", "bf16", 30, 16, 999, path="few"),
     # b2h_train_step_dp, world 1, grad_scale 0.5: the fused tail (tile) / reduce_* + adam_dp_kernel (three launches)
     _case("train_step_dp-tile-bf16-C30-B200", "dp", "bf16", 30, 200, 9, path="one-pass"),
     _case("train_step_dp-tile-fp32-C30-B8", "dp", "fp32", 30, 8, 99999, loss="confL1", path="multi-pass"),
-    _case("train_step_dp-ffma-C64-B4", "dp", "fp32-ffma", 64, 4, 0),
+    _case("train_step_dp-ffma-C64-B4", "dp", "fp32-ffma", 64, 4, 0, path="few"),
 ]
 
 
@@ -85,19 +88,17 @@ def _assert_path(c):
     pe = 1 if c["pe"] else 0
     choice = lib.b2h_kernel_choice(c["T"], N_IN, c["C"], pe, _lib.PRECISIONS[c["prec"]], 1)
     path = c["path"]
-    if c["prec"] == "fp32-ffma":
-        assert choice == FFMA
-        return
     slots = gp_total(N_IN, c["C"], pe)
     if path.startswith("slots"):
         assert choice == WIDE_TRAIN
         assert (slots <= 100000) == (path == "slots<=1e5"), slots
         return
-    assert choice == TILE
-    n = tile_nparts(c["B"], c["T"], N_IN, c["C"], pe, c["prec"])
+    assert choice == (FFMA if c["prec"] == "fp32-ffma" else TILE)
+    n = train_nparts(c["B"], c["T"], N_IN, c["C"], pe, c["prec"])
     per = ((slots + n - 1) // n + 3) // 4 * 4          # fused tail: slots per CTA (one pass while <= 256 threads)
-    if path == "few":
+    if path.startswith("few"):
         assert n <= 64, n
+        assert (slots <= 100000) == (path == "few"), slots
     elif path == "many":
         assert n > 64, n
     elif path == "multi-pass":

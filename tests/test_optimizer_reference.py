@@ -6,7 +6,7 @@ import pytest
 import torch
 
 from hand_pose_sl_b200 import _lib
-from optim_ref import adam_step_f64, gp_total, pack_reference, packed_layout, tile_nparts
+from optim_ref import adam_step_f64, gp_total, pack_reference, packed_layout, train_nparts
 
 
 @pytest.mark.parametrize("t", [1, 2, 10, 1000, 100000])
@@ -82,5 +82,5 @@ def test_tile_nparts_follows_the_batch():
     assumes 148 when no device is present)."""
     for B in (1, 2, 4, 127, 128, 130, 166, 168, 256, 296, 300):
         for prec in ("fp32", "bf16"):
-            assert tile_nparts(B, 64, 24, 30, 0, prec) == min(148, (B + 1) // 2), (B, prec)
+            assert train_nparts(B, 64, 24, 30, 0, prec) == min(148, (B + 1) // 2), (B, prec)
     assert gp_total(24, 30, 0) == 21260 and gp_total(24, 80, 0) == 93884 and gp_total(24, 96, 0) == 128012
