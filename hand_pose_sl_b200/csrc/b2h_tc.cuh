@@ -72,6 +72,11 @@ __device__ __forceinline__ bool mbar_wait_warp(uint64_t* bar, uint32_t parity, i
 }
 #endif  // B2H_TC_NO_STATUS
 
+// named barrier `id` (1..15; 0 is __syncthreads) over `nthreads` (whole warps)
+__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+
 // ---- proxies / fences -------------------------------------------------------------------------
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 // Programmatic dependent launch (sm_90+).  `launch_dependents`: the next kernel on the stream, if it was launched with the

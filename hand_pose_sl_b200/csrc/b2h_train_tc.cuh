@@ -20,8 +20,10 @@
 //
 // Per tile: F1 F2 F3 F4(+loss,+dY) | D4,W4 | D3,W3 | D2,W2 | W1.   F/D = conv GEMM + epilogue
 // (tcgen05.ld -> bias/ReLU or ReLU-mask -> bf16 -> st.shared); W = weight/bias-gradient GEMMs that keep
-// accumulating in TMEM across all tiles of the CTA (issued right after D so they run under D's epilogue) and
-// are read out once at the end into the CTA's slice of the partials workspace (deterministic 2-stage sum).
+// accumulating in TMEM across all tiles of the CTA and are read out once at the end into the CTA's slice of the
+// partials workspace (deterministic 2-stage sum).  In the backward warps 0/1 only issue MMAs and warps 2..7 run the
+// D epilogues, each under the W GEMMs issued right after its D, so the tensor pipe runs D4 W4 D3 W3 D2 W2 W1 back to
+// back; an mbarrier handshake (not __syncthreads) tells the issuers that the next D's operand is ready.
 //
 // Measured on B200: one tcgen05.mma costs >= ~25 (M=64) / ~40 (M=128) cycles whatever N <= 64 is, so the MMA
 // phases are instruction-count bound at C=30: descriptors are pre-encoded (one integer add per MMA) and the
@@ -222,6 +224,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
   __shared__ __align__(8) uint64_t bar;      // MMAs of the current phase complete (one arrival per issuing warp)
   __shared__ __align__(8) uint64_t wbar;     // weights + biases landed (bulk async copies)
   __shared__ __align__(8) uint64_t tbar;     // target tile landed (train)
+  __shared__ __align__(8) uint64_t ebar;     // backward: dZ_{l-1} stored and the dgrad accumulator read (one arrival per epilogue warp)
   __shared__ uint32_t tmem_slot;
   __shared__ __align__(16) float bias_s[4][64];
   __shared__ float red_s[8];
@@ -349,6 +352,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
     mbar_init(&bar, nissue);
     mbar_init(&wbar, 1);
     mbar_init(&tbar, 1);
+    if (TRAIN) mbar_init(&ebar, kTileThreads / 32 - 2);
     fence_barrier_init();
   }
   auto zero_buffers = [&]() {   // zero every activation / gradient buffer once: pad rows and pad channels stay zero
@@ -405,7 +409,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
   __syncthreads();
   tc_fence_after();
   const uint32_t tbase = tmem_slot;
-  uint32_t phase = 0, tphase = 0;
+  uint32_t phase = 0, tphase = 0, ephase = 0;
   float loss_acc = 0.0f;
   bool wg_started = false, weights_ready = false;
   B2H_STAMP();   // setup done
@@ -417,9 +421,9 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
 
   // Read one layer pair's weight / bias gradient accumulators out into this CTA's partial slice.  A pair shares its
   // TMEM columns: lanes 32q+i hold layer 2p (co = 16q+i), lanes 32q+16+i layer 2p+1, so one tcgen05.ld per tap
-  // serves both layers and every lane has a row to store.
-  bool pair1_done = false;
-  auto readout_pair = [&](int pr) {
+  // serves both layers and every lane has a row to store.  Column half 0 holds taps 0..2, half 1 taps 3..4 and the bias
+  // column; the warp reads halves h0..h1 of its lane quadrant.
+  auto readout_pair = [&](int pr, int h0, int h1) {
     float* part = p.partials + (size_t)blockIdx.x * gp_total(g);
     const int l = 2 * pr + (lane >> 4);
     const int co = (warp & 3) * 16 + (lane & 15);
@@ -429,29 +433,30 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
     float4* lp4 = reinterpret_cast<float4*>(lp);
     const int q4 = Nw >> 2, cout_l = g.cout[l];
     const uint32_t dcol = tbase + lane_addr + kWgCol + pr * kWgPairCols;
-    // column half 0 reads taps 0..2, half 1 taps 3..4 and the bias column
-    const int k0 = ch == 0 ? 0 : 3, nk = ch == 0 ? 3 : 2;
-    uint32_t v[3][32];
+    for (int hc = h0; hc <= h1; ++hc) {
+      const int k0 = hc == 0 ? 0 : 3, nk = hc == 0 ? 3 : 2;
+      uint32_t v[3][32];
 #pragma unroll
-    for (int k = 0; k < 3; ++k)
-      if (k < nk) tmem_ld32(dcol + (k0 + k) * 32, v[k]);
-    uint32_t vb[16];
-    if (ch == 1) tmem_ld16(dcol + 5 * 32, vb);      // 8 valid columns; column 0 holds db (ones sits in element 0)
-    tmem_ld_wait();
-    if (mine) {
+      for (int k = 0; k < 3; ++k)
+        if (k < nk) tmem_ld32(dcol + (k0 + k) * 32, v[k]);
+      uint32_t vb[16];
+      if (hc == 1) tmem_ld16(dcol + 5 * 32, vb);      // 8 valid columns; column 0 holds db (ones sits in element 0)
+      tmem_ld_wait();
+      if (mine) {
 #pragma unroll
-      for (int k = 0; k < 3; ++k) {
-        if (k >= nk) continue;
-        // slot layout [k][ci/4][co][4] (gp_slot_in_layer, b2h_common.cuh) as float4s: for a fixed (k, q) the 16 lanes
-        // of a layer store 16 consecutive float4s
-        float4* dst = lp4 + (size_t)(k0 + k) * q4 * cout_l + co;
+        for (int k = 0; k < 3; ++k) {
+          if (k >= nk) continue;
+          // slot layout [k][ci/4][co][4] (gp_slot_in_layer, b2h_common.cuh) as float4s: for a fixed (k, q) the 16 lanes
+          // of a layer store 16 consecutive float4s
+          float4* dst = lp4 + (size_t)(k0 + k) * q4 * cout_l + co;
 #pragma unroll
-        for (int q = 0; q < 8; ++q)
-          if (q * 4 < Nw)
-            dst[(size_t)q * cout_l] = make_float4(__uint_as_float(v[k][4 * q]), __uint_as_float(v[k][4 * q + 1]),
-                                                  __uint_as_float(v[k][4 * q + 2]), __uint_as_float(v[k][4 * q + 3]));
+          for (int q = 0; q < 8; ++q)
+            if (q * 4 < Nw)
+              dst[(size_t)q * cout_l] = make_float4(__uint_as_float(v[k][4 * q]), __uint_as_float(v[k][4 * q + 1]),
+                                                    __uint_as_float(v[k][4 * q + 2]), __uint_as_float(v[k][4 * q + 3]));
+        }
+        if (hc == 1) lp[B2H_KW * g.cout[l] * Nw + co] = __uint_as_float(vb[0]);
       }
-      if (ch == 1) lp[B2H_KW * g.cout[l] * Nw + co] = __uint_as_float(vb[0]);
     }
   };
 
@@ -764,13 +769,24 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
 
     if (TRAIN) {
       // =========================== backward ===========================
-      // dZ_l (grad wrt layer l's pre-activation) ping-pongs G0 (l=3) -> G1 (l=2) -> G0 (l=1) -> G1 (l=0)
+      // dZ_l (grad wrt layer l's pre-activation) ping-pongs G0 (l=3) -> G1 (l=2) -> G0 (l=1) -> G1 (l=0).
+      // Warps 0/1 only issue: the tensor pipe runs D4 W4 D3 W3 D2 W2 W1 back to back, and the issuers wait only for the
+      // epilogue handshake (ebar) before each dgrad and for each other between dgrad and wgrad.  Warps 2..7 wait for dgrad_l's commit and run its ReLU-mask
+      // epilogue while wgrad_l is in the pipe; warps 4/5 take all columns of lane quadrants 0/1.  The epilogue's only
+      // write hazard, the dZ buffer wgrad_{l+1} read, is clear: that commit also covers wgrad_{l+1}.
+      const bool last_tile = tile + (int)gridDim.x >= p.n_tiles;
+      const bool both = warp == 4 || warp == 5;
       for (int l = 3; l >= 0; --l) {
         unsigned char* gz = ((3 - l) & 1) ? G1 : G0;          // dZ_l
         unsigned char* gnext = ((3 - l) & 1) ? G0 : G1;       // dZ_{l-1}
         unsigned char* ain = (l == 0) ? X : (l == 1) ? A1 : (l == 2) ? A2 : A3;   // layer l's input activation
         if (warp < nissue) {
           if (elect_one()) {
+            if (l < 3) {                         // dZ_l is in shared memory and the dgrad accumulator has been read
+              mbar_wait(&ebar, ephase, 40 + l);
+              tc_fence_after();
+              B2H_STAMP();   // bwd layer: epilogue handshake passed
+            }
             if (l > 0) {  // dgrad: dA_{l-1}[r][ci] = sum_{k',co} dZ_l[r+k'-2][co] * W_l[co][ci][4-k']
               const int KSd = round_up(g.cout[l], 16) >> 4, Nd = round_up(g.cin[l], 16);
               const uint32_t a_lo = desc_lo(smem_u32(gz), (uint32_t)CH) + warp * seg_row;
@@ -801,6 +817,12 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
               }
               umma_commit(&bar);
             }
+          }
+          __syncwarp();
+          // both segments' dgrad enter the tensor pipe ahead of either warp's wgrad, so that the epilogue can start as
+          // soon as possible
+          if (nissue == 2 && l > 0) named_bar_sync(1, 64);
+          if (elect_one()) {
             // wgrad: dW_l[k][co][ci] += sum_r dZ_l[r][co] * in_l[r+k-2][ci];  db_l[co] += sum_r dZ_l[r][co]
             // A = dZ_l read MN-major (M = co, 8 chunks), B = in_l read MN-major (N = ci), K = 16 frames per MMA.
             // The six accumulators (5 taps + bias) are split between the issuing warps (disjoint TMEM columns).
@@ -835,12 +857,14 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
           }
           __syncwarp();
         }
-        B2H_STAMP();   // bwd layer: MMAs issued
-        mbar_wait(&bar, phase, 30 + l);
-        phase ^= 1;
-        tc_fence_after();
-        B2H_STAMP();   // bwd layer: dgrad accumulator ready
-        if (l > 0) {
+        if (warp < 2) {                          // (warp 1 idles when one warp issues: nissue == 1)
+          if (l < 3) ephase ^= 1;
+          if (l > 0) phase ^= 1;                 // the issuers do not wait for the dgrad commits
+          B2H_STAMP();   // bwd layer: MMAs issued
+        } else if (l > 0) {
+          mbar_wait_warp(&bar, phase, 30 + l);   // dgrad_l complete (and with it wgrad_{l+1}, issued before it)
+          phase ^= 1;
+          tc_fence_after();
           // dZ_{l-1} = dA_{l-1} * (a_{l-1} > 0)     (ReLU backward on the saved activation)
           const int Nd = round_up(g.cin[l], 16);
           for (int j = 0; j < NT; ++j) {
@@ -848,7 +872,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
           const int row = rc.row;
           const bool valid = rc.valid;
           const uint32_t taddr = tbase + lane_addr + kAccCol + 64 * j;
-          for (int c0 = 16 * ch; c0 < Nd; c0 += 32) {
+          for (int c0 = both ? 0 : 16 * ch; c0 < Nd; c0 += both ? 16 : 32) {
             uint32_t v[16];
             tmem_ld16(taddr + c0, v);
             tmem_ld_wait();
@@ -861,19 +885,26 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
             store8_act<SPLIT>(gnext, LO, CH, row, (c0 >> 3) + 1, f + 8);
           }
           }   // MMA tiles j
+          // hand dZ_{l-1} (generic-proxy stores) and the free dgrad accumulator to the issuers
+          fence_proxy_async_smem();
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive(&ebar);
+          if (l == 1 && last_tile) {
+            // last tile of this CTA: W_4 and W_3 (layer pair 1) are final (their MMAs precede dgrad_1's commit) -> read
+            // them out under the tensor-pipe time of W_2 / W_1
+            readout_pair(1, both ? 0 : ch, both ? 1 : ch);
+          }
         }
-        if (l == 1 && tile + (int)gridDim.x >= p.n_tiles) {
-          // last tile of this CTA: W_4 and W_3 (layer pair 1) are final (their MMAs precede the commit just waited
-          // on) -> read them out now, under the tensor-pipe time of W_2 / W_1 instead of after the loop
-          readout_pair(1);
-          pair1_done = true;
-        }
-        fence_proxy_async_smem();
-        tc_fence_before();
-        __syncthreads();
-        tc_fence_after();
-        B2H_STAMP();   // bwd layer: epilogue done
       }
+      mbar_wait(&bar, phase, 30);                // wgrad_0: every MMA of the tile is complete
+      phase ^= 1;
+      B2H_STAMP();   // bwd: last weight-gradient MMA complete
+      fence_proxy_async_smem();
+      tc_fence_before();
+      __syncthreads();
+      tc_fence_after();
+      B2H_STAMP();   // bwd: epilogue warps done (pair-1 read-out)
       wg_started = true;
     }
   }
@@ -884,8 +915,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
       float* part = p.partials + (size_t)blockIdx.x * gp_total(g);
       for (int i = tid; i < gp_total(g); i += kTileThreads) part[i] = 0.0f;
     } else {
-      readout_pair(0);
-      if (!pair1_done) readout_pair(1);
+      readout_pair(0, ch, ch);                     // (pair 1 was read out under the last tile's W2 / W1)
     }
     if (tid == 0 && p.loss_partials)
       p.loss_partials[blockIdx.x] = (p.loss_kind == B2H_LOSS_L1) ? loss_acc / (float)p.loss_B : loss_acc;

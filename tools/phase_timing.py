@@ -26,7 +26,9 @@ FWD = (["start", "pre-wait", "setup", "staging", "weights"] + [f"F{l}:{p}" for l
        + ["F3:issued", "F3:ready", "F3:target", "F3:chunk0", "F3:chunk1", "F3:epilogue"])
 TRAIN = (["start", "pre-wait", "setup", "staging", "weights"] + [f"F{l}:{p}" for l in range(3) for p in ("issued", "ready", "epilogue")]
          + ["F3:issued", "F3:ready", "F3:target", "F3:chunk0", "F3:chunk1", "F3:epilogue"]
-         + [f"B{l}:{p}" for l in (3, 2, 1, 0) for p in ("issued", "ready", "epilogue")]
+         # backward, stamped by the issuing thread: "wait" = for the epilogue handshake before dgrad / wgrad_0 (the tensor
+         # pipe still works off the previous wgrad), "ready" = wgrad_0 complete, "sync" = epilogue warps done
+         + ["B3:issued"] + [f"B{l}:{p}" for l in (2, 1, 0) for p in ("wait", "issued")] + ["B0:ready", "B:sync"]
          + ["readout", "barrier", "gather"])
 TAIL1 = ["adam", "end"]
 TAILDP = ["pushed", "collected", "adam", "end"]
