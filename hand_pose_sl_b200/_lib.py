@@ -52,6 +52,11 @@ _SIGNATURES = {
                                  c_int, c_int, c_int, c_float, c_void_p]),
     "b2h_conv_forward_windows": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                          c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p]),
+    "b2h_conv_forward_utterances": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int,
+                                            c_int, c_int, c_int, c_float, c_void_p, c_int64, c_void_p]),
+    "b2h_utterances_workspace_bytes": (c_int64, [c_int64, c_int, c_int, c_int, c_int, c_int]),
+    "b2h_utterances_plan": (c_int, [c_int64, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "b2h_utterance_subwindows": (c_int, [c_int, c_int, c_int, c_void_p]),
     "b2h_train_forward_backward": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                            c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p,
                                            c_void_p, c_int64, c_void_p]),

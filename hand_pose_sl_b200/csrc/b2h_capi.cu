@@ -92,6 +92,45 @@ static TrainPlan train_plan(const Geo& g, int B, int T, int precision) {
   return t;
 }
 
+// Which kernel and sub-window length b2h_conv_forward_utterances runs for n_utt utterances in a stream of n_frames frames:
+// the ONE place that decides.  Per length Ts of the menu the family is the tile forward where it fits (bf16 and fp32 mode),
+// else the wide forward (bf16 mode); the plan takes the Ts whose family computes the fewest MMA rows for an utterance of the
+// mean length n_frames / n_utt under the cut rule (ties: the longer Ts, fewer sub-windows).  Rows per sub-window are the
+// tile's rows over the windows it holds: 64 / 128 / 256 in the tile kernel, 256 / floor(258 / (Ts + 2)) in the wide one.
+static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int precision) {
+  static const int kMenu[3] = {256, 128, 64};
+  UttPlan best{};
+  best.kernel = B2H_KERNEL_NONE;
+  if (precision != B2H_BF16 && precision != B2H_FP32) return best;   // the FFMA kernel reads dense windows only
+  const int64_t mean = n_frames / (n_utt > 0 ? n_utt : 1);
+  double best_rows = 0.0;
+  for (int Ts : kMenu) {
+    const int64_t max_sub = (int64_t)(n_utt > 0 ? n_utt : 0) + n_frames / (Ts - 32);
+    if (max_sub > (int64_t)INT32_MAX / 2) continue;
+    UttPlan c{};
+    c.Ts = Ts;
+    c.max_sub = (int)max_sub;
+    const int B = c.max_sub > 0 ? c.max_sub : 1;
+    c.tile = plan_tile(g, B, Ts, false, is_split(precision));
+    double rows_per_sub = 0.0;
+    if (c.tile.ok) {
+      c.kernel = B2H_KERNEL_TC_TILE;
+      rows_per_sub = (double)c.tile.MB / c.tile.gh;
+    } else if (precision == B2H_BF16 && (c.wide = plan_wide(g, B, Ts)).ok) {
+      c.kernel = B2H_KERNEL_TC_WIDE;
+      rows_per_sub = 256.0 / c.wide.gh;
+    } else {
+      continue;
+    }
+    const double rows = rows_per_sub * sub_window_count(mean > 0 ? mean : 1, Ts);
+    if (best.kernel != B2H_KERNEL_NONE && rows >= best_rows) continue;
+    c.ws_bytes = (utt_prefix_offset(c.max_sub) + 4 * ((int64_t)n_utt + 1) + 255) / 256 * 256;
+    best = c;
+    best_rows = rows;
+  }
+  return best;
+}
+
 }  // namespace b2h
 
 using namespace b2h;
@@ -256,6 +295,76 @@ extern "C" int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t
   const WindowView wv = window_view(win_start, win_end, n_frames, pad_mode);
   return conv_forward(frames, x_dtype, &wv, params, packed, lengths, y, n_win, T, n_in, C, pos_emb, precision, apply_mask,
                       out_scale, (cudaStream_t)stream, "b2h_conv_forward_windows");
+}
+
+static const char* const kUttServed =
+    "utterances are served in bf16 mode for conv_channels <= 256 and in fp32 mode for conv_channels <= 32 with at most 32 "
+    "input channels";
+
+extern "C" int b2h_utterances_plan(int64_t n_frames, int n_utt, int n_in, int C, int pos_emb, int precision, int* seg_len) {
+  if (seg_len) *seg_len = 0;
+  if (!geo_ok(n_in, C, pos_emb) || n_frames < 0 || n_frames > INT32_MAX || n_utt < 0) return B2H_KERNEL_NONE;
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), n_frames, n_utt, precision);
+  if (seg_len && u.kernel != B2H_KERNEL_NONE) *seg_len = u.Ts;
+  return u.kernel;
+}
+
+extern "C" int b2h_utterance_subwindows(int L, int Ts, int i, int* out3) {
+  if (L < 0 || Ts <= 32) { set_error("b2h_utterance_subwindows: bad L=%d Ts=%d", L, Ts); return B2H_ESHAPE; }
+  const int n = sub_window_count(L, Ts);
+  if (out3) {
+    if (i < 0 || i >= n) { set_error("b2h_utterance_subwindows: sub-window %d of %d", i, n); return B2H_EINVAL; }
+    if (n == 1) { out3[0] = 0; out3[1] = 0; out3[2] = L; }
+    else {
+      const SubWindow s = sub_window(L, Ts, n, i);
+      out3[0] = s.start; out3[1] = s.clo; out3[2] = s.chi;
+    }
+  }
+  return n;
+}
+
+extern "C" int64_t b2h_utterances_workspace_bytes(int64_t n_frames, int n_utt, int n_in, int C, int pos_emb, int precision) {
+  const char* who = "b2h_utterances_workspace_bytes";
+  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
+  if (n_frames < 0 || n_frames > INT32_MAX || n_utt < 0) { set_error("%s: bad n_frames=%lld n_utt=%d", who, (long long)n_frames, n_utt); return B2H_ESHAPE; }
+  if (n_utt == 0) return 256;
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), n_frames, n_utt, precision);
+  if (u.kernel == B2H_KERNEL_NONE) { set_error("%s: %s (C=%d, n_in=%d, precision=%d)", who, kUttServed, C, n_in, precision); return B2H_ESHAPE; }
+  return u.ws_bytes;
+}
+
+extern "C" int b2h_conv_forward_utterances(const void* frames, int x_dtype, int64_t n_frames, const int64_t* offsets, int n_utt,
+                                           const float* params, const void* packed, float* y, int n_in, int C, int pos_emb,
+                                           int precision, float out_scale, void* workspace, int64_t workspace_bytes,
+                                           void* stream) {
+  const char* who = "b2h_conv_forward_utterances";
+  if (!offsets || !workspace) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  if (int rc = check_common(frames, x_dtype, nullptr, params, packed, y, 1, 0, 1, n_in, C, pos_emb, who)) return rc;
+  if (n_utt < 0 || n_frames < 0 || n_frames > INT32_MAX) {
+    set_error("%s: bad n_utt=%d n_frames=%lld", who, n_utt, (long long)n_frames);
+    return B2H_ESHAPE;
+  }
+  if (n_utt == 0) return B2H_OK;
+  if (misaligned(frames, 15) || misaligned(y, 15) || misaligned(packed, 15) || misaligned(workspace, 15) || misaligned(offsets, 7)) {
+    set_error("%s: frames, y, packed and workspace must be 16-byte aligned, offsets 8-byte aligned", who);
+    return B2H_EALIGN;
+  }
+  if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
+  const Geo g = make_geo(n_in, C, pos_emb);
+  const UttPlan plan = utterance_plan(g, n_frames, n_utt, precision);
+  if (plan.kernel == B2H_KERNEL_NONE) {
+    set_error("%s: %s; no kernel for C=%d, n_in=%d, precision=%d", who, kUttServed, C, n_in, precision);
+    return B2H_ESHAPE;
+  }
+  if (workspace_bytes < plan.ws_bytes) {
+    set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.ws_bytes);
+    return B2H_EWORKSPACE;
+  }
+  ConvArgs a{};
+  a.x = frames; a.x_dtype = x_dtype; a.params = params; a.packed = reinterpret_cast<const char*>(packed);
+  a.y = y; a.mode = 0; a.out_scale = out_scale; a.geo = g;
+  return launch_utterances(a, plan, reinterpret_cast<const long long*>(offsets), n_utt, (long long)n_frames, workspace,
+                           (cudaStream_t)stream);
 }
 
 // What a training launch left for the reduction / Adam launches that follow it (rc != B2H_OK: nothing was launched).

@@ -214,6 +214,16 @@ __host__ __device__ inline SubWindow sub_window(int T, int Ts, int n_sub, int i)
   s.start = st; s.clo = cb0 - st; s.chi = cb1 - st;
   return s;
 }
+// Number of sub-windows of Ts frames the cut rule above makes of a sequence of L frames (n_sub of sub_window): 0 for an empty
+// one, 1 for L <= Ts (one sub-window, core [0, L)), otherwise the least n >= 2 whose cores (Ts - 16) * 2 + (n - 2) * (Ts - 32)
+// = n (Ts - 32) + 32 frames cover L.  So n <= 1 + L / (Ts - 32) for every L, and a set of sequences with F frames in all
+// is cut into at most n_seq + F / (Ts - 32) sub-windows (the bound that sizes the utterance forward's grid and workspace).
+__host__ __device__ inline int sub_window_count(long long L, int Ts) {
+  if (L <= 0) return 0;
+  if (L <= Ts) return 1;
+  const long long n = (L - 32 + (Ts - 32) - 1) / (Ts - 32);
+  return n < 2 ? 2 : (int)n;
+}
 
 // Workspace header of the fused train kernel (first B2H_WS_HEADER bytes of the caller's workspace, zeroed once when the
 // workspace is allocated and owned by the kernels afterwards; FIXED offset, so runners of different (B, T) that share
@@ -327,6 +337,7 @@ struct ConvArgs {
   float out_scale;
   Geo geo;
   WindowView wv;            // tensor-core kernels only: win_start set = x (and target / conf) are frame streams, B = windows
+  const int4* utt;          // forward over utterances (b2h_utterances.cuh): the device-side plan, x a frame stream; else nullptr
 };
 int launch_fp32(const ConvArgs& a, const FfmaPlan& plan, cudaStream_t stream);
 int launch_tc_fwd(const ConvArgs& a, const RowspacePlan& plan, cudaStream_t stream);
@@ -338,6 +349,23 @@ int launch_tc_wide_fwd(const ConvArgs& a, const WidePlan& plan, cudaStream_t str
 int launch_tc_wide_train(const ConvArgs& a, const WidePlan& plan, unsigned char* scratch, cudaStream_t stream);
 int launch_tc_probe(const void* a, const void* b, float* out, int n, int ksteps, int shift, int variant, cudaStream_t stream);
 int tc_status_and_clear();
+
+// Forward over packed utterances (b2h_conv_forward_utterances): every utterance is cut into sub-windows of Ts frames by
+// sub_window(); the forward kernels read sub-window g from a table that a one-CTA planning kernel builds on the device.
+// Workspace: [int4 {sub-window count, 0, 0, 0}][int4 per sub-window, max_sub of them][int prefix[n_utt + 1]], where
+// sub-window g = {stream row of its first frame, its first frame in the utterance, clo | chi << 16, frames before the
+// utterance end (<= Ts)}.
+struct UttPlan {
+  int kernel;               // B2H_KERNEL_TC_TILE | B2H_KERNEL_TC_WIDE | B2H_KERNEL_NONE
+  int Ts;                   // sub-window length
+  int max_sub;              // upper bound on the sub-window count: n_utt + n_frames / (Ts - 32)
+  TilePlan tile; WidePlan wide;   // planned for max_sub windows of Ts frames
+  int64_t ws_bytes;
+};
+__host__ __device__ inline int64_t utt_prefix_offset(int max_sub) { return (int64_t)(1 + max_sub) * 16; }
+// planning kernel, then the forward of a.B = plan.max_sub sub-windows of a.T = plan.Ts frames over the table it wrote
+int launch_utterances(ConvArgs a, const UttPlan& plan, const long long* offsets, int n_utt, long long n_frames, void* workspace,
+                      cudaStream_t stream);
 
 void set_debug_timing(long long* p);
 int launch_format_prediction(const float* pred, float* out, int64_t rows, int mode, cudaStream_t stream);

@@ -360,3 +360,4 @@ int tc_status_and_clear() {
 
 #include "b2h_train_tc.cuh"
 #include "b2h_wide_tc.cuh"
+#include "b2h_utterances.cuh"

@@ -63,6 +63,9 @@ struct TcTileArgs {
   float out_scale;
   int n_tiles, nhalf, MB, HR, gh, NT;      // tile geometry (NT = 128-row MMA tiles per segment: 2 for 128 < T <= 256)
   Geo geo;
+  // Forward over utterances (UTT instantiations): x is a frame stream and window g < utt[0].x is sub-window utt[1 + g] of the
+  // plan (UttPlan, b2h_common.cuh); B / n_tiles are the host's upper bound on the sub-window count.
+  const int4* utt;
 };
 
 constexpr int kTileThreads = 256;   // 8 warps: two per TMEM lane quadrant (each takes every other 16-column chunk)
@@ -217,8 +220,12 @@ __device__ __forceinline__ long long global_ns() { long long t; asm volatile("mo
 // VIEW (training only) = window views of frame streams: target / confidence rows through the view, per-window staging of
 // the target tile.  A separate instantiation: the same code behind a run-time test made the dense 256x64 step 1.9 us
 // slower (27.4 -> 29.3 us) with the same register count.  The forward kernel tests p.win_start at run time.
-template <bool TRAIN, int NT, bool SPLIT, bool VIEW = false>
+// UTT (forward only) = sub-windows of utterances (b2h_conv_forward_utterances): window g reads its rows from the plan's
+// table, rows at or past the utterance end are zero in every layer (the sequence ends there), and only the core rows
+// are written, to y at their stream rows.
+template <bool TRAIN, int NT, bool SPLIT, bool VIEW = false, bool UTT = false>
 __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArgs p) {
+  static_assert(!(UTT && TRAIN), "utterances are a forward-only view");
   int dbg_n = 0;
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) uint64_t bar;      // MMAs of the current phase complete (one arrival per issuing warp)
@@ -255,7 +262,9 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
   const int hh = (nhalf == 2) ? ((r128 >> 4) & 1) : 0;
   const int m = (nhalf == 2) ? ((r128 >> 5) * 16 + (r128 & 15)) : r128;
   // row context of this thread in MMA tile j of its segment (NT > 1 only with one 128*NT-row segment per tile)
-  struct RowCtx { int row, t, gw; bool valid; };
+  // UTT: us = the row's sub-window {stream row of frame 0, frame 0 in the utterance, clo | chi << 16, frames before the end}
+  int utt_n = 0;                                 // UTT: sub-windows in the plan (read after griddep_wait)
+  struct RowCtx { int row, t, gw; bool valid; int4 us; };
   auto rowctx = [&](int j, int wbase) {
     const int mm = m + 128 * j;
     const int wjj = mm / (T + 2);
@@ -264,18 +273,23 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
     r.row = hh * HR + 2 + mm;
     r.gw = wbase + hh * gh + wjj;
     r.valid = (r.t < T) && (wjj < gh) && (r.gw < p.B);
+    if constexpr (UTT) {
+      const bool in = (wjj < gh) && (r.gw < utt_n);
+      r.us = in ? __ldg(p.utt + 1 + r.gw) : make_int4(0, 0, 0, 0);
+      r.valid = in && r.t < r.us.w;
+    }
     return r;
   };
   const int wj = m / (T + 2), t = m - wj * (T + 2);     // tile 0 (prefetch path, NT == 1)
   const uint32_t lane_addr = (uint32_t)((warp & 3) * 32) << 16;
   const int srow = hh * MB + m;                  // row of this thread in the fp32 staging tile
-  const bool bulk_io = (T & 1) == 0 && NT == 1 && !(SPLIT && TRAIN);  // T*168 B and the staging row offsets are 16-B multiples; the split training kernel has no staging tile
+  const bool bulk_io = (T & 1) == 0 && NT == 1 && !(SPLIT && TRAIN) && !UTT;  // T*168 B and the staging row offsets are 16-B multiples; the split training kernel has no staging tile; utterances write core rows only
   const int wpt = nhalf * gh;                    // windows per tile
   const int nissue = (nhalf == 2) ? 2 : NT;      // issuing warps: one per row segment / per 128-row MMA tile
   const uint32_t idesc_M = (nhalf == 2) ? 64 : 128;
   const int n_in = g.n_in;
   const bool vec_in = (g.pos_emb == 0) && ((n_in & 7) == 0) && n_in <= 32;   // <= 4 chunks: 16-B vector loads
-  const bool fast_in = vec_in && NT == 1;        // + register prefetch one tile ahead
+  const bool fast_in = vec_in && NT == 1 && !UTT;   // + register prefetch one tile ahead
   const int seg_row = (nhalf == 2) ? HR : 128;   // row offset / TMEM offset of issuing warp w's accumulator
   const uint32_t seg_d = (nhalf == 2) ? (16u << 16) : 64u;
   const int cpr = n_in >> 3;
@@ -367,8 +381,14 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
   // ---- part 2: the previous kernel has completed and its writes (weights, Adam state, counters, inputs) are visible ----
   griddep_wait();
   B2H_STAMP();   // predecessor complete
+  int utt_tiles = 0;
+  if constexpr (UTT) {                           // the plan's count: CTAs past it have no tile and load no weights
+    utt_n = __ldg(&p.utt->x);
+    const int need = (utt_n + wpt - 1) / wpt;
+    utt_tiles = need < p.n_tiles ? need : p.n_tiles;
+  }
   prefetch_x(blockIdx.x);
-  if (tid == 0) {
+  if (tid == 0 && (!UTT || (int)blockIdx.x < utt_tiles)) {
     // weights (packed bf16 UMMA blocks) + zero-padded biases -> smem once per CTA: 1-D bulk async copies (TMA engine)
     // that run under the first tile's input staging; completion is signalled on wbar.
     uint32_t total = 4 * 64 * 4;
@@ -460,7 +480,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
     }
   };
 
-  for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
+  for (int tile = blockIdx.x; tile < (UTT ? utt_tiles : p.n_tiles); tile += gridDim.x) {
     const int wbase = tile * wpt;
     // sequence lengths of this thread's rows, fetched at tile start so the load is long complete at the layer-4 epilogue
     int lens[NT];
@@ -505,7 +525,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
       const int pe = g.pos_emb;
       const int nch0 = g.kp[0] / 8;
       if (rc.valid && vec_in) {
-        if (!fast_in) load_x_row(xrow_of(rc.gw, rc.t));   // no prefetch (NT > 1): load this row now
+        if (!fast_in) load_x_row(UTT ? (long long)rc.us.x + rc.t : xrow_of(rc.gw, rc.t));   // no prefetch: load this row now
         if (p.x_dtype == B2H_DT_F32) {
 #pragma unroll
           for (int c8 = 0; c8 < 4; ++c8)
@@ -523,14 +543,14 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
             }
         }
       } else if (rc.valid) {
-        const long long xr = xrow_of(rc.gw, rc.t);
+        const long long xr = UTT ? (long long)rc.us.x + rc.t : xrow_of(rc.gw, rc.t);
         for (int c8 = ch; c8 < nch0; c8 += 2) {
           float v[8];
 #pragma unroll
           for (int e = 0; e < 8; ++e) {
             const int cc = c8 * 8 + e;            // channel in the conv1 input (pos-emb row first)
             float val = 0.0f;
-            if (pe && cc == 0) val = __fdiv_rn((float)(subw(rc.gw).start + rc.t), (float)g.pe_len);   // HandPoseModels.py:70-82
+            if (pe && cc == 0) val = __fdiv_rn((float)((UTT ? rc.us.y : subw(rc.gw).start) + rc.t), (float)g.pe_len);   // HandPoseModels.py:70-82
             else if (cc - pe < n_in && cc - pe >= 0 && xr >= 0) {
               const size_t gi = (size_t)xr * n_in + (cc - pe);
               val = (p.x_dtype == B2H_DT_F32) ? __ldg(reinterpret_cast<const float*>(p.x) + gi)
@@ -614,8 +634,9 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
         int len = lens[j];
         float n_el = 0.f, scale = 0.f;
         const float* tg = nullptr; const float* cf = nullptr; const float* dy = nullptr;
-        const size_t drow = valid ? (size_t)dense_row(gw, t) : 0;       // row of this frame in the dense (B, T, .) arrays
-        bool in_core = true, zrow = false;
+        // row of this frame in the dense (B, T, .) arrays; UTT: its stream row, written only in the sub-window's core
+        const size_t drow = valid ? (UTT ? (size_t)rc.us.x + t : (size_t)dense_row(gw, t)) : 0;
+        bool in_core = UTT ? (t >= (rc.us.z & 0xFFFF) && t < (rc.us.z >> 16)) : true, zrow = false;
         if (TRAIN && valid) {
           n_el = (float)len * (float)B2H_COUT;                      // (sub-window mode: len = the WINDOW's sequence length)
           scale = (p.loss_kind == B2H_LOSS_L1) ? (1.0f / (float)p.loss_B) / n_el : 1.0f / n_el;
@@ -1142,20 +1163,23 @@ int launch_tc_tile(const ConvArgs& a, const TilePlan& plan, cudaStream_t stream)
   p.loss_kind = a.loss_kind; p.apply_mask = a.apply_mask; p.mode = a.mode; p.out_scale = a.out_scale; p.geo = a.geo;
   p.B = plan.B; p.T = plan.T;
   p.nhalf = plan.nhalf; p.MB = plan.MB; p.NT = plan.NT; p.HR = plan.HR; p.gh = plan.gh; p.n_tiles = plan.n_tiles;
+  p.utt = a.utt;
   const bool train = plan.train, split = plan.split;
   const size_t smem = plan.smem;
   const int grid = plan.grid;
-  // twelve instantiations: {forward, train, train over window views} x {NT = 1, 2} x {bf16 operands, bf16 high/low pairs
-  // (fp32 mode)}
+  // sixteen instantiations: {forward, train, train over window views, forward over utterances} x {NT = 1, 2} x {bf16
+  // operands, bf16 high/low pairs (fp32 mode)}
   const int nt2 = p.NT == 2 ? 1 : 0;
-  const int kind = !train ? 0 : p.win_start ? 2 : 1;
-  const void* fns[3][2][2] = {
+  const int kind = !train ? (p.utt ? 3 : 0) : p.win_start ? 2 : 1;
+  const void* fns[4][2][2] = {
       {{(const void*)conv_tc_tile_kernel<false, 1, false>, (const void*)conv_tc_tile_kernel<false, 1, true>},
        {(const void*)conv_tc_tile_kernel<false, 2, false>, (const void*)conv_tc_tile_kernel<false, 2, true>}},
       {{(const void*)conv_tc_tile_kernel<true, 1, false>, (const void*)conv_tc_tile_kernel<true, 1, true>},
        {(const void*)conv_tc_tile_kernel<true, 2, false>, (const void*)conv_tc_tile_kernel<true, 2, true>}},
       {{(const void*)conv_tc_tile_kernel<true, 1, false, true>, (const void*)conv_tc_tile_kernel<true, 1, true, true>},
-       {(const void*)conv_tc_tile_kernel<true, 2, false, true>, (const void*)conv_tc_tile_kernel<true, 2, true, true>}}};
+       {(const void*)conv_tc_tile_kernel<true, 2, false, true>, (const void*)conv_tc_tile_kernel<true, 2, true, true>}},
+      {{(const void*)conv_tc_tile_kernel<false, 1, false, false, true>, (const void*)conv_tc_tile_kernel<false, 1, true, false, true>},
+       {(const void*)conv_tc_tile_kernel<false, 2, false, false, true>, (const void*)conv_tc_tile_kernel<false, 2, true, false, true>}}};
   const void* fn = fns[kind][nt2][split ? 1 : 0];
   if (int rc = ensure_dyn_smem(fn, smem)) return rc;
   void* kargs[] = {&p};

@@ -1,0 +1,106 @@
+// Forward over packed utterances (b2h_conv_forward_utterances): the device-side plan and the launch.  Included by
+// b2h_conv_tc.cu after the tile and wide kernels.
+//
+// Utterance u owns stream rows [offsets[u], offsets[u+1]) and is predicted as ONE sequence, like the reference's
+// infer_utterance (steps/traintest.py:214-300): it is cut into sub-windows of Ts frames by the training cut rule
+// (sub_window(), b2h_common.cuh), every interior cut with >= 16 real frames of context on both sides.  The receptive field
+// of the four convolutions is +-8 frames, so a sub-window's core rows equal the whole sequence's rows there; the utterance
+// start is the window's own leading zero rows, and rows at or past the utterance end are zero in every layer.
+//
+// The offsets live on the device, so the host sizes the launch from a bound (UttPlan::max_sub) and a one-CTA planning
+// kernel turns the offsets into the sub-window table the forward kernels read (layout: UttPlan).  The forward kernels end
+// their tile loops at the table's count.
+#pragma once
+
+namespace b2h {
+
+constexpr int kUttPlanThreads = 1024;
+constexpr int kUttBadOffsets = 80;   // b2h_tc_status id: offsets not non-decreasing within [0, n_frames]
+
+__global__ void __launch_bounds__(kUttPlanThreads) utt_plan_kernel(const long long* __restrict__ off, int n_utt, long long n_frames,
+                                                                   int Ts, int max_sub, int4* ws) {
+  __shared__ int warp_sum[32];
+  __shared__ int s_bad;
+  int4* table = ws + 1;
+  int* prefix = reinterpret_cast<int*>(reinterpret_cast<char*>(ws) + utt_prefix_offset(max_sub));
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  griddep_launch_dependents();       // the forward behind it may start its set-up; it reads the table after griddep_wait
+  if (tid == 0) s_bad = 0;
+  __syncthreads();
+  // pass 1: check the offsets, count each utterance's sub-windows, exclusive prefix sum (1024 utterances per round)
+  long long carry = 0;
+  for (int base = 0; base < n_utt; base += kUttPlanThreads) {
+    const int u = base + tid;
+    int cnt = 0;
+    if (u < n_utt) {
+      const long long a = off[u], b = off[u + 1];
+      if (a < 0 || b < a || b > n_frames) s_bad = 1;
+      else cnt = sub_window_count(b - a, Ts);
+    }
+    int v = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int n = __shfl_up_sync(0xffffffffu, v, o);
+      if (lane >= o) v += n;
+    }
+    if (lane == 31) warp_sum[warp] = v;
+    __syncthreads();
+    if (warp == 0) {
+      int w = warp_sum[lane];
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const int n = __shfl_up_sync(0xffffffffu, w, o);
+        if (lane >= o) w += n;
+      }
+      warp_sum[lane] = w;
+    }
+    __syncthreads();
+    const long long excl = carry + (v - cnt) + (warp ? warp_sum[warp - 1] : 0);
+    if (u < n_utt) prefix[u] = excl < max_sub ? (int)excl : max_sub;
+    carry += warp_sum[31];
+    __syncthreads();
+  }
+  // valid offsets hold at most n_frames frames, so carry <= max_sub (sub_window_count); bad ones plan nothing
+  const bool bad = s_bad || carry > max_sub;
+  const int count = bad ? 0 : (int)carry;
+  if (tid == 0) {
+    prefix[n_utt] = count;
+    ws[0] = make_int4(count, 0, 0, 0);
+    if (bad) atomicExch(&g_tc_status, kUttBadOffsets);
+  }
+  __syncthreads();                   // the prefix sums are visible to the whole CTA
+  // pass 2: sub-window g -> (utterance u, index i) by binary search over the prefix sums -> sub_window()
+  for (int gi = tid; gi < count; gi += kUttPlanThreads) {
+    int lo = 0, hi = n_utt - 1;      // the last u with prefix[u] <= gi (empty utterances share their successor's prefix)
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (prefix[mid] <= gi) lo = mid;
+      else hi = mid - 1;
+    }
+    const int n = prefix[lo + 1] - prefix[lo], i = gi - prefix[lo];
+    const long long a = off[lo];
+    const int L = (int)(off[lo + 1] - a);
+    int start = 0, clo = 0, chi = L;
+    if (n > 1) {
+      const SubWindow s = sub_window(L, Ts, n, i);
+      start = s.start; clo = s.clo; chi = s.chi;
+    }
+    const int len = L - start < Ts ? L - start : Ts;
+    table[gi] = make_int4((int)(a + start), start, clo | (chi << 16), len);
+  }
+}
+
+int launch_utterances(ConvArgs a, const UttPlan& plan, const long long* offsets, int n_utt, long long n_frames, void* workspace,
+                      cudaStream_t stream) {
+  int4* ws = reinterpret_cast<int4*>(workspace);
+  utt_plan_kernel<<<1, kUttPlanThreads, 0, stream>>>(offsets, n_utt, n_frames, plan.Ts, plan.max_sub, ws);
+  count_launch();
+  if (int rc = check_launch("utt_plan_kernel")) return rc;
+  a.utt = ws;
+  a.B = plan.max_sub; a.T = plan.Ts;
+  a.lengths = nullptr; a.apply_mask = 0;
+  if (plan.kernel == B2H_KERNEL_TC_TILE) return launch_tc_tile(a, plan.tile, stream);
+  return launch_tc_wide_fwd(a, plan.wide, stream);
+}
+
+}  // namespace b2h

@@ -45,6 +45,7 @@ struct WideArgs {
   const float* target; const float* conf; const float* d_y;
   int loss_kind, train_mode;    // train_mode 1 = criterion inside, 2 = backward of a given d_y
   unsigned char* scratch;       // per tile: the layer inputs ACT[0..3] and the pre-activation gradients DZ[0..3], each a
+                                // (MODE 0 over utterances: the plan, see UttPlan in b2h_common.cuh)
   long long tile_bytes;         // dump of the shared-memory operand layout [channel/8][264 rows][8 ch] bf16
   long long act_off[4], dz_off[4];
   float* loss_partials;         // [grid]
@@ -117,8 +118,12 @@ __device__ __forceinline__ bool wait_addr(uint32_t bar, uint32_t parity, int sit
 //         over the dumps (conv_tc_wide_wgrad_kernel).
 // VIEW (MODE 1 only): training over window views, a separate instantiation so that the dense training forward keeps its
 // code (the run-time test cost the C = 256 step ~0.6 %).  MODE 0 tests p.wv.win_start at run time.
-template <int MODE, bool VIEW = false>
+// UTT (MODE 0 only) = sub-windows of utterances (b2h_conv_forward_utterances): window g reads its rows from the plan's
+// table in p.scratch, rows at or past the utterance end are zero in every layer, and only the core rows are written, to y
+// at their stream rows.  p.B / p.n_tiles are the host's upper bound; the plan's count ends the tile loops.
+template <int MODE, bool VIEW = false, bool UTT = false>
 __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs p, const __grid_constant__ CUtensorMap wmap) {
+  static_assert(!UTT || MODE == 0, "utterances are a forward-only view");
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) uint64_t full_bar[kWideMaxStages];    // stage landed (TMA complete_tx)
   __shared__ __align__(8) uint64_t empty_bar[kWideMaxStages];   // stage consumed (tcgen05.commit)
@@ -164,6 +169,13 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
   __syncthreads();
   tc_fence_after();
   const uint32_t tbase = tmem_slot;
+  const int4* utt = reinterpret_cast<const int4*>(p.scratch);
+  int utt_n = 0, utt_tiles = 0;
+  if constexpr (UTT) {
+    utt_n = __ldg(&utt->x);
+    const int need = (utt_n + gh - 1) / gh;
+    utt_tiles = need < p.n_tiles ? need : p.n_tiles;
+  }
 
   // Both single-thread loops below are latency-bound scalar code (every instruction waits for the previous one): a
   // first version that recomputed slot = stage % S, the barrier addresses and the descriptors per stage needed ~540
@@ -174,7 +186,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
     // ===================== weight producer: one thread, runs ahead by the ring depth =====================
     if (elect_one()) {
       uint32_t slot = 0, ph = 1;                     // parity 1 on a fresh barrier = "already free" (first lap)
-      for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x)
+      for (int tile = blockIdx.x; tile < (UTT ? utt_tiles : p.n_tiles); tile += gridDim.x)
         for (int l = 0; l < NL; ++l) {
           const WideSched sc = wide_sched(p.st[l].KS, p.st[l].N);
           int row = p.st[l].row0;                                        // 128-byte rows of the weight tensor map
@@ -199,7 +211,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
       const uint32_t hi_k = desc_hi(128);
       const uint32_t a_lo0 = desc_lo(smem_u32(A), (uint32_t)CH);
       const uint32_t acc_addr = smem_u32(&acc_full);
-      for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x)
+      for (int tile = blockIdx.x; tile < (UTT ? utt_tiles : p.n_tiles); tile += gridDim.x)
         for (int l = 0; l < NL; ++l) {
           const WideSched sc = wide_sched(p.st[l].KS, p.st[l].N);
           const uint32_t idesc = make_idesc_bf16(128, sc.N, 0, 0);
@@ -262,7 +274,8 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
     const int nch0 = g.kp[0] / 8;
     const bool vec_in = (pe == 0) && ((n_in & 7) == 0);
     float loss_run = 0.0f;                                     // MODE 1: this thread's share of the criterion
-    struct RowCtx { int row, t, gw; bool valid; };
+    // UTT: us = the row's sub-window {stream row of frame 0, frame 0 in the utterance, clo | chi << 16, frames before the end}
+    struct RowCtx { int row, t, gw; bool valid; int4 us; };
     auto rowctx = [&](int j, int tile) {
       const int mm = r128 + 128 * j;
       const int wjj = mm / (T + 2);
@@ -271,6 +284,11 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
       r.row = 2 + mm;
       r.gw = tile * gh + wjj;
       r.valid = (r.t < T) && (wjj < gh) && (r.gw < p.B) && tile < p.n_tiles;
+      if constexpr (UTT) {
+        const bool in = (wjj < gh) && (r.gw < utt_n) && tile < utt_tiles;
+        r.us = in ? __ldg(utt + 1 + r.gw) : make_int4(0, 0, 0, 0);
+        r.valid = in && r.t < r.us.w;
+      }
       return r;
     };
     // scratch dumps of tile `tile` (training): same [chunk][row][8 ch] layout as the shared-memory buffer
@@ -299,6 +317,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
           uint4 q = make_uint4(0, 0, 0, 0);
           if (rc.valid) {
             size_t base = ((size_t)rc.gw * T + rc.t) * n_in;
+            if constexpr (UTT) base = ((size_t)rc.us.x + rc.t) * n_in;
             if constexpr (MODE == 0 || VIEW) {
               if (p.wv.win_start) {                  // window view: the source row in the frame stream
                 const long long f = window_src_row(p.wv, rc.gw, rc.t);
@@ -325,7 +344,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
               for (int e = 0; e < 8; ++e) {
                 const int cc = c8 * 8 + e;          // channel in the conv1 input (pos-emb row first)
                 float val = 0.0f;
-                if (pe && cc == 0) val = __fdiv_rn((float)rc.t, (float)g.pe_len);             // HandPoseModels.py:70-82
+                if (pe && cc == 0) val = __fdiv_rn((float)(UTT ? rc.us.y + rc.t : rc.t), (float)g.pe_len);   // HandPoseModels.py:70-82
                 else if (cc - pe < n_in && cc - pe >= 0)
                   val = (p.x_dtype == B2H_DT_F32) ? __ldg(reinterpret_cast<const float*>(p.x) + base + (cc - pe))
                                                   : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(p.x)[base + (cc - pe)]);
@@ -356,7 +375,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
     publish();
     uint32_t acc_phase = 0;
     int en = 64;
-    for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
+    for (int tile = blockIdx.x; tile < (UTT ? utt_tiles : p.n_tiles); tile += gridDim.x) {
       for (int l = 0; l < NL; ++l) {
         const int N = p.st[l].N;
         const int layer = p.st[l].layer;      // model layer this stage belongs to (forward: l; backward: 3, 2, 1)
@@ -456,6 +475,10 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
             int len = T;
             if (rc.valid && p.lengths) { len = p.lengths[rc.gw]; len = len < 0 ? 0 : (len > T ? T : len); }
             float* yrow = rc.valid ? p.y + ((size_t)rc.gw * T + rc.t) * B2H_COUT : nullptr;
+            if constexpr (UTT) {                 // the core rows only, at their stream rows
+              const bool core = rc.valid && rc.t >= (rc.us.z & 0xFFFF) && rc.t < (rc.us.z >> 16);
+              yrow = core ? p.y + ((size_t)rc.us.x + rc.t) * B2H_COUT : nullptr;
+            }
             const bool masked = p.apply_mask && (rc.t >= len);
             for (int c0 = 16 * ch; c0 < N; c0 += 32) {
               uint32_t v[16];
@@ -808,13 +831,15 @@ static WideArgs wide_args(const ConvArgs& a, const WidePlan& plan) {
 
 int launch_tc_wide_fwd(const ConvArgs& a, const WidePlan& plan, cudaStream_t stream) {
   const Geo& g = a.geo;
-  const WideArgs p = wide_args(a, plan);
-  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(conv_tc_wide_kernel<0>), plan.smem)) return rc;
+  WideArgs p = wide_args(a, plan);
+  p.scratch = reinterpret_cast<unsigned char*>(const_cast<int4*>(a.utt));
+  auto* fn = a.utt ? conv_tc_wide_kernel<0, false, true> : conv_tc_wide_kernel<0>;
+  if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), plan.smem)) return rc;
   CUtensorMap wmap;
   if (int rc = wide_weight_map(a.packed + g.tf_off[0], g.td_off[0] - g.tf_off[0], &wmap)) return rc;
-  conv_tc_wide_kernel<0><<<plan.grid, kWideThreads, plan.smem, stream>>>(p, wmap);
+  fn<<<plan.grid, kWideThreads, plan.smem, stream>>>(p, wmap);
   count_launch();
-  return check_launch("conv_tc_wide_kernel<fwd>");
+  return check_launch(a.utt ? "conv_tc_wide_kernel<fwd, utterances>" : "conv_tc_wide_kernel<fwd>");
 }
 
 // ---- wide training: forward+criterion (saves layer inputs), dgrad chain, split-K wgrad; the caller reduces + applies Adam ----

@@ -11,6 +11,7 @@ from __future__ import annotations
 
 import weakref
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -98,6 +99,7 @@ class ConvModel(nn.Module):
         self._packed = None
         self._packed_versions = None
         self._workspace = None
+        self._utt_workspace = None
         self._flatten()
 
     # ------------------------------------------------------------------ flat parameter storage
@@ -126,7 +128,7 @@ class ConvModel(nn.Module):
 
     def __getstate__(self):
         st = dict(self.__dict__)
-        for k in ("_flat", "_packed", "_packed_versions", "_workspace"):
+        for k in ("_flat", "_packed", "_packed_versions", "_workspace", "_utt_workspace"):
             st[k] = None
         return st
 
@@ -293,6 +295,59 @@ class ConvModel(nn.Module):
             _lib.ptr(self._flat), _lib.ptr(self.packed_weights()), _lib.ptr(len32), _lib.ptr(y), W, T, n_in, C, pe,
             _lib.PRECISIONS[self.precision], 1 if len32 is not None else 0, 1.0 if denormalize is None else float(denormalize),
             _lib.stream_ptr(dev)))
+        return y
+
+    def utterances_workspace(self, n_frames, n_utt):
+        """The workspace of predict_utterances (the device-side sub-window plan), cached on the model like workspace()."""
+        n_in, C, pe = self._geometry()
+        n = _lib.load().b2h_utterances_workspace_bytes(int(n_frames), int(n_utt), n_in, C, pe, _lib.PRECISIONS[self.precision])
+        if n < 0:
+            raise _lib.B2HError(_lib.last_error())
+        dev = self._flat.device
+        if self._utt_workspace is None or self._utt_workspace.numel() < n or self._utt_workspace.device != dev:
+            self._utt_workspace = torch.empty(n, dtype=torch.uint8, device=dev)
+        return self._utt_workspace
+
+    @torch.no_grad()
+    def predict_utterances(self, frames, offsets, denormalize=None, out=None):
+        """Inference over packed utterances of any length, one prediction per frame: the reference's infer_utterance
+        (steps/traintest.py:214-300) for every utterance at once.  `frames` (F, K, 2) is a frame stream
+        (`PreprocessRightHand.frame_stream`), `offsets` (S + 1,) int64 non-decreasing (`PackedClips.offsets`): utterance u
+        owns rows [offsets[u], offsets[u+1]).  Returns (F, 21, 2) fp32 (`out` if given): row f of utterance u is
+        ConvModel.forward of frames[offsets[u]:offsets[u+1]] as one sequence at that frame (times `denormalize`, e.g. 1280);
+        rows outside [offsets[0], offsets[S]) are not written (zeros when `out` is None).  Host offsets (numpy, list, CPU
+        tensor) are checked here (ValueError) and uploaded; device offsets are used as given, checked by the kernels (bad ones
+        write nothing and set b2h_tc_status).  Served in bf16 mode for conv_channels <= 256 and in fp32 mode for
+        conv_channels <= 32 with at most 32 input channels; other shapes raise B2HError."""
+        if not self._is_flat():
+            self._flatten()
+        if self.pos_emb is not None and not self.pos_emb_any_length:
+            # the reference's torch.cat fails unless T == max_len (HandPoseModels.py:82): utterances of any length need
+            # pos_emb_any_length=True
+            raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {self.pos_emb.max_len} "
+                               "(predict_utterances needs pos_emb_any_length=True)")
+        F, _ = self._check_input(frames, 1)
+        dev = frames.device
+        x = frames.contiguous()
+        if isinstance(offsets, torch.Tensor) and offsets.is_cuda:
+            if offsets.dtype != torch.int64 or offsets.dim() != 1 or offsets.numel() < 1 or offsets.device != dev:
+                raise ValueError("device offsets must be a 1-D int64 tensor of S + 1 entries on the frames' device")
+            off = offsets.contiguous()
+        else:
+            o = np.asarray(offsets.cpu() if isinstance(offsets, torch.Tensor) else offsets)
+            if o.ndim != 1 or o.size < 1 or not np.issubdtype(o.dtype, np.integer):
+                raise ValueError("offsets must be a 1-D integer array of S + 1 entries")
+            if (np.diff(o) < 0).any() or o[0] < 0 or o[-1] > F:
+                raise ValueError(f"offsets must be non-decreasing within [0, {F}]")
+            off = torch.from_numpy(o.astype(np.int64)).to(dev)
+        S = off.numel() - 1
+        n_in, C, pe = self._geometry()
+        y = out if out is not None else torch.zeros((F, 21, 2), dtype=torch.float32, device=dev)
+        ws = self.utterances_workspace(F, S)
+        _lib.check(_lib.load().b2h_conv_forward_utterances(
+            _lib.ptr(x), _lib.dtype_code(x.dtype), F, _lib.ptr(off), S, _lib.ptr(self._flat), _lib.ptr(self.packed_weights()),
+            _lib.ptr(y), n_in, C, pe, _lib.PRECISIONS[self.precision], 1.0 if denormalize is None else float(denormalize),
+            _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
         return y
 
 

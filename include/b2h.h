@@ -161,6 +161,35 @@ int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t n_frames, 
                              int pad_mode, const float* params, const void* packed, const int32_t* lengths, float* y, int n_win,
                              int T, int n_in, int C, int pos_emb, int precision, int apply_mask, float out_scale, void* stream);
 
+/* ConvModel.forward over PACKED UTTERANCES of any length, one prediction per frame -- the reference's infer_utterance
+ * (steps/traintest.py:214-300), which runs each utterance as one zero-padded sequence.  frames (n_frames, n_in) fp32 or
+ * bf16; offsets (n_utt + 1) int64 on the device, non-decreasing within [0, n_frames]: utterance u owns rows
+ * [offsets[u], offsets[u+1]) (PackedClips.offsets).  y (n_frames, 42) fp32: row f of utterance u is ConvModel.forward of
+ * frames[offsets[u]:offsets[u+1]] as one sequence at that frame, times out_scale; rows outside [offsets[0], offsets[n_utt])
+ * are not written, nor are rows of empty utterances; n_utt = 0 does nothing.  No mask_output (inference has none); the
+ * positional row is t / max_len with t counted from the utterance's first frame.
+ * Each utterance is cut into sub-windows of Ts frames by the training cut rule (>= 16 real context frames at every interior
+ * cut, b2h_utterance_subwindows) and each sub-window writes its core rows.  A planning kernel checks the offsets on the
+ * device: bad ones write nothing and set b2h_tc_status to 80.  Enqueues only (no allocation, no synchronisation; graph
+ * capturable).  workspace: b2h_utterances_workspace_bytes, 16-byte aligned.  Served in bf16 mode for conv_channels <= 256
+ * and in fp32 mode for conv_channels <= 32 with at most 32 input channels (B2H_ESHAPE otherwise: fp32 mode with wider
+ * models and B2H_FP32_FFMA, whose kernel reads dense windows only). */
+int b2h_conv_forward_utterances(const void* frames, int x_dtype, int64_t n_frames, const int64_t* offsets, int n_utt,
+                                const float* params, const void* packed, float* y, int n_in, int C, int pos_emb,
+                                int precision, float out_scale, void* workspace, int64_t workspace_bytes, void* stream);
+/* bytes of workspace b2h_conv_forward_utterances needs (the plan's sub-window table, sized from the bound
+ * n_utt + n_frames / (Ts - 32) on the sub-window count); B2H_ESHAPE for an unserved shape */
+int64_t b2h_utterances_workspace_bytes(int64_t n_frames, int n_utt, int n_in, int C, int pos_emb, int precision);
+/* Host-only: the kernel family b2h_conv_forward_utterances runs (B2H_KERNEL_TC_TILE / _TC_WIDE / _NONE) and, into
+ * *seg_len (nullable), the sub-window length Ts it uses: from the menu 64 / 128 / 256, the one that computes the fewest
+ * MMA rows for an utterance of the mean length n_frames / n_utt. */
+int b2h_utterances_plan(int64_t n_frames, int n_utt, int n_in, int C, int pos_emb, int precision, int* seg_len);
+/* Host-only: the number of sub-windows an utterance of L frames is cut into at sub-window length Ts (0 for L = 0, 1 for
+ * L <= Ts) and, when out3 is non-NULL, sub-window i as {first frame, first core row, end of the core rows} (sub-window
+ * coordinates); the cores partition [0, L).  tests/test_utterances_host.py proves on the CPU that each core equals the
+ * whole sequence's rows. */
+int b2h_utterance_subwindows(int L, int Ts, int i, int* out3);
+
 /* LinearPositionalEmbedding.forward as a stand-alone call (models/HandPoseModels.py:78-84): inp (B, channels, T) fp32
  * -> out (B, channels+1, T) with out[:,0,t] = t / max_len (fp32 division) and the input channels behind it.  Like the
  * reference's torch.cat it only works for T == max_len (B2H_ESHAPE otherwise).  ConvModel(pos_emb=True) does not
