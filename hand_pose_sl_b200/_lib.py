@@ -63,6 +63,15 @@ _SIGNATURES = {
     "b2h_train_forward_backward_windows": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int,
                                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                                    c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int64, c_void_p]),
+    "b2h_train_forward_backward_utterances": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int,
+                                                      c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                                      c_int, c_int, c_int, c_void_p, c_void_p, c_int64, c_void_p]),
+    "b2h_train_step_utterances": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int,
+                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
+                                          c_double, c_double, c_double, c_double, c_int64, c_void_p, c_void_p, c_void_p,
+                                          c_int64, c_void_p]),
+    "b2h_train_utterances_workspace_bytes": (c_int64, [c_int, c_int, c_int, c_int, c_int, c_int]),
+    "b2h_train_utterances_plan": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "b2h_conv_backward": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                   c_int, c_int, c_void_p, c_int64, c_void_p]),
     "b2h_mask_output": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),

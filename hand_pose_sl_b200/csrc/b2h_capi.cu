@@ -97,25 +97,33 @@ static TrainPlan train_plan(const Geo& g, int B, int T, int precision) {
 // else the wide forward (bf16 mode); the plan takes the Ts whose family computes the fewest MMA rows for an utterance of the
 // mean length n_frames / n_utt under the cut rule (ties: the longer Ts, fewer sub-windows).  Rows per sub-window are the
 // tile's rows over the windows it holds: 64 / 128 / 256 in the tile kernel, 256 / floor(258 / (Ts + 2)) in the wide one.
-static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int precision) {
+// Training over segments (max_len > 0, b2h_train_*_utterances): n_utt segments of at most max_len frames, the same rule for a
+// segment of max_len frames over the lengths the tile kernel trains as whole windows (bf16: 64 / 128 / 256, fp32 mode: 64 /
+// 128), sized for n_utt * n(max_len) sub-windows; the workspace is the training one (header, gradient and loss partials of
+// the plan's grid) followed by the table and one {segment, length} pair per sub-window.
+static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int precision, int max_len = 0) {
   static const int kMenu[3] = {256, 128, 64};
   UttPlan best{};
   best.kernel = B2H_KERNEL_NONE;
   if (precision != B2H_BF16 && precision != B2H_FP32) return best;   // the FFMA kernel reads dense windows only
-  const int64_t mean = n_frames / (n_utt > 0 ? n_utt : 1);
+  const bool train = max_len > 0;
+  const int64_t mean = train ? max_len : n_frames / (n_utt > 0 ? n_utt : 1);
   double best_rows = 0.0;
   for (int Ts : kMenu) {
-    const int64_t max_sub = (int64_t)(n_utt > 0 ? n_utt : 0) + n_frames / (Ts - 32);
+    const int64_t max_sub = train ? (int64_t)n_utt * sub_window_count(max_len, Ts)
+                                  : (int64_t)(n_utt > 0 ? n_utt : 0) + n_frames / (Ts - 32);
     if (max_sub > (int64_t)INT32_MAX / 2) continue;
     UttPlan c{};
     c.Ts = Ts;
     c.max_sub = (int)max_sub;
     const int B = c.max_sub > 0 ? c.max_sub : 1;
-    c.tile = plan_tile(g, B, Ts, false, is_split(precision));
+    c.tile = plan_tile(g, B, Ts, train, is_split(precision));
     double rows_per_sub = 0.0;
-    if (c.tile.ok) {
+    if (c.tile.ok && c.tile.n_sub == 1) {
       c.kernel = B2H_KERNEL_TC_TILE;
       rows_per_sub = (double)c.tile.MB / c.tile.gh;
+    } else if (train) {
+      continue;
     } else if (precision == B2H_BF16 && (c.wide = plan_wide(g, B, Ts)).ok) {
       c.kernel = B2H_KERNEL_TC_WIDE;
       rows_per_sub = 256.0 / c.wide.gh;
@@ -125,6 +133,11 @@ static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int pre
     const double rows = rows_per_sub * sub_window_count(mean > 0 ? mean : 1, Ts);
     if (best.kernel != B2H_KERNEL_NONE && rows >= best_rows) continue;
     c.ws_bytes = (utt_prefix_offset(c.max_sub) + 4 * ((int64_t)n_utt + 1) + 255) / 256 * 256;
+    if (train) {
+      c.plan_off = (B2H_WS_HEADER + ((int64_t)c.tile.grid * gp_total(g) + c.tile.grid) * 4 + 255) / 256 * 256;
+      c.seg_off = (utt_prefix_offset(c.max_sub) + 4 * ((int64_t)n_utt + 1) + 15) / 16 * 16;
+      c.ws_bytes = (c.plan_off + c.seg_off + 8 * (int64_t)c.max_sub + 255) / 256 * 256;
+    }
     best = c;
     best_rows = rows;
   }
@@ -559,6 +572,119 @@ extern "C" int b2h_train_step_windows(const void* frames, int x_dtype, const flo
   return train_step(frames, x_dtype, &wv, target_frames, conf_frames, lengths, params, packed, exp_avg, exp_avg_sq, loss_out,
                     n_win, T, n_in, C, pos_emb, loss_kind, precision, lr, beta1, beta2, eps, step, step_dev, lr_dev, workspace,
                     workspace_bytes, stream, "b2h_train_step_windows");
+}
+
+static const char* const kUttTrainServed =
+    "segments are trained by the tile kernel: conv_channels <= 32 with at most 32 input channels, in bf16 or fp32 mode "
+    "(wider models and fp32-ffma have no segment path)";
+
+extern "C" int b2h_train_utterances_plan(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision, int* seg_len) {
+  if (seg_len) *seg_len = 0;
+  if (!geo_ok(n_in, C, pos_emb) || n_seg < 1 || max_len < 1) return B2H_KERNEL_NONE;
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, max_len);
+  if (seg_len && u.kernel != B2H_KERNEL_NONE) *seg_len = u.Ts;
+  return u.kernel;
+}
+
+extern "C" int64_t b2h_train_utterances_workspace_bytes(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision) {
+  const char* who = "b2h_train_utterances_workspace_bytes";
+  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
+  if (n_seg < 1 || max_len < 1) { set_error("%s: bad n_seg=%d max_len=%d", who, n_seg, max_len); return B2H_ESHAPE; }
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, max_len);
+  if (u.kernel == B2H_KERNEL_NONE) { set_error("%s: %s (C=%d, n_in=%d, precision=%d)", who, kUttTrainServed, C, n_in, precision); return B2H_ESHAPE; }
+  return u.ws_bytes;
+}
+
+// The checks and the launch shared by b2h_train_forward_backward_utterances and b2h_train_step_utterances (fuse != nullptr:
+// the fused step), in the order and style of train_common.
+static int train_utterances(const void* frames, int x_dtype, const float* target, const float* conf, int64_t n_frames,
+                            const int64_t* seg_start, const int64_t* seg_end, int n_seg, int max_len, const float* params,
+                            const void* packed, float* pred_out, int n_in, int C, int pos_emb, int loss_kind, int precision,
+                            int64_t* step_dev, void* workspace, int64_t workspace_bytes, cudaStream_t stream, const char* who,
+                            const FuseAdam* fuse, UttPlan* plan_out, Geo* g_out) {
+  if (!seg_start || !seg_end) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  if (int rc = check_common(frames, x_dtype, nullptr, params, packed, workspace, 1, 0, 1, n_in, C, pos_emb, who)) return rc;
+  if (n_seg < 1 || max_len < 1 || n_frames < 0 || n_frames > INT32_MAX) {
+    set_error("%s: bad n_seg=%d max_len=%d n_frames=%lld", who, n_seg, max_len, (long long)n_frames);
+    return B2H_ESHAPE;
+  }
+  if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
+  if (!target) { set_error("%s: null target", who); return B2H_EINVAL; }
+  if (loss_kind != B2H_LOSS_L1 && loss_kind != B2H_LOSS_CONFL1) { set_error("%s: bad loss_kind %d", who, loss_kind); return B2H_EINVAL; }
+  if (loss_kind == B2H_LOSS_CONFL1 && !conf) { set_error("%s: confL1 needs scores", who); return B2H_EINVAL; }
+  if (misaligned(frames, 15) || misaligned(target, 7) || misaligned(conf, 3) || misaligned(packed, 15) || misaligned(pred_out, 15) ||
+      misaligned(workspace, 15) || misaligned(seg_start, 7) || misaligned(seg_end, 7)) {
+    set_error("%s: frames, packed, pred_out and workspace must be 16-byte aligned, target_frames, seg_start and seg_end 8-byte "
+              "and conf_frames 4-byte aligned", who);
+    return B2H_EALIGN;
+  }
+  const Geo g = make_geo(n_in, C, pos_emb);
+  const UttPlan plan = utterance_plan(g, n_frames, n_seg, precision, max_len);
+  if (plan.kernel == B2H_KERNEL_NONE) {
+    set_error("%s: %s; no kernel for C=%d, n_in=%d, precision=%d", who, kUttTrainServed, C, n_in, precision);
+    return B2H_ESHAPE;
+  }
+  if (workspace_bytes < plan.ws_bytes) {
+    set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.ws_bytes);
+    return B2H_EWORKSPACE;
+  }
+  if (pred_out) {
+    const cudaError_t e = cudaMemsetAsync(pred_out, 0, (size_t)n_seg * max_len * B2H_COUT * 4, stream);
+    if (e != cudaSuccess) { cudaGetLastError(); set_error("%s: cudaMemsetAsync: %s", who, cudaGetErrorString(e)); return B2H_ECUDA; }
+  }
+  ConvArgs a{};
+  a.x = frames; a.x_dtype = x_dtype; a.target = target; a.conf = conf; a.params = params;
+  a.packed = reinterpret_cast<const char*>(packed); a.y = pred_out;
+  a.partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + B2H_WS_HEADER);
+  a.loss_partials = a.partials + (size_t)plan.tile.grid * gp_total(g);
+  a.loss_kind = loss_kind; a.mode = 1; a.out_scale = 1.0f; a.geo = g;
+  a.step_dev = reinterpret_cast<long long*>(step_dev);
+  if (fuse) {
+    if (plan.tile.grid > B2H_WS_MAX_CTA) { set_error("%s: %d CTAs exceed the %d arrival flags of the workspace header", who, plan.tile.grid, B2H_WS_MAX_CTA); return B2H_ESHAPE; }
+    a.fuse = *fuse;
+    a.fuse.enabled = 1;
+    a.fuse.hdr = reinterpret_cast<unsigned*>(workspace);
+  }
+  if (plan_out) *plan_out = plan;
+  if (g_out) *g_out = g;
+  return launch_train_utterances(a, plan, reinterpret_cast<const long long*>(seg_start), reinterpret_cast<const long long*>(seg_end),
+                                 n_seg, (long long)n_frames, max_len, workspace, stream);
+}
+
+extern "C" int b2h_train_forward_backward_utterances(const void* frames, int x_dtype, const float* target_frames,
+                                                     const float* conf_frames, int64_t n_frames, const int64_t* seg_start,
+                                                     const int64_t* seg_end, int n_seg, int max_len, const float* params,
+                                                     const void* packed, float* grads_out, float* loss_out, float* pred_out,
+                                                     int n_in, int C, int pos_emb, int loss_kind, int precision,
+                                                     int64_t* step_dev, void* workspace, int64_t workspace_bytes, void* stream) {
+  const char* who = "b2h_train_forward_backward_utterances";
+  if (!grads_out || !loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  UttPlan plan{};
+  Geo g{};
+  if (int rc = train_utterances(frames, x_dtype, target_frames, conf_frames, n_frames, seg_start, seg_end, n_seg, max_len, params,
+                                packed, pred_out, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace, workspace_bytes,
+                                (cudaStream_t)stream, who, nullptr, &plan, &g))
+    return rc;
+  float* partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + B2H_WS_HEADER);
+  return launch_reduce(partials, plan.tile.grid, g, grads_out, partials + (size_t)plan.tile.grid * gp_total(g), plan.tile.grid,
+                       loss_out, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int b2h_train_step_utterances(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
+                                         int64_t n_frames, const int64_t* seg_start, const int64_t* seg_end, int n_seg,
+                                         int max_len, float* params, void* packed, float* exp_avg, float* exp_avg_sq,
+                                         float* loss_out, int n_in, int C, int pos_emb, int loss_kind, int precision, double lr,
+                                         double beta1, double beta2, double eps, int64_t step, int64_t* step_dev,
+                                         const double* lr_dev, void* workspace, int64_t workspace_bytes, void* stream) {
+  const char* who = "b2h_train_step_utterances";
+  if (!exp_avg || !exp_avg_sq || !loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  if (step < 1 && !step_dev) { set_error("%s: step must be >= 1", who); return B2H_EINVAL; }
+  // the fused step reads the Adam step from the device counter and advances it (a refused segment list leaves it alone)
+  if (!step_dev) { set_error("%s: null step_dev (the fused step reads and advances the device-side step counter)", who); return B2H_EINVAL; }
+  const FuseAdam fuse = fuse_adam(params, packed, exp_avg, exp_avg_sq, loss_out, lr, beta1, beta2, eps, 1.0f, step_dev, lr_dev);
+  return train_utterances(frames, x_dtype, target_frames, conf_frames, n_frames, seg_start, seg_end, n_seg, max_len, params, packed,
+                          nullptr, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace, workspace_bytes,
+                          (cudaStream_t)stream, who, &fuse, nullptr, nullptr);
 }
 
 extern "C" int b2h_train_step_dp(const void* x, int x_dtype, const float* target, const float* conf, const int32_t* lengths,

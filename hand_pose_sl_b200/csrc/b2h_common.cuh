@@ -338,6 +338,8 @@ struct ConvArgs {
   Geo geo;
   WindowView wv;            // tensor-core kernels only: win_start set = x (and target / conf) are frame streams, B = windows
   const int4* utt;          // forward over utterances (b2h_utterances.cuh): the device-side plan, x a frame stream; else nullptr
+  const int2* utt_seg;      // training over segments: per sub-window {segment, segment length} (UttPlan); else nullptr
+  int utt_max_len;          // training over segments: row stride of the masked prediction (n_seg, max_len, 42)
 };
 int launch_fp32(const ConvArgs& a, const FfmaPlan& plan, cudaStream_t stream);
 int launch_tc_fwd(const ConvArgs& a, const RowspacePlan& plan, cudaStream_t stream);
@@ -352,20 +354,27 @@ int tc_status_and_clear();
 
 // Forward over packed utterances (b2h_conv_forward_utterances): every utterance is cut into sub-windows of Ts frames by
 // sub_window(); the forward kernels read sub-window g from a table that a one-CTA planning kernel builds on the device.
-// Workspace: [int4 {sub-window count, 0, 0, 0}][int4 per sub-window, max_sub of them][int prefix[n_utt + 1]], where
+// Workspace: [int4 {sub-window count, bad, 0, 0}][int4 per sub-window, max_sub of them][int prefix[n_utt + 1]], where
 // sub-window g = {stream row of its first frame, its first frame in the utterance, clo | chi << 16, frames before the
-// utterance end (<= Ts)}.
+// utterance end (<= Ts)} and bad = 1 when the planning kernel refused the offsets / segments (count = 0 then).
+// Training over segments (b2h_train_*_utterances) plans the same table at plan_off of the training workspace, followed at
+// seg_off (from the table's start) by one int2 per sub-window: {segment, segment length}.
 struct UttPlan {
   int kernel;               // B2H_KERNEL_TC_TILE | B2H_KERNEL_TC_WIDE | B2H_KERNEL_NONE
   int Ts;                   // sub-window length
-  int max_sub;              // upper bound on the sub-window count: n_utt + n_frames / (Ts - 32)
+  int max_sub;              // upper bound on the sub-window count: n_utt + n_frames / (Ts - 32); training: n_seg * n(max_len)
   TilePlan tile; WidePlan wide;   // planned for max_sub windows of Ts frames
   int64_t ws_bytes;
+  int64_t plan_off, seg_off; // training: byte offset of the table in the workspace, of the segment array from the table
 };
 __host__ __device__ inline int64_t utt_prefix_offset(int max_sub) { return (int64_t)(1 + max_sub) * 16; }
 // planning kernel, then the forward of a.B = plan.max_sub sub-windows of a.T = plan.Ts frames over the table it wrote
 int launch_utterances(ConvArgs a, const UttPlan& plan, const long long* offsets, int n_utt, long long n_frames, void* workspace,
                       cudaStream_t stream);
+// planning kernel over the segments [seg_start[s], seg_end[s]) (each 1..max_len frames), then the training launch of the
+// tile kernel (a.fuse.enabled: the fused step) over the table it wrote; a.B = n_seg
+int launch_train_utterances(ConvArgs a, const UttPlan& plan, const long long* seg_start, const long long* seg_end, int n_seg,
+                            long long n_frames, int max_len, void* workspace, cudaStream_t stream);
 
 void set_debug_timing(long long* p);
 int launch_format_prediction(const float* pred, float* out, int64_t rows, int mode, cudaStream_t stream);

@@ -66,6 +66,10 @@ struct TcTileArgs {
   // Forward over utterances (UTT instantiations): x is a frame stream and window g < utt[0].x is sub-window utt[1 + g] of the
   // plan (UttPlan, b2h_common.cuh); B / n_tiles are the host's upper bound on the sub-window count.
   const int4* utt;
+  // Training over segments (TRAIN && UTT): sub-window g belongs to segment utt_seg[g].x of utt_seg[g].y frames (loss weight
+  // 1 / (42 L_s), masked-prediction row utt_seg[g].x * utt_max_len + frame); B is the bound on the sub-window count and
+  // loss_B the segment count.
+  const int2* utt_seg; int utt_max_len;
 };
 
 constexpr int kTileThreads = 256;   // 8 warps: two per TMEM lane quadrant (each takes every other 16-column chunk)
@@ -220,12 +224,14 @@ __device__ __forceinline__ long long global_ns() { long long t; asm volatile("mo
 // VIEW (training only) = window views of frame streams: target / confidence rows through the view, per-window staging of
 // the target tile.  A separate instantiation: the same code behind a run-time test made the dense 256x64 step 1.9 us
 // slower (27.4 -> 29.3 us) with the same register count.  The forward kernel tests p.win_start at run time.
-// UTT (forward only) = sub-windows of utterances (b2h_conv_forward_utterances): window g reads its rows from the plan's
-// table, rows at or past the utterance end are zero in every layer (the sequence ends there), and only the core rows
-// are written, to y at their stream rows.
+// UTT = sub-windows of utterances / training segments: window g reads its rows from the plan's table, rows at or past the
+// sequence end are zero in every layer (the sequence ends there).  Forward (b2h_conv_forward_utterances): only the core rows
+// are written, to y at their stream rows.  Training (b2h_train_*_utterances): target and confidence rows are read at the
+// stream rows, the criterion covers the core rows with the weight 1 / (42 L_s) of the row's segment, the masked prediction
+// goes to row (segment, frame in the segment) of y, and a plan the planning kernel refused ("bad") makes the step a no-op.
 template <bool TRAIN, int NT, bool SPLIT, bool VIEW = false, bool UTT = false>
 __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArgs p) {
-  static_assert(!(UTT && TRAIN), "utterances are a forward-only view");
+  static_assert(!(UTT && VIEW), "utterances and window views are separate instantiations");
   int dbg_n = 0;
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) uint64_t bar;      // MMAs of the current phase complete (one arrival per issuing warp)
@@ -381,9 +387,10 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
   // ---- part 2: the previous kernel has completed and its writes (weights, Adam state, counters, inputs) are visible ----
   griddep_wait();
   B2H_STAMP();   // predecessor complete
-  int utt_tiles = 0;
+  int utt_tiles = 0, utt_bad = 0;
   if constexpr (UTT) {                           // the plan's count: CTAs past it have no tile and load no weights
     utt_n = __ldg(&p.utt->x);
+    if constexpr (TRAIN) utt_bad = __ldg(&p.utt->y);   // refused plan (count 0): no Adam update, no counter, NaN loss
     const int need = (utt_n + wpt - 1) / wpt;
     utt_tiles = need < p.n_tiles ? need : p.n_tiles;
   }
@@ -419,7 +426,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
         abort_flag = *reinterpret_cast<volatile int*>(&g_dp_abort);
       }
       sync_tok = *reinterpret_cast<const volatile unsigned*>(p.fuse.hdr) + 1u;
-    } else if (blockIdx.x == 0 && tid == 0) {
+    } else if (blockIdx.x == 0 && tid == 0 && !utt_bad) {
       if (p.step_dev) *p.step_dev += 1;
       if (p.epoch_dev) *p.epoch_dev += 1;
     }
@@ -490,6 +497,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
       const int Tw = p.n_sub > 1 ? p.T_orig : T;              // length of the window the sequence length refers to
       lens[j] = Tw;
       if (rc.valid && p.lengths) { const int v = p.lengths[p.n_sub > 1 ? rc.gw / p.n_sub : rc.gw]; lens[j] = v < 0 ? 0 : (v > Tw ? Tw : v); }
+      if constexpr (UTT && TRAIN) if (rc.valid) lens[j] = __ldg(&p.utt_seg[rc.gw].y);   // the segment's length L_s
     }
 
     const bool tgt_smem = TRAIN && p.mode == 1 && bulk_io && p.n_sub <= 1;
@@ -659,7 +667,9 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
           }
         }
         const bool y_smem = !TRAIN && bulk_io;
-        float* yrow = (valid && p.y && in_core) ? p.y + drow * B2H_COUT : nullptr;                // global row
+        size_t prow = drow;                                         // training over segments: (segment, frame in it)
+        if constexpr (UTT && TRAIN) prow = valid ? (size_t)__ldg(&p.utt_seg[gw].x) * p.utt_max_len + rc.us.y + t : 0;
+        float* yrow = (valid && p.y && in_core) ? p.y + prow * B2H_COUT : nullptr;                // global row
         float* ys_row = YS + (size_t)srow * B2H_COUT;                                            // shared staging row
         if (tgt_smem && j == 0) { mbar_wait(&tbar, tphase, 18); tphase ^= 1; }
         B2H_STAMP();   // layer-4 epilogue: target tile landed
@@ -795,7 +805,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
       // epilogue handshake (ebar) before each dgrad and for each other between dgrad and wgrad.  Warps 2..7 wait for dgrad_l's commit and run its ReLU-mask
       // epilogue while wgrad_l is in the pipe; warps 4/5 take all columns of lane quadrants 0/1.  The epilogue's only
       // write hazard, the dZ buffer wgrad_{l+1} read, is clear: that commit also covers wgrad_{l+1}.
-      const bool last_tile = tile + (int)gridDim.x >= p.n_tiles;
+      const bool last_tile = tile + (int)gridDim.x >= (UTT ? utt_tiles : p.n_tiles);
       const bool both = warp == 4 || warp == 5;
       for (int l = 3; l >= 0; --l) {
         unsigned char* gz = ((3 - l) & 1) ? G1 : G0;          // dZ_l
@@ -938,8 +948,11 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
     } else {
       readout_pair(0, ch, ch);                     // (pair 1 was read out under the last tile's W2 / W1)
     }
-    if (tid == 0 && p.loss_partials)
-      p.loss_partials[blockIdx.x] = (p.loss_kind == B2H_LOSS_L1) ? loss_acc / (float)p.loss_B : loss_acc;
+    if (tid == 0 && p.loss_partials) {
+      float lp = (p.loss_kind == B2H_LOSS_L1) ? loss_acc / (float)p.loss_B : loss_acc;
+      if constexpr (UTT) if (utt_bad) lp = __int_as_float(0x7fffffff);   // a refused segment list: the loss is NaN
+      p.loss_partials[blockIdx.x] = lp;
+    }
     B2H_STAMP();   // partial slice written
 
     if (p.fuse.enabled) {
@@ -979,7 +992,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
       B2H_MARK(2);
       if (blockIdx.x == 0 && tid == 0) {                 // publish the counters for the next launch
         *reinterpret_cast<volatile unsigned*>(f.hdr) = sync_tok;
-        *p.step_dev = step_next;
+        if (!utt_bad) *p.step_dev = step_next;
         if (dp) *p.epoch_dev = epoch_next;
       }
       if (blockIdx.x == 0 && warp == 7 && f.loss_out) {  // loss = sum of the CTAs' loss partials (fixed order)
@@ -1032,7 +1045,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
         for (int j = jb + tid; j < jn; j += kTileThreads) {
           float gr = 0.f;
           for (int pg = 0; pg < groups; ++pg) gr += red[(size_t)pg * ncol * 4 + (j - jb)];
-          bool apply = true;
+          bool apply = !utt_bad;                         // a refused segment list leaves params, m, v and packed as they are
           // padding slots of the slot layout (ci >= cin, bias pad: ~10 % at C = 30) carry no parameter: neither pushed nor polled
           const bool real_slot = one_pass ? (my_i >= 0) : (flat_index_of_gp(g, j) >= 0);
           if (dp && real_slot) {
@@ -1163,15 +1176,16 @@ int launch_tc_tile(const ConvArgs& a, const TilePlan& plan, cudaStream_t stream)
   p.loss_kind = a.loss_kind; p.apply_mask = a.apply_mask; p.mode = a.mode; p.out_scale = a.out_scale; p.geo = a.geo;
   p.B = plan.B; p.T = plan.T;
   p.nhalf = plan.nhalf; p.MB = plan.MB; p.NT = plan.NT; p.HR = plan.HR; p.gh = plan.gh; p.n_tiles = plan.n_tiles;
-  p.utt = a.utt;
+  p.utt = a.utt; p.utt_seg = a.utt_seg; p.utt_max_len = a.utt_max_len;
   const bool train = plan.train, split = plan.split;
   const size_t smem = plan.smem;
   const int grid = plan.grid;
-  // sixteen instantiations: {forward, train, train over window views, forward over utterances} x {NT = 1, 2} x {bf16
-  // operands, bf16 high/low pairs (fp32 mode)}
+  // nineteen instantiations: {forward, train, train over window views, forward over utterances} x {NT = 1, 2} x {bf16
+  // operands, bf16 high/low pairs (fp32 mode)}, and training over segments with bf16 operands at NT = 1, 2 and with bf16
+  // high/low pairs at NT = 1 (split training holds 128 rows, utterance_plan offers it no longer sub-window)
   const int nt2 = p.NT == 2 ? 1 : 0;
-  const int kind = !train ? (p.utt ? 3 : 0) : p.win_start ? 2 : 1;
-  const void* fns[4][2][2] = {
+  const int kind = !train ? (p.utt ? 3 : 0) : p.utt ? 4 : p.win_start ? 2 : 1;
+  const void* fns[5][2][2] = {
       {{(const void*)conv_tc_tile_kernel<false, 1, false>, (const void*)conv_tc_tile_kernel<false, 1, true>},
        {(const void*)conv_tc_tile_kernel<false, 2, false>, (const void*)conv_tc_tile_kernel<false, 2, true>}},
       {{(const void*)conv_tc_tile_kernel<true, 1, false>, (const void*)conv_tc_tile_kernel<true, 1, true>},
@@ -1179,8 +1193,11 @@ int launch_tc_tile(const ConvArgs& a, const TilePlan& plan, cudaStream_t stream)
       {{(const void*)conv_tc_tile_kernel<true, 1, false, true>, (const void*)conv_tc_tile_kernel<true, 1, true, true>},
        {(const void*)conv_tc_tile_kernel<true, 2, false, true>, (const void*)conv_tc_tile_kernel<true, 2, true, true>}},
       {{(const void*)conv_tc_tile_kernel<false, 1, false, false, true>, (const void*)conv_tc_tile_kernel<false, 1, true, false, true>},
-       {(const void*)conv_tc_tile_kernel<false, 2, false, false, true>, (const void*)conv_tc_tile_kernel<false, 2, true, false, true>}}};
+       {(const void*)conv_tc_tile_kernel<false, 2, false, false, true>, (const void*)conv_tc_tile_kernel<false, 2, true, false, true>}},
+      {{(const void*)conv_tc_tile_kernel<true, 1, false, false, true>, (const void*)conv_tc_tile_kernel<true, 1, true, false, true>},
+       {(const void*)conv_tc_tile_kernel<true, 2, false, false, true>, nullptr}}};
   const void* fn = fns[kind][nt2][split ? 1 : 0];
+  if (!fn) { set_error("tile kernel: no instantiation for this plan"); return B2H_ESHAPE; }
   if (int rc = ensure_dyn_smem(fn, smem)) return rc;
   void* kargs[] = {&p};
   cudaError_t le;

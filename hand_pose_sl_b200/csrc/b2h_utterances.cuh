@@ -10,15 +10,23 @@
 // The offsets live on the device, so the host sizes the launch from a bound (UttPlan::max_sub) and a one-CTA planning
 // kernel turns the offsets into the sub-window table the forward kernels read (layout: UttPlan).  The forward kernels end
 // their tile loops at the table's count.
+//
+// Training over segments (b2h_train_*_utterances) plans the same way: segment s = stream rows [seg_start[s], seg_end[s]),
+// 1..max_len frames, trained as one sequence; the planning kernel also writes each sub-window's segment and its length
+// (loss weight 1 / (42 L_s)) and the "bad" word the fused step reads before its Adam update.
 #pragma once
 
 namespace b2h {
 
 constexpr int kUttPlanThreads = 1024;
 constexpr int kUttBadOffsets = 80;   // b2h_tc_status id: offsets not non-decreasing within [0, n_frames]
+constexpr int kUttBadSegments = 81;  // b2h_tc_status id: a training segment outside [0, n_frames] or not of 1..max_len frames
 
-__global__ void __launch_bounds__(kUttPlanThreads) utt_plan_kernel(const long long* __restrict__ off, int n_utt, long long n_frames,
-                                                                   int Ts, int max_sub, int4* ws) {
+// Sequence u is rows [seg_a[u], seg_b[u]): the offsets form of the forward passes (off, off + 1).  max_len > 0 (training):
+// every sequence must hold 1..max_len frames, and seg_out receives {u, L_u} per sub-window.
+__global__ void __launch_bounds__(kUttPlanThreads) utt_plan_kernel(const long long* __restrict__ seg_a, const long long* __restrict__ seg_b,
+                                                                   int n_utt, long long n_frames, int Ts, int max_sub, int max_len,
+                                                                   int bad_id, int4* ws, int2* seg_out) {
   __shared__ int warp_sum[32];
   __shared__ int s_bad;
   int4* table = ws + 1;
@@ -33,8 +41,8 @@ __global__ void __launch_bounds__(kUttPlanThreads) utt_plan_kernel(const long lo
     const int u = base + tid;
     int cnt = 0;
     if (u < n_utt) {
-      const long long a = off[u], b = off[u + 1];
-      if (a < 0 || b < a || b > n_frames) s_bad = 1;
+      const long long a = seg_a[u], b = seg_b[u];
+      if (a < 0 || b < a || b > n_frames || (max_len > 0 && (b == a || b - a > max_len))) s_bad = 1;
       else cnt = sub_window_count(b - a, Ts);
     }
     int v = cnt;
@@ -65,8 +73,8 @@ __global__ void __launch_bounds__(kUttPlanThreads) utt_plan_kernel(const long lo
   const int count = bad ? 0 : (int)carry;
   if (tid == 0) {
     prefix[n_utt] = count;
-    ws[0] = make_int4(count, 0, 0, 0);
-    if (bad) atomicExch(&g_tc_status, kUttBadOffsets);
+    ws[0] = make_int4(count, bad ? 1 : 0, 0, 0);
+    if (bad) atomicExch(&g_tc_status, bad_id);
   }
   __syncthreads();                   // the prefix sums are visible to the whole CTA
   // pass 2: sub-window g -> (utterance u, index i) by binary search over the prefix sums -> sub_window()
@@ -78,8 +86,8 @@ __global__ void __launch_bounds__(kUttPlanThreads) utt_plan_kernel(const long lo
       else hi = mid - 1;
     }
     const int n = prefix[lo + 1] - prefix[lo], i = gi - prefix[lo];
-    const long long a = off[lo];
-    const int L = (int)(off[lo + 1] - a);
+    const long long a = seg_a[lo];
+    const int L = (int)(seg_b[lo] - a);
     int start = 0, clo = 0, chi = L;
     if (n > 1) {
       const SubWindow s = sub_window(L, Ts, n, i);
@@ -87,13 +95,15 @@ __global__ void __launch_bounds__(kUttPlanThreads) utt_plan_kernel(const long lo
     }
     const int len = L - start < Ts ? L - start : Ts;
     table[gi] = make_int4((int)(a + start), start, clo | (chi << 16), len);
+    if (seg_out) seg_out[gi] = make_int2(lo, L);
   }
 }
 
 int launch_utterances(ConvArgs a, const UttPlan& plan, const long long* offsets, int n_utt, long long n_frames, void* workspace,
                       cudaStream_t stream) {
   int4* ws = reinterpret_cast<int4*>(workspace);
-  utt_plan_kernel<<<1, kUttPlanThreads, 0, stream>>>(offsets, n_utt, n_frames, plan.Ts, plan.max_sub, ws);
+  utt_plan_kernel<<<1, kUttPlanThreads, 0, stream>>>(offsets, offsets + 1, n_utt, n_frames, plan.Ts, plan.max_sub, 0, kUttBadOffsets,
+                                                     ws, nullptr);
   count_launch();
   if (int rc = check_launch("utt_plan_kernel")) return rc;
   a.utt = ws;
@@ -101,6 +111,20 @@ int launch_utterances(ConvArgs a, const UttPlan& plan, const long long* offsets,
   a.lengths = nullptr; a.apply_mask = 0;
   if (plan.kernel == B2H_KERNEL_TC_TILE) return launch_tc_tile(a, plan.tile, stream);
   return launch_tc_wide_fwd(a, plan.wide, stream);
+}
+
+int launch_train_utterances(ConvArgs a, const UttPlan& plan, const long long* seg_start, const long long* seg_end, int n_seg,
+                            long long n_frames, int max_len, void* workspace, cudaStream_t stream) {
+  int4* ws = reinterpret_cast<int4*>(reinterpret_cast<char*>(workspace) + plan.plan_off);
+  int2* seg = reinterpret_cast<int2*>(reinterpret_cast<char*>(ws) + plan.seg_off);
+  utt_plan_kernel<<<1, kUttPlanThreads, 0, stream>>>(seg_start, seg_end, n_seg, n_frames, plan.Ts, plan.max_sub, max_len,
+                                                     kUttBadSegments, ws, seg);
+  count_launch();
+  if (int rc = check_launch("utt_plan_kernel")) return rc;
+  a.utt = ws; a.utt_seg = seg; a.utt_max_len = max_len;
+  a.B = n_seg; a.T = plan.Ts;
+  a.lengths = nullptr; a.apply_mask = 1;
+  return launch_tc_tile(a, plan.tile, stream);
 }
 
 }  // namespace b2h

@@ -120,6 +120,13 @@ class GpuPoseDataset(Dataset):
         return {"win_start": torch.tensor(starts, dtype=torch.int64), "win_end": torch.tensor(ends, dtype=torch.int64),
                 "n_frames": torch.tensor(nf, dtype=torch.int64)}
 
+    def utterance_segments(self, indices):
+        """The segment list of a training step on whole utterances over `training_streams()`: (seg_start, seg_end) as CPU
+        int64 (S,) tensors, utterance `indices[s]` = frames [offsets[idx], offsets[idx + 1]) (no crop, no pad frames)."""
+        idx = np.asarray(indices, dtype=np.int64).reshape(-1)
+        off = np.asarray(self.packed.offsets, dtype=np.int64)
+        return torch.from_numpy(off[idx].copy()), torch.from_numpy(off[idx + 1].copy())
+
     def training_streams(self, dtype=torch.bfloat16):
         """Per-frame training data of ALL packed frames, built once per dtype and cached ({input_kp, target_kp,
         target_conf}, `PreprocessRightHand.training_stream`).  Per-frame preprocessing does not depend on the window, so the

@@ -183,9 +183,16 @@ class ConvModel(nn.Module):
             self._packed_versions = versions
         return self._packed
 
-    def workspace(self, B, T):
+    def workspace(self, B, T, segments=False):
+        """The training workspace for a batch of B windows of T frames, or (segments=True) for B segments of at most T
+        frames (b2h_train_utterances_workspace_bytes).  One buffer, grown on demand: its header is shared by every step."""
         n_in, C, pe = self._geometry()
-        need = _lib.workspace_bytes(B, T, n_in, C, pe, _lib.PRECISIONS[self.precision])
+        if segments:
+            need = _lib.load().b2h_train_utterances_workspace_bytes(int(B), int(T), n_in, C, pe, _lib.PRECISIONS[self.precision])
+            if need < 0:
+                raise _lib.B2HError(_lib.last_error())
+        else:
+            need = _lib.workspace_bytes(B, T, n_in, C, pe, _lib.PRECISIONS[self.precision])
         dev = self._flat.device
         if self._workspace is None or self._workspace.numel() < need or self._workspace.device != dev:
             self._workspace = torch.zeros(need, dtype=torch.uint8, device=dev)    # holds the fused kernel's grid-barrier words

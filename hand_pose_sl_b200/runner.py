@@ -5,7 +5,8 @@ what a training / serving loop uses once shapes are fixed (SURVEY.md §0.7: laun
 tensor pipe or HBM, bounds every BASELINE config).
 
 Input staging: every slot is ONE contiguous device buffer  [input_kp | target_kp | target_conf? | n_frames(int32)]
-(WindowTrainStepRunner, over frame streams resident on the device: [win_start | win_end | n_frames])
+(WindowTrainStepRunner, over frame streams resident on the device: [win_start | win_end | n_frames];
+UtteranceTrainStepRunner: [seg_start | seg_end])
 and `host_stage(batch)` builds the same layout in pinned host memory, so a step's inputs travel with ONE
 cudaMemcpyAsync (`load_staged`).  With `x_dtype=torch.bfloat16` the keypoint input is shipped as bf16 -- the bf16
 kernels round it to bf16 on the way into shared memory anyway (cvt.rn == torch's CPU rounding), so the result is
@@ -16,7 +17,7 @@ import torch
 
 from . import _lib
 from .models import ConvModel
-from .steps import FusedAdam, _dense_inputs, _view_inputs
+from .steps import FusedAdam, _dense_inputs, _segment_inputs, _view_inputs
 
 
 def _align(n, a=256):
@@ -165,6 +166,9 @@ class _StepBuffers:
         """Raise if a device-side wait gave up (grid barrier, MMA completion, data-parallel peer wait).  Synchronises."""
         tc = int(self.lib.b2h_tc_status())
         dp = int(self.lib.b2h_dp_status())
+        if tc == 81 and not dp:
+            raise _lib.B2HError("bad segment list (tc_status=81): a segment outside the streams or not of 1..max_len frames; "
+                                "that step changed no parameter, moment or step counter and its loss is NaN")
         if tc or dp:
             raise _lib.B2HError(f"device-side wait timed out (tc_status={tc}, dp_status={dp}): "
                                 + ("a data-parallel peer never delivered its gradients; parameter updates were suppressed "
@@ -237,6 +241,36 @@ class WindowTrainStepRunner(_StepBuffers):
             model, streams, crops["win_start"], T, crops["n_frames"], crops["win_end"], pad_mode, loss))
         self.win_end.fill_(streams["input_kp"].shape[0])
         self.lengths.fill_(T)
+
+
+class UtteranceTrainStepRunner(_StepBuffers):
+    """TrainStepRunner over SEGMENTS of device-resident frame streams, each trained as one whole sequence
+    (`steps.fused_train_step_utterances`): a slot holds the step's segment list, ONE buffer [seg_start int64 | seg_end int64]
+    of n_seg segments of at most max_len frames each, loaded from a dict {seg_start, seg_end} or the pair
+    `GpuPoseDataset.utterance_segments` returns, by `load` / `host_stage` + `load_staged`.  Steps, capture, replay,
+    `pipelined_steps` and finish behave as TrainStepRunner's; a bad segment list makes its step a no-op that
+    `check_status` reports.  `streams` stay referenced by the runner (a captured graph reads them by address)."""
+
+    def __init__(self, model: ConvModel, optimizer: FusedAdam, streams, n_seg: int, max_len: int, loss: str = "L1",
+                 n_slots: int = 1):
+        _check_x_dtype(model, streams["input_kp"].dtype)
+        self._init_common(model, optimizer, n_seg, max_len, loss, n_slots, (
+            ("seg_start", "seg_start", torch.int64, (n_seg,)), ("seg_end", "seg_end", torch.int64, (n_seg,))))
+        self.ws = model.workspace(n_seg, max_len, segments=True)
+        self._bind(self.lib.b2h_train_step_utterances, lambda segs: _segment_inputs(
+            model, streams, segs["seg_start"], segs["seg_end"], max_len, loss))
+        self._shape = self._shape[2:]               # (n_seg, max_len) travel with the segment list, not after the loss
+        self.seg_end.fill_(1)                       # a valid list until the first load: segment s = frame 0
+
+    @staticmethod
+    def _as_dict(segs):
+        return segs if isinstance(segs, dict) else {"seg_start": segs[0], "seg_end": segs[1]}
+
+    def load(self, segs, slot=0, non_blocking=True):
+        super().load(self._as_dict(segs), slot, non_blocking)
+
+    def host_stage(self, segs, out=None):
+        return super().host_stage(self._as_dict(segs), out)
 
 
 def pipelined_steps(runner, batches, status_every=0, copy_streams=1):

@@ -248,9 +248,8 @@ def _dense_inputs(model: ConvModel, batch, loss):
     return (x.contiguous(), _lib.dtype_code(x.dtype), tgt, conf, _lib.lengths_i32(batch["n_frames"], dev, B)), B, T, dev
 
 
-def _view_inputs(model: ConvModel, streams, win_start, T, lengths, win_end, pad_mode, loss):
-    """`_dense_inputs` of the *_windows entry points: (frames, x_dtype, target_frames, conf_frames, n_frames, win_start,
-    win_end, pad_mode, lengths), and the number of windows, T and the device."""
+def _stream_inputs(model: ConvModel, streams, T, loss):
+    """The three training streams, checked: (frames, x_dtype, target_frames, conf_frames, n_frames) and the device."""
     x = streams["input_kp"]
     F, T = model._check_input(x, T)
     dev = x.device
@@ -262,33 +261,69 @@ def _view_inputs(model: ConvModel, streams, win_start, T, lengths, win_end, pad_
         conf = streams["target_conf"].to(device=dev, dtype=torch.float32).contiguous()
         if conf.numel() != F * 21:
             raise RuntimeError(f"target_conf stream has {conf.numel()} values for {F} frames (expected (F, 21))")
+    return (x.contiguous(), _lib.dtype_code(x.dtype), tgt, conf, F), dev
+
+
+def _view_inputs(model: ConvModel, streams, win_start, T, lengths, win_end, pad_mode, loss):
+    """`_dense_inputs` of the *_windows entry points: (frames, x_dtype, target_frames, conf_frames, n_frames, win_start,
+    win_end, pad_mode, lengths), and the number of windows, T and the device."""
+    head, dev = _stream_inputs(model, streams, T, loss)
     ws = torch.as_tensor(win_start).to(device=dev, dtype=torch.int64).contiguous()
     W = ws.numel()
     we = None if win_end is None else torch.as_tensor(win_end).to(device=dev, dtype=torch.int64).contiguous()
     if we is not None and we.numel() != W:
         raise RuntimeError("win_end must have one entry per window")
-    return (x.contiguous(), _lib.dtype_code(x.dtype), tgt, conf, F, ws, we, _lib.PAD_MODES[pad_mode],
-            _lib.lengths_i32(lengths, dev, W)), W, T, dev
+    return (*head, ws, we, _lib.PAD_MODES[pad_mode], _lib.lengths_i32(lengths, dev, W)), W, T, dev
+
+
+def _segment_inputs(model: ConvModel, streams, seg_start, seg_end, max_len, loss):
+    """`_view_inputs` of the *_utterances entry points: (frames, x_dtype, target_frames, conf_frames, n_frames, seg_start,
+    seg_end, n_seg, max_len), and the number of segments, max_len and the device.  max_len defaults to the longest host-side
+    segment; device segments need it given."""
+    if model.pos_emb is not None and not model.pos_emb_any_length:
+        raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {model.pos_emb.max_len} "
+                           "(training on segments needs pos_emb_any_length=True)")
+    head, dev = _stream_inputs(model, streams, 1, loss)
+    on_device = any(isinstance(t, torch.Tensor) and t.is_cuda for t in (seg_start, seg_end))
+    if max_len is None:
+        if on_device:
+            raise ValueError("max_len is required when the segments are already on the device")
+        lens = torch.as_tensor(seg_end).reshape(-1).to(torch.int64) - torch.as_tensor(seg_start).reshape(-1).to(torch.int64)
+        max_len = int(lens.max()) if lens.numel() else 1
+    ss = torch.as_tensor(seg_start).to(device=dev, dtype=torch.int64).contiguous()
+    se = torch.as_tensor(seg_end).to(device=dev, dtype=torch.int64).contiguous()
+    S = ss.numel()
+    if S < 1 or se.numel() != S:
+        raise RuntimeError("seg_start and seg_end must have one entry per segment (at least one)")
+    return (*head, ss, se, S, int(max_len)), S, int(max_len), dev
 
 
 def _train_step(entry, model, optimizer, inputs, loss, who):
-    """forward + criterion + backward + reduction + Adam + re-pack through C entry point `entry` (b2h_train_step[_windows])."""
+    """forward + criterion + backward + reduction + Adam + re-pack through C entry point `entry`
+    (b2h_train_step[_windows|_utterances]).  The segment step takes its shape in `inputs` and the Adam step from the
+    device-side counter, which it advances."""
     args, W, T, dev = inputs
+    segments = entry.endswith("_utterances")
     group = optimizer.param_groups[0]
     if optimizer._owner(group) is not model:
         raise RuntimeError(f"{who} needs FusedAdam(model.parameters()) over exactly this model")
     st = optimizer._group_state(0, group, model)
+    if segments and st["dev_step_mirror"] != st["step"]:
+        st["step_dev"].fill_(int(st["step"]))
     st["step"] += 1
     n_in, C, pe = model._geometry()
     packed = model.packed_weights()
-    ws = model.workspace(W, T)
+    ws = model.workspace(W, T, segments)
     flat = model.flat_parameters()
     loss_out = torch.empty((), dtype=torch.float32, device=dev)
     b1, b2 = group["betas"]
     _lib.check(getattr(_lib.load(), entry)(
-        *_lib.ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(st["m"]), _lib.ptr(st["v"]), _lib.ptr(loss_out), W, T,
-        n_in, C, pe, _lib.LOSSES[loss], _lib.PRECISIONS[model.precision], float(group["lr"]), b1, b2, group["eps"], st["step"],
-        None, None, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
+        *_lib.ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(st["m"]), _lib.ptr(st["v"]), _lib.ptr(loss_out),
+        *(() if segments else (W, T)), n_in, C, pe, _lib.LOSSES[loss], _lib.PRECISIONS[model.precision], float(group["lr"]),
+        b1, b2, group["eps"], st["step"], _lib.ptr(st["step_dev"]) if segments else None, None, _lib.ptr(ws), ws.numel(),
+        _lib.stream_ptr(dev)))
+    if segments:
+        st["dev_step_mirror"] = st["step"]
     model.packed_weights(fresh_from_kernel=True)
     st["step_t"].fill_(float(st["step"]))
     return loss_out
@@ -296,18 +331,20 @@ def _train_step(entry, model, optimizer, inputs, loss, who):
 
 def _forward_backward(entry, model, inputs, loss, want_pred):
     """forward + criterion + backward and the gradient reduction through C entry point `entry`
-    (b2h_train_forward_backward[_windows])."""
+    (b2h_train_forward_backward[_windows|_utterances])."""
     args, W, T, dev = inputs
+    segments = entry.endswith("_utterances")
     n_in, C, pe = model._geometry()
     packed = model.packed_weights()
-    ws = model.workspace(W, T)
+    ws = model.workspace(W, T, segments)
     flat = model.flat_parameters()
     grads = torch.empty_like(flat)
     loss_out = torch.empty((), dtype=torch.float32, device=dev)
     pred = torch.empty((W, T, 21, 2), dtype=torch.float32, device=dev) if want_pred else None
     _lib.check(getattr(_lib.load(), entry)(
-        *_lib.ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(grads), _lib.ptr(loss_out), _lib.ptr(pred), W, T,
-        n_in, C, pe, _lib.LOSSES[loss], _lib.PRECISIONS[model.precision], None, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
+        *_lib.ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(grads), _lib.ptr(loss_out), _lib.ptr(pred),
+        *(() if segments else (W, T)), n_in, C, pe, _lib.LOSSES[loss], _lib.PRECISIONS[model.precision], None, _lib.ptr(ws),
+        ws.numel(), _lib.stream_ptr(dev)))
     return (loss_out, grads, pred) if want_pred else (loss_out, grads)
 
 
@@ -343,6 +380,26 @@ def forward_backward_windows(model: ConvModel, streams, win_start, T, lengths, w
     [, masked prediction (W, T, 21, 2)]), bit-identical to `forward_backward` on the materialised windows."""
     inputs = _view_inputs(model, streams, win_start, T, lengths, win_end, pad_mode, loss)
     return _forward_backward("b2h_train_forward_backward_windows", model, inputs, loss, want_pred)
+
+
+def fused_train_step_utterances(model: ConvModel, streams, seg_start, seg_end, optimizer: FusedAdam, max_len=None, loss="L1"):
+    """`fused_train_step` on SEGMENTS of device-resident frame streams, each trained as one whole sequence (utterances of
+    any length): `streams` as in `fused_train_step_windows`; segment s = frames [seg_start[s], seg_end[s]) of all three
+    streams, zero-padded only at its own two ends -- the reference's forward on a batch of one window of exactly L_s frames
+    with lengths = [L_s].  L1 = (1/S) sum_s (per-segment mean), confL1 = sum_s (per-segment confidence-weighted mean).
+    Whole utterances: `GpuPoseDataset.utterance_segments`.  `max_len` bounds every L_s (default: the longest host-side
+    segment; required for device segments).  A segment outside [0, F] or not of 1..max_len frames (checked on the device)
+    makes the step a no-op with a NaN loss and b2h_tc_status 81.  Served where the tile kernel trains (conv_channels <= 32,
+    at most 32 input channels, bf16 or fp32 mode); B2HError otherwise.  Two launches; returns the 0-dim device loss."""
+    inputs = _segment_inputs(model, streams, seg_start, seg_end, max_len, loss)
+    return _train_step("b2h_train_step_utterances", model, optimizer, inputs, loss, "fused_train_step_utterances")
+
+
+def forward_backward_utterances(model: ConvModel, streams, seg_start, seg_end, max_len=None, loss="L1", want_pred=False):
+    """`forward_backward` on segments (see `fused_train_step_utterances`): returns (loss, flat gradients [, masked
+    prediction (S, max_len, 21, 2): row t of segment s, zero for t >= L_s])."""
+    inputs = _segment_inputs(model, streams, seg_start, seg_end, max_len, loss)
+    return _forward_backward("b2h_train_forward_backward_utterances", model, inputs, loss, want_pred)
 
 
 @torch.no_grad()

@@ -318,6 +318,45 @@ int b2h_train_step_windows(const void* frames, int x_dtype, const float* target_
                            double lr, double beta1, double beta2, double eps, int64_t step, int64_t* step_dev,
                            const double* lr_dev, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* Training on SEGMENTS of device-resident frame streams, each trained as one whole sequence (utterances of any length):
+ * frames (n_frames, n_in) fp32 or bf16, target_frames (n_frames, 42) and conf_frames (n_frames, 21, confL1 only) fp32 as in
+ * b2h_train_forward_backward_windows; seg_start / seg_end (n_seg) int64 on the device: segment s is rows
+ * [seg_start[s], seg_end[s]) of all three streams, L_s frames, zero-padded only at its own two ends -- ConvModel.forward on
+ * a batch of one window of exactly L_s frames with lengths = [L_s].  The positional row is t / max_len of the model (t from
+ * the segment start).  Loss L1: (1/n_seg) sum_s sum_rows |pred - target| / (42 L_s); confL1: sum_s sum_rows
+ * |pred - target| conf / (42 L_s) (the reference's sum of per-sample means).  Segments may overlap or repeat.
+ * max_len >= every L_s bounds the grid, the workspace and the plan.  A segment with L_s < 1, L_s > max_len, seg_start < 0
+ * or seg_end > n_frames (checked on the device) makes the call a no-op: no parameter, moment, packed weight or step counter
+ * changes, the loss is NaN and b2h_tc_status reads 81.
+ * Each segment is cut into sub-windows of Ts frames (b2h_train_utterances_plan, b2h_utterance_subwindows) whose core rows
+ * carry the criterion.  Enqueues only (no allocation, no synchronisation; graph capturable).  workspace:
+ * b2h_train_utterances_workspace_bytes, 16-byte aligned, the first B2H_WS_HEADER bytes shared with the other train steps.
+ * Served by the tile kernel: conv_channels <= 32 with at most 32 input channels, bf16 or fp32 mode (B2H_ESHAPE otherwise).
+ * b2h_train_forward_backward_utterances: planning kernel, training kernel, gradient reduction into grads_out (flat, P) and
+ * *loss_out; pred_out (n_seg, max_len, 42) fp32, nullable: row t of segment s is the masked prediction, zero for t >= L_s. */
+int b2h_train_forward_backward_utterances(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
+                                          int64_t n_frames, const int64_t* seg_start, const int64_t* seg_end, int n_seg,
+                                          int max_len, const float* params, const void* packed, float* grads_out,
+                                          float* loss_out, float* pred_out, int n_in, int C, int pos_emb, int loss_kind,
+                                          int precision, int64_t* step_dev, void* workspace, int64_t workspace_bytes,
+                                          void* stream);
+/* The whole training step on segments in two launches: the planning kernel, then ONE cooperative launch of forward,
+ * criterion, backward, gradient reduction, Adam (lr or *lr_dev) and weight re-pack.  step_dev is required: the step reads the
+ * Adam step from it and advances it (`step` is checked as in b2h_train_step_windows and not read otherwise). */
+int b2h_train_step_utterances(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
+                              int64_t n_frames, const int64_t* seg_start, const int64_t* seg_end, int n_seg, int max_len,
+                              float* params, void* packed, float* exp_avg, float* exp_avg_sq, float* loss_out, int n_in, int C,
+                              int pos_emb, int loss_kind, int precision, double lr, double beta1, double beta2, double eps,
+                              int64_t step, int64_t* step_dev, const double* lr_dev, void* workspace, int64_t workspace_bytes,
+                              void* stream);
+/* bytes of workspace the *_utterances training calls need for n_seg segments of at most max_len frames; B2H_ESHAPE for an
+ * unserved shape */
+int64_t b2h_train_utterances_workspace_bytes(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision);
+/* Host-only: the kernel family the *_utterances training calls run (B2H_KERNEL_TC_TILE / _NONE) and, into *seg_len
+ * (nullable), the sub-window length Ts: the rule of b2h_utterances_plan for a segment of max_len frames, over the lengths the
+ * tile kernel trains as whole windows (bf16 64 / 128 / 256, fp32 mode 64 / 128). */
+int b2h_train_utterances_plan(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision, int* seg_len);
+
 /* tcgen05 / TMEM / descriptor self-test (tests/test_tc_probe.py): D = A·B^T for one 128xNx(16*ksteps)
  * bf16 tile staged in the no-swizzle K-major layout the conv kernels use, A rows shifted by `shift`
  * rows (the implicit-im2col trick).  out (128,N) fp32. */
