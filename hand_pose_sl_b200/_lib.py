@@ -72,6 +72,11 @@ _SIGNATURES = {
                                           c_int64, c_void_p]),
     "b2h_train_utterances_workspace_bytes": (c_int64, [c_int, c_int, c_int, c_int, c_int, c_int]),
     "b2h_train_utterances_plan": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "b2h_validate_utterances": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int, c_void_p,
+                                        c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int64,
+                                        c_void_p]),
+    "b2h_validate_utterances_workspace_bytes": (c_int64, [c_int, c_int, c_int, c_int, c_int, c_int]),
+    "b2h_validate_utterances_plan": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "b2h_conv_backward": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                   c_int, c_int, c_void_p, c_int64, c_void_p]),
     "b2h_mask_output": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),

@@ -97,21 +97,26 @@ static TrainPlan train_plan(const Geo& g, int B, int T, int precision) {
 // else the wide forward (bf16 mode); the plan takes the Ts whose family computes the fewest MMA rows for an utterance of the
 // mean length n_frames / n_utt under the cut rule (ties: the longer Ts, fewer sub-windows).  Rows per sub-window are the
 // tile's rows over the windows it holds: 64 / 128 / 256 in the tile kernel, 256 / floor(258 / (Ts + 2)) in the wide one.
-// Training over segments (max_len > 0, b2h_train_*_utterances): n_utt segments of at most max_len frames, the same rule for a
+// Training over segments (kUttTrain, b2h_train_*_utterances): n_utt segments of at most max_len frames, the same rule for a
 // segment of max_len frames over the lengths the tile kernel trains as whole windows (bf16: 64 / 128 / 256, fp32 mode: 64 /
 // 128), sized for n_utt * n(max_len) sub-windows; the workspace is the training one (header, gradient and loss partials of
 // the plan's grid) followed by the table and one {segment, length} pair per sub-window.
-static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int precision, int max_len = 0) {
+// Validation over segments (kUttValidate, b2h_validate_utterances): the forward's families, the training's sizing (a segment
+// of max_len frames, n_utt * n(max_len) sub-windows); the workspace is the table, one {segment, length} pair and one float
+// (the sub-window's criterion sum) per sub-window.
+enum UttPurpose { kUttForward, kUttTrain, kUttValidate };
+static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int precision, UttPurpose purpose, int max_len = 0) {
   static const int kMenu[3] = {256, 128, 64};
   UttPlan best{};
   best.kernel = B2H_KERNEL_NONE;
   if (precision != B2H_BF16 && precision != B2H_FP32) return best;   // the FFMA kernel reads dense windows only
-  const bool train = max_len > 0;
-  const int64_t mean = train ? max_len : n_frames / (n_utt > 0 ? n_utt : 1);
+  const bool train = purpose == kUttTrain, segments = purpose != kUttForward;
+  if (segments && max_len < 1) return best;
+  const int64_t mean = segments ? max_len : n_frames / (n_utt > 0 ? n_utt : 1);
   double best_rows = 0.0;
   for (int Ts : kMenu) {
-    const int64_t max_sub = train ? (int64_t)n_utt * sub_window_count(max_len, Ts)
-                                  : (int64_t)(n_utt > 0 ? n_utt : 0) + n_frames / (Ts - 32);
+    const int64_t max_sub = segments ? (int64_t)n_utt * sub_window_count(max_len, Ts)
+                                     : (int64_t)(n_utt > 0 ? n_utt : 0) + n_frames / (Ts - 32);
     if (max_sub > (int64_t)INT32_MAX / 2) continue;
     UttPlan c{};
     c.Ts = Ts;
@@ -133,10 +138,13 @@ static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int pre
     const double rows = rows_per_sub * sub_window_count(mean > 0 ? mean : 1, Ts);
     if (best.kernel != B2H_KERNEL_NONE && rows >= best_rows) continue;
     c.ws_bytes = (utt_prefix_offset(c.max_sub) + 4 * ((int64_t)n_utt + 1) + 255) / 256 * 256;
+    if (segments) c.seg_off = (utt_prefix_offset(c.max_sub) + 4 * ((int64_t)n_utt + 1) + 15) / 16 * 16;
     if (train) {
       c.plan_off = (B2H_WS_HEADER + ((int64_t)c.tile.grid * gp_total(g) + c.tile.grid) * 4 + 255) / 256 * 256;
-      c.seg_off = (utt_prefix_offset(c.max_sub) + 4 * ((int64_t)n_utt + 1) + 15) / 16 * 16;
       c.ws_bytes = (c.plan_off + c.seg_off + 8 * (int64_t)c.max_sub + 255) / 256 * 256;
+    } else if (segments) {
+      c.part_off = c.seg_off + 8 * (int64_t)c.max_sub;
+      c.ws_bytes = (c.part_off + 4 * (int64_t)c.max_sub + 255) / 256 * 256;
     }
     best = c;
     best_rows = rows;
@@ -317,7 +325,7 @@ static const char* const kUttServed =
 extern "C" int b2h_utterances_plan(int64_t n_frames, int n_utt, int n_in, int C, int pos_emb, int precision, int* seg_len) {
   if (seg_len) *seg_len = 0;
   if (!geo_ok(n_in, C, pos_emb) || n_frames < 0 || n_frames > INT32_MAX || n_utt < 0) return B2H_KERNEL_NONE;
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), n_frames, n_utt, precision);
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), n_frames, n_utt, precision, kUttForward);
   if (seg_len && u.kernel != B2H_KERNEL_NONE) *seg_len = u.Ts;
   return u.kernel;
 }
@@ -341,7 +349,7 @@ extern "C" int64_t b2h_utterances_workspace_bytes(int64_t n_frames, int n_utt, i
   if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
   if (n_frames < 0 || n_frames > INT32_MAX || n_utt < 0) { set_error("%s: bad n_frames=%lld n_utt=%d", who, (long long)n_frames, n_utt); return B2H_ESHAPE; }
   if (n_utt == 0) return 256;
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), n_frames, n_utt, precision);
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), n_frames, n_utt, precision, kUttForward);
   if (u.kernel == B2H_KERNEL_NONE) { set_error("%s: %s (C=%d, n_in=%d, precision=%d)", who, kUttServed, C, n_in, precision); return B2H_ESHAPE; }
   return u.ws_bytes;
 }
@@ -364,7 +372,7 @@ extern "C" int b2h_conv_forward_utterances(const void* frames, int x_dtype, int6
   }
   if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
   const Geo g = make_geo(n_in, C, pos_emb);
-  const UttPlan plan = utterance_plan(g, n_frames, n_utt, precision);
+  const UttPlan plan = utterance_plan(g, n_frames, n_utt, precision, kUttForward);
   if (plan.kernel == B2H_KERNEL_NONE) {
     set_error("%s: %s; no kernel for C=%d, n_in=%d, precision=%d", who, kUttServed, C, n_in, precision);
     return B2H_ESHAPE;
@@ -581,7 +589,7 @@ static const char* const kUttTrainServed =
 extern "C" int b2h_train_utterances_plan(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision, int* seg_len) {
   if (seg_len) *seg_len = 0;
   if (!geo_ok(n_in, C, pos_emb) || n_seg < 1 || max_len < 1) return B2H_KERNEL_NONE;
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, max_len);
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, kUttTrain, max_len);
   if (seg_len && u.kernel != B2H_KERNEL_NONE) *seg_len = u.Ts;
   return u.kernel;
 }
@@ -590,7 +598,7 @@ extern "C" int64_t b2h_train_utterances_workspace_bytes(int n_seg, int max_len, 
   const char* who = "b2h_train_utterances_workspace_bytes";
   if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
   if (n_seg < 1 || max_len < 1) { set_error("%s: bad n_seg=%d max_len=%d", who, n_seg, max_len); return B2H_ESHAPE; }
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, max_len);
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, kUttTrain, max_len);
   if (u.kernel == B2H_KERNEL_NONE) { set_error("%s: %s (C=%d, n_in=%d, precision=%d)", who, kUttTrainServed, C, n_in, precision); return B2H_ESHAPE; }
   return u.ws_bytes;
 }
@@ -619,7 +627,7 @@ static int train_utterances(const void* frames, int x_dtype, const float* target
     return B2H_EALIGN;
   }
   const Geo g = make_geo(n_in, C, pos_emb);
-  const UttPlan plan = utterance_plan(g, n_frames, n_seg, precision, max_len);
+  const UttPlan plan = utterance_plan(g, n_frames, n_seg, precision, kUttTrain, max_len);
   if (plan.kernel == B2H_KERNEL_NONE) {
     set_error("%s: %s; no kernel for C=%d, n_in=%d, precision=%d", who, kUttTrainServed, C, n_in, precision);
     return B2H_ESHAPE;
@@ -685,6 +693,67 @@ extern "C" int b2h_train_step_utterances(const void* frames, int x_dtype, const 
   return train_utterances(frames, x_dtype, target_frames, conf_frames, n_frames, seg_start, seg_end, n_seg, max_len, params, packed,
                           nullptr, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace, workspace_bytes,
                           (cudaStream_t)stream, who, &fuse, nullptr, nullptr);
+}
+
+static const char* const kUttValidateServed =
+    "segments are validated by the utterance forward: in bf16 mode for conv_channels <= 256, in fp32 mode for "
+    "conv_channels <= 32 with at most 32 input channels (fp32-ffma has no segment path)";
+
+extern "C" int b2h_validate_utterances_plan(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision, int* seg_len) {
+  if (seg_len) *seg_len = 0;
+  if (!geo_ok(n_in, C, pos_emb) || n_seg < 1 || max_len < 1) return B2H_KERNEL_NONE;
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, kUttValidate, max_len);
+  if (seg_len && u.kernel != B2H_KERNEL_NONE) *seg_len = u.Ts;
+  return u.kernel;
+}
+
+extern "C" int64_t b2h_validate_utterances_workspace_bytes(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision) {
+  const char* who = "b2h_validate_utterances_workspace_bytes";
+  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
+  if (n_seg < 1 || max_len < 1) { set_error("%s: bad n_seg=%d max_len=%d", who, n_seg, max_len); return B2H_ESHAPE; }
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, kUttValidate, max_len);
+  if (u.kernel == B2H_KERNEL_NONE) { set_error("%s: %s (C=%d, n_in=%d, precision=%d)", who, kUttValidateServed, C, n_in, precision); return B2H_ESHAPE; }
+  return u.ws_bytes;
+}
+
+extern "C" int b2h_validate_utterances(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
+                                       int64_t n_frames, const int64_t* seg_start, const int64_t* seg_end, int n_seg, int max_len,
+                                       const float* params, const void* packed, float* seg_loss_out, float* loss_out, int n_in,
+                                       int C, int pos_emb, int loss_kind, int precision, void* workspace,
+                                       int64_t workspace_bytes, void* stream) {
+  const char* who = "b2h_validate_utterances";
+  if (!seg_start || !seg_end || !loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  if (int rc = check_common(frames, x_dtype, nullptr, params, packed, workspace, 1, 0, 1, n_in, C, pos_emb, who)) return rc;
+  if (n_seg < 1 || max_len < 1 || n_frames < 0 || n_frames > INT32_MAX) {
+    set_error("%s: bad n_seg=%d max_len=%d n_frames=%lld", who, n_seg, max_len, (long long)n_frames);
+    return B2H_ESHAPE;
+  }
+  if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
+  if (!target_frames) { set_error("%s: null target", who); return B2H_EINVAL; }
+  if (loss_kind != B2H_LOSS_L1 && loss_kind != B2H_LOSS_CONFL1) { set_error("%s: bad loss_kind %d", who, loss_kind); return B2H_EINVAL; }
+  if (loss_kind == B2H_LOSS_CONFL1 && !conf_frames) { set_error("%s: confL1 needs scores", who); return B2H_EINVAL; }
+  if (misaligned(frames, 15) || misaligned(target_frames, 7) || misaligned(conf_frames, 3) || misaligned(packed, 15) ||
+      misaligned(workspace, 15) || misaligned(seg_start, 7) || misaligned(seg_end, 7) || misaligned(seg_loss_out, 3) ||
+      misaligned(loss_out, 3)) {
+    set_error("%s: frames, packed and workspace must be 16-byte aligned, target_frames, seg_start and seg_end 8-byte, "
+              "conf_frames, seg_loss_out and loss_out 4-byte aligned", who);
+    return B2H_EALIGN;
+  }
+  const Geo g = make_geo(n_in, C, pos_emb);
+  const UttPlan plan = utterance_plan(g, n_frames, n_seg, precision, kUttValidate, max_len);
+  if (plan.kernel == B2H_KERNEL_NONE) {
+    set_error("%s: %s; no kernel for C=%d, n_in=%d, precision=%d", who, kUttValidateServed, C, n_in, precision);
+    return B2H_ESHAPE;
+  }
+  if (workspace_bytes < plan.ws_bytes) {
+    set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.ws_bytes);
+    return B2H_EWORKSPACE;
+  }
+  ConvArgs a{};
+  a.x = frames; a.x_dtype = x_dtype; a.target = target_frames; a.conf = conf_frames; a.params = params;
+  a.packed = reinterpret_cast<const char*>(packed); a.loss_kind = loss_kind; a.mode = 0; a.out_scale = 1.0f; a.geo = g;
+  return launch_validate_utterances(a, plan, reinterpret_cast<const long long*>(seg_start), reinterpret_cast<const long long*>(seg_end),
+                                    n_seg, (long long)n_frames, max_len, seg_loss_out, loss_out, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int b2h_train_step_dp(const void* x, int x_dtype, const float* target, const float* conf, const int32_t* lengths,

@@ -329,7 +329,7 @@ struct ConvArgs {
   const float* params; const char* packed;
   float* y;                 // forward output / masked prediction (nullable in train mode)
   float* partials;          // [grid][gp_total]
-  float* loss_partials;     // [grid]
+  float* loss_partials;     // [grid]; a forward over utterances: nullptr, or one criterion sum per sub-window (validation)
   long long* step_dev;      // nullable: device step counter, incremented by block 0 (read by the Adam kernel)
   long long* epoch_dev;     // nullable: data-parallel exchange epoch, incremented the same way (never rewound)
   FuseAdam fuse;            // tensor-core train kernel only: reduce + exchange + Adam in the same launch
@@ -358,7 +358,9 @@ int tc_status_and_clear();
 // sub-window g = {stream row of its first frame, its first frame in the utterance, clo | chi << 16, frames before the
 // utterance end (<= Ts)} and bad = 1 when the planning kernel refused the offsets / segments (count = 0 then).
 // Training over segments (b2h_train_*_utterances) plans the same table at plan_off of the training workspace, followed at
-// seg_off (from the table's start) by one int2 per sub-window: {segment, segment length}.
+// seg_off (from the table's start) by one int2 per sub-window: {segment, segment length}.  Validation over segments
+// (b2h_validate_utterances) plans the same table and segment array at the workspace's start, followed at part_off by one
+// float per sub-window: its criterion sum, written by the forward.
 struct UttPlan {
   int kernel;               // B2H_KERNEL_TC_TILE | B2H_KERNEL_TC_WIDE | B2H_KERNEL_NONE
   int Ts;                   // sub-window length
@@ -366,6 +368,7 @@ struct UttPlan {
   TilePlan tile; WidePlan wide;   // planned for max_sub windows of Ts frames
   int64_t ws_bytes;
   int64_t plan_off, seg_off; // training: byte offset of the table in the workspace, of the segment array from the table
+  int64_t part_off;         // validation: byte offset of the per-sub-window sums from the table
 };
 __host__ __device__ inline int64_t utt_prefix_offset(int max_sub) { return (int64_t)(1 + max_sub) * 16; }
 // planning kernel, then the forward of a.B = plan.max_sub sub-windows of a.T = plan.Ts frames over the table it wrote
@@ -375,6 +378,12 @@ int launch_utterances(ConvArgs a, const UttPlan& plan, const long long* offsets,
 // tile kernel (a.fuse.enabled: the fused step) over the table it wrote; a.B = n_seg
 int launch_train_utterances(ConvArgs a, const UttPlan& plan, const long long* seg_start, const long long* seg_end, int n_seg,
                             long long n_frames, int max_len, void* workspace, cudaStream_t stream);
+
+// planning kernel over the segments (each 1..max_len frames), the forward over the table it wrote with the criterion per
+// sub-window instead of predictions (a.loss_partials = the sums), then the per-segment means and the loss
+int launch_validate_utterances(ConvArgs a, const UttPlan& plan, const long long* seg_start, const long long* seg_end, int n_seg,
+                               long long n_frames, int max_len, float* seg_loss, float* loss_out, void* workspace,
+                               cudaStream_t stream);
 
 void set_debug_timing(long long* p);
 int launch_format_prediction(const float* pred, float* out, int64_t rows, int mode, cudaStream_t stream);

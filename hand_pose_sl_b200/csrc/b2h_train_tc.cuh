@@ -229,9 +229,13 @@ __device__ __forceinline__ long long global_ns() { long long t; asm volatile("mo
 // are written, to y at their stream rows.  Training (b2h_train_*_utterances): target and confidence rows are read at the
 // stream rows, the criterion covers the core rows with the weight 1 / (42 L_s) of the row's segment, the masked prediction
 // goes to row (segment, frame in the segment) of y, and a plan the planning kernel refused ("bad") makes the step a no-op.
-template <bool TRAIN, int NT, bool SPLIT, bool VIEW = false, bool UTT = false>
+// CRIT (forward over utterances only) = validation over segments (b2h_validate_utterances): the layer-4 epilogue stores no
+// prediction; it sums the criterion term |a s - t s| over the core rows of every sub-window against the target (and
+// confidence) rows at the stream rows, and writes one sum per sub-window, reduced in a fixed order, to loss_partials[g].
+template <bool TRAIN, int NT, bool SPLIT, bool VIEW = false, bool UTT = false, bool CRIT = false>
 __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArgs p) {
   static_assert(!(UTT && VIEW), "utterances and window views are separate instantiations");
+  static_assert(!CRIT || (UTT && !TRAIN), "the validation criterion is a view of the forward over utterances");
   int dbg_n = 0;
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) uint64_t bar;      // MMAs of the current phase complete (one arrival per issuing warp)
@@ -241,6 +245,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
   __shared__ uint32_t tmem_slot;
   __shared__ __align__(16) float bias_s[4][64];
   __shared__ float red_s[8];
+  __shared__ float crit_s[8][2];             // CRIT: per warp, per row segment: the sub-window's criterion sum
   const Geo& g = p.geo;
   const int T = p.T, MB = p.MB, HR = p.HR, nhalf = p.nhalf, gh = p.gh;
   constexpr int kWgCol = 64 * NT;
@@ -679,7 +684,30 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
         // and the body is straight-line code -- the generic loop below executed ~4x the instructions of a hidden
         // layer's epilogue (per-element predicates for the confidence weights, the given-d_y mode and the y store).
         const bool l4_fast = TRAIN && p.mode == 1 && p.loss_kind == B2H_LOSS_L1 && tgt_smem && p.y == nullptr;
-        if (TRAIN && l4_fast) {
+        if constexpr (CRIT) {
+          // validation: the criterion term of the training epilogue (L1 = the weighted form with s = 1) on the core rows
+          // before the segment end; target rows are 168 B, 8-B aligned at odd stream rows: float2 loads
+          const bool live = valid && in_core;
+          const float* trow = p.target + (live ? drow : 0) * B2H_COUT;
+          const float* crow = (p.loss_kind == B2H_LOSS_CONFL1) ? p.conf + (live ? drow : 0) * (B2H_COUT / 2) : nullptr;
+          for (int c0 = 16 * ch; c0 < N; c0 += 32) {
+            uint32_t v[16];
+            tmem_ld16(taddr + c0, v);
+            tmem_ld_wait();
+#pragma unroll
+            for (int q = 0; q < 16; q += 2) {
+              const int c = c0 + q;
+              if (live && c < B2H_COUT) {
+                const float2 tv = __ldg(reinterpret_cast<const float2*>(trow + c));
+                const float sv = crow ? __ldg(crow + (c >> 1)) : 1.0f;
+                const float a0 = __uint_as_float(v[q]) + bias_s[3][c], a1 = __uint_as_float(v[q + 1]) + bias_s[3][c + 1];
+                sum += fabsf(__fsub_rn(__fmul_rn(a0, sv), __fmul_rn(tv.x, sv)));
+                sum += fabsf(__fsub_rn(__fmul_rn(a1, sv), __fmul_rn(tv.y, sv)));
+              }
+            }
+          }
+          contrib += sum;
+        } else if (TRAIN && l4_fast) {
           const bool live = valid && (t < len) && in_core;   // rows t >= len are zeroed by mask_output and carry no loss
           auto chunk = [&](auto c0_tag) {
             constexpr int C0 = decltype(c0_tag)::value;
@@ -782,6 +810,12 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
         for (int o = 16; o > 0; o >>= 1) contrib += __shfl_xor_sync(0xffffffffu, contrib, o);
         if (lane == 0) red_s[warp] = contrib;
       }
+      if constexpr (CRIT) if (l == 3) {
+        // lanes 0-15 / 16-31 of a warp hold rows of row segment 0 / 1 when a tile holds two (nhalf == 2)
+#pragma unroll
+        for (int o = 8; o > 0; o >>= 1) contrib += __shfl_xor_sync(0xffffffffu, contrib, o);
+        if ((lane & 15) == 0) crit_s[warp][lane >> 4] = contrib;
+      }
       fence_proxy_async_smem();
       tc_fence_before();
       __syncthreads();
@@ -793,6 +827,11 @@ __global__ void __launch_bounds__(kTileThreads, 1) conv_tc_tile_kernel(TcTileArg
           bulk_s2g(p.y + (size_t)(wbase + w) * T * B2H_COUT, YS + (size_t)(h * MB + j * (T + 2)) * B2H_COUT, (uint32_t)T * B2H_COUT * 4);
         }
         bulk_commit();
+      }
+      if constexpr (CRIT) if (l == 3 && tid < nhalf) {   // one sub-window per row segment (gh == 1: Ts >= 64, launch_tc_tile)
+        float s = 0.f;
+        for (int w = 0; w < 8; ++w) s += nhalf == 2 ? crit_s[w][tid] : crit_s[w][0] + crit_s[w][1];
+        if (wbase + tid < utt_n) p.loss_partials[wbase + tid] = s;
       }
       B2H_STAMP();   // fwd layer: epilogue done
     }
@@ -1180,12 +1219,15 @@ int launch_tc_tile(const ConvArgs& a, const TilePlan& plan, cudaStream_t stream)
   const bool train = plan.train, split = plan.split;
   const size_t smem = plan.smem;
   const int grid = plan.grid;
-  // nineteen instantiations: {forward, train, train over window views, forward over utterances} x {NT = 1, 2} x {bf16
+  // twenty-three instantiations: {forward, train, train over window views, forward over utterances} x {NT = 1, 2} x {bf16
   // operands, bf16 high/low pairs (fp32 mode)}, and training over segments with bf16 operands at NT = 1, 2 and with bf16
-  // high/low pairs at NT = 1 (split training holds 128 rows, utterance_plan offers it no longer sub-window)
+  // high/low pairs at NT = 1 (split training holds 128 rows, utterance_plan offers it no longer sub-window), and validation
+  // over segments (a forward over utterances with loss_partials set) at NT = 1, 2 with both operand kinds
   const int nt2 = p.NT == 2 ? 1 : 0;
-  const int kind = !train ? (p.utt ? 3 : 0) : p.utt ? 4 : p.win_start ? 2 : 1;
-  const void* fns[5][2][2] = {
+  const bool crit = !train && p.utt && p.loss_partials;
+  const int kind = !train ? (p.utt ? (crit ? 5 : 3) : 0) : p.utt ? 4 : p.win_start ? 2 : 1;
+  if (crit && p.gh != 1) { set_error("tile kernel: validation needs one sub-window per row segment (gh = %d)", p.gh); return B2H_ESHAPE; }
+  const void* fns[6][2][2] = {
       {{(const void*)conv_tc_tile_kernel<false, 1, false>, (const void*)conv_tc_tile_kernel<false, 1, true>},
        {(const void*)conv_tc_tile_kernel<false, 2, false>, (const void*)conv_tc_tile_kernel<false, 2, true>}},
       {{(const void*)conv_tc_tile_kernel<true, 1, false>, (const void*)conv_tc_tile_kernel<true, 1, true>},
@@ -1195,7 +1237,9 @@ int launch_tc_tile(const ConvArgs& a, const TilePlan& plan, cudaStream_t stream)
       {{(const void*)conv_tc_tile_kernel<false, 1, false, false, true>, (const void*)conv_tc_tile_kernel<false, 1, true, false, true>},
        {(const void*)conv_tc_tile_kernel<false, 2, false, false, true>, (const void*)conv_tc_tile_kernel<false, 2, true, false, true>}},
       {{(const void*)conv_tc_tile_kernel<true, 1, false, false, true>, (const void*)conv_tc_tile_kernel<true, 1, true, false, true>},
-       {(const void*)conv_tc_tile_kernel<true, 2, false, false, true>, nullptr}}};
+       {(const void*)conv_tc_tile_kernel<true, 2, false, false, true>, nullptr}},
+      {{(const void*)conv_tc_tile_kernel<false, 1, false, false, true, true>, (const void*)conv_tc_tile_kernel<false, 1, true, false, true, true>},
+       {(const void*)conv_tc_tile_kernel<false, 2, false, false, true, true>, (const void*)conv_tc_tile_kernel<false, 2, true, false, true, true>}}};
   const void* fn = fns[kind][nt2][split ? 1 : 0];
   if (!fn) { set_error("tile kernel: no instantiation for this plan"); return B2H_ESHAPE; }
   if (int rc = ensure_dyn_smem(fn, smem)) return rc;

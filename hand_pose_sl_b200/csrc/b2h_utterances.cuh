@@ -127,4 +127,72 @@ int launch_train_utterances(ConvArgs a, const UttPlan& plan, const long long* se
   return launch_tc_tile(a, plan.tile, stream);
 }
 
+// Validation over segments, the last launch: seg_loss[s] = (the sums of segment s's sub-windows, in table order) / (42 L_s);
+// loss = the sum over s in a fixed order (per-thread strided sums, then a fixed tree), times 1 / S for L1.  A refused plan:
+// NaN in loss and every seg_loss entry.
+__global__ void __launch_bounds__(kUttPlanThreads) utt_validate_finish_kernel(const int4* __restrict__ ws, const int2* __restrict__ seg,
+                                                                              const float* __restrict__ part, int n_seg, int max_sub,
+                                                                              int loss_kind, float* seg_loss, float* loss_out) {
+  __shared__ float warp_sum[32];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  griddep_wait();                    // the forward's sums are complete and visible
+  const bool bad = __ldg(&ws->y) != 0;
+  const int* prefix = reinterpret_cast<const int*>(reinterpret_cast<const char*>(ws) + utt_prefix_offset(max_sub));
+  const float nan = __int_as_float(0x7fffffff);
+  float acc = 0.f;
+  for (int s = tid; s < n_seg; s += kUttPlanThreads) {
+    float v = nan;
+    if (!bad) {
+      const int g0 = __ldg(prefix + s), g1 = __ldg(prefix + s + 1);
+      float sum = 0.f;
+      for (int gi = g0; gi < g1; ++gi) sum += __ldg(part + gi);
+      v = sum / ((float)__ldg(&seg[g0].y) * (float)B2H_COUT);   // every segment has >= 1 sub-window: seg[g0] is its own
+      acc += v;
+    }
+    if (seg_loss) seg_loss[s] = v;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if (lane == 0) warp_sum[warp] = acc;
+  __syncthreads();
+  if (tid == 0) {
+    float total = 0.f;
+    for (int w = 0; w < kUttPlanThreads / 32; ++w) total += warp_sum[w];
+    *loss_out = bad ? nan : (loss_kind == B2H_LOSS_L1 ? total / (float)n_seg : total);
+  }
+}
+
+int launch_validate_utterances(ConvArgs a, const UttPlan& plan, const long long* seg_start, const long long* seg_end, int n_seg,
+                               long long n_frames, int max_len, float* seg_loss, float* loss_out, void* workspace,
+                               cudaStream_t stream) {
+  int4* ws = reinterpret_cast<int4*>(workspace);
+  int2* seg = reinterpret_cast<int2*>(reinterpret_cast<char*>(ws) + plan.seg_off);
+  float* part = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + plan.part_off);
+  utt_plan_kernel<<<1, kUttPlanThreads, 0, stream>>>(seg_start, seg_end, n_seg, n_frames, plan.Ts, plan.max_sub, max_len,
+                                                     kUttBadSegments, ws, seg);
+  count_launch();
+  if (int rc = check_launch("utt_plan_kernel")) return rc;
+  a.utt = ws; a.loss_partials = part;
+  a.B = plan.max_sub; a.T = plan.Ts;
+  a.lengths = nullptr; a.apply_mask = 0; a.y = nullptr;
+  const int rc = plan.kernel == B2H_KERNEL_TC_TILE ? launch_tc_tile(a, plan.tile, stream) : launch_tc_wide_fwd(a, plan.wide, stream);
+  if (rc) return rc;
+  // programmatic dependent launch: its set-up overlaps the forward's tail; it reads the sums after griddepcontrol.wait
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(1); cfg.blockDim = dim3(kUttPlanThreads); cfg.dynamicSmemBytes = 0; cfg.stream = stream;
+  cudaLaunchAttribute at;
+  at.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at.val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = &at; cfg.numAttrs = 1;
+  const int4* cws = ws;
+  const int2* cseg = seg;
+  const float* cpart = part;
+  int lk = a.loss_kind, ms = plan.max_sub;
+  void* kargs[] = {&cws, &cseg, &cpart, &n_seg, &ms, &lk, &seg_loss, &loss_out};
+  const cudaError_t le = cudaLaunchKernelExC(&cfg, (const void*)utt_validate_finish_kernel, kargs);
+  if (le != cudaSuccess) { cudaGetLastError(); set_error("utt_validate_finish_kernel launch: %s", cudaGetErrorString(le)); return B2H_ECUDA; }
+  count_launch();
+  return check_launch("utt_validate_finish_kernel");
+}
+
 }  // namespace b2h

@@ -121,9 +121,13 @@ __device__ __forceinline__ bool wait_addr(uint32_t bar, uint32_t parity, int sit
 // UTT (MODE 0 only) = sub-windows of utterances (b2h_conv_forward_utterances): window g reads its rows from the plan's
 // table in p.scratch, rows at or past the utterance end are zero in every layer, and only the core rows are written, to y
 // at their stream rows.  p.B / p.n_tiles are the host's upper bound; the plan's count ends the tile loops.
-template <int MODE, bool VIEW = false, bool UTT = false>
+// CRIT (UTT only) = validation over segments (b2h_validate_utterances): layer 4 stores no prediction; it sums the criterion
+// term |a s - t s| over the core rows of every sub-window against the target (and confidence) rows at the stream rows and
+// writes one sum per sub-window, reduced in a fixed order, to p.loss_partials[g].
+template <int MODE, bool VIEW = false, bool UTT = false, bool CRIT = false>
 __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs p, const __grid_constant__ CUtensorMap wmap) {
   static_assert(!UTT || MODE == 0, "utterances are a forward-only view");
+  static_assert(!CRIT || UTT, "the validation criterion is a view of the forward over utterances");
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) uint64_t full_bar[kWideMaxStages];    // stage landed (TMA complete_tx)
   __shared__ __align__(8) uint64_t empty_bar[kWideMaxStages];   // stage consumed (tcgen05.commit)
@@ -132,6 +136,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
   __shared__ uint32_t tmem_slot;
   __shared__ __align__(16) float bias_s[4][256];
   __shared__ float loss_w[8];
+  __shared__ float crit_w[8][3];                                // CRIT: per epilogue warp, per window of the tile
   const Geo& g = p.geo;
   const int T = p.T, gh = p.gh;
   const int tid = threadIdx.x, lane = tid & 31;
@@ -466,6 +471,52 @@ __global__ void __launch_bounds__(kWideThreads, 1) conv_tc_wide_kernel(WideArgs 
               *reinterpret_cast<uint4*>(out + o0) = q0;
               *reinterpret_cast<uint4*>(out + o1) = q1;
             }
+          }
+        } else if constexpr (CRIT) {
+          // layer 4, validation: the criterion term of the training epilogue (L1 = the weighted form with s = 1) on the core
+          // rows before the segment end, summed per window of the tile; target rows are 168 B, 8-B aligned at odd stream
+          // rows: float2 loads
+          float wsum[3] = {0.f, 0.f, 0.f};                     // gh <= 3 windows per tile
+          for (int j = 0; j < 2; ++j) {
+            const RowCtx rc = rowctx(j, tile);
+            const uint32_t taddr = tbase + lane_addr + 256 * j;
+            const bool live = rc.valid && rc.t >= (rc.us.z & 0xFFFF) && rc.t < (rc.us.z >> 16);
+            const size_t tro = live ? (size_t)rc.us.x + rc.t : 0;
+            const float* tg = p.target + tro * B2H_COUT;
+            const float* cf = (p.loss_kind == B2H_LOSS_CONFL1) ? p.conf + tro * (B2H_COUT / 2) : nullptr;
+            float sum = 0.f;
+            for (int c0 = 16 * ch; c0 < N; c0 += 32) {
+              uint32_t v[16];
+              tmem_ld16(taddr + c0, v);
+              tmem_ld_wait();
+#pragma unroll
+              for (int q = 0; q < 16; q += 2) {
+                const int c = c0 + q;
+                if (live && c < B2H_COUT) {
+                  const float2 tv = __ldg(reinterpret_cast<const float2*>(tg + c));
+                  const float sv = cf ? __ldg(cf + (c >> 1)) : 1.0f;
+                  const float a0 = __uint_as_float(v[q]) + bias_s[3][c], a1 = __uint_as_float(v[q + 1]) + bias_s[3][c + 1];
+                  sum += fabsf(__fsub_rn(__fmul_rn(a0, sv), __fmul_rn(tv.x, sv)));
+                  sum += fabsf(__fsub_rn(__fmul_rn(a1, sv), __fmul_rn(tv.y, sv)));
+                }
+              }
+            }
+            const int wj = (r128 + 128 * j) / (T + 2);
+#pragma unroll
+            for (int k = 0; k < 3; ++k) wsum[k] += k == wj ? sum : 0.f;
+          }
+#pragma unroll
+          for (int k = 0; k < 3; ++k) {
+            float s = wsum[k];
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+            if (lane == 0) crit_w[warp][k] = s;
+          }
+          named_bar_sync(1, kWideEpiThreads);               // the epilogue warps only
+          if (tid < gh) {                                   // (crit_w is rewritten only after this thread's next arrival)
+            float s = 0.f;
+            for (int w = 0; w < 8; ++w) s += crit_w[w][tid];
+            if (tile * gh + tid < utt_n) p.loss_partials[tile * gh + tid] = s;
           }
         } else if (MODE == 0) {
           for (int j = 0; j < 2; ++j) {
@@ -833,13 +884,15 @@ int launch_tc_wide_fwd(const ConvArgs& a, const WidePlan& plan, cudaStream_t str
   const Geo& g = a.geo;
   WideArgs p = wide_args(a, plan);
   p.scratch = reinterpret_cast<unsigned char*>(const_cast<int4*>(a.utt));
-  auto* fn = a.utt ? conv_tc_wide_kernel<0, false, true> : conv_tc_wide_kernel<0>;
+  // a forward over utterances with loss_partials set: validation (the criterion per sub-window, no prediction)
+  const bool crit = a.utt && a.loss_partials;
+  auto* fn = crit ? conv_tc_wide_kernel<0, false, true, true> : a.utt ? conv_tc_wide_kernel<0, false, true> : conv_tc_wide_kernel<0>;
   if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), plan.smem)) return rc;
   CUtensorMap wmap;
   if (int rc = wide_weight_map(a.packed + g.tf_off[0], g.td_off[0] - g.tf_off[0], &wmap)) return rc;
   fn<<<plan.grid, kWideThreads, plan.smem, stream>>>(p, wmap);
   count_launch();
-  return check_launch(a.utt ? "conv_tc_wide_kernel<fwd, utterances>" : "conv_tc_wide_kernel<fwd>");
+  return check_launch(crit ? "conv_tc_wide_kernel<fwd, validation>" : a.utt ? "conv_tc_wide_kernel<fwd, utterances>" : "conv_tc_wide_kernel<fwd>");
 }
 
 // ---- wide training: forward+criterion (saves layer inputs), dgrad chain, split-K wgrad; the caller reduces + applies Adam ----

@@ -100,6 +100,7 @@ class ConvModel(nn.Module):
         self._packed_versions = None
         self._workspace = None
         self._utt_workspace = None
+        self._val_workspace = None
         self._flatten()
 
     # ------------------------------------------------------------------ flat parameter storage
@@ -128,7 +129,7 @@ class ConvModel(nn.Module):
 
     def __getstate__(self):
         st = dict(self.__dict__)
-        for k in ("_flat", "_packed", "_packed_versions", "_workspace", "_utt_workspace"):
+        for k in ("_flat", "_packed", "_packed_versions", "_workspace", "_utt_workspace", "_val_workspace"):
             st[k] = None
         return st
 
@@ -314,6 +315,20 @@ class ConvModel(nn.Module):
         if self._utt_workspace is None or self._utt_workspace.numel() < n or self._utt_workspace.device != dev:
             self._utt_workspace = torch.empty(n, dtype=torch.uint8, device=dev)
         return self._utt_workspace
+
+    def validate_workspace(self, n_seg, max_len):
+        """The workspace of steps.validate_utterances (sub-window table, segment pairs, per-sub-window sums) for n_seg
+        segments of at most max_len frames, cached on the model like utterances_workspace() and apart from the training
+        workspace, so a validation pass may sit between training steps (and graphs) on the same stream."""
+        n_in, C, pe = self._geometry()
+        n = _lib.load().b2h_validate_utterances_workspace_bytes(int(n_seg), int(max_len), n_in, C, pe,
+                                                                 _lib.PRECISIONS[self.precision])
+        if n < 0:
+            raise _lib.B2HError(_lib.last_error())
+        dev = self._flat.device
+        if self._val_workspace is None or self._val_workspace.numel() < n or self._val_workspace.device != dev:
+            self._val_workspace = torch.empty(n, dtype=torch.uint8, device=dev)
+        return self._val_workspace
 
     @torch.no_grad()
     def predict_utterances(self, frames, offsets, denormalize=None, out=None):

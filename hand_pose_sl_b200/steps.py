@@ -403,6 +403,39 @@ def forward_backward_utterances(model: ConvModel, streams, seg_start, seg_end, m
 
 
 @torch.no_grad()
+def validate_utterances(model: ConvModel, streams, seg_start, seg_end, max_len=None, loss="L1", per_segment=False):
+    """validate() (traintest.py:168-211) on SEGMENTS of device-resident frame streams, each evaluated as one whole sequence:
+    the loss `fused_train_step_utterances` computes for the same streams and segments (L1 = (1/S) sum_s per-segment mean,
+    confL1 = sum_s per-segment confidence-weighted mean), from one forward and no backward.  Segment s is frames
+    [seg_start[s], seg_end[s]) zero-padded only at its own two ends, the sequence `predict_utterances` sees at inference, so
+    no pad frame reaches the last frames of a short utterance as it does in `validate_batch`'s padded crops.  Arguments as in
+    `fused_train_step_utterances` (segments may overlap, repeat or leave gaps; `max_len` is required for device segments).
+    Returns the 0-dim device loss, or (loss, seg_loss (S,)) with per_segment=True.  Parameters, packed weights and the
+    optimiser state are only read; the workspace is `model.validate_workspace`, apart from the training one.  A segment
+    outside [0, F] or not of 1..max_len frames (checked on the device) gives NaN in loss and every seg_loss entry and
+    b2h_tc_status 81.  Deterministic (fixed summation order); three launches, graph capturable.  Served in bf16 mode for
+    conv_channels <= 256 and in fp32 mode for conv_channels <= 32 with at most 32 input channels; B2HError otherwise.
+
+    A validation split of whole utterances, reported in pixels as traintest.py:207 does:
+
+        val_s, val_e = dataset.utterance_segments(val_indices)
+        l1 = validate_utterances(model, dataset.training_streams(), val_s, val_e, loss="L1")
+        print(L12Pixels(21, 1280)(l1.item()))
+    """
+    args, S, max_len, dev = _segment_inputs(model, streams, seg_start, seg_end, max_len, loss)
+    n_in, C, pe = model._geometry()
+    packed = model.packed_weights()
+    flat = model.flat_parameters()
+    ws = model.validate_workspace(S, max_len)
+    loss_out = torch.empty((), dtype=torch.float32, device=dev)
+    seg_loss = torch.empty(S, dtype=torch.float32, device=dev) if per_segment else None
+    _lib.check(_lib.load().b2h_validate_utterances(
+        *_lib.ptrs(args), _lib.ptr(flat), _lib.ptr(packed), _lib.ptr(seg_loss), _lib.ptr(loss_out), n_in, C, pe,
+        _lib.LOSSES[loss], _lib.PRECISIONS[model.precision], _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)))
+    return (loss_out, seg_loss) if per_segment else loss_out
+
+
+@torch.no_grad()
 def validate_batch(model: ConvModel, batch, loss="L1"):
     """validate() body, traintest.py:174-207, for one batch: forward + mask_output + criterion."""
     pred = model.predict(batch["input_kp"], lengths=batch["n_frames"])

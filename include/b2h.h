@@ -357,6 +357,29 @@ int64_t b2h_train_utterances_workspace_bytes(int n_seg, int max_len, int n_in, i
  * tile kernel trains as whole windows (bf16 64 / 128 / 256, fp32 mode 64 / 128). */
 int b2h_train_utterances_plan(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision, int* seg_len);
 
+/* Validation on SEGMENTS: the loss the segment training step computes, for the same streams and segment list, from one
+ * forward and no backward.  Segment s is evaluated as one sequence of L_s frames zero-padded at its two ends (ConvModel.forward
+ * on one window of exactly L_s frames with lengths = [L_s], then mask_output and the criterion).  seg_loss_out (n_seg) fp32,
+ * nullable: the per-sample term of maskedPoseL1 / poderatedPoseL1, sum_rows |pred s - target s| / (42 L_s) (s = 1 for L1);
+ * *loss_out: their mean (L1) or sum (confL1), each summed in a fixed order (bit-identical reruns).  Segment rules and
+ * max_len as in b2h_train_forward_backward_utterances; a refused segment list (checked on the device, b2h_tc_status 81)
+ * writes NaN to *loss_out and every seg_loss_out entry.  Parameters, packed weights and every training buffer are only
+ * read.  Three launches (planning kernel, forward with the criterion, finishing kernel); enqueues only (graph capturable).
+ * workspace: b2h_validate_utterances_workspace_bytes, 16-byte aligned, its own (no training workspace header).  Served in
+ * bf16 mode for conv_channels <= 256 and in fp32 mode for conv_channels <= 32 with at most 32 input channels (B2H_ESHAPE
+ * otherwise, fp32-ffma included). */
+int b2h_validate_utterances(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
+                            int64_t n_frames, const int64_t* seg_start, const int64_t* seg_end, int n_seg, int max_len,
+                            const float* params, const void* packed, float* seg_loss_out, float* loss_out, int n_in, int C,
+                            int pos_emb, int loss_kind, int precision, void* workspace, int64_t workspace_bytes, void* stream);
+/* bytes of workspace b2h_validate_utterances needs for n_seg segments of at most max_len frames (the sub-window table, one
+ * {segment, length} pair and one float per sub-window); B2H_ESHAPE for an unserved shape */
+int64_t b2h_validate_utterances_workspace_bytes(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision);
+/* Host-only: the kernel family b2h_validate_utterances runs (B2H_KERNEL_TC_TILE / _TC_WIDE / _NONE) and, into *seg_len
+ * (nullable), the sub-window length Ts: the family rule of b2h_utterances_plan (tile where it fits, else wide in bf16 mode)
+ * for a segment of max_len frames. */
+int b2h_validate_utterances_plan(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision, int* seg_len);
+
 /* tcgen05 / TMEM / descriptor self-test (tests/test_tc_probe.py): D = A·B^T for one 128xNx(16*ksteps)
  * bf16 tile staged in the no-swizzle K-major layout the conv kernels use, A rows shifted by `shift`
  * rows (the implicit-im2col trick).  out (128,N) fp32. */
