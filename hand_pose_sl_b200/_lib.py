@@ -184,29 +184,25 @@ def launch_count() -> int:
     return int(load().b2h_launch_count())
 
 
-def param_count(n_in, C, pos_emb) -> int:
-    n = load().b2h_param_count(n_in, C, int(pos_emb))
+def query(name, *args) -> int:
+    """The count or byte size C-ABI query `name` returns for `args`; a negative result is an error code: B2HError."""
+    n = getattr(load(), name)(*args)
     if n < 0:
         raise B2HError(last_error())
     return int(n)
+
+
+def param_count(n_in, C, pos_emb) -> int:
+    return query("b2h_param_count", n_in, C, int(pos_emb))
 
 
 def param_offset(n_in, C, pos_emb, layer, is_bias) -> int:
-    n = load().b2h_param_offset(n_in, C, int(pos_emb), layer, int(is_bias))
-    if n < 0:
-        raise B2HError(last_error())
-    return int(n)
+    return query("b2h_param_offset", n_in, C, int(pos_emb), layer, int(is_bias))
 
 
 def packed_bytes(n_in, C, pos_emb) -> int:
-    n = load().b2h_packed_bytes(n_in, C, int(pos_emb))
-    if n < 0:
-        raise B2HError(last_error())
-    return int(n)
+    return query("b2h_packed_bytes", n_in, C, int(pos_emb))
 
 
 def workspace_bytes(B, T, n_in, C, pos_emb, precision) -> int:
-    n = load().b2h_workspace_bytes(B, T, n_in, C, int(pos_emb), precision)
-    if n < 0:
-        raise B2HError(last_error())
-    return int(n)
+    return query("b2h_workspace_bytes", B, T, n_in, C, int(pos_emb), precision)

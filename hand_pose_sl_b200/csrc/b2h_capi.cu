@@ -99,13 +99,10 @@ static TrainPlan train_plan(const Geo& g, int B, int T, int precision) {
 // tile's rows over the windows it holds: 64 / 128 / 256 in the tile kernel, 256 / floor(258 / (Ts + 2)) in the wide one.
 // Training over segments (kUttTrain, b2h_train_*_utterances): n_utt segments of at most max_len frames, the same rule for a
 // segment of max_len frames over the lengths the tile kernel trains as whole windows (bf16: 64 / 128 / 256, fp32 mode: 64 /
-// 128), sized for n_utt * n(max_len) sub-windows; the workspace is the training one (header, gradient and loss partials of
-// the plan's grid) followed by the table and one {segment, length} pair per sub-window.
-// Validation over segments (kUttValidate, b2h_validate_utterances): the forward's families, the training's sizing (a segment
-// of max_len frames, n_utt * n(max_len) sub-windows); the workspace is the table, one {segment, length} pair and one float
-// (the sub-window's criterion sum) per sub-window.
+// 128), sized for n_utt * n(max_len) sub-windows.  Validation over segments (kUttValidate, b2h_validate_utterances): the
+// forward's families, the training's sizing.  The workspace layout is UttPlan's.
 enum UttPurpose { kUttForward, kUttTrain, kUttValidate };
-static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int precision, UttPurpose purpose, int max_len = 0) {
+static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int precision, UttPurpose purpose, int max_len) {
   static const int kMenu[3] = {256, 128, 64};
   UttPlan best{};
   best.kernel = B2H_KERNEL_NONE;
@@ -137,19 +134,65 @@ static UttPlan utterance_plan(const Geo& g, int64_t n_frames, int n_utt, int pre
     }
     const double rows = rows_per_sub * sub_window_count(mean > 0 ? mean : 1, Ts);
     if (best.kernel != B2H_KERNEL_NONE && rows >= best_rows) continue;
-    c.ws_bytes = (utt_prefix_offset(c.max_sub) + 4 * ((int64_t)n_utt + 1) + 255) / 256 * 256;
-    if (segments) c.seg_off = (utt_prefix_offset(c.max_sub) + 4 * ((int64_t)n_utt + 1) + 15) / 16 * 16;
-    if (train) {
-      c.plan_off = (B2H_WS_HEADER + ((int64_t)c.tile.grid * gp_total(g) + c.tile.grid) * 4 + 255) / 256 * 256;
-      c.ws_bytes = (c.plan_off + c.seg_off + 8 * (int64_t)c.max_sub + 255) / 256 * 256;
-    } else if (segments) {
-      c.part_off = c.seg_off + 8 * (int64_t)c.max_sub;
-      c.ws_bytes = (c.part_off + 4 * (int64_t)c.max_sub + 255) / 256 * 256;
-    }
+    if (train) c.plan_off = (B2H_WS_HEADER + ((int64_t)c.tile.grid * gp_total(g) + c.tile.grid) * 4 + 255) / 256 * 256;
+    c.seg_off = (utt_prefix_offset(c.max_sub) + 4 * ((int64_t)n_utt + 1) + 15) / 16 * 16;
+    c.part_off = c.seg_off + (segments ? 8 * (int64_t)c.max_sub : 0);
+    const int64_t end = c.part_off + (purpose == kUttValidate ? 4 * (int64_t)c.max_sub : 0);
+    c.ws_bytes = (c.plan_off + end + 255) / 256 * 256;
     best = c;
     best_rows = rows;
   }
   return best;
+}
+
+// What utterance_plan serves, by purpose (the refusals of the queries and of the run entry points).
+static const char* const kUttServed[3] = {
+    "utterances are served in bf16 mode for conv_channels <= 256 and in fp32 mode for conv_channels <= 32 with at most 32 "
+    "input channels",
+    "segments are trained by the tile kernel: conv_channels <= 32 with at most 32 input channels, in bf16 or fp32 mode "
+    "(wider models and fp32-ffma have no segment path)",
+    "segments are validated by the utterance forward: in bf16 mode for conv_channels <= 256, in fp32 mode for "
+    "conv_channels <= 32 with at most 32 input channels (fp32-ffma has no segment path)"};
+
+// The six utterance queries: n utterances in a stream of n_frames frames (forward), or n segments of at most max_len frames.
+// who == nullptr: a *_plan query, which leaves the error string alone, returns the kernel and writes the sub-window length
+// to seg_len; else a *_workspace_bytes query, which returns the workspace size or B2H_ESHAPE.
+static int64_t utterance_query(UttPurpose purpose, int64_t n_frames, int n, int max_len, int n_in, int C, int pos_emb,
+                               int precision, int* seg_len, const char* who) {
+  const int64_t refused = who ? B2H_ESHAPE : B2H_KERNEL_NONE;
+  if (seg_len) *seg_len = 0;
+  if (!geo_ok(n_in, C, pos_emb, who)) return refused;
+  if (purpose == kUttForward ? n_frames < 0 || n_frames > INT32_MAX || n < 0 : n < 1 || max_len < 1) {
+    if (who && purpose == kUttForward) set_error("%s: bad n_frames=%lld n_utt=%d", who, (long long)n_frames, n);
+    else if (who) set_error("%s: bad n_seg=%d max_len=%d", who, n, max_len);
+    return refused;
+  }
+  if (who && n == 0) return 256;     // the forward over no utterances launches nothing
+  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), n_frames, n, precision, purpose, max_len);
+  if (!who) {
+    if (seg_len && u.kernel != B2H_KERNEL_NONE) *seg_len = u.Ts;
+    return u.kernel;
+  }
+  if (u.kernel == B2H_KERNEL_NONE) {
+    set_error("%s: %s (C=%d, n_in=%d, precision=%d)", who, kUttServed[purpose], C, n_in, precision);
+    return B2H_ESHAPE;
+  }
+  return u.ws_bytes;
+}
+
+// The plan of an utterance run entry point over the sequences of sv: served, and the workspace large enough.
+static int utterance_run_plan(const Geo& g, const SegmentView& sv, int precision, UttPurpose purpose, int64_t workspace_bytes,
+                              const char* who, UttPlan* u) {
+  *u = utterance_plan(g, sv.n_frames, sv.n, precision, purpose, sv.max_len);
+  if (u->kernel == B2H_KERNEL_NONE) {
+    set_error("%s: %s; no kernel for C=%d, n_in=%d, precision=%d", who, kUttServed[purpose], g.C, g.n_in, precision);
+    return B2H_ESHAPE;
+  }
+  if (workspace_bytes < u->ws_bytes) {
+    set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)u->ws_bytes);
+    return B2H_EWORKSPACE;
+  }
+  return B2H_OK;
 }
 
 }  // namespace b2h
@@ -254,30 +297,52 @@ static WindowView window_view(const int64_t* win_start, const int64_t* win_end, 
   return WindowView{reinterpret_cast<const long long*>(win_start), reinterpret_cast<const long long*>(win_end), (long long)n_frames, pad_mode};
 }
 
+// The segment view of the *_utterances entry points (the forward's offsets: seg_end = offsets + 1, max_len = 0).
+static SegmentView segment_view(const int64_t* seg_start, const int64_t* seg_end, int n, int64_t n_frames, int max_len) {
+  return SegmentView{reinterpret_cast<const long long*>(seg_start), reinterpret_cast<const long long*>(seg_end), n, (long long)n_frames, max_len};
+}
+
 // The checks every forward and training entry point makes first, in this order: pointers (`out` = y in the forward, the
-// workspace in training), x_dtype, pad_mode, geometry, shape (B >= B_min).
-static int check_common(const void* x, int x_dtype, const WindowView* wv, const float* params, const void* packed,
-                        const void* out, int B, int B_min, int T, int n_in, int C, int pos_emb, const char* who) {
-  if (!x || (wv && !wv->win_start) || !params || !packed || !out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+// workspace in training), x_dtype, pad_mode, geometry, shape (B >= B_min; a segment view: n >= B_min sequences in a stream
+// of at most INT32_MAX frames, and with B_min = 1, segments of max_len >= 1 frames).
+static int check_common(const void* x, int x_dtype, const WindowView* wv, const SegmentView* sv, const float* params,
+                        const void* packed, const void* out, int B, int B_min, int T, int n_in, int C, int pos_emb,
+                        const char* who) {
+  if (!x || (wv && !wv->win_start) || (sv && (!sv->seg_a || !sv->seg_b)) || !params || !packed || !out) {
+    set_error("%s: null pointer", who);
+    return B2H_EINVAL;
+  }
   if (x_dtype != B2H_DT_F32 && x_dtype != B2H_DT_BF16) { set_error("%s: bad x_dtype %d", who, x_dtype); return B2H_EINVAL; }
   if (wv && wv->pad_mode != B2H_PAD_REPEAT_FIRST && wv->pad_mode != B2H_PAD_ZEROS) { set_error("%s: bad pad_mode %d", who, wv->pad_mode); return B2H_EINVAL; }
   if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
-  if (B < B_min || T < 1 || (wv && wv->n_frames < 0)) { set_error("%s: bad B=%d T=%d", who, B, T); return B2H_ESHAPE; }
+  if (sv) {
+    if (sv->n < B_min || sv->n_frames < 0 || sv->n_frames > INT32_MAX || (B_min > 0 && sv->max_len < 1)) {
+      if (B_min > 0) set_error("%s: bad n_seg=%d max_len=%d n_frames=%lld", who, sv->n, sv->max_len, sv->n_frames);
+      else set_error("%s: bad n_utt=%d n_frames=%lld", who, sv->n, sv->n_frames);
+      return B2H_ESHAPE;
+    }
+  } else if (B < B_min || T < 1 || (wv && wv->n_frames < 0)) {
+    set_error("%s: bad B=%d T=%d", who, B, T);
+    return B2H_ESHAPE;
+  }
   return B2H_OK;
 }
 
 static bool misaligned(const void* p, uintptr_t mask) { return reinterpret_cast<uintptr_t>(p) & mask; }
 
-// The forward of B dense windows x (wv == nullptr) or of B windows viewed in the frame stream x.  Window views are read by
-// the tensor-core kernels only: fp32 mode beyond the tile kernel runs on FFMA, which reads dense windows.
-static int conv_forward(const void* x, int x_dtype, const WindowView* wv, const float* params, const void* packed,
-                        const int32_t* lengths, float* y, int B, int T, int n_in, int C, int pos_emb, int precision,
-                        int apply_mask, float out_scale, cudaStream_t stream, const char* who) {
-  if (int rc = check_common(x, x_dtype, wv, params, packed, y, B, 0, T, n_in, C, pos_emb, who)) return rc;
+// The forward of B dense windows x (wv == nullptr), of B windows viewed in the frame stream x, or of the B = sv->n
+// utterances of a segment view (T unused; the plan's table lives in the workspace).  Views are read by the tensor-core
+// kernels only: fp32 mode beyond the tile kernel runs on FFMA, which reads dense windows.
+static int conv_forward(const void* x, int x_dtype, const WindowView* wv, const SegmentView* sv, const float* params,
+                        const void* packed, const int32_t* lengths, float* y, int B, int T, int n_in, int C, int pos_emb,
+                        int precision, int apply_mask, float out_scale, void* workspace, int64_t workspace_bytes,
+                        cudaStream_t stream, const char* who) {
+  if (int rc = check_common(x, x_dtype, wv, sv, params, packed, y, B, 0, T, n_in, C, pos_emb, who)) return rc;
   if (apply_mask && !lengths) { set_error("%s: apply_mask needs lengths", who); return B2H_EINVAL; }
   if (B == 0) return B2H_OK;
-  if (misaligned(x, 15) || misaligned(y, 15) || misaligned(packed, 15)) {
-    set_error("%s: %s, y and packed must be 16-byte aligned", who, wv ? "frames" : "x");
+  if (misaligned(x, 15) || misaligned(y, 15) || misaligned(packed, 15) || (sv && (misaligned(workspace, 15) || misaligned(sv->seg_a, 7)))) {
+    if (sv) set_error("%s: frames, y, packed and workspace must be 16-byte aligned, offsets 8-byte aligned", who);
+    else set_error("%s: %s, y and packed must be 16-byte aligned", who, wv ? "frames" : "x");
     return B2H_EALIGN;
   }
   if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
@@ -286,6 +351,11 @@ static int conv_forward(const void* x, int x_dtype, const WindowView* wv, const 
   a.y = y; a.B = B; a.T = T; a.apply_mask = apply_mask; a.mode = 0; a.out_scale = out_scale;
   a.geo = make_geo(n_in, C, pos_emb);
   if (wv) a.wv = *wv;
+  if (sv) {
+    UttPlan u;
+    if (int rc = utterance_run_plan(a.geo, *sv, precision, kUttForward, workspace_bytes, who, &u)) return rc;
+    return launch_utterances(a, u, *sv, workspace, nullptr, nullptr, stream);
+  }
   const ForwardPlan f = forward_plan(a.geo, B, T, precision);
   if (f.kernel == B2H_KERNEL_TC_TILE) return launch_tc_tile(a, f.tile, stream);
   if (f.kernel == B2H_KERNEL_TC_WIDE) return launch_tc_wide_fwd(a, f.wide, stream);
@@ -305,8 +375,8 @@ static int conv_forward(const void* x, int x_dtype, const WindowView* wv, const 
 extern "C" int b2h_conv_forward(const void* x, int x_dtype, const float* params, const void* packed, const int32_t* lengths,
                                 float* y, int B, int T, int n_in, int C, int pos_emb, int precision, int apply_mask,
                                 float out_scale, void* stream) {
-  return conv_forward(x, x_dtype, nullptr, params, packed, lengths, y, B, T, n_in, C, pos_emb, precision, apply_mask, out_scale,
-                      (cudaStream_t)stream, "b2h_conv_forward");
+  return conv_forward(x, x_dtype, nullptr, nullptr, params, packed, lengths, y, B, T, n_in, C, pos_emb, precision, apply_mask,
+                      out_scale, nullptr, 0, (cudaStream_t)stream, "b2h_conv_forward");
 }
 
 extern "C" int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t n_frames, const int64_t* win_start,
@@ -314,20 +384,12 @@ extern "C" int b2h_conv_forward_windows(const void* frames, int x_dtype, int64_t
                                         const int32_t* lengths, float* y, int n_win, int T, int n_in, int C, int pos_emb,
                                         int precision, int apply_mask, float out_scale, void* stream) {
   const WindowView wv = window_view(win_start, win_end, n_frames, pad_mode);
-  return conv_forward(frames, x_dtype, &wv, params, packed, lengths, y, n_win, T, n_in, C, pos_emb, precision, apply_mask,
-                      out_scale, (cudaStream_t)stream, "b2h_conv_forward_windows");
+  return conv_forward(frames, x_dtype, &wv, nullptr, params, packed, lengths, y, n_win, T, n_in, C, pos_emb, precision,
+                      apply_mask, out_scale, nullptr, 0, (cudaStream_t)stream, "b2h_conv_forward_windows");
 }
 
-static const char* const kUttServed =
-    "utterances are served in bf16 mode for conv_channels <= 256 and in fp32 mode for conv_channels <= 32 with at most 32 "
-    "input channels";
-
 extern "C" int b2h_utterances_plan(int64_t n_frames, int n_utt, int n_in, int C, int pos_emb, int precision, int* seg_len) {
-  if (seg_len) *seg_len = 0;
-  if (!geo_ok(n_in, C, pos_emb) || n_frames < 0 || n_frames > INT32_MAX || n_utt < 0) return B2H_KERNEL_NONE;
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), n_frames, n_utt, precision, kUttForward);
-  if (seg_len && u.kernel != B2H_KERNEL_NONE) *seg_len = u.Ts;
-  return u.kernel;
+  return (int)utterance_query(kUttForward, n_frames, n_utt, 0, n_in, C, pos_emb, precision, seg_len, nullptr);
 }
 
 extern "C" int b2h_utterance_subwindows(int L, int Ts, int i, int* out3) {
@@ -345,13 +407,7 @@ extern "C" int b2h_utterance_subwindows(int L, int Ts, int i, int* out3) {
 }
 
 extern "C" int64_t b2h_utterances_workspace_bytes(int64_t n_frames, int n_utt, int n_in, int C, int pos_emb, int precision) {
-  const char* who = "b2h_utterances_workspace_bytes";
-  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
-  if (n_frames < 0 || n_frames > INT32_MAX || n_utt < 0) { set_error("%s: bad n_frames=%lld n_utt=%d", who, (long long)n_frames, n_utt); return B2H_ESHAPE; }
-  if (n_utt == 0) return 256;
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), n_frames, n_utt, precision, kUttForward);
-  if (u.kernel == B2H_KERNEL_NONE) { set_error("%s: %s (C=%d, n_in=%d, precision=%d)", who, kUttServed, C, n_in, precision); return B2H_ESHAPE; }
-  return u.ws_bytes;
+  return utterance_query(kUttForward, n_frames, n_utt, 0, n_in, C, pos_emb, precision, nullptr, "b2h_utterances_workspace_bytes");
 }
 
 extern "C" int b2h_conv_forward_utterances(const void* frames, int x_dtype, int64_t n_frames, const int64_t* offsets, int n_utt,
@@ -359,33 +415,10 @@ extern "C" int b2h_conv_forward_utterances(const void* frames, int x_dtype, int6
                                            int precision, float out_scale, void* workspace, int64_t workspace_bytes,
                                            void* stream) {
   const char* who = "b2h_conv_forward_utterances";
-  if (!offsets || !workspace) { set_error("%s: null pointer", who); return B2H_EINVAL; }
-  if (int rc = check_common(frames, x_dtype, nullptr, params, packed, y, 1, 0, 1, n_in, C, pos_emb, who)) return rc;
-  if (n_utt < 0 || n_frames < 0 || n_frames > INT32_MAX) {
-    set_error("%s: bad n_utt=%d n_frames=%lld", who, n_utt, (long long)n_frames);
-    return B2H_ESHAPE;
-  }
-  if (n_utt == 0) return B2H_OK;
-  if (misaligned(frames, 15) || misaligned(y, 15) || misaligned(packed, 15) || misaligned(workspace, 15) || misaligned(offsets, 7)) {
-    set_error("%s: frames, y, packed and workspace must be 16-byte aligned, offsets 8-byte aligned", who);
-    return B2H_EALIGN;
-  }
-  if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
-  const Geo g = make_geo(n_in, C, pos_emb);
-  const UttPlan plan = utterance_plan(g, n_frames, n_utt, precision, kUttForward);
-  if (plan.kernel == B2H_KERNEL_NONE) {
-    set_error("%s: %s; no kernel for C=%d, n_in=%d, precision=%d", who, kUttServed, C, n_in, precision);
-    return B2H_ESHAPE;
-  }
-  if (workspace_bytes < plan.ws_bytes) {
-    set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.ws_bytes);
-    return B2H_EWORKSPACE;
-  }
-  ConvArgs a{};
-  a.x = frames; a.x_dtype = x_dtype; a.params = params; a.packed = reinterpret_cast<const char*>(packed);
-  a.y = y; a.mode = 0; a.out_scale = out_scale; a.geo = g;
-  return launch_utterances(a, plan, reinterpret_cast<const long long*>(offsets), n_utt, (long long)n_frames, workspace,
-                           (cudaStream_t)stream);
+  if (!workspace) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  const SegmentView sv = segment_view(offsets, offsets ? offsets + 1 : nullptr, n_utt, n_frames, 0);
+  return conv_forward(frames, x_dtype, nullptr, &sv, params, packed, nullptr, y, n_utt, 0, n_in, C, pos_emb, precision, 0,
+                      out_scale, workspace, workspace_bytes, (cudaStream_t)stream, who);
 }
 
 // What a training launch left for the reduction / Adam launches that follow it (rc != B2H_OK: nothing was launched).
@@ -397,50 +430,76 @@ struct TrainResult {
   float* loss_partials;   // plan.n_loss floats
 };
 
-// The training forward + criterion + backward of B dense windows (wv == nullptr) or of B windows viewed in the frame
-// streams x / target / conf (mode 1 only; the tensor-core kernels only: the FFMA kernel reads dense windows).  fuse != nullptr
-// asks the tile kernel to reduce and apply Adam in the same launch.
-static TrainResult train_common(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
-                                const float* d_y, const int32_t* lengths, const float* params, const void* packed,
-                                float* pred_out, int B, int T, int n_in, int C, int pos_emb, int loss_kind, int precision,
-                                int mode, void* workspace, int64_t workspace_bytes, cudaStream_t stream, const char* who,
-                                long long* step_dev, long long* epoch_dev, const FuseAdam* fuse) {
+// The criterion's inputs of training and validation: target rows, the windows' lengths (not for segments, which carry their
+// own), loss_kind and, for confL1, the confidence rows.
+static int check_criterion(const float* target, const float* conf, const int32_t* lengths, bool need_lengths, int loss_kind,
+                           const char* who) {
+  if (!target || (need_lengths && !lengths)) { set_error(need_lengths ? "%s: null target/lengths" : "%s: null target", who); return B2H_EINVAL; }
+  if (loss_kind != B2H_LOSS_L1 && loss_kind != B2H_LOSS_CONFL1) { set_error("%s: bad loss_kind %d", who, loss_kind); return B2H_EINVAL; }
+  if (loss_kind == B2H_LOSS_CONFL1 && !conf) { set_error("%s: confL1 needs scores", who); return B2H_EINVAL; }
+  return B2H_OK;
+}
+
+// The training forward + criterion + backward of B dense windows (wv == nullptr), of B windows viewed in the frame streams
+// x / target / conf, or of the segments of sv in them, each trained as one sequence (views: mode 1 only; the tensor-core
+// kernels only: the FFMA kernel reads dense windows; segments: the tile kernel, the plan's table in the workspace past the
+// partials).  fuse != nullptr asks the tile kernel to reduce and apply Adam in the same launch.
+static TrainResult train_common(const void* x, int x_dtype, const WindowView* wv, const SegmentView* sv, const float* target,
+                                const float* conf, const float* d_y, const int32_t* lengths, const float* params,
+                                const void* packed, float* pred_out, int B, int T, int n_in, int C, int pos_emb, int loss_kind,
+                                int precision, int mode, void* workspace, int64_t workspace_bytes, cudaStream_t stream,
+                                const char* who, long long* step_dev, long long* epoch_dev, const FuseAdam* fuse) {
   TrainResult r{};
   auto result = [&r](int rc) { r.rc = rc; return r; };
-  if (int rc = check_common(x, x_dtype, wv, params, packed, workspace, B, 1, T, n_in, C, pos_emb, who)) return result(rc);
+  if (int rc = check_common(x, x_dtype, wv, sv, params, packed, workspace, B, 1, T, n_in, C, pos_emb, who)) return result(rc);
   if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return result(B2H_EINVAL); }
   if (mode == 1) {
-    if (!target || !lengths) { set_error("%s: null target/lengths", who); return result(B2H_EINVAL); }
-    if (loss_kind != B2H_LOSS_L1 && loss_kind != B2H_LOSS_CONFL1) { set_error("%s: bad loss_kind %d", who, loss_kind); return result(B2H_EINVAL); }
-    if (loss_kind == B2H_LOSS_CONFL1 && !conf) { set_error("%s: confL1 needs scores", who); return result(B2H_EINVAL); }
+    if (int rc = check_criterion(target, conf, lengths, !sv, loss_kind, who)) return result(rc);
   } else if (!d_y) { set_error("%s: null d_y", who); return result(B2H_EINVAL); }
   // A stream's target row (168 B) and confidence row (84 B) start 8 / 4 bytes past a 16-B boundary at odd frames: the
   // kernels read them with float2 / float loads and use a bulk copy only where the address allows it.
-  if (misaligned(x, 15) || misaligned(target, wv ? 7 : 15) || misaligned(conf, wv ? 3 : 0) || misaligned(packed, 15)) {
-    if (wv) set_error("%s: frames and packed must be 16-byte aligned, target_frames 8-byte and conf_frames 4-byte aligned", who);
+  const bool stream_rows = wv || sv;
+  if (misaligned(x, 15) || misaligned(target, stream_rows ? 7 : 15) || misaligned(conf, stream_rows ? 3 : 0) || misaligned(packed, 15) ||
+      (sv && (misaligned(pred_out, 15) || misaligned(workspace, 15) || misaligned(sv->seg_a, 7) || misaligned(sv->seg_b, 7)))) {
+    if (sv)
+      set_error("%s: frames, packed, pred_out and workspace must be 16-byte aligned, target_frames, seg_start and seg_end 8-byte "
+                "and conf_frames 4-byte aligned", who);
+    else if (wv) set_error("%s: frames and packed must be 16-byte aligned, target_frames 8-byte and conf_frames 4-byte aligned", who);
     else set_error("%s: x, target and packed must be 16-byte aligned", who);
     return result(B2H_EALIGN);
   }
   r.g = make_geo(n_in, C, pos_emb);
-  const TrainPlan& plan = r.plan = train_plan(r.g, B, T, precision);
-  if (wv && plan.kernel != B2H_KERNEL_TC_TILE && plan.kernel != B2H_KERNEL_TC_WIDE_TRAIN) {
-    set_error("%s: window views are trained on the tensor cores: in bf16 mode for conv_channels <= 32 with at most 32 input "
-              "channels and T <= 4096, and for conv_channels <= 256 with T <= 256; in fp32 mode for conv_channels <= 32 with at "
-              "most 32 input channels and T <= 4096; materialise the windows (b2h_preprocess) for C=%d, T=%d, precision=%d",
-              who, C, T, precision);
-    return result(B2H_ESHAPE);
+  TrainPlan& plan = r.plan;
+  UttPlan u{};
+  if (sv) {
+    if (int rc = utterance_run_plan(r.g, *sv, precision, kUttTrain, workspace_bytes, who, &u)) return result(rc);
+    plan.kernel = B2H_KERNEL_TC_TILE; plan.tile = u.tile; plan.nparts = plan.n_loss = u.tile.grid;
+  } else {
+    plan = train_plan(r.g, B, T, precision);
+    if (wv && plan.kernel != B2H_KERNEL_TC_TILE && plan.kernel != B2H_KERNEL_TC_WIDE_TRAIN) {
+      set_error("%s: window views are trained on the tensor cores: in bf16 mode for conv_channels <= 32 with at most 32 input "
+                "channels and T <= 4096, and for conv_channels <= 256 with T <= 256; in fp32 mode for conv_channels <= 32 with "
+                "at most 32 input channels and T <= 4096; materialise the windows (b2h_preprocess) for C=%d, T=%d, precision=%d",
+                who, C, T, precision);
+      return result(B2H_ESHAPE);
+    }
+    if (plan.kernel == B2H_KERNEL_NONE) {
+      set_error("%s: no training kernel for conv_channels=%d, T=%d, precision=%d (tcgen05 training: C <= 32 in the one-launch "
+                "tile kernel, C <= 256 in bf16 mode through the wide kernels, T <= 256; the FFMA kernel would need %zu B of "
+                "shared memory)", who, C, T, precision, plan.ffma.smem);
+      return result(B2H_ESHAPE);
+    }
+    if (workspace_bytes < plan.total - 256) { set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.total); return result(B2H_EWORKSPACE); }
+    if (misaligned(workspace, 15)) { set_error("%s: workspace must be 16-byte aligned", who); return result(B2H_EALIGN); }
   }
-  if (plan.kernel == B2H_KERNEL_NONE) {
-    set_error("%s: no training kernel for conv_channels=%d, T=%d, precision=%d (tcgen05 training: C <= 32 in the one-launch tile "
-              "kernel, C <= 256 in bf16 mode through the wide kernels, T <= 256; the FFMA kernel would need %zu B of shared memory)",
-              who, C, T, precision, plan.ffma.smem);
-    return result(B2H_ESHAPE);
-  }
-  if (workspace_bytes < plan.total - 256) { set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.total); return result(B2H_EWORKSPACE); }
-  if (misaligned(workspace, 15)) { set_error("%s: workspace must be 16-byte aligned", who); return result(B2H_EALIGN); }
-  // [header: launch sequence + per-CTA arrival flags of the fused kernel, FIXED offset][gradient partials][loss partials][scratch]
+  // [header: launch sequence + per-CTA arrival flags of the fused kernel, FIXED offset][gradient partials][loss partials]
+  // [scratch (wide) | the utterance plan's table (segments)]
   r.partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + B2H_WS_HEADER);
   r.loss_partials = r.partials + (size_t)plan.nparts * gp_total(r.g);
+  if (sv && pred_out) {   // the masked prediction (n_seg, max_len, 42): rows at or past a segment's end stay zero
+    const cudaError_t e = cudaMemsetAsync(pred_out, 0, (size_t)sv->n * sv->max_len * B2H_COUT * 4, stream);
+    if (e != cudaSuccess) { cudaGetLastError(); set_error("%s: cudaMemsetAsync: %s", who, cudaGetErrorString(e)); return result(B2H_ECUDA); }
+  }
   ConvArgs a{};
   a.x = x; a.x_dtype = x_dtype; a.target = target; a.conf = conf; a.d_y = d_y; a.lengths = lengths; a.params = params;
   a.packed = reinterpret_cast<const char*>(packed); a.y = pred_out; a.partials = r.partials; a.loss_partials = r.loss_partials;
@@ -455,6 +514,9 @@ static TrainResult train_common(const void* x, int x_dtype, const WindowView* wv
       a.fuse.enabled = 1;
       a.fuse.hdr = reinterpret_cast<unsigned*>(workspace);
     }
+    if (sv) {
+      return result(launch_utterances(a, u, *sv, reinterpret_cast<char*>(workspace) + u.plan_off, nullptr, nullptr, stream));
+    }
     return result(launch_tc_tile(a, plan.tile, stream));
   }
   if (plan.kernel == B2H_KERNEL_TC_WIDE_TRAIN) {
@@ -464,13 +526,13 @@ static TrainResult train_common(const void* x, int x_dtype, const WindowView* wv
   return result(launch_fp32(a, plan.ffma, stream));
 }
 
-static int train_forward_backward(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
-                                  const int32_t* lengths, const float* params, const void* packed, float* grads_out,
-                                  float* loss_out, float* pred_out, int B, int T, int n_in, int C, int pos_emb, int loss_kind,
-                                  int precision, int64_t* step_dev, void* workspace, int64_t workspace_bytes, void* stream,
-                                  const char* who) {
+static int train_forward_backward(const void* x, int x_dtype, const WindowView* wv, const SegmentView* sv, const float* target,
+                                  const float* conf, const int32_t* lengths, const float* params, const void* packed,
+                                  float* grads_out, float* loss_out, float* pred_out, int B, int T, int n_in, int C, int pos_emb,
+                                  int loss_kind, int precision, int64_t* step_dev, void* workspace, int64_t workspace_bytes,
+                                  void* stream, const char* who) {
   if (grads_out && !loss_out) { set_error("%s: null loss_out", who); return B2H_EINVAL; }
-  const TrainResult r = train_common(x, x_dtype, wv, target, conf, nullptr, lengths, params, packed, pred_out, B, T, n_in, C,
+  const TrainResult r = train_common(x, x_dtype, wv, sv, target, conf, nullptr, lengths, params, packed, pred_out, B, T, n_in, C,
                                      pos_emb, loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, who,
                                      reinterpret_cast<long long*>(step_dev), nullptr, nullptr);
   if (r.rc || !grads_out) return r.rc;   // grads_out == NULL: only the fused kernel runs, partials stay in the workspace
@@ -483,9 +545,9 @@ extern "C" int b2h_train_forward_backward(const void* x, int x_dtype, const floa
                                           float* grads_out, float* loss_out, float* pred_out, int B, int T, int n_in,
                                           int C, int pos_emb, int loss_kind, int precision, int64_t* step_dev,
                                           void* workspace, int64_t workspace_bytes, void* stream) {
-  return train_forward_backward(x, x_dtype, nullptr, target, conf, lengths, params, packed, grads_out, loss_out, pred_out, B, T,
-                                n_in, C, pos_emb, loss_kind, precision, step_dev, workspace, workspace_bytes, stream,
-                                "b2h_train_forward_backward");
+  return train_forward_backward(x, x_dtype, nullptr, nullptr, target, conf, lengths, params, packed, grads_out, loss_out,
+                                pred_out, B, T, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace, workspace_bytes,
+                                stream, "b2h_train_forward_backward");
 }
 
 extern "C" int b2h_train_forward_backward_windows(const void* frames, int x_dtype, const float* target_frames,
@@ -496,8 +558,8 @@ extern "C" int b2h_train_forward_backward_windows(const void* frames, int x_dtyp
                                                   int loss_kind, int precision, int64_t* step_dev, void* workspace,
                                                   int64_t workspace_bytes, void* stream) {
   const WindowView wv = window_view(win_start, win_end, n_frames, pad_mode);
-  return train_forward_backward(frames, x_dtype, &wv, target_frames, conf_frames, lengths, params, packed, grads_out, loss_out,
-                                pred_out, n_win, T, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace,
+  return train_forward_backward(frames, x_dtype, &wv, nullptr, target_frames, conf_frames, lengths, params, packed, grads_out,
+                                loss_out, pred_out, n_win, T, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace,
                                 workspace_bytes, stream, "b2h_train_forward_backward_windows");
 }
 
@@ -522,8 +584,8 @@ extern "C" int b2h_conv_backward(const void* x, int x_dtype, const float* d_y, c
                                  float* grads_out, int B, int T, int n_in, int C, int pos_emb, int precision,
                                  void* workspace, int64_t workspace_bytes, void* stream) {
   if (!grads_out) { set_error("b2h_conv_backward: null output"); return B2H_EINVAL; }
-  const TrainResult r = train_common(x, x_dtype, nullptr, nullptr, nullptr, d_y, nullptr, params, packed, nullptr, B, T, n_in, C,
-                                     pos_emb, 0, precision, 2, workspace, workspace_bytes, (cudaStream_t)stream,
+  const TrainResult r = train_common(x, x_dtype, nullptr, nullptr, nullptr, nullptr, d_y, nullptr, params, packed, nullptr, B, T,
+                                     n_in, C, pos_emb, 0, precision, 2, workspace, workspace_bytes, (cudaStream_t)stream,
                                      "b2h_conv_backward", nullptr, nullptr, nullptr);
   if (r.rc) return r.rc;
   return launch_reduce(r.partials, r.plan.nparts, r.g, grads_out, nullptr, r.plan.n_loss, nullptr, nullptr, (cudaStream_t)stream);
@@ -540,16 +602,19 @@ static FuseAdam fuse_adam(float* params, void* packed, float* exp_avg, float* ex
   return f;
 }
 
-static int train_step(const void* x, int x_dtype, const WindowView* wv, const float* target, const float* conf,
-                      const int32_t* lengths, float* params, void* packed, float* exp_avg, float* exp_avg_sq, float* loss_out,
-                      int B, int T, int n_in, int C, int pos_emb, int loss_kind, int precision, double lr, double beta1,
-                      double beta2, double eps, int64_t step, int64_t* step_dev, const double* lr_dev, void* workspace,
-                      int64_t workspace_bytes, void* stream, const char* who) {
+static int train_step(const void* x, int x_dtype, const WindowView* wv, const SegmentView* sv, const float* target,
+                      const float* conf, const int32_t* lengths, float* params, void* packed, float* exp_avg, float* exp_avg_sq,
+                      float* loss_out, int B, int T, int n_in, int C, int pos_emb, int loss_kind, int precision, double lr,
+                      double beta1, double beta2, double eps, int64_t step, int64_t* step_dev, const double* lr_dev,
+                      void* workspace, int64_t workspace_bytes, void* stream, const char* who) {
   if (!exp_avg || !exp_avg_sq || !loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
   if (step < 1 && !step_dev) { set_error("%s: step must be >= 1", who); return B2H_EINVAL; }
+  // segments have the fused step only: it reads the Adam step from the device counter and advances it (a refused segment
+  // list leaves it alone)
+  if (sv && !step_dev) { set_error("%s: null step_dev (the fused step reads and advances the device-side step counter)", who); return B2H_EINVAL; }
   // tile kernel + device-side step counter: ONE cooperative launch (reduction + Adam + re-pack in its tail)
   const FuseAdam fuse = fuse_adam(params, packed, exp_avg, exp_avg_sq, loss_out, lr, beta1, beta2, eps, 1.0f, step_dev, lr_dev);
-  const TrainResult r = train_common(x, x_dtype, wv, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C,
+  const TrainResult r = train_common(x, x_dtype, wv, sv, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C,
                                      pos_emb, loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream, who,
                                      reinterpret_cast<long long*>(step_dev), nullptr, step_dev ? &fuse : nullptr);
   if (r.rc) return r.rc;
@@ -564,8 +629,8 @@ extern "C" int b2h_train_step(const void* x, int x_dtype, const float* target, c
                               int T, int n_in, int C, int pos_emb, int loss_kind, int precision, double lr, double beta1,
                               double beta2, double eps, int64_t step, int64_t* step_dev, const double* lr_dev, void* workspace,
                               int64_t workspace_bytes, void* stream) {
-  return train_step(x, x_dtype, nullptr, target, conf, lengths, params, packed, exp_avg, exp_avg_sq, loss_out, B, T, n_in, C,
-                    pos_emb, loss_kind, precision, lr, beta1, beta2, eps, step, step_dev, lr_dev, workspace, workspace_bytes,
+  return train_step(x, x_dtype, nullptr, nullptr, target, conf, lengths, params, packed, exp_avg, exp_avg_sq, loss_out, B, T, n_in,
+                    C, pos_emb, loss_kind, precision, lr, beta1, beta2, eps, step, step_dev, lr_dev, workspace, workspace_bytes,
                     stream, "b2h_train_step");
 }
 
@@ -577,86 +642,17 @@ extern "C" int b2h_train_step_windows(const void* frames, int x_dtype, const flo
                                       int64_t* step_dev, const double* lr_dev, void* workspace, int64_t workspace_bytes,
                                       void* stream) {
   const WindowView wv = window_view(win_start, win_end, n_frames, pad_mode);
-  return train_step(frames, x_dtype, &wv, target_frames, conf_frames, lengths, params, packed, exp_avg, exp_avg_sq, loss_out,
-                    n_win, T, n_in, C, pos_emb, loss_kind, precision, lr, beta1, beta2, eps, step, step_dev, lr_dev, workspace,
-                    workspace_bytes, stream, "b2h_train_step_windows");
+  return train_step(frames, x_dtype, &wv, nullptr, target_frames, conf_frames, lengths, params, packed, exp_avg, exp_avg_sq,
+                    loss_out, n_win, T, n_in, C, pos_emb, loss_kind, precision, lr, beta1, beta2, eps, step, step_dev, lr_dev,
+                    workspace, workspace_bytes, stream, "b2h_train_step_windows");
 }
 
-static const char* const kUttTrainServed =
-    "segments are trained by the tile kernel: conv_channels <= 32 with at most 32 input channels, in bf16 or fp32 mode "
-    "(wider models and fp32-ffma have no segment path)";
-
 extern "C" int b2h_train_utterances_plan(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision, int* seg_len) {
-  if (seg_len) *seg_len = 0;
-  if (!geo_ok(n_in, C, pos_emb) || n_seg < 1 || max_len < 1) return B2H_KERNEL_NONE;
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, kUttTrain, max_len);
-  if (seg_len && u.kernel != B2H_KERNEL_NONE) *seg_len = u.Ts;
-  return u.kernel;
+  return (int)utterance_query(kUttTrain, 0, n_seg, max_len, n_in, C, pos_emb, precision, seg_len, nullptr);
 }
 
 extern "C" int64_t b2h_train_utterances_workspace_bytes(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision) {
-  const char* who = "b2h_train_utterances_workspace_bytes";
-  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
-  if (n_seg < 1 || max_len < 1) { set_error("%s: bad n_seg=%d max_len=%d", who, n_seg, max_len); return B2H_ESHAPE; }
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, kUttTrain, max_len);
-  if (u.kernel == B2H_KERNEL_NONE) { set_error("%s: %s (C=%d, n_in=%d, precision=%d)", who, kUttTrainServed, C, n_in, precision); return B2H_ESHAPE; }
-  return u.ws_bytes;
-}
-
-// The checks and the launch shared by b2h_train_forward_backward_utterances and b2h_train_step_utterances (fuse != nullptr:
-// the fused step), in the order and style of train_common.
-static int train_utterances(const void* frames, int x_dtype, const float* target, const float* conf, int64_t n_frames,
-                            const int64_t* seg_start, const int64_t* seg_end, int n_seg, int max_len, const float* params,
-                            const void* packed, float* pred_out, int n_in, int C, int pos_emb, int loss_kind, int precision,
-                            int64_t* step_dev, void* workspace, int64_t workspace_bytes, cudaStream_t stream, const char* who,
-                            const FuseAdam* fuse, UttPlan* plan_out, Geo* g_out) {
-  if (!seg_start || !seg_end) { set_error("%s: null pointer", who); return B2H_EINVAL; }
-  if (int rc = check_common(frames, x_dtype, nullptr, params, packed, workspace, 1, 0, 1, n_in, C, pos_emb, who)) return rc;
-  if (n_seg < 1 || max_len < 1 || n_frames < 0 || n_frames > INT32_MAX) {
-    set_error("%s: bad n_seg=%d max_len=%d n_frames=%lld", who, n_seg, max_len, (long long)n_frames);
-    return B2H_ESHAPE;
-  }
-  if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
-  if (!target) { set_error("%s: null target", who); return B2H_EINVAL; }
-  if (loss_kind != B2H_LOSS_L1 && loss_kind != B2H_LOSS_CONFL1) { set_error("%s: bad loss_kind %d", who, loss_kind); return B2H_EINVAL; }
-  if (loss_kind == B2H_LOSS_CONFL1 && !conf) { set_error("%s: confL1 needs scores", who); return B2H_EINVAL; }
-  if (misaligned(frames, 15) || misaligned(target, 7) || misaligned(conf, 3) || misaligned(packed, 15) || misaligned(pred_out, 15) ||
-      misaligned(workspace, 15) || misaligned(seg_start, 7) || misaligned(seg_end, 7)) {
-    set_error("%s: frames, packed, pred_out and workspace must be 16-byte aligned, target_frames, seg_start and seg_end 8-byte "
-              "and conf_frames 4-byte aligned", who);
-    return B2H_EALIGN;
-  }
-  const Geo g = make_geo(n_in, C, pos_emb);
-  const UttPlan plan = utterance_plan(g, n_frames, n_seg, precision, kUttTrain, max_len);
-  if (plan.kernel == B2H_KERNEL_NONE) {
-    set_error("%s: %s; no kernel for C=%d, n_in=%d, precision=%d", who, kUttTrainServed, C, n_in, precision);
-    return B2H_ESHAPE;
-  }
-  if (workspace_bytes < plan.ws_bytes) {
-    set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.ws_bytes);
-    return B2H_EWORKSPACE;
-  }
-  if (pred_out) {
-    const cudaError_t e = cudaMemsetAsync(pred_out, 0, (size_t)n_seg * max_len * B2H_COUT * 4, stream);
-    if (e != cudaSuccess) { cudaGetLastError(); set_error("%s: cudaMemsetAsync: %s", who, cudaGetErrorString(e)); return B2H_ECUDA; }
-  }
-  ConvArgs a{};
-  a.x = frames; a.x_dtype = x_dtype; a.target = target; a.conf = conf; a.params = params;
-  a.packed = reinterpret_cast<const char*>(packed); a.y = pred_out;
-  a.partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + B2H_WS_HEADER);
-  a.loss_partials = a.partials + (size_t)plan.tile.grid * gp_total(g);
-  a.loss_kind = loss_kind; a.mode = 1; a.out_scale = 1.0f; a.geo = g;
-  a.step_dev = reinterpret_cast<long long*>(step_dev);
-  if (fuse) {
-    if (plan.tile.grid > B2H_WS_MAX_CTA) { set_error("%s: %d CTAs exceed the %d arrival flags of the workspace header", who, plan.tile.grid, B2H_WS_MAX_CTA); return B2H_ESHAPE; }
-    a.fuse = *fuse;
-    a.fuse.enabled = 1;
-    a.fuse.hdr = reinterpret_cast<unsigned*>(workspace);
-  }
-  if (plan_out) *plan_out = plan;
-  if (g_out) *g_out = g;
-  return launch_train_utterances(a, plan, reinterpret_cast<const long long*>(seg_start), reinterpret_cast<const long long*>(seg_end),
-                                 n_seg, (long long)n_frames, max_len, workspace, stream);
+  return utterance_query(kUttTrain, 0, n_seg, max_len, n_in, C, pos_emb, precision, nullptr, "b2h_train_utterances_workspace_bytes");
 }
 
 extern "C" int b2h_train_forward_backward_utterances(const void* frames, int x_dtype, const float* target_frames,
@@ -667,15 +663,10 @@ extern "C" int b2h_train_forward_backward_utterances(const void* frames, int x_d
                                                      int64_t* step_dev, void* workspace, int64_t workspace_bytes, void* stream) {
   const char* who = "b2h_train_forward_backward_utterances";
   if (!grads_out || !loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
-  UttPlan plan{};
-  Geo g{};
-  if (int rc = train_utterances(frames, x_dtype, target_frames, conf_frames, n_frames, seg_start, seg_end, n_seg, max_len, params,
-                                packed, pred_out, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace, workspace_bytes,
-                                (cudaStream_t)stream, who, nullptr, &plan, &g))
-    return rc;
-  float* partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + B2H_WS_HEADER);
-  return launch_reduce(partials, plan.tile.grid, g, grads_out, partials + (size_t)plan.tile.grid * gp_total(g), plan.tile.grid,
-                       loss_out, nullptr, (cudaStream_t)stream);
+  const SegmentView sv = segment_view(seg_start, seg_end, n_seg, n_frames, max_len);
+  return train_forward_backward(frames, x_dtype, nullptr, &sv, target_frames, conf_frames, nullptr, params, packed, grads_out,
+                                loss_out, pred_out, n_seg, 1, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace,
+                                workspace_bytes, stream, who);
 }
 
 extern "C" int b2h_train_step_utterances(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
@@ -684,54 +675,34 @@ extern "C" int b2h_train_step_utterances(const void* frames, int x_dtype, const 
                                          float* loss_out, int n_in, int C, int pos_emb, int loss_kind, int precision, double lr,
                                          double beta1, double beta2, double eps, int64_t step, int64_t* step_dev,
                                          const double* lr_dev, void* workspace, int64_t workspace_bytes, void* stream) {
-  const char* who = "b2h_train_step_utterances";
-  if (!exp_avg || !exp_avg_sq || !loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
-  if (step < 1 && !step_dev) { set_error("%s: step must be >= 1", who); return B2H_EINVAL; }
-  // the fused step reads the Adam step from the device counter and advances it (a refused segment list leaves it alone)
-  if (!step_dev) { set_error("%s: null step_dev (the fused step reads and advances the device-side step counter)", who); return B2H_EINVAL; }
-  const FuseAdam fuse = fuse_adam(params, packed, exp_avg, exp_avg_sq, loss_out, lr, beta1, beta2, eps, 1.0f, step_dev, lr_dev);
-  return train_utterances(frames, x_dtype, target_frames, conf_frames, n_frames, seg_start, seg_end, n_seg, max_len, params, packed,
-                          nullptr, n_in, C, pos_emb, loss_kind, precision, step_dev, workspace, workspace_bytes,
-                          (cudaStream_t)stream, who, &fuse, nullptr, nullptr);
+  const SegmentView sv = segment_view(seg_start, seg_end, n_seg, n_frames, max_len);
+  return train_step(frames, x_dtype, nullptr, &sv, target_frames, conf_frames, nullptr, params, packed, exp_avg, exp_avg_sq,
+                    loss_out, n_seg, 1, n_in, C, pos_emb, loss_kind, precision, lr, beta1, beta2, eps, step, step_dev, lr_dev,
+                    workspace, workspace_bytes, stream, "b2h_train_step_utterances");
 }
 
-static const char* const kUttValidateServed =
-    "segments are validated by the utterance forward: in bf16 mode for conv_channels <= 256, in fp32 mode for "
-    "conv_channels <= 32 with at most 32 input channels (fp32-ffma has no segment path)";
-
 extern "C" int b2h_validate_utterances_plan(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision, int* seg_len) {
-  if (seg_len) *seg_len = 0;
-  if (!geo_ok(n_in, C, pos_emb) || n_seg < 1 || max_len < 1) return B2H_KERNEL_NONE;
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, kUttValidate, max_len);
-  if (seg_len && u.kernel != B2H_KERNEL_NONE) *seg_len = u.Ts;
-  return u.kernel;
+  return (int)utterance_query(kUttValidate, 0, n_seg, max_len, n_in, C, pos_emb, precision, seg_len, nullptr);
 }
 
 extern "C" int64_t b2h_validate_utterances_workspace_bytes(int n_seg, int max_len, int n_in, int C, int pos_emb, int precision) {
-  const char* who = "b2h_validate_utterances_workspace_bytes";
-  if (!geo_ok(n_in, C, pos_emb, who)) return B2H_ESHAPE;
-  if (n_seg < 1 || max_len < 1) { set_error("%s: bad n_seg=%d max_len=%d", who, n_seg, max_len); return B2H_ESHAPE; }
-  const UttPlan u = utterance_plan(make_geo(n_in, C, pos_emb), 0, n_seg, precision, kUttValidate, max_len);
-  if (u.kernel == B2H_KERNEL_NONE) { set_error("%s: %s (C=%d, n_in=%d, precision=%d)", who, kUttValidateServed, C, n_in, precision); return B2H_ESHAPE; }
-  return u.ws_bytes;
+  return utterance_query(kUttValidate, 0, n_seg, max_len, n_in, C, pos_emb, precision, nullptr,
+                         "b2h_validate_utterances_workspace_bytes");
 }
 
+// Validation over segments: the forward over them with the criterion per sub-window instead of predictions, then the
+// per-segment means and the loss.
 extern "C" int b2h_validate_utterances(const void* frames, int x_dtype, const float* target_frames, const float* conf_frames,
                                        int64_t n_frames, const int64_t* seg_start, const int64_t* seg_end, int n_seg, int max_len,
                                        const float* params, const void* packed, float* seg_loss_out, float* loss_out, int n_in,
                                        int C, int pos_emb, int loss_kind, int precision, void* workspace,
                                        int64_t workspace_bytes, void* stream) {
   const char* who = "b2h_validate_utterances";
-  if (!seg_start || !seg_end || !loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
-  if (int rc = check_common(frames, x_dtype, nullptr, params, packed, workspace, 1, 0, 1, n_in, C, pos_emb, who)) return rc;
-  if (n_seg < 1 || max_len < 1 || n_frames < 0 || n_frames > INT32_MAX) {
-    set_error("%s: bad n_seg=%d max_len=%d n_frames=%lld", who, n_seg, max_len, (long long)n_frames);
-    return B2H_ESHAPE;
-  }
+  if (!loss_out) { set_error("%s: null pointer", who); return B2H_EINVAL; }
+  const SegmentView sv = segment_view(seg_start, seg_end, n_seg, n_frames, max_len);
+  if (int rc = check_common(frames, x_dtype, nullptr, &sv, params, packed, workspace, n_seg, 1, 1, n_in, C, pos_emb, who)) return rc;
   if (!prec_ok(precision)) { set_error("%s: bad precision %d", who, precision); return B2H_EINVAL; }
-  if (!target_frames) { set_error("%s: null target", who); return B2H_EINVAL; }
-  if (loss_kind != B2H_LOSS_L1 && loss_kind != B2H_LOSS_CONFL1) { set_error("%s: bad loss_kind %d", who, loss_kind); return B2H_EINVAL; }
-  if (loss_kind == B2H_LOSS_CONFL1 && !conf_frames) { set_error("%s: confL1 needs scores", who); return B2H_EINVAL; }
+  if (int rc = check_criterion(target_frames, conf_frames, nullptr, false, loss_kind, who)) return rc;
   if (misaligned(frames, 15) || misaligned(target_frames, 7) || misaligned(conf_frames, 3) || misaligned(packed, 15) ||
       misaligned(workspace, 15) || misaligned(seg_start, 7) || misaligned(seg_end, 7) || misaligned(seg_loss_out, 3) ||
       misaligned(loss_out, 3)) {
@@ -739,21 +710,14 @@ extern "C" int b2h_validate_utterances(const void* frames, int x_dtype, const fl
               "conf_frames, seg_loss_out and loss_out 4-byte aligned", who);
     return B2H_EALIGN;
   }
-  const Geo g = make_geo(n_in, C, pos_emb);
-  const UttPlan plan = utterance_plan(g, n_frames, n_seg, precision, kUttValidate, max_len);
-  if (plan.kernel == B2H_KERNEL_NONE) {
-    set_error("%s: %s; no kernel for C=%d, n_in=%d, precision=%d", who, kUttValidateServed, C, n_in, precision);
-    return B2H_ESHAPE;
-  }
-  if (workspace_bytes < plan.ws_bytes) {
-    set_error("%s: workspace %lld B < %lld B", who, (long long)workspace_bytes, (long long)plan.ws_bytes);
-    return B2H_EWORKSPACE;
-  }
   ConvArgs a{};
   a.x = frames; a.x_dtype = x_dtype; a.target = target_frames; a.conf = conf_frames; a.params = params;
-  a.packed = reinterpret_cast<const char*>(packed); a.loss_kind = loss_kind; a.mode = 0; a.out_scale = 1.0f; a.geo = g;
-  return launch_validate_utterances(a, plan, reinterpret_cast<const long long*>(seg_start), reinterpret_cast<const long long*>(seg_end),
-                                    n_seg, (long long)n_frames, max_len, seg_loss_out, loss_out, workspace, (cudaStream_t)stream);
+  a.packed = reinterpret_cast<const char*>(packed); a.loss_kind = loss_kind; a.mode = 0; a.out_scale = 1.0f;
+  a.geo = make_geo(n_in, C, pos_emb);
+  UttPlan u;
+  if (int rc = utterance_run_plan(a.geo, sv, precision, kUttValidate, workspace_bytes, who, &u)) return rc;
+  a.loss_partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + u.part_off);
+  return launch_utterances(a, u, sv, workspace, seg_loss_out, loss_out, (cudaStream_t)stream);
 }
 
 extern "C" int b2h_train_step_dp(const void* x, int x_dtype, const float* target, const float* conf, const int32_t* lengths,
@@ -771,8 +735,8 @@ extern "C" int b2h_train_step_dp(const void* x, int x_dtype, const float* target
   fuse.peer_bufs = reinterpret_cast<const float* const*>(peer_bufs_dev); fuse.sym_grads = sym_grads;
   fuse.mc_buf = reinterpret_cast<unsigned long long*>(multicast_buf);
   fuse.epoch_dev = reinterpret_cast<const long long*>(epoch_dev); fuse.rank = rank; fuse.world = world;
-  const TrainResult r = train_common(x, x_dtype, nullptr, target, conf, nullptr, lengths, params, packed, nullptr, B, T, n_in, C,
-                                     pos_emb, loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream,
+  const TrainResult r = train_common(x, x_dtype, nullptr, nullptr, target, conf, nullptr, lengths, params, packed, nullptr, B, T,
+                                     n_in, C, pos_emb, loss_kind, precision, 1, workspace, workspace_bytes, (cudaStream_t)stream,
                                      "b2h_train_step_dp", reinterpret_cast<long long*>(step_dev),
                                      reinterpret_cast<long long*>(epoch_dev), &fuse);
   if (r.rc) return r.rc;

@@ -276,6 +276,11 @@ __device__ __forceinline__ long long window_src_row(const WindowView& v, int w, 
   return f;
 }
 
+// Utterances and segments (host side; the planning kernel turns them into the table of UttPlan): sequence s of n is stream
+// rows [seg_a[s], seg_b[s]), predicted or trained as one sequence.  The forward's offsets are (off, off + 1, n_utt, n_frames,
+// max_len = 0); training and validation segments hold 1..max_len frames each.
+struct SegmentView { const long long* seg_a; const long long* seg_b; int n; long long n_frames; int max_len; };
+
 // ---- launch plans: for each kernel family, one host function (in the file that owns the kernel) decides whether a
 // shape fits and how it launches.  The C-ABI queries, the workspace layout and the launchers all read the same plan, so
 // the number of gradient / loss partial slices a launch writes is the number the workspace was sized for. ----
@@ -354,36 +359,30 @@ int tc_status_and_clear();
 
 // Forward over packed utterances (b2h_conv_forward_utterances): every utterance is cut into sub-windows of Ts frames by
 // sub_window(); the forward kernels read sub-window g from a table that a one-CTA planning kernel builds on the device.
-// Workspace: [int4 {sub-window count, bad, 0, 0}][int4 per sub-window, max_sub of them][int prefix[n_utt + 1]], where
-// sub-window g = {stream row of its first frame, its first frame in the utterance, clo | chi << 16, frames before the
-// utterance end (<= Ts)} and bad = 1 when the planning kernel refused the offsets / segments (count = 0 then).
-// Training over segments (b2h_train_*_utterances) plans the same table at plan_off of the training workspace, followed at
-// seg_off (from the table's start) by one int2 per sub-window: {segment, segment length}.  Validation over segments
-// (b2h_validate_utterances) plans the same table and segment array at the workspace's start, followed at part_off by one
-// float per sub-window: its criterion sum, written by the forward.
+// One workspace layout for the forward, training and validation, from the table at plan_off (0 unless training, where the
+// header and the gradient and loss partials of the plan's grid come first):
+//   [int4 {sub-window count, bad, 0, 0}][int4 per sub-window, max_sub of them][int prefix[n + 1]]
+//   segments (training, validation): at seg_off, the next 16-byte boundary, one int2 {segment, segment length} per sub-window
+//   validation: at part_off, right after them, one float per sub-window: its criterion sum, written by the forward
+// and the whole rounded up to 256 B.  Sub-window g = {stream row of its first frame, its first frame in the sequence,
+// clo | chi << 16, frames before the sequence end (<= Ts)}; bad = 1 when the planning kernel refused the offsets / segments
+// (count = 0 then).
 struct UttPlan {
   int kernel;               // B2H_KERNEL_TC_TILE | B2H_KERNEL_TC_WIDE | B2H_KERNEL_NONE
   int Ts;                   // sub-window length
-  int max_sub;              // upper bound on the sub-window count: n_utt + n_frames / (Ts - 32); training: n_seg * n(max_len)
+  int max_sub;              // upper bound on the sub-window count: n_utt + n_frames / (Ts - 32); segments: n_seg * n(max_len)
   TilePlan tile; WidePlan wide;   // planned for max_sub windows of Ts frames
   int64_t ws_bytes;
-  int64_t plan_off, seg_off; // training: byte offset of the table in the workspace, of the segment array from the table
-  int64_t part_off;         // validation: byte offset of the per-sub-window sums from the table
+  int64_t plan_off;         // byte offset of the table in the workspace
+  int64_t seg_off, part_off;  // byte offsets of the segment pairs and of the per-sub-window sums from the table
 };
 __host__ __device__ inline int64_t utt_prefix_offset(int max_sub) { return (int64_t)(1 + max_sub) * 16; }
-// planning kernel, then the forward of a.B = plan.max_sub sub-windows of a.T = plan.Ts frames over the table it wrote
-int launch_utterances(ConvArgs a, const UttPlan& plan, const long long* offsets, int n_utt, long long n_frames, void* workspace,
+// The planning kernel over the sequences of `sv` into `table` (the workspace at plan.plan_off), then the kernel the plan
+// names over the table it wrote: training (a.mode 1) the tile kernel with a.B = sv.n segments (a.fuse.enabled: the fused
+// step); the forward the tile or wide kernel with a.B = plan.max_sub sub-windows; validation (the forward with
+// a.loss_partials = the per-sub-window sums) that forward, then the kernel that writes seg_loss (nullable) and *loss_out.
+int launch_utterances(ConvArgs a, const UttPlan& plan, const SegmentView& sv, void* table, float* seg_loss, float* loss_out,
                       cudaStream_t stream);
-// planning kernel over the segments [seg_start[s], seg_end[s]) (each 1..max_len frames), then the training launch of the
-// tile kernel (a.fuse.enabled: the fused step) over the table it wrote; a.B = n_seg
-int launch_train_utterances(ConvArgs a, const UttPlan& plan, const long long* seg_start, const long long* seg_end, int n_seg,
-                            long long n_frames, int max_len, void* workspace, cudaStream_t stream);
-
-// planning kernel over the segments (each 1..max_len frames), the forward over the table it wrote with the criterion per
-// sub-window instead of predictions (a.loss_partials = the sums), then the per-segment means and the loss
-int launch_validate_utterances(ConvArgs a, const UttPlan& plan, const long long* seg_start, const long long* seg_end, int n_seg,
-                               long long n_frames, int max_len, float* seg_loss, float* loss_out, void* workspace,
-                               cudaStream_t stream);
 
 void set_debug_timing(long long* p);
 int launch_format_prediction(const float* pred, float* out, int64_t rows, int mode, cudaStream_t stream);

@@ -1,5 +1,6 @@
-// Forward over packed utterances (b2h_conv_forward_utterances): the device-side plan and the launch.  Included by
-// b2h_conv_tc.cu after the tile and wide kernels.
+// Forward, training and validation over packed utterances and segments (b2h_conv_forward_utterances,
+// b2h_train_*_utterances, b2h_validate_utterances): the device-side plan and the one launcher.  Included by b2h_conv_tc.cu
+// after the tile and wide kernels.
 //
 // Utterance u owns stream rows [offsets[u], offsets[u+1]) and is predicted as ONE sequence, like the reference's
 // infer_utterance (steps/traintest.py:214-300): it is cut into sub-windows of Ts frames by the training cut rule
@@ -99,34 +100,6 @@ __global__ void __launch_bounds__(kUttPlanThreads) utt_plan_kernel(const long lo
   }
 }
 
-int launch_utterances(ConvArgs a, const UttPlan& plan, const long long* offsets, int n_utt, long long n_frames, void* workspace,
-                      cudaStream_t stream) {
-  int4* ws = reinterpret_cast<int4*>(workspace);
-  utt_plan_kernel<<<1, kUttPlanThreads, 0, stream>>>(offsets, offsets + 1, n_utt, n_frames, plan.Ts, plan.max_sub, 0, kUttBadOffsets,
-                                                     ws, nullptr);
-  count_launch();
-  if (int rc = check_launch("utt_plan_kernel")) return rc;
-  a.utt = ws;
-  a.B = plan.max_sub; a.T = plan.Ts;
-  a.lengths = nullptr; a.apply_mask = 0;
-  if (plan.kernel == B2H_KERNEL_TC_TILE) return launch_tc_tile(a, plan.tile, stream);
-  return launch_tc_wide_fwd(a, plan.wide, stream);
-}
-
-int launch_train_utterances(ConvArgs a, const UttPlan& plan, const long long* seg_start, const long long* seg_end, int n_seg,
-                            long long n_frames, int max_len, void* workspace, cudaStream_t stream) {
-  int4* ws = reinterpret_cast<int4*>(reinterpret_cast<char*>(workspace) + plan.plan_off);
-  int2* seg = reinterpret_cast<int2*>(reinterpret_cast<char*>(ws) + plan.seg_off);
-  utt_plan_kernel<<<1, kUttPlanThreads, 0, stream>>>(seg_start, seg_end, n_seg, n_frames, plan.Ts, plan.max_sub, max_len,
-                                                     kUttBadSegments, ws, seg);
-  count_launch();
-  if (int rc = check_launch("utt_plan_kernel")) return rc;
-  a.utt = ws; a.utt_seg = seg; a.utt_max_len = max_len;
-  a.B = n_seg; a.T = plan.Ts;
-  a.lengths = nullptr; a.apply_mask = 1;
-  return launch_tc_tile(a, plan.tile, stream);
-}
-
 // Validation over segments, the last launch: seg_loss[s] = (the sums of segment s's sub-windows, in table order) / (42 L_s);
 // loss = the sum over s in a fixed order (per-thread strided sums, then a fixed tree), times 1 / S for L1.  A refused plan:
 // NaN in loss and every seg_loss entry.
@@ -162,22 +135,25 @@ __global__ void __launch_bounds__(kUttPlanThreads) utt_validate_finish_kernel(co
   }
 }
 
-int launch_validate_utterances(ConvArgs a, const UttPlan& plan, const long long* seg_start, const long long* seg_end, int n_seg,
-                               long long n_frames, int max_len, float* seg_loss, float* loss_out, void* workspace,
-                               cudaStream_t stream) {
-  int4* ws = reinterpret_cast<int4*>(workspace);
-  int2* seg = reinterpret_cast<int2*>(reinterpret_cast<char*>(ws) + plan.seg_off);
-  float* part = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + plan.part_off);
-  utt_plan_kernel<<<1, kUttPlanThreads, 0, stream>>>(seg_start, seg_end, n_seg, n_frames, plan.Ts, plan.max_sub, max_len,
-                                                     kUttBadSegments, ws, seg);
+int launch_utterances(ConvArgs a, const UttPlan& plan, const SegmentView& sv, void* table, float* seg_loss, float* loss_out,
+                      cudaStream_t stream) {
+  int4* ws = reinterpret_cast<int4*>(table);
+  int2* seg = sv.max_len > 0 ? reinterpret_cast<int2*>(reinterpret_cast<char*>(table) + plan.seg_off) : nullptr;
+  utt_plan_kernel<<<1, kUttPlanThreads, 0, stream>>>(sv.seg_a, sv.seg_b, sv.n, sv.n_frames, plan.Ts, plan.max_sub, sv.max_len,
+                                                     sv.max_len > 0 ? kUttBadSegments : kUttBadOffsets, ws, seg);
   count_launch();
   if (int rc = check_launch("utt_plan_kernel")) return rc;
-  a.utt = ws; a.loss_partials = part;
-  a.B = plan.max_sub; a.T = plan.Ts;
-  a.lengths = nullptr; a.apply_mask = 0; a.y = nullptr;
+  a.utt = ws; a.T = plan.Ts; a.lengths = nullptr;
+  if (a.mode == 1) {
+    a.utt_seg = seg; a.utt_max_len = sv.max_len;
+    a.B = sv.n; a.apply_mask = 1;
+    return launch_tc_tile(a, plan.tile, stream);
+  }
+  a.B = plan.max_sub; a.apply_mask = 0;
   const int rc = plan.kernel == B2H_KERNEL_TC_TILE ? launch_tc_tile(a, plan.tile, stream) : launch_tc_wide_fwd(a, plan.wide, stream);
-  if (rc) return rc;
-  // programmatic dependent launch: its set-up overlaps the forward's tail; it reads the sums after griddepcontrol.wait
+  if (rc || !a.loss_partials) return rc;
+  // validation: programmatic dependent launch, its set-up overlaps the forward's tail; it reads the sums after
+  // griddepcontrol.wait
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(1); cfg.blockDim = dim3(kUttPlanThreads); cfg.dynamicSmemBytes = 0; cfg.stream = stream;
   cudaLaunchAttribute at;
@@ -186,8 +162,8 @@ int launch_validate_utterances(ConvArgs a, const UttPlan& plan, const long long*
   cfg.attrs = &at; cfg.numAttrs = 1;
   const int4* cws = ws;
   const int2* cseg = seg;
-  const float* cpart = part;
-  int lk = a.loss_kind, ms = plan.max_sub;
+  const float* cpart = a.loss_partials;
+  int n_seg = sv.n, lk = a.loss_kind, ms = plan.max_sub;
   void* kargs[] = {&cws, &cseg, &cpart, &n_seg, &ms, &lk, &seg_loss, &loss_out};
   const cudaError_t le = cudaLaunchKernelExC(&cfg, (const void*)utt_validate_finish_kernel, kargs);
   if (le != cudaSuccess) { cudaGetLastError(); set_error("utt_validate_finish_kernel launch: %s", cudaGetErrorString(le)); return B2H_ECUDA; }

@@ -18,6 +18,7 @@ import torch.nn as nn
 from . import _lib
 
 _OWNERS = weakref.WeakValueDictionary()   # id(model) -> model, looked up through Parameter._b2h_owner_id
+ANY_LENGTH = object()                      # ConvModel._check_input's T of a frame stream read as sequences of any length
 
 
 def owner_of(param):
@@ -184,26 +185,29 @@ class ConvModel(nn.Module):
             self._packed_versions = versions
         return self._packed
 
+    def _cached_workspace(self, attr, query, a, b, zero=False):
+        """The buffer cached in `attr`, grown on demand (zeroed if `zero`) to the size C-ABI `query`(a, b, geometry,
+        precision) returns."""
+        n_in, C, pe = self._geometry()
+        need = _lib.query(query, int(a), int(b), n_in, C, pe, _lib.PRECISIONS[self.precision])
+        buf, dev = getattr(self, attr), self._flat.device
+        if buf is None or buf.numel() < need or buf.device != dev:
+            buf = (torch.zeros if zero else torch.empty)(need, dtype=torch.uint8, device=dev)
+            setattr(self, attr, buf)
+        return buf
+
     def workspace(self, B, T, segments=False):
         """The training workspace for a batch of B windows of T frames, or (segments=True) for B segments of at most T
         frames (b2h_train_utterances_workspace_bytes).  One buffer, grown on demand: its header is shared by every step."""
-        n_in, C, pe = self._geometry()
-        if segments:
-            need = _lib.load().b2h_train_utterances_workspace_bytes(int(B), int(T), n_in, C, pe, _lib.PRECISIONS[self.precision])
-            if need < 0:
-                raise _lib.B2HError(_lib.last_error())
-        else:
-            need = _lib.workspace_bytes(B, T, n_in, C, pe, _lib.PRECISIONS[self.precision])
-        dev = self._flat.device
-        if self._workspace is None or self._workspace.numel() < need or self._workspace.device != dev:
-            self._workspace = torch.zeros(need, dtype=torch.uint8, device=dev)    # holds the fused kernel's grid-barrier words
-        return self._workspace
+        query = "b2h_train_utterances_workspace_bytes" if segments else "b2h_workspace_bytes"
+        return self._cached_workspace("_workspace", query, B, T, zero=True)    # holds the fused kernel's grid-barrier words
 
     # ------------------------------------------------------------------ kernels
     def _check_input(self, x, T=None):
         """The model-level checks of every entry point, on windows x (B, T, K, 2) or, with T given, on a frame stream
-        x (F, K, 2) read as windows of T frames: a CUDA tensor on an sm_100 device and on the model's device, K * 2 =
-        n_in channels, float32 / bfloat16, and the pos_emb window length.  Returns (B or F, T)."""
+        x (F, K, 2) read as windows of T frames (T = ANY_LENGTH: as sequences of any length): a CUDA tensor on an sm_100
+        device and on the model's device, K * 2 = n_in channels, float32 / bfloat16, and the pos_emb window length.
+        Returns (B or F, T)."""
         stream = T is not None
         _lib.require_device(x, "frame stream" if stream else "ConvModel input")
         _lib.require_sm100(x.device)
@@ -216,7 +220,8 @@ class ConvModel(nn.Module):
         T = T if stream else x.shape[1]
         if self.pos_emb is not None and T != self.pos_emb.max_len and not self.pos_emb_any_length:
             # torch.cat in LinearPositionalEmbedding.forward fails unless T == max_len (HandPoseModels.py:82)
-            raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {self.pos_emb.max_len}, got {T}")
+            got = " (sequences of any length need pos_emb_any_length=True)" if T is ANY_LENGTH else f", got {T}"
+            raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {self.pos_emb.max_len}{got}")
         if x.dtype not in (torch.float32, torch.bfloat16):
             raise RuntimeError(f"ConvModel input must be float32 or bfloat16, got {x.dtype}")
         if self._flat.device != x.device:
@@ -307,28 +312,13 @@ class ConvModel(nn.Module):
 
     def utterances_workspace(self, n_frames, n_utt):
         """The workspace of predict_utterances (the device-side sub-window plan), cached on the model like workspace()."""
-        n_in, C, pe = self._geometry()
-        n = _lib.load().b2h_utterances_workspace_bytes(int(n_frames), int(n_utt), n_in, C, pe, _lib.PRECISIONS[self.precision])
-        if n < 0:
-            raise _lib.B2HError(_lib.last_error())
-        dev = self._flat.device
-        if self._utt_workspace is None or self._utt_workspace.numel() < n or self._utt_workspace.device != dev:
-            self._utt_workspace = torch.empty(n, dtype=torch.uint8, device=dev)
-        return self._utt_workspace
+        return self._cached_workspace("_utt_workspace", "b2h_utterances_workspace_bytes", n_frames, n_utt)
 
     def validate_workspace(self, n_seg, max_len):
         """The workspace of steps.validate_utterances (sub-window table, segment pairs, per-sub-window sums) for n_seg
         segments of at most max_len frames, cached on the model like utterances_workspace() and apart from the training
         workspace, so a validation pass may sit between training steps (and graphs) on the same stream."""
-        n_in, C, pe = self._geometry()
-        n = _lib.load().b2h_validate_utterances_workspace_bytes(int(n_seg), int(max_len), n_in, C, pe,
-                                                                 _lib.PRECISIONS[self.precision])
-        if n < 0:
-            raise _lib.B2HError(_lib.last_error())
-        dev = self._flat.device
-        if self._val_workspace is None or self._val_workspace.numel() < n or self._val_workspace.device != dev:
-            self._val_workspace = torch.empty(n, dtype=torch.uint8, device=dev)
-        return self._val_workspace
+        return self._cached_workspace("_val_workspace", "b2h_validate_utterances_workspace_bytes", n_seg, max_len)
 
     @torch.no_grad()
     def predict_utterances(self, frames, offsets, denormalize=None, out=None):
@@ -343,12 +333,7 @@ class ConvModel(nn.Module):
         conv_channels <= 32 with at most 32 input channels; other shapes raise B2HError."""
         if not self._is_flat():
             self._flatten()
-        if self.pos_emb is not None and not self.pos_emb_any_length:
-            # the reference's torch.cat fails unless T == max_len (HandPoseModels.py:82): utterances of any length need
-            # pos_emb_any_length=True
-            raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {self.pos_emb.max_len} "
-                               "(predict_utterances needs pos_emb_any_length=True)")
-        F, _ = self._check_input(frames, 1)
+        F, _ = self._check_input(frames, ANY_LENGTH)
         dev = frames.device
         x = frames.contiguous()
         if isinstance(offsets, torch.Tensor) and offsets.is_cuda:

@@ -8,7 +8,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from .models import ConvModel, owner_of
+from .models import ANY_LENGTH, ConvModel, owner_of
 
 
 class _MaskOutput(torch.autograd.Function):
@@ -280,10 +280,7 @@ def _segment_inputs(model: ConvModel, streams, seg_start, seg_end, max_len, loss
     """`_view_inputs` of the *_utterances entry points: (frames, x_dtype, target_frames, conf_frames, n_frames, seg_start,
     seg_end, n_seg, max_len), and the number of segments, max_len and the device.  max_len defaults to the longest host-side
     segment; device segments need it given."""
-    if model.pos_emb is not None and not model.pos_emb_any_length:
-        raise RuntimeError(f"Sizes of tensors must match: pos_emb requires T == {model.pos_emb.max_len} "
-                           "(training on segments needs pos_emb_any_length=True)")
-    head, dev = _stream_inputs(model, streams, 1, loss)
+    head, dev = _stream_inputs(model, streams, ANY_LENGTH, loss)
     on_device = any(isinstance(t, torch.Tensor) and t.is_cuda for t in (seg_start, seg_end))
     if max_len is None:
         if on_device:

@@ -163,6 +163,11 @@ def test_workspace_query():
         # header, >= 1 gradient + loss partial slice, the table (count + max_sub int4), prefix sums, max_sub {segment, length}
         floor = 1024 + 4 * (19032 + 1) + 16 * (1 + max_sub) + 4 * (S + 1) + 8 * max_sub
         assert need % 256 == 0 and need >= floor, (S, L, need, floor)
+        # exactly: the table starts where the tile kernel's training of max_sub windows of Ts frames ends its partials (the
+        # dense workspace without its trailing 256 B), the pairs at the 16-byte boundary after the prefix sums
+        plan_off = lib.b2h_workspace_bytes(max_sub, Ts, 24, 30, 0, prec) - 256
+        pairs = (16 * (1 + max_sub) + 4 * (S + 1) + 15) // 16 * 16
+        assert need == (plan_off + pairs + 8 * max_sub + 255) // 256 * 256, (S, L, need)
         assert lib.b2h_train_utterances_workspace_bytes(S + 1, L, 24, 30, 0, prec) >= need
     assert lib.b2h_train_utterances_workspace_bytes(0, 100, 24, 30, 0, BF16) == ESHAPE and "bad n_seg=0" in _lib.last_error()
     assert lib.b2h_train_utterances_workspace_bytes(4, 0, 24, 30, 0, BF16) == ESHAPE

@@ -114,6 +114,8 @@ def test_workspace_query():
         need = lib.b2h_utterances_workspace_bytes(F, S, 24, C, 0, prec)
         bound = S + F // (Ts - 32)
         assert need % 256 == 0 and need >= 16 * (1 + bound) + 4 * (S + 1), (F, S, C, need)
+        # exactly: the table (count + bound int4) and the prefix sums, rounded to 256 B
+        assert need == (16 * (1 + bound) + 4 * (S + 1) + 255) // 256 * 256, (F, S, C, need)
 
 
 # ---------------------------------------------------------------------------------------------------- the plan
